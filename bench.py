@@ -7,6 +7,7 @@ the configuration the metric's "4K frame time at 1/2/4/8 B200" is quoted on), ti
 GPUs of one box, frame assembled on rank 0.  A ray = one nearest-hit query (ray_color call with depth > 0).
 
   python bench.py --gpus 1 --steps K --warmup W          # this repo's CUDA path
+  python bench.py ... --dump-outputs DIR                  # + what the last timed step computed, as DIR/<name>.npy
   python bench.py --impl reference ...                    # the reference algorithm on the host cores (oracle port)
   python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
@@ -42,6 +43,8 @@ import numpy as np  # noqa: E402
 METRIC = "Mrays/s"
 UNIT = "Mrays/s"
 FLUSH_BYTES = 160 << 20   # > 126 MB L2
+# --dump-outputs: at most this many pixels of the frame (2 Mi: 24 MiB of float32 channels + 16 MiB of float64 indices)
+DUMP_PIXELS = 1 << 21
 
 # --------------------------------------------------------------------------------------------------------
 # FLOP model (SURVEY.md Appendix C; add/sub/mul/div/sqrt = 1, FMA = 2, compares/min/max/int = 0), applied to
@@ -239,6 +242,20 @@ def ncu_block(path):
     return out
 
 
+def dump_outputs(path, frame, rays):
+    """Write what one render step computed, so that two builds can be compared output for output:
+    frame_pixels.npy      (n, 3) float32, the frame's 8-bit channels at n pixels, row-major order
+    frame_pixel_index.npy (n,) float64, the flat index (y * width + x) of each of those pixels
+    rays.npy              (1,) float64, the step's nearest-hit query count (all ranks)
+    The pixels are the whole frame when it has at most DUMP_PIXELS of them, else a fixed sample (seed 0) of that many."""
+    os.makedirs(path, exist_ok=True)
+    h, w, _ = frame.shape
+    idx = np.sort(np.random.default_rng(0).choice(h * w, size=min(h * w, DUMP_PIXELS), replace=False))
+    np.save(os.path.join(path, "frame_pixels.npy"), frame.reshape(-1, 3)[idx].astype(np.float32))
+    np.save(os.path.join(path, "frame_pixel_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(path, "rays.npy"), np.array([rays], dtype=np.float64))
+
+
 # --------------------------------------------------------------------------------------------------------
 def _claim_stdout():
     """Keep fd 1 for the ONE JSON line: libraries (NCCL prints its version banner there) get stderr instead."""
@@ -299,7 +316,11 @@ def main():
     ap.add_argument("--intersector", type=int, default=0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the frame and ray count of the last timed step to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the CUDA path computed: it needs --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     from rt_b200 import scenes
@@ -388,10 +409,14 @@ def main():
     barrier()
     elapsed = time.perf_counter() - t0
     clocks = sampler.stop() if rank == 0 else None
+    # read back before the all-reduce below: until rank 0 joins it, no rank can start a frame into this buffer again
+    last_frame = sched.download(np.empty((H, W, 3), dtype=np.uint8)) if args.dump_outputs and rank == 0 else None
 
     ROp = dist.ReduceOp if dist is not None else None
     elapsed_max = allreduce(elapsed, ROp.MAX if ROp else None)
     rays_total = allreduce(float(rays_step), ROp.SUM if ROp else None)
+    if last_frame is not None:
+        dump_outputs(args.dump_outputs, last_frame, rays_total)
     value = rays_total * args.steps / elapsed_max / 1e6
     ms_per_step = elapsed_max / args.steps * 1e3
 
