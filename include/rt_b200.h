@@ -197,6 +197,38 @@ int rt_render_tiles_device(rt_ctx* ctx, const rt_scene* scene, const rt_params* 
 int rt_render_tiles_collect(rt_ctx* ctx, const rt_scene* scene, const rt_params* params, uint32_t tile_rank,
                             uint32_t tile_ranks, void* frame_dev, uint64_t seq, uint8_t* out_rgb, size_t out_len,
                             rt_stats* stats);
+
+/* ---- progressive rendering: resumable per-pixel sample chains, rendered in chunks ------------------ */
+/* A pixel's chain is sequential but resumable: between two samples its whole state is the xoshiro256++ state and three
+ * running sums, and the samples of a render at spp = k are the first k samples of a render at any larger spp.  So a band
+ * rendered in chunks of samples is byte-identical at every step to rt_render_division at the cumulative count: a cheap
+ * preview that improves (1 sample, then 2, 4, 8 ...), or more samples added to a finished frame without paying again for
+ * the samples it has. */
+typedef struct rt_accum rt_accum;
+/* Sample state of the rows rt_render_division would render for *params (divisions / division_no honoured; 1 = whole
+ * frame), every pixel at sample 0.  Binds width, height, band, seed, camera, max_bounces, flags, intersector;
+ * params->spp and collect_counters are ignored.  Device memory: 2 x 48 bytes per pixel. */
+int rt_accum_create(rt_ctx* ctx, const rt_params* params, rt_accum** out);
+void rt_accum_destroy(rt_ctx* ctx, rt_accum* acc);
+/* Back to sample 0, optionally re-bound to new params (same width, height and band; NULL = keep): a camera move.
+ * RT_ERR_INVALID_ARG for another size or band. */
+int rt_accum_reset(rt_ctx* ctx, rt_accum* acc, const rt_params* params);
+int rt_accum_samples(const rt_accum* acc, uint32_t* samples_out);
+/* Advances every pixel by n_samples (samples [done, done + n) of its chain) and, if out_rgb != NULL, writes the band as
+ * it now stands: byte-identical to rt_render_division with spp = done + n.  Every chunk since the last create / reset
+ * must render the same scene (another one, a re-created one included, is RT_ERR_INVALID_ARG; RT_INTERSECT_AUTO is
+ * resolved against the scene of each call).  RT_ERR_INVALID_ARG also for n_samples == 0, done + n_samples above
+ * 2^32 - 1, out_len != rows*width*3 with out_rgb != NULL, and an accum of another context; RT_ERR_UNSUPPORTED in the
+ * experiments build while an A/B kernel is selected (they have no resumable form).  On any error the state is
+ * unchanged.  stats (nullable): rays, primary (pixels * n_samples), kernel_ms, total_ms, intersector_used,
+ * kernel_launches, the launch shape and redo_pixels; the counters of collect_counters are not filled (0). */
+int rt_render_samples(rt_ctx* ctx, const rt_scene* scene, rt_accum* acc, uint32_t n_samples, uint8_t* out_rgb,
+                      size_t out_len, rt_stats* stats);
+/* Linear radiance of the band: rows*width*3 float32 (out_len in bytes), sum / samples per channel (the exact-domain
+ * division quantise() does: sqrt, * 255.999, truncate, saturate, NaN -> 0 give the RGB8 band).  RT_ERR_INVALID_ARG before
+ * the first chunk. */
+int rt_accum_read_linear(rt_ctx* ctx, const rt_accum* acc, float* out, size_t out_len);
+
 int rt_sync(rt_ctx* ctx);
 /* The ctx stream as a cudaStream_t, for callers that order their own work (NCCL, copies) after a render. */
 void* rt_stream(rt_ctx* ctx);

@@ -36,6 +36,15 @@ constexpr uint32_t kBruteMaxPrims = 16;
 
 int resolve(rt_ctx* ctx, const rt_scene* scene, const rt_params* in, bool whole_frame, Resolved* r) {
     if (!scene || !in) return set_err(ctx, RT_ERR_INVALID_ARG, "NULL scene or params");
+    const int rc = resolve_params(ctx, in, whole_frame, r);
+    if (rc) return rc;
+    r->isect = r->p.intersector == RT_INTERSECT_AUTO ? (scene->n <= kBruteMaxPrims ? RT_INTERSECT_BRUTE : RT_INTERSECT_BVH)
+                                                     : (int)r->p.intersector;
+    return RT_OK;
+}
+
+int resolve_params(rt_ctx* ctx, const rt_params* in, bool whole_frame, Resolved* r) {
+    if (!in) return set_err(ctx, RT_ERR_INVALID_ARG, "NULL params");
     rt_params p = *in;
     if (whole_frame) {  // division fields do not apply to a whole-frame call
         p.divisions = 1;
@@ -59,8 +68,6 @@ int resolve(rt_ctx* ctx, const rt_scene* scene, const rt_params* in, bool whole_
     if ((uint64_t)p.width * p.height > 0x7fffffffu) return set_err(ctx, RT_ERR_UNSUPPORTED, "frame too large");
     if (p.intersector > RT_INTERSECT_BVH) return set_err(ctx, RT_ERR_INVALID_ARG, "unknown intersector");
     r->p = p;
-    r->isect = p.intersector == RT_INTERSECT_AUTO ? (scene->n <= kBruteMaxPrims ? RT_INTERSECT_BRUTE : RT_INTERSECT_BVH)
-                                                  : (int)p.intersector;
     // Camera::new (camera.rs:19-47) with the arguments of main.rs:42-50, single f32 ops in order
     DevCamera& c = r->cam;
     const float aspect = (float)p.width / (float)p.height;
@@ -154,6 +161,9 @@ int launch(rt_ctx* ctx, const rt_scene* scene, const Resolved& r, const LaunchAr
     pr.redo_cap = RT_REDO_CAP;
     pr.pixel_list = a.pixel_list;
     pr.list_count = a.list_count;
+    pr.state_in = static_cast<const uint4*>(a.state_in);
+    pr.state_out = static_cast<uint4*>(a.state_out);
+    pr.s0 = a.s0;
     pr.done = a.ctl ? a.ctl->done : nullptr;
     pr.stage_hint = a.stream ? 1 : 0;
     pr.redo_slab = ctx->d_ctr + RT_CTR_REDO_SLAB;
@@ -708,6 +718,145 @@ int rt_render_tiles_collect(rt_ctx* ctx, const rt_scene* scene, const rt_params*
     a.ctl = reinterpret_cast<rt_frame_ctl*>((uint8_t*)frame_dev + rt_frame_ctl_offset(bytes));
     return render_and_collect(ctx, scene, r, a, (const uint8_t*)frame_dev, seq, out_rgb, bytes,
                               (uint64_t)r.p.width * r.p.height / tile_ranks, stats, t0);
+    RT_GUARD_END(ctx)
+}
+
+// -------------------------------------------------------------------------------------------------
+// Progressive rendering: resumable per-pixel sample chains
+// -------------------------------------------------------------------------------------------------
+// The samples of a render at spp = k are the first k samples of a render at any larger spp (no draw depends on spp, the
+// sum is folded in order, quantise() divides at the end), so chunks of samples reproduce rt_render_division at the
+// cumulative count byte for byte.
+int rt_accum_create(rt_ctx* ctx, const rt_params* params, rt_accum** out) {
+    if (!ctx) return RT_ERR_INVALID_ARG;
+    RT_GUARD_BEGIN
+    if (!out) return set_err(ctx, RT_ERR_INVALID_ARG, "rt_accum_create: out is NULL");
+    *out = nullptr;
+    Resolved r;
+    const int rc = resolve_params(ctx, params, false, &r);
+    if (rc) return rc;
+    std::unique_ptr<rt_accum> acc(new rt_accum());
+    acc->ctx = ctx;
+    acc->params = *params;
+    acc->params.collect_counters = 0;
+    const uint32_t band = r.p.height / r.p.divisions;
+    acc->row0 = band * r.p.division_no;
+    acc->row1 = acc->row0 + band;
+    const size_t bytes = (size_t)band * r.p.width * STATE_RECORD_BYTES;
+    CK(ctx, cudaSetDevice(ctx->device));
+    for (int i = 0; i < 2; i++) {
+        const cudaError_t e = cudaMalloc(&acc->state[i], bytes);
+        if (e != cudaSuccess) {
+            if (i) cudaFree(acc->state[0]);
+            (void)cudaGetLastError();
+            return set_err(ctx, RT_ERR_CUDA, "rt_accum_create: cudaMalloc of %zu bytes failed: %s", bytes, cudaGetErrorString(e));
+        }
+    }
+    *out = acc.release();
+    return RT_OK;
+    RT_GUARD_END(ctx)
+}
+
+void rt_accum_destroy(rt_ctx* ctx, rt_accum* acc) {
+    if (!acc) return;
+    rt_ctx* c = ctx ? ctx : acc->ctx;
+    cudaSetDevice(c->device);
+    cudaStreamSynchronize(c->stream);
+    cudaFree(acc->state[0]);
+    cudaFree(acc->state[1]);
+    delete acc;
+}
+
+int rt_accum_reset(rt_ctx* ctx, rt_accum* acc, const rt_params* params) {
+    if (!ctx) return RT_ERR_INVALID_ARG;
+    RT_GUARD_BEGIN
+    if (!acc || acc->ctx != ctx) return set_err(ctx, RT_ERR_INVALID_ARG, "rt_accum_reset: accum is NULL or of another context");
+    if (params) {
+        Resolved r;
+        const int rc = resolve_params(ctx, params, false, &r);
+        if (rc) return rc;
+        const uint32_t band = r.p.height / r.p.divisions, row0 = band * r.p.division_no;
+        if (r.p.width != acc->params.width || r.p.height != acc->params.height || row0 != acc->row0 || row0 + band != acc->row1)
+            return set_err(ctx, RT_ERR_INVALID_ARG, "rt_accum_reset: width, height and band must stay %ux%u, rows [%u, %u)",
+                           acc->params.width, acc->params.height, acc->row0, acc->row1);
+        acc->params = *params;
+        acc->params.collect_counters = 0;
+    }
+    acc->samples = 0;
+    acc->scene_serial = 0;
+    return RT_OK;
+    RT_GUARD_END(ctx)
+}
+
+int rt_accum_samples(const rt_accum* acc, uint32_t* samples_out) {
+    if (!acc || !samples_out) return RT_ERR_INVALID_ARG;
+    *samples_out = acc->samples;
+    return RT_OK;
+}
+
+int rt_render_samples(rt_ctx* ctx, const rt_scene* scene, rt_accum* acc, uint32_t n_samples, uint8_t* out_rgb,
+                      size_t out_len, rt_stats* stats) {
+    if (!ctx) return RT_ERR_INVALID_ARG;
+    RT_GUARD_BEGIN
+    const auto t0 = std::chrono::steady_clock::now();
+    if (!acc || acc->ctx != ctx) return set_err(ctx, RT_ERR_INVALID_ARG, "rt_render_samples: accum is NULL or of another context");
+    if (!scene) return set_err(ctx, RT_ERR_INVALID_ARG, "rt_render_samples: scene is NULL");
+    if (n_samples == 0) return set_err(ctx, RT_ERR_INVALID_ARG, "rt_render_samples: n_samples is 0");
+    if ((uint64_t)acc->samples + n_samples > 0xffffffffull)
+        return set_err(ctx, RT_ERR_INVALID_ARG, "rt_render_samples: %u + %u samples overflow 32 bits", acc->samples, n_samples);
+    if (acc->samples && scene->serial != acc->scene_serial)
+        return set_err(ctx, RT_ERR_INVALID_ARG, "rt_render_samples: not the scene of the chunks since the last create / reset");
+#ifdef RT_B200_EXPERIMENTS
+    if (tunables().bvh_variant != 3)
+        return set_err(ctx, RT_ERR_UNSUPPORTED, "rt_render_samples: the A/B kernels (RT_B200_BVH_KERNEL) have no resumable form");
+#endif
+    rt_params p = acc->params;
+    p.spp = acc->samples + n_samples;
+    Resolved r;
+    int rc = resolve(ctx, scene, &p, false, &r);
+    if (rc) return rc;
+    const uint32_t rows = acc->row1 - acc->row0;
+    const size_t bytes = (size_t)rows * r.p.width * 3;
+    if (out_rgb && out_len != bytes)
+        return set_err(ctx, RT_ERR_INVALID_ARG, "out_len %zu != (rows %u * width %u * 3) = %zu", out_len, rows, r.p.width, bytes);
+    CK(ctx, cudaSetDevice(ctx->device));
+    LaunchArgs a;
+    a.row0 = acc->row0;
+    a.row1 = acc->row1;
+    a.out_row0 = acc->row0;
+    rc = own_frame(ctx, r.p.width, rows, &a);
+    if (rc) return rc;
+    a.stream = false;  // the band is copied after the kernel
+    a.state_in = acc->state[acc->cur];
+    a.state_out = acc->state[acc->cur ^ 1];
+    a.s0 = acc->samples;
+    const uint64_t pixels = (uint64_t)rows * r.p.width;
+    rc = render_and_collect(ctx, scene, r, a, ctx->d_out, ctx->out_seq, out_rgb, bytes, pixels, stats, t0);
+    if (rc) return rc;
+    acc->cur ^= 1;
+    acc->samples += n_samples;
+    acc->scene_serial = scene->serial;
+    if (stats) stats->primary = pixels * n_samples;
+    return RT_OK;
+    RT_GUARD_END(ctx)
+}
+
+int rt_accum_read_linear(rt_ctx* ctx, const rt_accum* acc, float* out, size_t out_len) {
+    if (!ctx) return RT_ERR_INVALID_ARG;
+    RT_GUARD_BEGIN
+    if (!acc || acc->ctx != ctx) return set_err(ctx, RT_ERR_INVALID_ARG, "rt_accum_read_linear: accum is NULL or of another context");
+    if (!out) return set_err(ctx, RT_ERR_INVALID_ARG, "rt_accum_read_linear: out is NULL");
+    if (acc->samples == 0) return set_err(ctx, RT_ERR_INVALID_ARG, "rt_accum_read_linear: no samples rendered yet");
+    const uint64_t pixels = (uint64_t)(acc->row1 - acc->row0) * acc->params.width;
+    const size_t bytes = (size_t)pixels * 3 * sizeof(float);
+    if (out_len != bytes) return set_err(ctx, RT_ERR_INVALID_ARG, "out_len %zu != rows * width * 3 * 4 = %zu", out_len, bytes);
+    CK(ctx, cudaSetDevice(ctx->device));
+    // the buffer the next chunk writes in full serves as the scratch (12 of its 48 bytes per pixel)
+    float* scratch = static_cast<float*>(acc->state[acc->cur ^ 1]);
+    CK(ctx, launch_accum_linear(acc->state[acc->cur], scratch, pixels, acc->samples, ctx->sm_count, ctx->stream));
+    CK(ctx, cudaMemcpyAsync(out, scratch, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(ctx, cudaStreamSynchronize(ctx->stream));
+    return RT_OK;
     RT_GUARD_END(ctx)
 }
 

@@ -101,6 +101,7 @@ struct rt_scene {
     bool device_tree = false;  // it was built on the device (LBVH)
     size_t o_rank = 0, o_up = 0, o_refbox = 0;  // blob offsets of the late tables
     std::unique_ptr<rt_aux> aux;
+    uint64_t serial = 0;  // unique per process (rt_scene_create): a re-created scene may reuse a destroyed one's address
 };
 
 namespace rtb {
@@ -117,6 +118,8 @@ struct Resolved {
     int isect;
 };
 int resolve(rt_ctx* ctx, const rt_scene* scene, const rt_params* in, bool whole_frame, Resolved* r);
+// resolve() without a scene: every check and default except the intersector's pick (r->isect is left unset)
+int resolve_params(rt_ctx* ctx, const rt_params* in, bool whole_frame, Resolved* r);
 
 // slab geometry of a launch that renders `rows` image rows: slabs of `tile_rows` tile rows each
 struct SlabPlan {
@@ -137,6 +140,9 @@ struct LaunchArgs {
     bool stream = false;          // the frame goes to the host slab by slab while it renders (stage + counters wanted)
     const unsigned int* pixel_list = nullptr;  // redo launch: render exactly these pixels (y * width + x)
     uint32_t list_count = 0;
+    const void* state_in = nullptr;  // resumable chains (rt_render_samples): samples [s0, spp) from state_in to state_out
+    void* state_out = nullptr;
+    uint32_t s0 = 0;
 };
 // The context's own staging frame (+ control block) for a launch of `rows` rows: fills dst / ctl / plan, bumps out_seq.
 int own_frame(rt_ctx* ctx, uint32_t width, uint32_t rows, LaunchArgs* a);
@@ -164,6 +170,19 @@ int enqueue_slab_copies(rt_ctx* ctx, const uint8_t* frame_dev, const rt_frame_ct
 int finish_slab_copies(rt_ctx* ctx, const SlabJob& job);
 
 }  // namespace rtb
+
+// Sample state of the rows of one frame or division (rt_accum_create).  Two buffers of STATE_RECORD_BYTES per pixel: a
+// chunk reads state[cur] and writes state[cur ^ 1], and cur flips only when the chunk has succeeded, so a second pass
+// (which starts over from state[cur]) and a failed call both leave the chain where it was.
+struct rt_accum {
+    rt_ctx* ctx = nullptr;
+    rt_params params{};         // as bound (spp and collect_counters ignored); resolved against the scene per chunk
+    uint32_t row0 = 0, row1 = 0;
+    void* state[2] = {nullptr, nullptr};
+    int cur = 0;
+    uint32_t samples = 0;       // samples of every pixel's chain done so far
+    uint64_t scene_serial = 0;  // the scene of the chunks since the last create / reset (0: none yet)
+};
 
 #define CK(ctx, call)                                                                                        \
     do {                                                                                                     \

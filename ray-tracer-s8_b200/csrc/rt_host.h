@@ -71,6 +71,9 @@ cudaError_t launch_wait_all_slabs(const unsigned long long* done, unsigned long 
 cudaError_t launch_set_u64(unsigned long long* p, unsigned long long v, cudaStream_t stream);
 cudaError_t launch_add_counts(unsigned long long* done, const unsigned long long* add, int n, cudaStream_t stream);
 cudaError_t launch_fp32_peak(float* scratch, int sm_count, int iters, cudaStream_t stream);
+// rows * width * 3 floats: sum / samples of each pixel's state record (rt_accum_read_linear)
+cudaError_t launch_accum_linear(const void* state, float* out, unsigned long long pixels, uint32_t samples, int sm_count,
+                                cudaStream_t stream);
 size_t scene_smem_bytes(const DevScene& sc, int isect);
 
 #ifdef RT_B200_EXPERIMENTS

@@ -153,7 +153,9 @@ constexpr uint32_t L_REDO = 8u;           constexpr int W_NEXT_SHIFT = 8;    // 
 constexpr int L_SLOT_SHIFT = 4;           // 3 bits: output-stage slot + 1 of this lane's pixel (0: straight to the frame)
 constexpr uint32_t L_SECOND = 128u;       // this pixel comes from the redo list: its first pass was held back, not counted
 
-template <int ISECT, bool SMEM, bool COUNT, bool STAGE, int MINB, int TPB>
+// RESUME: the launch renders samples [pr.s0, pr.spp) of each pixel's chain from the state in pr.state_in and leaves the
+// state in pr.state_out (rt_render_samples); the other instantiations render samples [0, pr.spp).
+template <int ISECT, bool SMEM, bool COUNT, bool STAGE, int MINB, int TPB, bool RESUME = false>
 __global__ void __launch_bounds__(TPB, MINB) render_kernel_lanes(const DevScene sc, const DevCamera cam,
                                                                 const DevParams pr) {
     extern __shared__ float4 smem_dyn[];
@@ -389,9 +391,25 @@ __global__ void __launch_bounds__(TPB, MINB) render_kernel_lanes(const DevScene 
                 if (x < pr.width && y < pr.row1) {
                     px = x; py = y;
                     st = L_HAVE | (slot1 << L_SLOT_SHIFT) | second;
-                    rng.seed_from_u64(pr.seed + ((uint64_t)y * pr.width + x));
-                    sr = sg = sb = 0.0f;
-                    s = 0;
+                    if constexpr (RESUME) {
+                        if (pr.s0 == 0) {  // the chain's start: nothing to read
+                            rng.seed_from_u64(pr.seed + ((uint64_t)y * pr.width + x));
+                            sr = sg = sb = 0.0f;
+                        } else {
+                            const uint4* rec = pr.state_in + ((size_t)(y - pr.row0) * pr.width + x) * 3;
+                            const uint4 a = __ldcs(rec), b = __ldcs(rec + 1), c = __ldcs(rec + 2);
+                            rng.s0 = ((uint64_t)a.y << 32) | a.x;
+                            rng.s1 = ((uint64_t)a.w << 32) | a.z;
+                            rng.s2 = ((uint64_t)b.y << 32) | b.x;
+                            rng.s3 = ((uint64_t)b.w << 32) | b.z;
+                            sr = __uint_as_float(c.x); sg = __uint_as_float(c.y); sb = __uint_as_float(c.z);
+                        }
+                        s = pr.s0;
+                    } else {
+                        rng.seed_from_u64(pr.seed + ((uint64_t)y * pr.width + x));
+                        sr = sg = sb = 0.0f;
+                        s = 0;
+                    }
                     left = 0;
                 }
                 want = __ballot_sync(FULL, (st & (L_HAVE | L_FINISHED)) == 0);
@@ -480,6 +498,15 @@ __global__ void __launch_bounds__(TPB, MINB) render_kernel_lanes(const DevScene 
                 s++;
                 left = 0;
                 if (s == pr.spp) {  // pixel finished (main.rs:78-81)
+                    if constexpr (RESUME) {
+                        // a pixel held back for the second pass leaves its state there (from the same state_in)
+                        if (!(st & L_REDO)) {
+                            uint4* rec = pr.state_out + ((size_t)(py - pr.row0) * pr.width + px) * 3;
+                            __stcs(rec, make_uint4((uint32_t)rng.s0, (uint32_t)(rng.s0 >> 32), (uint32_t)rng.s1, (uint32_t)(rng.s1 >> 32)));
+                            __stcs(rec + 1, make_uint4((uint32_t)rng.s2, (uint32_t)(rng.s2 >> 32), (uint32_t)rng.s3, (uint32_t)(rng.s3 >> 32)));
+                            __stcs(rec + 2, make_uint4(__float_as_uint(sr), __float_as_uint(sg), __float_as_uint(sb), 0u));
+                        }
+                    }
                     const uint32_t rgb = quantise(sr, spp_f) | (quantise(sg, spp_f) << 8) | (quantise(sb, spp_f) << 16);
                     // a pixel that goes to the second pass is counted there: a slab whose count is complete is final
                     const bool hold = (st & L_REDO) != 0;
@@ -602,6 +629,18 @@ __global__ void add_counts_kernel(unsigned long long* done, const unsigned long 
     }
 }
 
+// rt_accum_read_linear: sum / samples per channel of every pixel's state record (the exact-domain division quantise()
+// starts with), rows * width * 3 floats.
+__global__ void accum_linear_kernel(const uint4* state, float* out, unsigned long long pixels, float samples) {
+    for (unsigned long long i = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; i < pixels;
+         i += (unsigned long long)gridDim.x * blockDim.x) {
+        const uint4 c = state[3 * i + 2];
+        out[3 * i + 0] = x_div(__uint_as_float(c.x), samples);
+        out[3 * i + 1] = x_div(__uint_as_float(c.y), samples);
+        out[3 * i + 2] = x_div(__uint_as_float(c.z), samples);
+    }
+}
+
 // ---------------------------------------------------------------------------------------------
 // FFMA-chain micro-benchmark for the FP32 roofline denominator
 // ---------------------------------------------------------------------------------------------
@@ -693,6 +732,19 @@ static KernelFn pick_lanes(bool count, bool stage, int* threads) {
                  : (KernelFn)render_kernel_lanes<ISECT, SMEM, false, false, 3, THREADS>;
 }
 
+// the resumable form (rt_render_samples): the same CTA shapes, no output stage and no instrumented variant
+template <int ISECT, bool SMEM>
+static KernelFn pick_resume(int* threads) {
+    if constexpr (SMEM) {
+        *threads = SMEM_TPB;
+        return (KernelFn)render_kernel_lanes<ISECT, SMEM, false, false, 1, SMEM_TPB, true>;
+    } else {
+        *threads = THREADS;
+        if constexpr (ISECT == RT_INTERSECT_BVH) return (KernelFn)render_kernel_lanes<ISECT, SMEM, false, false, 4, THREADS, true>;
+        else return (KernelFn)render_kernel_lanes<ISECT, SMEM, false, false, 3, THREADS, true>;
+    }
+}
+
 size_t scene_smem_bytes(const DevScene& sc, int isect) {
     size_t b = (size_t)sc.ns * 16 + (size_t)sc.nt * 64;
     if (isect == RT_INTERSECT_BVH) b += (size_t)sc.lni * NODE_BYTES;
@@ -714,6 +766,11 @@ cudaError_t preload_kernels() {
             RT_TOUCH((pick_lanes<RT_INTERSECT_BRUTE, true>(count, stage, &th)));
             RT_TOUCH((pick_lanes<RT_INTERSECT_BRUTE, false>(count, stage, &th)));
         }
+    RT_TOUCH((pick_resume<RT_INTERSECT_BVH, true>(&th)));
+    RT_TOUCH((pick_resume<RT_INTERSECT_BVH, false>(&th)));
+    RT_TOUCH((pick_resume<RT_INTERSECT_BRUTE, true>(&th)));
+    RT_TOUCH((pick_resume<RT_INTERSECT_BRUTE, false>(&th)));
+    RT_TOUCH(accum_linear_kernel);
     RT_TOUCH(wait_slab_kernel);
     RT_TOUCH(wait_all_slabs_kernel);
     RT_TOUCH(add_counts_kernel);
@@ -726,6 +783,8 @@ cudaError_t preload_kernels() {
 cudaError_t launch_render(const DevScene& sc, const DevCamera& cam, const DevParams& pr, int isect, bool count,
                           int sm_count, int smem_optin, cudaStream_t stream, LaunchInfo* info) {
     const Tunables& tn = tunables();
+    const bool resume = pr.state_out != nullptr;  // rt_render_samples
+    if (resume) count = false;
 #ifdef RT_B200_EXPERIMENTS
     {
         cudaError_t ee;
@@ -745,10 +804,12 @@ cudaError_t launch_render(const DevScene& sc, const DevCamera& cam, const DevPar
     // the copy they let the owner overlap costs 0.06 ns per pixel.  On for frames shared between ranks and for frames the
     // caller streams to the host; a frame that stays on one device keeps round 1's byte stores.
     // RT_B200_STAGE_OUT=0|1 forces it (profiles/r2_notes.md).
-    const bool stage = !count && (tn.stage_out < 0 ? ((pr.tile_ranks > 1 || pr.stage_hint) && pr.done != nullptr) : tn.stage_out != 0);
+    const bool stage = !count && !resume && (tn.stage_out < 0 ? ((pr.tile_ranks > 1 || pr.stage_hint) && pr.done != nullptr) : tn.stage_out != 0);
     int threads = THREADS;
     KernelFn fn;
-    if (isect == RT_INTERSECT_BRUTE) fn = smem ? pick_lanes<RT_INTERSECT_BRUTE, true>(count, stage, &threads) : pick_lanes<RT_INTERSECT_BRUTE, false>(count, stage, &threads);
+    if (resume) fn = isect == RT_INTERSECT_BRUTE ? (smem ? pick_resume<RT_INTERSECT_BRUTE, true>(&threads) : pick_resume<RT_INTERSECT_BRUTE, false>(&threads))
+                                                 : (smem ? pick_resume<RT_INTERSECT_BVH, true>(&threads) : pick_resume<RT_INTERSECT_BVH, false>(&threads));
+    else if (isect == RT_INTERSECT_BRUTE) fn = smem ? pick_lanes<RT_INTERSECT_BRUTE, true>(count, stage, &threads) : pick_lanes<RT_INTERSECT_BRUTE, false>(count, stage, &threads);
     else fn = smem ? pick_lanes<RT_INTERSECT_BVH, true>(count, stage, &threads) : pick_lanes<RT_INTERSECT_BVH, false>(count, stage, &threads);
     const size_t dyn = smem ? need : 0;
     cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
@@ -812,6 +873,14 @@ cudaError_t launch_set_u64(unsigned long long* p, unsigned long long v, cudaStre
 
 cudaError_t launch_add_counts(unsigned long long* done, const unsigned long long* add, int n, cudaStream_t stream) {
     add_counts_kernel<<<1, MAX_SLABS, 0, stream>>>(done, add, n);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_accum_linear(const void* state, float* out, unsigned long long pixels, uint32_t samples, int sm_count,
+                                cudaStream_t stream) {
+    const unsigned long long blocks = std::min<unsigned long long>((pixels + 255) / 256, (unsigned long long)sm_count * 8);
+    accum_linear_kernel<<<(unsigned)std::max<unsigned long long>(1, blocks), 256, 0, stream>>>(
+        static_cast<const uint4*>(state), out, pixels, (float)samples);
     return cudaGetLastError();
 }
 

@@ -212,8 +212,10 @@ int rt_scene_create(rt_ctx* ctx, const rt_sphere* spheres, uint32_t n_spheres, c
         t_prev = now;
     };
 
+    static std::atomic<uint64_t> next_serial{1};
     std::unique_ptr<rt_scene> sc(new rt_scene());
     sc->ctx = ctx;
+    sc->serial = next_serial++;
     sc->n = n;
     sc->aux.reset(new rt_aux());
     rt_aux* aux = sc->aux.get();

@@ -14,6 +14,10 @@ pub struct rt_ctx {
     _private: [u8; 0],
 }
 #[repr(C)]
+pub struct rt_accum {
+    _private: [u8; 0],
+}
+#[repr(C)]
 pub struct rt_scene {
     _private: [u8; 0],
 }
@@ -147,6 +151,20 @@ extern "C" {
         sync: c_int,
         stats: *mut rt_stats,
     ) -> c_int;
+    pub fn rt_accum_create(ctx: *mut rt_ctx, params: *const rt_params, out: *mut *mut rt_accum) -> c_int;
+    pub fn rt_accum_destroy(ctx: *mut rt_ctx, acc: *mut rt_accum);
+    pub fn rt_accum_reset(ctx: *mut rt_ctx, acc: *mut rt_accum, params: *const rt_params) -> c_int;
+    pub fn rt_accum_samples(acc: *const rt_accum, samples_out: *mut u32) -> c_int;
+    pub fn rt_render_samples(
+        ctx: *mut rt_ctx,
+        scene: *const rt_scene,
+        acc: *mut rt_accum,
+        n_samples: u32,
+        out_rgb: *mut u8,
+        out_len: usize,
+        stats: *mut rt_stats,
+    ) -> c_int;
+    pub fn rt_accum_read_linear(ctx: *mut rt_ctx, acc: *const rt_accum, out: *mut f32, out_len: usize) -> c_int;
 }
 
 /// Error of any call: the negative `rt_status` and the library's message.
@@ -173,6 +191,14 @@ unsafe impl Send for Context {}
 pub struct Scene<'c> {
     ctx: &'c Context,
     raw: *mut rt_scene,
+}
+
+/// Resumable per-pixel sample chains of one band (`rt_accum`): chunks rendered with `render` add up, byte for byte, to
+/// `render_division` at the cumulative sample count.
+pub struct Accum<'c> {
+    ctx: &'c Context,
+    raw: *mut rt_accum,
+    len: usize,
 }
 
 impl Context {
@@ -235,6 +261,37 @@ impl Context {
         self.check(rc)?;
         Ok(out)
     }
+
+    /// Sample state of the band `params` selects (`params.spp` is ignored), every pixel at sample 0.
+    pub fn accum(&self, params: &rt_params) -> Result<Accum<'_>, Error> {
+        let div = params.divisions.max(1);
+        let mut raw = ptr::null_mut();
+        self.check(unsafe { rt_accum_create(self.raw, params, &mut raw) })?;
+        Ok(Accum { ctx: self, raw, len: (params.height / div) as usize * params.width as usize * 3 })
+    }
+}
+
+impl Accum<'_> {
+    /// Advances every pixel by `n_samples` and returns the band as it now stands: the bytes of `render_division` at
+    /// `spp = self.samples()`.
+    pub fn render(&mut self, scene: &Scene<'_>, n_samples: u32) -> Result<Vec<u8>, Error> {
+        let mut out = vec![0u8; self.len];
+        let rc = unsafe { rt_render_samples(self.ctx.raw, scene.raw, self.raw, n_samples, out.as_mut_ptr(), out.len(), ptr::null_mut()) };
+        self.ctx.check(rc)?;
+        Ok(out)
+    }
+
+    /// Back to sample 0, optionally with new params of the same size and band.
+    pub fn reset(&mut self, params: Option<&rt_params>) -> Result<(), Error> {
+        let p = params.map_or(ptr::null(), |p| p as *const rt_params);
+        self.ctx.check(unsafe { rt_accum_reset(self.ctx.raw, self.raw, p) })
+    }
+
+    pub fn samples(&self) -> u32 {
+        let mut n = 0u32;
+        unsafe { rt_accum_samples(self.raw, &mut n) };
+        n
+    }
 }
 
 /// One frame over several GPUs from this process (`rt_render_frame_multi`): `ctxs[i]` renders rank i's share of the
@@ -254,6 +311,11 @@ pub fn render_frame_multi(ctxs: &[&Context], scenes: &[&Scene<'_>], params: &rt_
 impl Drop for Context {
     fn drop(&mut self) {
         unsafe { rt_shutdown(self.raw) }
+    }
+}
+impl Drop for Accum<'_> {
+    fn drop(&mut self) {
+        unsafe { rt_accum_destroy(self.ctx.raw, self.raw) }
     }
 }
 impl Drop for Scene<'_> {

@@ -10,6 +10,6 @@
 """
 from . import scenes  # noqa: F401
 from .api import (  # noqa: F401
-    INTERSECT_AUTO, INTERSECT_BRUTE, INTERSECT_BVH, Context, RtError, RtParams, RtStats, Scene, make_params,
+    INTERSECT_AUTO, INTERSECT_BRUTE, INTERSECT_BVH, Accum, Context, RtError, RtParams, RtStats, Scene, make_params,
     render_frame_multi,
 )

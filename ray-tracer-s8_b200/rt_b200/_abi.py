@@ -74,6 +74,7 @@ EXPORTS = [
     "rt_host_alloc", "rt_host_free", "rt_frame_alloc", "rt_frame_open", "rt_frame_close", "rt_frame_free",
     "rt_frame_download", "rt_measure_fp32_peak", "rt_device_info", "rt_bvh_build_host", "rt_struct_sizes", "rt_scene_device_bytes",
     "rt_scene_wait_ready", "rt_render_frame_multi", "rt_frame_collect", "rt_render_tiles_collect", "rt_frame_wait_consumed", "rt_l2_flush",
+    "rt_accum_create", "rt_accum_destroy", "rt_accum_reset", "rt_accum_samples", "rt_render_samples", "rt_accum_read_linear",
 ]
 # only in the experiments build (csrc/experiments/rt_experiments_api.h)
 EXPERIMENT_EXPORTS = ["rt_debug_trace_bench"]
@@ -159,6 +160,18 @@ def lib():
     L.rt_bvh_build_host.restype = i32
     L.rt_scene_device_bytes.argtypes = [vp]
     L.rt_scene_device_bytes.restype = sz
+    L.rt_accum_create.argtypes = [vp, C.POINTER(RtParams), pp]
+    L.rt_accum_create.restype = i32
+    L.rt_accum_destroy.argtypes = [vp, vp]
+    L.rt_accum_destroy.restype = None
+    L.rt_accum_reset.argtypes = [vp, vp, C.POINTER(RtParams)]
+    L.rt_accum_reset.restype = i32
+    L.rt_accum_samples.argtypes = [vp, C.POINTER(u32)]
+    L.rt_accum_samples.restype = i32
+    L.rt_render_samples.argtypes = [vp, vp, vp, u32, vp, sz, C.POINTER(RtStats)]
+    L.rt_render_samples.restype = i32
+    L.rt_accum_read_linear.argtypes = [vp, vp, vp, sz]
+    L.rt_accum_read_linear.restype = i32
     L.rt_struct_sizes.argtypes = [C.POINTER(sz)]
     L.rt_struct_sizes.restype = None
     sizes = (sz * 4)()

@@ -197,6 +197,34 @@ class Context:
                                                       0 if out is None else out.nbytes, C.byref(st)))
         return st.as_dict() if want_stats else None
 
+    # -- progressive rendering ---------------------------------------------------------------------------
+    def accum(self, params: RtParams) -> "Accum":
+        """Sample state (device memory, 96 bytes per pixel) of the band `params` selects, every pixel at sample 0."""
+        return Accum(self, params)
+
+    def render_samples(self, scene: "Scene", acc: "Accum", n: int, out: np.ndarray | None = None, download=True,
+                       want_stats=False):
+        """Advance every pixel of `acc` by `n` samples of its chain.  The band as it now stands (byte-identical to
+        render_division at spp = acc.samples) goes to `out` (None: a new array); download=False skips the copy and
+        returns None in its place."""
+        if download:
+            out = self._out_buffer(out, (acc.rows, acc.width, 3))
+        else:
+            out = None
+        st = RtStats()
+        self._check(self._lib.rt_render_samples(self._h, scene._h, acc._h, int(n),
+                                                None if out is None else out.ctypes.data_as(C.c_void_p),
+                                                0 if out is None else out.nbytes, C.byref(st)))
+        return (out, st.as_dict()) if want_stats else out
+
+    def render_progressive(self, scene: "Scene", params: RtParams, schedule=(1, 1, 2, 4, 8)):
+        """Preview that improves: yields (samples_done, frame) after each chunk of `schedule` samples; each frame equals
+        render_division at spp = samples_done."""
+        with self.accum(params) as acc:
+            for n in schedule:
+                frame = self.render_samples(scene, acc, n)
+                yield acc.samples, frame
+
     # -- shared frame (one NVLink box, one process per GPU) ----------------------------------------------
     def frame_alloc(self, nbytes: int):
         p = C.c_void_p()
@@ -249,6 +277,56 @@ def render_frame_multi(ctxs, scenes, params: RtParams, out: np.ndarray | None = 
     ctxs[0]._check(ctxs[0]._lib.rt_render_frame_multi(ch, sh, n, C.byref(params), out.ctypes.data_as(C.c_void_p),
                                                       out.nbytes, C.byref(st)))
     return (out, st.as_dict()) if want_stats else out
+
+
+class Accum:
+    """Resumable per-pixel sample chains of one frame or division (rt_accum): chunks rendered with
+    Context.render_samples add up to the frame render_division renders at the cumulative sample count."""
+
+    def __init__(self, ctx: Context, params: RtParams):
+        self._ctx = ctx
+        self._h = None
+        div = params.divisions or 1
+        if params.height % div != 0:
+            raise RtError(_abi.RT_ERR_INVALID_ARG, f"height {params.height} is not a multiple of divisions {div}")
+        h = C.c_void_p()
+        ctx._check(ctx._lib.rt_accum_create(ctx._h, C.byref(params), C.byref(h)))
+        self._h = h
+        self.width, self.rows = params.width, params.height // div
+
+    @property
+    def samples(self) -> int:
+        n = C.c_uint32()
+        self._ctx._check(self._ctx._lib.rt_accum_samples(self._h, C.byref(n)))
+        return n.value
+
+    def reset(self, params: RtParams | None = None):
+        """Back to sample 0, optionally with new params of the same size and band (a camera move, another seed)."""
+        self._ctx._check(self._ctx._lib.rt_accum_reset(self._ctx._h, self._h, None if params is None else C.byref(params)))
+
+    def read_linear(self) -> np.ndarray:
+        """float32 (rows, width, 3): sum / samples per channel, before the gamma and 8-bit quantisation."""
+        out = np.empty((self.rows, self.width, 3), dtype=np.float32)
+        self._ctx._check(self._ctx._lib.rt_accum_read_linear(self._ctx._h, self._h, out.ctypes.data_as(C.c_void_p),
+                                                             out.nbytes))
+        return out
+
+    def close(self):
+        if self._h and self._ctx._h:
+            self._ctx._lib.rt_accum_destroy(self._ctx._h, self._h)
+        self._h = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *a):
+        self.close()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
 
 
 class Scene:
