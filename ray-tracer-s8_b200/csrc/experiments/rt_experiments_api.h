@@ -12,6 +12,13 @@ extern "C" {
  * both.  The scene must fit shared memory. */
 int rt_debug_trace_bench(rt_ctx* ctx, const rt_scene* scene, const rt_params* params, uint64_t max_rays, int with_big,
                          uint64_t* n_rays_out, float* ms_while_while, float* ms_state_machine, uint64_t* mismatches_out);
+/* Test aid (csrc/experiments/rt_exact_fastpath.cuh): the guarded fast divisions, square roots, normalisations and sphere
+ * roots of rt_device.cuh against the plain __fdiv_rn / __fsqrt_rn forms, on the device.  Every float32 bit pattern is a
+ * numerator against each of the n_div divisors, and a square-root argument; vecs holds n_vec 3-vectors, sph n_sph
+ * records d.xyz, oc.xyz, r*r.  out[0] / out[1] = bitwise mismatches (scalars / vectors and sphere roots), out[2] = the
+ * number of (numerator, divisor) pairs inside the guarded domain that were compared. */
+int rt_debug_exact_fastpath(const float* divisors, uint32_t n_div, const float* vecs, uint32_t n_vec, const float* sph,
+                            uint32_t n_sph, uint64_t* out);
 #ifdef __cplusplus
 }
 #endif

@@ -664,6 +664,7 @@ __global__ void __launch_bounds__(256) fp32_peak_kernel(float* out, int iters, f
 
 #ifdef RT_B200_EXPERIMENTS
 #include "experiments/rt_experiments.cuh"
+#include "experiments/rt_exact_fastpath.cuh"
 #endif
 
 namespace rtb {

@@ -140,7 +140,9 @@ __device__ __forceinline__ void consider(const HitCtx& hc, V3 o, V3 d, float t, 
             return;
         }
     }
-    float dist = x_length(x_sub(p, o));
+    const V3 po = x_sub(p, o);
+    const float dist2 = x_dot(po, po);
+    const float dist = x_sqrt_domain(dist2) ? x_sqrt_fast(dist2) : x_sqrt_ool(dist2);  // = x_length(po)
     bool take;
     if (best.pid < 0) {
         take = true;
@@ -408,13 +410,24 @@ __device__ __forceinline__ void trace_brute_impl(const DevScene& sc, const Scene
 // ---------------------------------------------------------------------------------------------
 // Camera::get_ray (camera.rs:109-129) — EXACT
 // ---------------------------------------------------------------------------------------------
+static __device__ __noinline__ float2 camera_uv_slow(float nu, float nv, float u_den, float v_den) {
+    return make_float2(x_div_ool(nu, u_den), x_div_ool(nv, v_den));
+}
 __device__ __forceinline__ void primary_ray(const DevCamera& cam, uint32_t x, uint32_t y_cam, Rng& rng, V3* o_out,
                                             V3* d_out) {
     float a, b;
     unit_disc(rng, a, b);
     V3 offset = mk(x_mul(a, cam.lens_radius), x_mul(b, cam.lens_radius), 0.0f);
-    float u = x_div(x_add((float)x, rng.gen_range_0_1()), cam.u_den);
-    float v = x_div(x_add((float)y_cam, rng.gen_range_0_1()), cam.v_den);
+    const float nu = x_add((float)x, rng.gen_range_0_1());
+    const float nv = x_add((float)y_cam, rng.gen_range_0_1());
+    // u = nu / u_den, v = nv / v_den behind one guard
+    float u = x_quot(nu, cam.u_den, x_rcp_refined(cam.u_den));
+    float v = x_quot(nv, cam.v_den, x_rcp_refined(cam.v_den));
+    if (!(x_div_num(nu) && x_div_num(nv) && x_div_mag(cam.u_den) && x_div_mag(cam.v_den))) {
+        const float2 uv = camera_uv_slow(nu, nv, cam.u_den, cam.v_den);
+        u = uv.x;
+        v = uv.y;
+    }
     V3 org = mk(cam.org[0], cam.org[1], cam.org[2]);
     V3 llc = mk(cam.llc[0], cam.llc[1], cam.llc[2]);
     V3 hor = mk(cam.hor[0], cam.hor[1], cam.hor[2]);
@@ -422,16 +435,20 @@ __device__ __forceinline__ void primary_ray(const DevCamera& cam, uint32_t x, ui
     // lower_left_corner + u*horizontal + v*vertical - origin
     V3 target = x_sub(x_add(x_add(llc, x_scale(hor, u)), x_scale(ver, v)), org);
     // Ray::new(origin, normalize_or_zero(target)).at(focus_distance); Ray::new renormalises by division
-    V3 d1 = x_normalize_div(x_normalize_or_zero(target));
+    V3 d1 = x_normalize_div_or_zero(target);
     V3 focal_point = x_add(org, x_scale(d1, cam.focus));
     V3 fo = x_add(org, offset);
     *o_out = fo;
-    *d_out = x_normalize_div(x_normalize_or_zero(x_sub(focal_point, fo)));
+    *d_out = x_normalize_div_or_zero(x_sub(focal_point, fo));
 }
 
 // `(c * 255.999) as u8`: truncation, saturation, NaN → 0 (color.rs:13-19)
-__device__ RT_NORM_FN uint32_t quantise(float sum, float spp_f) {
-    float c = x_sqrt(x_div(sum, spp_f));
+static __device__ __noinline__ float x_sqrt_div_slow(float a, float b) { return x_sqrt_ool(x_div_ool(a, b)); }
+__device__ __forceinline__ uint32_t quantise(float sum, float spp_f) {
+    // sqrt(sum / spp): a zero mean (a black pixel) is its own square root, and the fast square root is NaN there
+    const float m = x_quot(sum, spp_f, x_rcp_refined(spp_f));
+    float c = (m == 0.0f) ? m : x_sqrt_fast(m);
+    if (!(x_div_num(sum) && x_div_mag(spp_f) && (m == 0.0f || x_sqrt_domain(m)))) c = x_sqrt_div_slow(sum, spp_f);
     float s = x_mul(c, 255.999f);
     uint32_t q = __float2uint_rz(s);  // saturating, NaN → 0
     return q > 255u ? 255u : q;
