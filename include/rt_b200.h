@@ -218,8 +218,7 @@ int rt_accum_samples(const rt_accum* acc, uint32_t* samples_out);
  * it now stands: byte-identical to rt_render_division with spp = done + n.  Every chunk since the last create / reset
  * must render the same scene (another one, a re-created one included, is RT_ERR_INVALID_ARG; RT_INTERSECT_AUTO is
  * resolved against the scene of each call).  RT_ERR_INVALID_ARG also for n_samples == 0, done + n_samples above
- * 2^32 - 1, out_len != rows*width*3 with out_rgb != NULL, and an accum of another context; RT_ERR_UNSUPPORTED in the
- * experiments build while an A/B kernel is selected (they have no resumable form).  On any error the state is
+ * 2^32 - 1, out_len != rows*width*3 with out_rgb != NULL, and an accum of another context.  On any error the state is
  * unchanged.  stats (nullable): rays, primary (pixels * n_samples), kernel_ms, total_ms, intersector_used,
  * kernel_launches, the launch shape and redo_pixels; the counters of collect_counters are not filled (0). */
 int rt_render_samples(rt_ctx* ctx, const rt_scene* scene, rt_accum* acc, uint32_t n_samples, uint8_t* out_rgb,

@@ -168,16 +168,6 @@ int launch(rt_ctx* ctx, const rt_scene* scene, const Resolved& r, const LaunchAr
     pr.stage_hint = a.stream ? 1 : 0;
     pr.redo_slab = ctx->d_ctr + RT_CTR_REDO_SLAB;
     pr.slab_tile_rows = a.plan.tile_rows ? a.plan.tile_rows : 1;
-#ifdef RT_B200_EXPERIMENTS
-    pr.ray_dump = ctx->dump_rays;
-    pr.ray_dump_n = ctx->dump_n;
-    pr.ray_dump_cap = ctx->dump_cap;
-    set_experiment_buffers(&ctx->xbuf);
-    if (tunables().bvh_variant != 3) {  // the A/B kernels have no second pass: they need the tie-break tables up front
-        const int src = scene_settle(ctx, scene);
-        if (src) return src;
-    }
-#endif
     const DevScene dev = scene_view(scene);
     CK(ctx, cudaMemsetAsync(ctx->d_ctr, 0, RT_CTR_SLOTS * sizeof(unsigned long long), ctx->stream));
     if (!a.pixel_list) CK(ctx, cudaMemsetAsync(ctx->d_redo, 0, RT_REDO_CAP * sizeof(unsigned int), ctx->stream));
@@ -269,7 +259,7 @@ int finish_stats(rt_ctx* ctx, const Resolved& r, uint64_t pixels, rt_stats* st,
     st->kernel_ms = ms + ctx->first_pass_ms;
     st->total_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
     st->intersector_used = (uint32_t)r.isect;
-    st->kernel_launches = li.launches + (redo ? 1u : 0u);
+    st->kernel_launches = 1u + (redo ? 1u : 0u);
     st->grid_ctas = li.grid;
     st->cta_threads = li.threads;
     st->ctas_per_sm = (uint32_t)li.ctas_per_sm;
@@ -588,9 +578,6 @@ void rt_shutdown(rt_ctx* ctx) {
     for (cudaEvent_t e : ctx->slab_events) cudaEventDestroy(e);
     if (ctx->d_scratch) cudaFree(ctx->d_scratch);
     if (ctx->d_flush) cudaFree(ctx->d_flush);
-#ifdef RT_B200_EXPERIMENTS
-    free_experiment_buffers(&ctx->xbuf);
-#endif
     free_device_build(&ctx->dbuild);
     for (auto& r : ctx->retired) cudaFree(r.p);
     ctx->retired.clear();
@@ -806,10 +793,6 @@ int rt_render_samples(rt_ctx* ctx, const rt_scene* scene, rt_accum* acc, uint32_
         return set_err(ctx, RT_ERR_INVALID_ARG, "rt_render_samples: %u + %u samples overflow 32 bits", acc->samples, n_samples);
     if (acc->samples && scene->serial != acc->scene_serial)
         return set_err(ctx, RT_ERR_INVALID_ARG, "rt_render_samples: not the scene of the chunks since the last create / reset");
-#ifdef RT_B200_EXPERIMENTS
-    if (tunables().bvh_variant != 3)
-        return set_err(ctx, RT_ERR_UNSUPPORTED, "rt_render_samples: the A/B kernels (RT_B200_BVH_KERNEL) have no resumable form");
-#endif
     rt_params p = acc->params;
     p.spp = acc->samples + n_samples;
     Resolved r;
@@ -1014,7 +997,3 @@ int rt_measure_fp32_peak(rt_ctx* ctx, double* tflops_out, float* ms_out) {
 }
 
 }  // extern "C"
-
-#ifdef RT_B200_EXPERIMENTS
-#include "experiments/rt_trace_bench_api.inc"
-#endif

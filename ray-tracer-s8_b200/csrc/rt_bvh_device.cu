@@ -101,7 +101,7 @@ __device__ __forceinline__ void centre_half_dev(const B6& b, float c[3], float h
 __global__ void refit(const unsigned long long* __restrict__ keys, const float* __restrict__ boxes,
                       const uint32_t* __restrict__ pid_of, int n, const int2* __restrict__ child,
                       const int* __restrict__ parent, unsigned int* __restrict__ arrived, B6* nbox,
-                      float4* __restrict__ lnode, float4* __restrict__ lnode_abc, int2* __restrict__ lnode_d) {
+                      float4* __restrict__ lnode) {
     const int p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= n) return;
     int node = parent[n - 1 + p];
@@ -146,12 +146,6 @@ __global__ void refit(const unsigned long long* __restrict__ keys, const float* 
         reinterpret_cast<int4*>(lnode)[NODE_F4 * (size_t)node + 3] =
             make_int4(cl >= 0 ? cl * NODE_BYTES : cl, cr >= 0 ? cr * NODE_BYTES : cr, 0, 0);
         for (int k = 4; k < NODE_F4; k++) lnode[NODE_F4 * (size_t)node + k] = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
-        if (lnode_abc) {  // experiment builds keep the index-coded form as well
-            lnode_abc[3 * (size_t)node + 0] = make_float4(lc[0], lc[1], lc[2], lh[0]);
-            lnode_abc[3 * (size_t)node + 1] = make_float4(lh[1], lh[2], rc[0], rc[1]);
-            lnode_abc[3 * (size_t)node + 2] = make_float4(rc[2], rh[0], rh[1], rh[2]);
-            lnode_d[node] = make_int2(cl, cr);
-        }
         B6 u;
         for (int a = 0; a < 3; a++) {
             u.lo[a] = fminf(bl.lo[a], br.lo[a]);
@@ -175,73 +169,16 @@ size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
 
 }  // namespace
 
-#ifdef RT_B200_EXPERIMENTS
-
-// ---- measurement aid for rt_debug_trace_bench: reorder recorded rays by (direction octant, origin cell) -----------
-namespace {
-__global__ void ray_keys(const float4* __restrict__ rays, unsigned long long n, float3 lo, float3 scale,
-                         unsigned int* __restrict__ keys, unsigned int* __restrict__ idx) {
-    const unsigned long long i = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    const float4 r0 = rays[2 * i], r1 = rays[2 * i + 1];
-    const uint32_t qx = (uint32_t)fminf(fmaxf((r0.x - lo.x) * scale.x, 0.0f), 127.0f);
-    const uint32_t qy = (uint32_t)fminf(fmaxf((r0.y - lo.y) * scale.y, 0.0f), 127.0f);
-    const uint32_t qz = (uint32_t)fminf(fmaxf((r0.z - lo.z) * scale.z, 0.0f), 127.0f);
-    const uint32_t oct = (r0.w < 0.0f ? 1u : 0u) | (r1.x < 0.0f ? 2u : 0u) | (r1.y < 0.0f ? 4u : 0u);
-    const uint32_t cell = (expand10(qx) << 2) | (expand10(qy) << 1) | expand10(qz);  // 21 bits
-    keys[i] = (oct << 21) | cell;
-    idx[i] = (unsigned int)i;
-}
-__global__ void ray_gather(const float4* __restrict__ in, const unsigned int* __restrict__ idx, unsigned long long n,
-                           float4* __restrict__ out) {
-    const unsigned long long i = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    const unsigned long long j = idx[i];
-    out[2 * i] = in[2 * j];
-    out[2 * i + 1] = in[2 * j + 1];
-}
-}  // namespace
-
-// Sorts n recorded rays (2 float4 each) by direction octant, then by the Morton code of the origin's cell in a 128^3 grid
-// over [lo, hi].  `out` receives the reordered rays.  Scratch is allocated and freed here (one-off measurement).
-cudaError_t sort_rays_device(const float4* rays, unsigned long long n, const float lo[3], const float hi[3], float4* out,
-                             cudaStream_t stream) {
-    if (n == 0 || n > 0xffffffffull) return cudaErrorInvalidValue;
-    unsigned int *k0 = nullptr, *k1 = nullptr, *i0 = nullptr, *i1 = nullptr;
-    void* tmp = nullptr;
-    size_t tmp_bytes = 0;
-    cudaError_t e = cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, k0, k1, i0, i1, (int)n, 0, 24, stream);
-    if (e == cudaSuccess) e = cudaMalloc(&k0, n * 4);
-    if (e == cudaSuccess) e = cudaMalloc(&k1, n * 4);
-    if (e == cudaSuccess) e = cudaMalloc(&i0, n * 4);
-    if (e == cudaSuccess) e = cudaMalloc(&i1, n * 4);
-    if (e == cudaSuccess) e = cudaMalloc(&tmp, tmp_bytes);
-    if (e == cudaSuccess) {
-        const float3 l = make_float3(lo[0], lo[1], lo[2]);
-        const float3 sc = make_float3(127.999f / fmaxf(hi[0] - lo[0], 1e-20f), 127.999f / fmaxf(hi[1] - lo[1], 1e-20f),
-                                      127.999f / fmaxf(hi[2] - lo[2], 1e-20f));
-        const unsigned G = (unsigned)((n + 255) / 256);
-        ray_keys<<<G, 256, 0, stream>>>(rays, n, l, sc, k0, i0);
-        e = cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, k0, k1, i0, i1, (int)n, 0, 24, stream);
-        if (e == cudaSuccess) ray_gather<<<G, 256, 0, stream>>>(rays, i1, n, out);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(stream);
-    }
-    cudaFree(k0); cudaFree(k1); cudaFree(i0); cudaFree(i1); cudaFree(tmp);
-    return e;
-}
-
-#endif  // RT_B200_EXPERIMENTS
-
 void free_device_build(DeviceBuild* b) {
     if (b->mem) cudaFree(b->mem);
     *b = DeviceBuild();
 }
 
 // boxes: n x (min xyz, max xyz) of the primitives the tree covers (host); pid_of: their primitive ids (host).
-// Writes n - 1 node records to lnode (device; and to legacy_abc / legacy_d when given); the root is node 0.
+// Writes n - 1 node records to lnode (device); the root is node 0.
 // *depth_out = deepest leaf.
 cudaError_t build_lbvh_device(DeviceBuild* buf, const float* h_boxes, const uint32_t* h_pid_of, uint32_t n,
-                              float4* lnode, float4* lnode_abc, int2* lnode_d, uint32_t* depth_out, cudaStream_t stream) {
+                              float4* lnode, uint32_t* depth_out, cudaStream_t stream) {
     if (n < 2) return cudaErrorInvalidValue;
     // centroid bounds on the host: one pass over data the host already holds
     float cmin[3] = {3.0e38f, 3.0e38f, 3.0e38f}, cmax[3] = {-3.0e38f, -3.0e38f, -3.0e38f};
@@ -296,7 +233,7 @@ cudaError_t build_lbvh_device(DeviceBuild* buf, const float* h_boxes, const uint
     morton_keys<<<G, T, 0, stream>>>(d_boxes, n, lo, sc, k0);
     if ((e = cub::DeviceRadixSort::SortKeys(m + o_sort, sort_bytes, k0, k1, (int)n, 0, 62, stream)) != cudaSuccess) return e;
     karras_nodes<<<G, T, 0, stream>>>(k1, (int)n, d_child, d_parent);
-    refit<<<G, T, 0, stream>>>(k1, d_boxes, d_pid, (int)n, d_child, d_parent, d_arr, d_nbox, lnode, lnode_abc, lnode_d);
+    refit<<<G, T, 0, stream>>>(k1, d_boxes, d_pid, (int)n, d_child, d_parent, d_arr, d_nbox, lnode);
     leaf_depths<<<G, T, 0, stream>>>(d_parent, (int)n, d_arr + n);
     unsigned int depth = 0;
     if ((e = cudaMemcpyAsync(&depth, d_arr + n, 4, cudaMemcpyDeviceToHost, stream)) != cudaSuccess) return e;

@@ -62,12 +62,6 @@ struct rt_ctx {
     std::vector<Retired> retired;
     std::vector<void*> host_allocs;  // rt_host_alloc'ed buffers still alive (freed at shutdown)
     std::string err;
-#ifdef RT_B200_EXPERIMENTS
-    rtb::ExperimentBuffers xbuf;
-    float4* dump_rays = nullptr;  // measurement aid: the instrumented kernel records its queries here
-    unsigned long long* dump_n = nullptr;
-    unsigned long long dump_cap = 0;
-#endif
 };
 constexpr uint32_t RT_REDO_CAP = 1u << 16;
 constexpr int RT_CTR_TICKETS = rtb::NUM_COUNTERS;      // two 32-bit tickets: whole tiles | the tail's pixels

@@ -31,14 +31,6 @@ struct Tunables {
     int aux_delay_ms = 0;        // RT_B200_AUX_DELAY_MS: the builder thread sleeps first (tests: frames rendered before the tables land)
     int wait_timeout_ms = 20000; // RT_B200_WAIT_TIMEOUT_MS: how long a frame owner waits for a slab / a rank for the owner
     bool count_done = true;      // RT_B200_COUNT_DONE=0: no completion counters (frames are copied after the kernel)
-#ifdef RT_B200_EXPERIMENTS
-    int bvh_variant = 3;         // RT_B200_BVH_KERNEL=lanes|simple|pools|deferred|wave|wq
-    int sched_minb = 2;
-    int w[4] = {1, 1, 1, 1}, node_num = 1, node_den = 2;
-    int wave_refill = 8;
-    int wq_warps = 24, wq_chains = 128, wq_min_active = 20, wq_min_node = 24, wq_burst = 2, wq_t_leaf = 4, wq_t_pend = 6,
-        wq_t_fin = 6, wq_sync = 0, wq_budget = 0, tb_alt = 0, tb_burst = 4;
-#endif
 };
 const Tunables& tunables();
 
@@ -47,8 +39,7 @@ struct LaunchInfo {
     size_t dyn_smem = 0;
     int ctas_per_sm = 0;
     bool scene_in_smem = false;
-    unsigned launches = 1;
-    bool counts_done = true;  // the kernel keeps the frame's completion counters (the A/B kernels do not)
+    bool counts_done = true;  // the kernel keeps the frame's completion counters
 };
 
 // rt_bvh_device.cu: LBVH + refit of the traversal tree on the device (scratch owned by the context)
@@ -58,7 +49,7 @@ struct DeviceBuild {
 };
 void free_device_build(DeviceBuild* b);
 cudaError_t build_lbvh_device(DeviceBuild* buf, const float* h_boxes, const uint32_t* h_pid_of, uint32_t n,
-                              float4* lnode, float4* legacy_abc, int2* legacy_d, uint32_t* depth_out, cudaStream_t stream);
+                              float4* lnode, uint32_t* depth_out, cudaStream_t stream);
 
 // rt_kernels.cu
 cudaError_t preload_kernels();
@@ -75,37 +66,6 @@ cudaError_t launch_fp32_peak(float* scratch, int sm_count, int iters, cudaStream
 cudaError_t launch_accum_linear(const void* state, float* out, unsigned long long pixels, uint32_t samples, int sm_count,
                                 cudaStream_t stream);
 size_t scene_smem_bytes(const DevScene& sc, int isect);
-
-#ifdef RT_B200_EXPERIMENTS
-// device buffers of the wavefront pipeline (owned by the context, grown on demand)
-struct WaveBuffers {
-    void* slots = nullptr;          // WSlot[capacity]
-    uint32_t* q_ray = nullptr;      // [capacity] each
-    uint32_t* q_hit = nullptr;
-    uint32_t* q_miss = nullptr;
-    uint32_t* path_ext = nullptr;   // [(ext_depth) * capacity] path entries beyond the 8 kept in the slot
-    void* counters = nullptr;       // WaveCounters[2]
-    size_t capacity = 0, ext_entries = 0;
-};
-void free_wave_buffers(WaveBuffers* wb);
-// device buffer of the warp-private wavefront kernel: per-chain state (rt_kernel_wq.cuh), grown on demand
-struct WqBuffers {
-    void* state = nullptr;
-    size_t bytes = 0;
-};
-void free_wq_buffers(WqBuffers* b);
-struct ExperimentBuffers {
-    WaveBuffers wave;
-    WqBuffers wq;
-};
-void set_experiment_buffers(ExperimentBuffers* b);  // the context whose launch follows (single-threaded tooling)
-void free_experiment_buffers(ExperimentBuffers* b);
-bool legacy_node_arrays_needed();  // true when RT_B200_BVH_KERNEL selects a kernel that reads node_* / cnode_*
-cudaError_t launch_trace_bench(const DevScene& sc, int variant, bool with_big, const float4* rays, unsigned long long n,
-                               unsigned long long* ticket, int2* out, int sm_count, int smem_optin, cudaStream_t stream);
-cudaError_t sort_rays_device(const float4* rays, unsigned long long n, const float lo[3], const float hi[3], float4* out,
-                             cudaStream_t stream);
-#endif
 
 // ---- rt_bvh_host.cpp: SAH BVH with the reference's topology ------------------------------------------
 struct Box {

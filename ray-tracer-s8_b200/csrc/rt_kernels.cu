@@ -28,11 +28,7 @@
 
 namespace rtb {
 
-#ifdef RT_AB_TPB
-constexpr int SMEM_TPB = RT_AB_TPB;  // A/B build: another CTA size for the shared-memory shape
-#else
 constexpr int SMEM_TPB = 1024;
-#endif
 constexpr int OUT_SLOTS = 4;                        // tiles a warp can have in flight in its output stage
 constexpr int TILE_PIX = TILE_W * TILE_H;
 constexpr int TILE_BYTES = TILE_PIX * 3;
@@ -193,12 +189,11 @@ __global__ void __launch_bounds__(TPB, MINB) render_kernel_lanes(const DevScene 
         sv.sph = reinterpret_cast<const float4*>(base);
         sv.tri = reinterpret_cast<const float4*>(base + sc.ns * 16u);
         sv.sph2 = reinterpret_cast<const float4*>(base + geom);
-        sv.na = nullptr; sv.nb = nullptr; sv.nc = nullptr; sv.nd = nullptr;
         sv.nodes_s = (uint32_t)__cvta_generic_to_shared(base + geom);
         sv.nodes_g = nullptr;
     } else {
         sv.sph2 = sc.sph2;
-        sv.sph = sc.sph; sv.tri = sc.tri; sv.na = nullptr; sv.nb = nullptr; sv.nc = nullptr; sv.nd = nullptr;
+        sv.sph = sc.sph; sv.tri = sc.tri;
         sv.nodes_s = 0;
         sv.nodes_g = reinterpret_cast<const char*>(sc.lnode);
     }
@@ -429,22 +424,10 @@ __global__ void __launch_bounds__(TPB, MINB) render_kernel_lanes(const DevScene 
                 ctr.v[CTR_ACTIVE_LANES]++;
                 unsigned am = __activemask();
                 if (lane == (__ffs(am) - 1)) ctr.v[CTR_TOTAL_LANES] += 32;
-#ifdef RT_B200_EXPERIMENTS
-                if (pr.ray_dump) {  // measurement aid: record the query (one atomic per warp)
-                    unsigned long long base = 0;
-                    if (lane == (__ffs(am) - 1)) base = atomicAdd(pr.ray_dump_n, (unsigned long long)__popc(am));
-                    base = __shfl_sync(am, base, __ffs(am) - 1);
-                    const unsigned long long at = base + __popc(am & lt_mask);
-                    if (at < pr.ray_dump_cap) {
-                        pr.ray_dump[2 * at] = make_float4(o.x, o.y, o.z, d.x);
-                        pr.ray_dump[2 * at + 1] = make_float4(d.y, d.z, 0.0f, 0.0f);
-                    }
-                }
-#endif
             }
             Hit h;
             if (ISECT == RT_INTERSECT_BRUTE) trace_brute<COUNT>(sc, sv, o, d, h, ctr);
-            else trace_bvh_ch<COUNT, true, SMEM>(sc, sv, o, d, h, ctr);
+            else trace_bvh_ch<COUNT, SMEM>(sc, sv, o, d, h, ctr);
             if (h.unsure) st |= L_REDO;
 
             bool done;
@@ -660,15 +643,6 @@ __global__ void __launch_bounds__(256) fp32_peak_kernel(float* out, int iters, f
     if (r == 123.456f) out[blockIdx.x * blockDim.x + threadIdx.x] = r;
 }
 
-}  // namespace rtb
-
-#ifdef RT_B200_EXPERIMENTS
-#include "experiments/rt_experiments.cuh"
-#include "experiments/rt_exact_fastpath.cuh"
-#endif
-
-namespace rtb {
-
 // ---------------------------------------------------------------------------------------------
 // Tunables: read from the environment ONCE (rt_init forces the read); measurement switches, not API
 // ---------------------------------------------------------------------------------------------
@@ -696,9 +670,6 @@ const Tunables& tunables() {
         v.pid_order = env_is("RT_B200_PID_ORDER", "world") ? 0 : 1;
         v.aux_delay_ms = std::max(0, env_int("RT_B200_AUX_DELAY_MS", 0));
         v.wait_timeout_ms = std::max(1, env_int("RT_B200_WAIT_TIMEOUT_MS", 20000));
-#ifdef RT_B200_EXPERIMENTS
-        read_experiment_tunables(&v);
-#endif
         return v;
     }();
     return t;
@@ -786,12 +757,6 @@ cudaError_t launch_render(const DevScene& sc, const DevCamera& cam, const DevPar
     const Tunables& tn = tunables();
     const bool resume = pr.state_out != nullptr;  // rt_render_samples
     if (resume) count = false;
-#ifdef RT_B200_EXPERIMENTS
-    {
-        cudaError_t ee;
-        if (launch_experiment(sc, cam, pr, isect, count, sm_count, smem_optin, stream, info, &ee)) return ee;
-    }
-#endif
     const size_t static_smem = (SMEM_TPB / 32) * (OUT_SLOTS * (TILE_BYTES + 16) + 4) + 64;
     const size_t need = scene_smem_bytes(sc, isect);
     // Stage the scene in shared memory when one 1024-thread CTA per SM fits with it (scenes up to ~200 KB); larger

@@ -229,10 +229,6 @@ int rt_scene_create(rt_ctx* ctx, const rt_sphere* spheres, uint32_t n_spheres, c
     lap("world order + boxes");
 
     // ---- which tree will be traversed ---------------------------------------------------------------------
-    bool legacy = false;
-#ifdef RT_B200_EXPERIMENTS
-    legacy = legacy_node_arrays_needed();
-#endif
     const int tree_mode = tn.tree_mode;
     std::vector<uint32_t> big_world;  // split layout: world positions of the primitives kept out of the tree
     std::vector<Box> rest_store;      // boxes and world positions of the primitives the tree covers (split layout only:
@@ -282,7 +278,7 @@ int rt_scene_create(rt_ctx* ctx, const rt_sphere* spheres, uint32_t n_spheres, c
                              (tn.build_mode == 2 || (tn.build_mode == 1 && rest.size() >= kDeviceBuildMin));
 
     // ---- the reference-topology tree: beside everything else when it is worth a thread -------------------
-    const bool ref_sync = !tn.async_ref || tree_mode == 0 || legacy || n < 256;
+    const bool ref_sync = !tn.async_ref || tree_mode == 0 || n < 256;
     HostBVH ref_bvh;  // synchronous case only
     AuxTables ref_tables;
     if (ref_sync) {
@@ -358,81 +354,8 @@ int rt_scene_create(rt_ctx* ctx, const rt_sphere* spheres, uint32_t n_spheres, c
     };
     const size_t o_sph = 0, o_tri = o_sph + (size_t)n_spheres * 16, o_ln = o_tri + (size_t)n_triangles * 64;
     off = align_up(o_ln + (size_t)lni * NODE_BYTES, 256);
-#ifdef RT_B200_EXPERIMENTS
-    const size_t o_la = take((size_t)lni * 48), o_ld = take((size_t)lni * 8);
-#endif
     const size_t o_sph2 = take((size_t)ns8 * 16), o_mat = take((size_t)n * 16), o_em = take((size_t)n * 4),
                  o_box = take((size_t)n * 32), o_big = take((size_t)MAX_BIG * 4);
-#ifdef RT_B200_EXPERIMENTS
-    // trace-bench experiment: the host tree collapsed to 4 children per node (greedy: open the child with the largest box)
-    std::vector<float> w4rec;
-    int32_t w4root = 0;
-    uint32_t w4n = 0;
-    if (T) {
-        auto area = [](const Box& b) {
-            const double sx = (double)b.max[0] - b.min[0], sy = (double)b.max[1] - b.min[1], sz = (double)b.max[2] - b.min[2];
-            return sx * sy + sx * sz + sy * sz;
-        };
-        struct Kid { int32_t code; Box box; };
-        struct Job { int32_t bin; uint32_t slot; };
-        std::vector<Job> jobs;
-        jobs.push_back({T->root, 0});
-        w4n = 1;
-        w4rec.assign(28, 0.0f);
-        for (size_t j = 0; j < jobs.size(); j++) {
-            const Job jb = jobs[j];
-            std::vector<Kid> kids;
-            const HostNode& hn = T->inner[(size_t)jb.bin];
-            kids.push_back({hn.left, hn.box_l});
-            kids.push_back({hn.right, hn.box_r});
-            while (kids.size() < 4) {
-                int best_k = -1;
-                double best_a = -1.0;
-                for (size_t k = 0; k < kids.size(); k++)
-                    if (kids[k].code >= 0 && area(kids[k].box) > best_a) {
-                        best_a = area(kids[k].box);
-                        best_k = (int)k;
-                    }
-                if (best_k < 0) break;
-                const HostNode& cn = T->inner[(size_t)kids[(size_t)best_k].code];
-                kids[(size_t)best_k] = {cn.left, cn.box_l};
-                kids.push_back({cn.right, cn.box_r});
-            }
-            float rec[28];
-            int32_t codes[4];
-            float cc[4][3], hh[4][3];
-            for (int k = 0; k < 4; k++) {
-                if (k < (int)kids.size()) {
-                    centre_half_of(kids[(size_t)k].box, cc[k], hh[k]);
-                    if (kids[(size_t)k].code < 0) {
-                        codes[k] = ~(int32_t)(pid_of_world[(uint32_t)~kids[(size_t)k].code] << 5);
-                    } else {
-                        codes[k] = (int32_t)w4n;
-                        jobs.push_back({kids[(size_t)k].code, w4n});
-                        w4n++;
-                        w4rec.resize((size_t)w4n * 28, 0.0f);
-                    }
-                } else {
-                    for (int a = 0; a < 3; a++) { cc[k][a] = 0.0f; hh[k][a] = -1.0f; }
-                    codes[k] = (int32_t)0x80000000;
-                }
-            }
-            for (int pr2 = 0; pr2 < 2; pr2++) {  // two boxes per three float4
-                const int k0 = 2 * pr2, k1 = 2 * pr2 + 1;
-                float* q = rec + 12 * pr2;
-                q[0] = cc[k0][0]; q[1] = cc[k0][1]; q[2] = cc[k0][2]; q[3] = hh[k0][0];
-                q[4] = hh[k0][1]; q[5] = hh[k0][2]; q[6] = cc[k1][0]; q[7] = cc[k1][1];
-                q[8] = cc[k1][2]; q[9] = hh[k1][0]; q[10] = hh[k1][1]; q[11] = hh[k1][2];
-            }
-            memcpy(rec + 24, codes, 16);
-            memcpy(w4rec.data() + (size_t)jb.slot * 28, rec, sizeof rec);
-        }
-    }
-    const size_t o_w4 = take((size_t)w4n * 112);
-    const size_t nl = legacy ? (size_t)ni_ref : 0;
-    const size_t o_na = take(nl * 16), o_nb = take(nl * 16), o_nc = take(nl * 16), o_nd = take(nl * 8);
-    const size_t o_ca = take(nl * 16), o_cb = take(nl * 16), o_cc = take(nl * 16);
-#endif
     const size_t sync_bytes = off;  // everything up to here is uploaded by this call
     const size_t o_rank = take((size_t)n * 4), o_up = take(((size_t)n + std::max(ni_ref, 1u)) * 4),
                  o_refbox = take((size_t)std::max(ni_ref, 1u) * 64), o_flag = take(4);
@@ -605,10 +528,6 @@ int rt_scene_create(rt_ctx* ctx, const rt_sphere* spheres, uint32_t n_spheres, c
     } else if (T) {
         float* ln = (float*)(h + o_ln);
         int32_t* lc = (int32_t*)(h + o_ln);  // the same records: words 12, 13 are the child codes
-#ifdef RT_B200_EXPERIMENTS
-        float* la = (float*)(h + o_la);
-        int32_t* ld = (int32_t*)(h + o_ld);
-#endif
         struct Item { int32_t code; uint32_t parent; int side; };
         std::vector<Item> todo;
         uint32_t next = 0;
@@ -619,9 +538,6 @@ int rt_scene_create(rt_ctx* ctx, const rt_sphere* spheres, uint32_t n_spheres, c
             const uint32_t me = next++;
             if (it.side < 0) lroot = (int32_t)me * NODE_BYTES;
             else lc[NODE_WORDS * (size_t)it.parent + 12 + it.side] = (int32_t)me * NODE_BYTES;
-#ifdef RT_B200_EXPERIMENTS
-            if (it.side >= 0) ld[2 * (size_t)it.parent + it.side] = (int32_t)me;
-#endif
             const HostNode& hn = T->inner[(size_t)it.code];
             float lcn[3], lhh[3], rcn[3], rhh[3];
             centre_half_of(hn.box_l, lcn, lhh);
@@ -629,21 +545,10 @@ int rt_scene_create(rt_ctx* ctx, const rt_sphere* spheres, uint32_t n_spheres, c
             float* pa = ln + NODE_WORDS * (size_t)me;
             node_box_words(lcn, lhh, rcn, rhh, pa);
             for (int k = 14; k < NODE_WORDS; k++) lc[NODE_WORDS * (size_t)me + k] = 0;
-#ifdef RT_B200_EXPERIMENTS
-            {   // the experiment kernels read the first layout
-                float* q = la + 12 * (size_t)me;
-                q[0] = lcn[0]; q[1] = lcn[1]; q[2] = lcn[2]; q[3] = lhh[0];
-                q[4] = lhh[1]; q[5] = lhh[2]; q[6] = rcn[0]; q[7] = rcn[1];
-                q[8] = rcn[2]; q[9] = rhh[0]; q[10] = rhh[1]; q[11] = rhh[2];
-            }
-#endif
             const int32_t kids[2] = {hn.left, hn.right};
             for (int side = 1; side >= 0; side--) {  // push right first so the left subtree is numbered first
                 if (kids[side] < 0) {
                     lc[NODE_WORDS * (size_t)me + 12 + side] = leaf_code(kids[side]);
-#ifdef RT_B200_EXPERIMENTS
-                    ld[2 * (size_t)me + side] = leaf_code(kids[side]);
-#endif
                 } else {
                     todo.push_back(Item{kids[side], me, side});
                 }
@@ -652,40 +557,6 @@ int rt_scene_create(rt_ctx* ctx, const rt_sphere* spheres, uint32_t n_spheres, c
     } else if (ltree) {  // a single primitive in the tree: the root is its leaf
         lroot = leaf_code(~(int32_t)rest_world[0]);
     }
-#ifdef RT_B200_EXPERIMENTS
-    if (w4n) memcpy(h + o_w4, w4rec.data(), (size_t)w4n * 112);
-    if (legacy) {  // the reference-topology tree in the first kernels' formats
-        float* h_na = (float*)(h + o_na); float* h_nb = (float*)(h + o_nb); float* h_nc = (float*)(h + o_nc);
-        int32_t* h_nd = (int32_t*)(h + o_nd);
-        auto code_of = [&](int32_t c) -> int32_t { return c >= 0 ? c : ~(int32_t)pid_of_world[(uint32_t)~c]; };
-        for (uint32_t i = 0; i < (uint32_t)ref_bvh.inner.size(); i++) {
-            const HostNode& hn = ref_bvh.inner[i];
-            const Box* bs[2] = {&hn.box_l, &hn.box_r};
-            float lo[2][3], hi[2][3], cc[2][3], hh[2][3];
-            for (int s = 0; s < 2; s++) {
-                float m = 0.0f;
-                for (int a = 0; a < 3; a++) m = fmaxf(m, fmaxf(fabsf(bs[s]->min[a]), fabsf(bs[s]->max[a])));
-                const float pad = m * 4e-6f + 1e-30f;
-                for (int a = 0; a < 3; a++) {
-                    lo[s][a] = bs[s]->min[a] - pad;
-                    hi[s][a] = bs[s]->max[a] + pad;
-                }
-                centre_half_of(*bs[s], cc[s], hh[s]);
-            }
-            float* a = h_na + 4 * (size_t)i; float* b = h_nb + 4 * (size_t)i; float* c = h_nc + 4 * (size_t)i;
-            a[0] = lo[0][0]; a[1] = lo[0][1]; a[2] = lo[0][2]; a[3] = hi[0][0];
-            b[0] = hi[0][1]; b[1] = hi[0][2]; b[2] = lo[1][0]; b[3] = lo[1][1];
-            c[0] = lo[1][2]; c[1] = hi[1][0]; c[2] = hi[1][1]; c[3] = hi[1][2];
-            h_nd[2 * (size_t)i] = code_of(hn.left);
-            h_nd[2 * (size_t)i + 1] = code_of(hn.right);
-            float* ca = (float*)(h + o_ca) + 4 * (size_t)i; float* cb = (float*)(h + o_cb) + 4 * (size_t)i;
-            float* c3 = (float*)(h + o_cc) + 4 * (size_t)i;
-            ca[0] = cc[0][0]; ca[1] = cc[0][1]; ca[2] = cc[0][2]; ca[3] = hh[0][0];
-            cb[0] = hh[0][1]; cb[1] = hh[0][2]; cb[2] = cc[1][0]; cb[3] = cc[1][1];
-            c3[0] = cc[1][2]; c3[1] = hh[1][0]; c3[2] = hh[1][1]; c3[3] = hh[1][2];
-        }
-    }
-#endif
     if (ref_sync) {
         memcpy(h + o_rank, ref_tables.rank.data(), ref_tables.rank.size() * 4);
         memcpy(h + o_up, ref_tables.up.data(), ref_tables.up.size() * 4);
@@ -721,13 +592,7 @@ int rt_scene_create(rt_ctx* ctx, const rt_sphere* spheres, uint32_t n_spheres, c
         }
         uint32_t depth = 0;
         e = build_lbvh_device(&ctx->dbuild, dev_boxes.data(), dev_pid.data(), (uint32_t)dev_pid.size(),
-                              (float4*)(sc->d_blob + o_ln),
-#ifdef RT_B200_EXPERIMENTS
-                              (float4*)(sc->d_blob + o_la), (int2*)(sc->d_blob + o_ld),
-#else
-                              nullptr, nullptr,
-#endif
-                              &depth, ctx->stream);
+                              (float4*)(sc->d_blob + o_ln), &depth, ctx->stream);
         if (e != cudaSuccess || depth > (uint32_t)MAX_STACK) {
             give_back();
             if (e != cudaSuccess) return set_err(ctx, RT_ERR_CUDA, "device BVH build failed: %s", cudaGetErrorString(e));
@@ -743,10 +608,6 @@ int rt_scene_create(rt_ctx* ctx, const rt_sphere* spheres, uint32_t n_spheres, c
     d.sph = (const float4*)(sc->d_blob + o_sph);
     d.tri = (const float4*)(sc->d_blob + o_tri);
     d.lnode = (const float4*)(sc->d_blob + o_ln);
-#ifdef RT_B200_EXPERIMENTS
-    d.lnode_a = (const float4*)(sc->d_blob + o_la);
-    d.lnode_d = (const int2*)(sc->d_blob + o_ld);
-#endif
     d.sph2 = (const float4*)(sc->d_blob + o_sph2);
     d.lni = lni;
     d.lroot = lroot;
@@ -764,20 +625,6 @@ int rt_scene_create(rt_ctx* ctx, const rt_sphere* spheres, uint32_t n_spheres, c
     d.ns = n_spheres;
     d.nt = n_triangles;
     d.ni = ni_ref;
-#ifdef RT_B200_EXPERIMENTS
-    for (size_t i = 0; i < (size_t)MAX_BIG; i++) d.big_pid[i] = i < big_world.size() ? pid_of_world[big_world[i]] : 0u;
-    d.w4 = (const float4*)(sc->d_blob + o_w4);
-    d.w4n = w4n;
-    d.w4root = w4root;
-    d.node_a = (const float4*)(sc->d_blob + o_na);
-    d.node_b = (const float4*)(sc->d_blob + o_nb);
-    d.node_c = (const float4*)(sc->d_blob + o_nc);
-    d.node_d = (const int2*)(sc->d_blob + o_nd);
-    d.cnode_a = (const float4*)(sc->d_blob + o_ca);
-    d.cnode_b = (const float4*)(sc->d_blob + o_cb);
-    d.cnode_c = (const float4*)(sc->d_blob + o_cc);
-    d.root = ref_sync ? (ref_bvh.root >= 0 ? ref_bvh.root : ~(int32_t)pid_of_world[(uint32_t)~ref_bvh.root]) : 0;
-#endif
     *out = sc.release();
     return RT_OK;
     RT_GUARD_END(ctx)

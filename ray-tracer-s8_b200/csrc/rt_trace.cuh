@@ -1,8 +1,7 @@
 // rt_trace.cuh — device code of the nearest-hit query and of the per-sample arithmetic (sm_100a).
 //
-// Shared by the product kernel (rt_kernels.cu) and, in the experiments build, by the A/B kernels under
-// csrc/experiments/.  Everything that decides a path is in the EXACT domain of rt_device.cuh; the FILTER-domain
-// tests here only cull.
+// Included by the render kernel (rt_kernels.cu).  Everything that decides a path is in the EXACT domain of
+// rt_device.cuh; the FILTER-domain tests here only cull.
 //
 //   K1 (trace_brute):  every primitive per query; the sphere FILTER runs on pairs of spheres in packed f32x2
 //                      arithmetic (FADD2 / FMUL2 / FFMA2), exact reference arithmetic only where it passes.
@@ -14,8 +13,7 @@
 
 namespace rtb {
 
-constexpr int THREADS = 256;  // CTA size of the instrumented (COUNT) instantiations and of the A/B kernels
-constexpr int WARPS = THREADS / 32;
+constexpr int THREADS = 256;  // CTA size of the instrumented (COUNT) instantiations and of the global-memory kernels
 
 struct Hit {
     float dist;  // length(point - origin), exact domain
@@ -41,10 +39,6 @@ struct SceneView {
     const float4* sph2;  // brute-force kernel only
     const float4* sph;
     const float4* tri;
-    const float4* na;   // experiment kernels: index-coded node arrays
-    const float4* nb;
-    const float4* nc;
-    const int2* nd;
     uint32_t nodes_s;       // shared-memory kernel: shared-window address of node record 0 (already inside the child codes)
     const char* nodes_g;    // global-memory kernel: DevScene::lnode
 };
@@ -101,11 +95,7 @@ __device__ __forceinline__ bool aux_now(const HitCtx& hc) {
     return v != 0;
 }
 __device__ __forceinline__ HitCtx hit_ctx(const DevScene& sc) {
-#ifdef RT_AB_NO_UNSURE  // A/B build: tables assumed present (no second-pass bookkeeping in the kernel)
-    return HitCtx{sc.leaf_box, sc.rank, sc.ref_up, sc.ref_box, sc.aux_flag, sc.ns + sc.nt, 1};
-#else
     return HitCtx{sc.leaf_box, sc.rank, sc.ref_up, sc.ref_box, sc.aux_flag, sc.ns + sc.nt, sc.aux_ready};
-#endif
 }
 
 // Rays with a direction component of exactly +-0 make the reference's slab test produce inf / NaN planes
@@ -167,74 +157,6 @@ __device__ __forceinline__ void consider(const HitCtx& hc, V3 o, V3 d, float t, 
         best.pid |= flag;  // best.pid >= 0 here: a candidate is only ever refused in favour of an incumbent
     }
 }
-__device__ __forceinline__ void consider(const DevScene& sc, V3 o, V3 d, float t, int pid, Hit& best) {
-    consider(hit_ctx(sc), o, d, t, pid, best);
-}
-
-template <bool COUNT>
-__device__ __forceinline__ void test_sphere(const DevScene& sc, const float4 s, int pid, V3 o, V3 d, Hit& best,
-                                            Ctr& ctr) {
-    // oc = origin - center is a single exact subtraction: shared by filter and exact path
-    V3 oc = mk(x_sub(o.x, s.x), x_sub(o.y, s.y), x_sub(o.z, s.z));
-    // FILTER: reference discriminant is 4*(bh*bh - (|oc|^2 - r^2)), bh = d.oc.  Evaluate it with FMAs
-    // and reject only when it is negative by more than a generous rounding bound (~300 ulp of |oc|^2).
-    float bh = fmaf(oc.z, d.z, fmaf(oc.y, d.y, oc.x * d.x));
-    float oc2 = fmaf(oc.z, oc.z, fmaf(oc.y, oc.y, oc.x * oc.x));
-    float cf = oc2 - s.w;
-    float disc = fmaf(bh, bh, -cf);
-    if (COUNT) ctr.v[CTR_SPH_TEST]++;
-    if (fmaf(oc2, 2e-5f, disc) < 0.0f) return;
-    // both roots behind the origin (ray points away, origin outside): cannot be in [T_MIN, T_MAX)
-    if (bh > 0.0f && cf > 1e-4f * oc2) return;
-    if (COUNT) ctr.v[CTR_SPH_EXACT]++;
-    float t;
-    if (!sphere_root_exact(d, oc, s.w, &t)) return;
-    if (COUNT) ctr.v[CTR_SPH_HIT]++;
-    consider(sc, o, d, t, pid, best);
-}
-
-template <bool COUNT>
-__device__ __forceinline__ void test_triangle(const DevScene& sc, const float4* tri, int tidx, int pid, V3 o, V3 d,
-                                              Hit& best, Ctr& ctr) {
-    V3 a = ld3(tri[4 * tidx + 0]);
-    V3 ab = ld3(tri[4 * tidx + 1]);
-    V3 ac = ld3(tri[4 * tidx + 2]);
-    if (COUNT) ctr.v[CTR_TRI_TEST]++;
-    float t;
-    int stage;
-    bool hit = triangle_root_exact(o, d, a, ab, ac, &t, &stage);
-    if (COUNT) {
-        if (stage >= 1) ctr.v[CTR_TRI_S1]++;
-        if (stage >= 2) ctr.v[CTR_TRI_S2]++;
-        if (stage >= 3) ctr.v[CTR_TRI_S3]++;
-        if (hit) ctr.v[CTR_TRI_HIT]++;
-    }
-    if (!hit) return;
-    consider(sc, o, d, t, pid, best);
-}
-
-// ---- the same tests split into a cheap FILTER stage and an EXACT stage (scheduled kernel) ----
-__device__ __forceinline__ bool sphere_filter(const float4 s, V3 o, V3 d) {
-    const float ocx = x_sub(o.x, s.x), ocy = x_sub(o.y, s.y), ocz = x_sub(o.z, s.z);
-    const float bh = fmaf(ocz, d.z, fmaf(ocy, d.y, ocx * d.x));
-    const float oc2 = fmaf(ocz, ocz, fmaf(ocy, ocy, ocx * ocx));
-    const float cf = oc2 - s.w;
-    const float disc = fmaf(bh, bh, -cf);
-    if (fmaf(oc2, 2e-5f, disc) < 0.0f) return false;
-    if (bh > 0.0f && cf > 1e-4f * oc2) return false;
-    return true;
-}
-
-template <bool COUNT>
-__device__ __forceinline__ void sphere_exact(const DevScene& sc, const float4 s, int pid, V3 o, V3 d, Hit& best,
-                                             Ctr& ctr) {
-    const V3 oc = mk(x_sub(o.x, s.x), x_sub(o.y, s.y), x_sub(o.z, s.z));
-    if (COUNT) ctr.v[CTR_SPH_EXACT]++;
-    float t;
-    if (!sphere_root_exact(d, oc, s.w, &t)) return;
-    if (COUNT) ctr.v[CTR_SPH_HIT]++;
-    consider(sc, o, d, t, pid, best);
-}
 
 // FMA Moeller-Trumbore with error-scaled margins: false only when the exact test (mesh.rs:109-161) must
 // reject, or when the hit would be farther than the current best by more than the tie margin.
@@ -260,23 +182,6 @@ __device__ __forceinline__ bool triangle_filter(const float4* tri, int tidx, V3 
     const float et = 1e-4f * mag * mab * mac * ainv + 1e-6f;
     if (t < 0.0009f - et || t > cull + et) return false;  // exact needs t in [T_MIN, T_MAX) and a chance to win
     return true;
-}
-
-template <bool COUNT>
-__device__ __forceinline__ void triangle_exact(const DevScene& sc, const float4* tri, int tidx, int pid, V3 o, V3 d,
-                                               Hit& best, Ctr& ctr) {
-    const V3 a = ld3(tri[4 * tidx + 0]), ab = ld3(tri[4 * tidx + 1]), ac = ld3(tri[4 * tidx + 2]);
-    float t;
-    int stage;
-    const bool hit = triangle_root_exact(o, d, a, ab, ac, &t, &stage);
-    if (COUNT) {
-        if (stage >= 1) ctr.v[CTR_TRI_S1]++;
-        if (stage >= 2) ctr.v[CTR_TRI_S2]++;
-        if (stage >= 3) ctr.v[CTR_TRI_S3]++;
-        if (hit) ctr.v[CTR_TRI_HIT]++;
-    }
-    if (!hit) return;
-    consider(sc, o, d, t, pid, best);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -475,7 +380,7 @@ __device__ __forceinline__ void load_node(const SceneView& sv, int cur, float4& 
     }
 }
 constexpr int TR_DONE = (int)0x80000000;  // traversal finished (never a leaf code: first_pid < 2^26)
-template <bool COUNT, bool WITH_BIG, bool SMEM>
+template <bool COUNT, bool SMEM>
 __device__ __forceinline__ void trace_bvh_ch_impl(const DevScene& sc, const SceneView& sv, V3 o, V3 d, Hit& best, Ctr& ctr) {
     best.pid = -1;
     best.dist = 0.0f;
@@ -491,11 +396,9 @@ __device__ __forceinline__ void trace_bvh_ch_impl(const DevScene& sc, const Scen
     const float qx = -o.x * ix, qy = -o.y * iy, qz = -o.z * iz;
     // rounding of the o-term: <= 3 * 2^-24 * |o*inv| per axis, in t (the c- and h-terms are padded on the host)
     const float slack = 4.8e-7f * fmaxf(fmaxf(fabsf(qx), fabsf(qy)), fabsf(qz)) + 1e-30f;
-#if RT_NODE_XY
     const f32x2 i_xy = pk2(ix, iy), q_xy = pk2(qx, qy), a_xy = pk2(ax, ay), na_xy = pk2(-ax, -ay);
     const f32x2 i_zz = pk2(iz, iz), q_zz = pk2(qz, qz), a_zz = pk2(az, az), na_zz = pk2(-az, -az);
     const f32x2 slack2 = pk2(slack, slack);
-#endif
     float cull = 1001.0f;  // a hit has t < T_MAX and length(p-o) ~ t
     const int ns = (int)sc.ns;
     const HitCtx hc = hit_ctx(sc);
@@ -508,14 +411,13 @@ __device__ __forceinline__ void trace_bvh_ch_impl(const DevScene& sc, const Scen
     int* top = stack + 1;  // next free entry
     if (sc.ltree) *top++ = (SMEM && sc.lroot >= 0) ? sc.lroot + (int)sv.nodes_s : sc.lroot;
 #pragma unroll 1
-    for (int i = (int)sc.nbig - 1; WITH_BIG && i >= 0; i--) *top++ = __ldg(&sc.big_code[i]);
+    for (int i = (int)sc.nbig - 1; i >= 0; i--) *top++ = __ldg(&sc.big_code[i]);
     int cur = *--top;
     for (;;) {
         while (cur >= 0) {
             float4 a, b, c;
             int2 ch;
             load_node<SMEM>(sv, cur, a, b, c, ch);
-#if RT_NODE_XY
             // a = l.c.xy | l.h.xy, b = r.c.xy | r.h.xy, c = l.c.z r.c.z | l.h.z r.h.z: the eighteen FMAs of the two slab
             // tests are nine packed ones (x|y of each box, z of both boxes); results are the scalar FMAs' bit for bit
             const f32x2 lc2 = fma2(pk2(a.x, a.y), i_xy, q_xy), rc2 = fma2(pk2(b.x, b.y), i_xy, q_xy);
@@ -534,17 +436,6 @@ __device__ __forceinline__ void trace_bvh_ch_impl(const DevScene& sc, const Scen
             upk2(add2(pk2(fl, fr), slack2), fls, frs);
             const bool hl = tl <= fls;
             const bool hr = tr <= frs;
-#else
-            // left box: c = (a.x,a.y,a.z) h = (a.w,b.x,b.y); right: c = (b.z,b.w,c.x) h = (c.y,c.z,c.w)
-            const float lcx = fmaf(a.x, ix, qx), lcy = fmaf(a.y, iy, qy), lcz = fmaf(a.z, iz, qz);
-            const float rcx = fmaf(b.z, ix, qx), rcy = fmaf(b.w, iy, qy), rcz = fmaf(c.x, iz, qz);
-            const float tl = fmaxf(fmaxf(fmaf(-a.w, ax, lcx), fmaf(-b.x, ay, lcy)), fmaxf(fmaf(-b.y, az, lcz), 0.0f));
-            const float fl = fminf(fminf(fmaf(a.w, ax, lcx), fmaf(b.x, ay, lcy)), fminf(fmaf(b.y, az, lcz), cull));
-            const float tr = fmaxf(fmaxf(fmaf(-c.y, ax, rcx), fmaf(-c.z, ay, rcy)), fmaxf(fmaf(-c.w, az, rcz), 0.0f));
-            const float fr = fminf(fminf(fmaf(c.y, ax, rcx), fmaf(c.z, ay, rcy)), fminf(fmaf(c.w, az, rcz), cull));
-            const bool hl = tl <= fl + slack;
-            const bool hr = tr <= fr + slack;
-#endif
             if (COUNT) ctr.v[CTR_SLAB] += 2;
             // branch-light step: push and pop are short predicated blocks, the loop has one exit
             const bool swap = tr < tl;
@@ -604,9 +495,9 @@ __device__ __forceinline__ void trace_brute(const DevScene& sc, const SceneView&
     trace_brute_impl<COUNT>(sc, sv, o, d, best, ctr);
     hit_finish(best);
 }
-template <bool COUNT, bool WITH_BIG, bool SMEM>
+template <bool COUNT, bool SMEM>
 __device__ __forceinline__ void trace_bvh_ch(const DevScene& sc, const SceneView& sv, V3 o, V3 d, Hit& best, Ctr& ctr) {
-    trace_bvh_ch_impl<COUNT, WITH_BIG, SMEM>(sc, sv, o, d, best, ctr);
+    trace_bvh_ch_impl<COUNT, SMEM>(sc, sv, o, d, best, ctr);
     hit_finish(best);
 }
 

@@ -10,11 +10,10 @@ import os
 
 PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 LIB_DIR = os.path.normpath(os.path.join(PKG_DIR, "..", "lib"))
-# RT_B200_LIB=exp selects the experiments build (product + the A/B kernels of csrc/experiments/, `make exp`): tooling and
-# the variant-agreement test only.  The product library is the default and carries no A/B code.
+# RT_B200_LIB=/path/to/lib.so loads a development build under another name (A/B measurements of `make EXTRA=-D...`
+# builds); the product library is the default.
 _sel = os.environ.get("RT_B200_LIB", "")
-LIB_PATH = (_sel if "/" in _sel else           # a development build under another name (A/B measurements)
-            os.path.join(LIB_DIR, "librt_b200_exp.so" if _sel == "exp" else "librt_b200.so"))
+LIB_PATH = _sel if "/" in _sel else os.path.join(LIB_DIR, "librt_b200.so")
 
 RT_OK = 0
 RT_ERR_INVALID_ARG = -1
@@ -76,8 +75,6 @@ EXPORTS = [
     "rt_scene_wait_ready", "rt_render_frame_multi", "rt_frame_collect", "rt_render_tiles_collect", "rt_frame_wait_consumed", "rt_l2_flush",
     "rt_accum_create", "rt_accum_destroy", "rt_accum_reset", "rt_accum_samples", "rt_render_samples", "rt_accum_read_linear",
 ]
-# only in the experiments build (csrc/experiments/rt_experiments_api.h)
-EXPERIMENT_EXPORTS = ["rt_debug_trace_bench"]
 
 _lib = None
 
@@ -138,10 +135,6 @@ def lib():
     L.rt_frame_download.restype = i32
     L.rt_measure_fp32_peak.argtypes = [vp, C.POINTER(C.c_double), C.POINTER(C.c_float)]
     L.rt_measure_fp32_peak.restype = i32
-    if hasattr(L, "rt_debug_trace_bench"):
-        L.rt_debug_trace_bench.argtypes = [vp, vp, C.c_void_p, C.c_uint64, i32, C.POINTER(C.c_uint64), C.POINTER(C.c_float),
-                                           C.POINTER(C.c_float), C.POINTER(C.c_uint64)]
-        L.rt_debug_trace_bench.restype = i32
     L.rt_scene_wait_ready.argtypes = [vp, vp]
     L.rt_scene_wait_ready.restype = i32
     L.rt_render_frame_multi.argtypes = [pp, pp, u32, C.POINTER(RtParams), vp, sz, C.POINTER(RtStats)]

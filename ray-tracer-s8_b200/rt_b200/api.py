@@ -112,17 +112,6 @@ class Context:
         self._check(self._lib.rt_l2_flush(self._h, nbytes, C.byref(ms) if timed else None))
         return ms.value if timed else None
 
-    def trace_bench(self, scene: "Scene", params: RtParams, max_rays: int, with_big: bool = True, sort: bool = False):
-        """Development aid (experiments build, RT_B200_LIB=exp): the nearest-hit query alone over the recorded queries of
-        one frame (csrc/experiments/rt_trace_bench.cuh)."""
-        if not hasattr(self._lib, "rt_debug_trace_bench"):
-            raise RtError(_abi.RT_ERR_UNSUPPORTED, "rt_debug_trace_bench exists only in librt_b200_exp.so (RT_B200_LIB=exp)")
-        n, bad = C.c_uint64(), C.c_uint64()
-        ms_ww, ms_sm = C.c_float(), C.c_float()
-        self._check(self._lib.rt_debug_trace_bench(self._h, scene._h, C.byref(params), int(max_rays), (1 if with_big else 0) + (2 if sort else 0),
-                                                   C.byref(n), C.byref(ms_ww), C.byref(ms_sm), C.byref(bad)))
-        return {"rays": n.value, "ms_while_while": ms_ww.value, "ms_state_machine": ms_sm.value, "mismatches": bad.value}
-
     def sync(self):
         self._check(self._lib.rt_sync(self._h))
 

@@ -2,7 +2,7 @@
 line) against the plain __fdiv_rn / __fsqrt_rn code they replace, bit for bit.
 
 GPU: every float32 bit pattern as numerator against divisors that straddle the guard's edges, every bit pattern as a
-square-root argument, seeded and built 3-vectors, and sphere roots (experiments build, rt_debug_exact_fastpath).
+square-root argument, seeded and built 3-vectors, and sphere roots (rt_debug_exact_fastpath of lib/librt_b200_check.so).
 CPU: the division guard, read from the header, accepts no exponent pair whose quotient or residual could leave the
 normal range.
 """
@@ -15,7 +15,7 @@ import pytest
 
 ROOT = os.path.abspath(os.path.join(os.path.dirname(__file__), ".."))
 HDR = os.path.join(ROOT, "ray-tracer-s8_b200", "csrc", "rt_device.cuh")
-EXP_LIB = os.path.join(ROOT, "ray-tracer-s8_b200", "lib", "librt_b200_exp.so")
+CHECK_LIB = os.path.join(ROOT, "ray-tracer-s8_b200", "lib", "librt_b200_check.so")
 
 
 def _const(name):
@@ -123,7 +123,7 @@ def _spheres():
 
 @pytest.mark.gpu
 def test_fast_paths_match_ieee_bit_for_bit():
-    L = C.CDLL(EXP_LIB)
+    L = C.CDLL(CHECK_LIB)
     f = L.rt_debug_exact_fastpath
     fp = C.POINTER(C.c_float)
     f.argtypes = [fp, C.c_uint32, fp, C.c_uint32, fp, C.c_uint32, C.POINTER(C.c_uint64)]

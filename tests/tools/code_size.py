@@ -23,12 +23,8 @@ print("total instructions", n, f"= {n * 16 / 1024:.1f} KB")
 src = {}
 def line_text(f, l):
     if f not in src:
-        for d in ("ray-tracer-s8_b200/csrc", "ray-tracer-s8_b200/csrc/experiments"):
-            p = os.path.join(d, f)
-            if os.path.exists(p):
-                src[f] = open(p).read().split("\n"); break
-        else:
-            src[f] = []
+        p = os.path.join("ray-tracer-s8_b200/csrc", f)
+        src[f] = open(p).read().split("\n") if os.path.exists(p) else []
     return src[f][l - 1].strip()[:90] if 0 < l <= len(src[f]) else ""
 for (f, l), c in cnt.most_common(int(sys.argv[3]) if len(sys.argv) > 3 else 45):
     print(f"{c:5d} {f}:{l:<5d} {line_text(f, l)}")

@@ -1,5 +1,5 @@
 """Dev tool (GPU box): kernel timings per workload + quick parity against the oracle.
-usage: python tests/tools/kbench.py [C2 C3 ...]   (env RT_B200_BVH_KERNEL=simple for the first BVH kernel)"""
+usage: python tests/tools/kbench.py [C2 C3 ...]"""
 import os, sys, time
 ROOT = os.path.abspath(os.path.join(os.path.dirname(__file__), "..", ".."))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "ray-tracer-s8_b200"))
@@ -12,7 +12,6 @@ from oracle import oracle as O
 def main():
     names = sys.argv[1:] or ["C2", "C3"]
     ctx = rt.Context(0)
-    print("variant", os.environ.get("RT_B200_BVH_KERNEL", "sched"))
     # parity on crops
     for name, w, h, spp, mb, n, plane in [("p1", 480, 270, 4, 5, 1024, True), ("p2", 320, 240, 2, 10, 64, False),
                                           ("p3", 101, 67, 3, 4, 32, True), ("p4", 64, 48, 2, 5, 1, False)]:
