@@ -88,19 +88,17 @@ int resolve_params(rt_ctx* ctx, const rt_params* in, bool whole_frame, Resolved*
     return RT_OK;
 }
 
-// A frame download is streamed in slabs of whole tile rows, about slab_bytes each and at most tunables().slabs.
+// A frame download is streamed in slabs of whole tile rows, about kSlabBytes each and at most kSlabs.
+constexpr size_t kSlabs = 16;
+constexpr size_t kSlabBytes = (size_t)1 << 20;
+static_assert(kSlabs <= (size_t)MAX_SLABS, "a frame's control block has MAX_SLABS counters");
 SlabPlan plan_slabs(uint32_t width, uint32_t rows) {
-    static const size_t slab_bytes = [] {
-        const char* e = std::getenv("RT_B200_SLAB_BYTES");
-        const long long v = e ? std::atoll(e) : (1ll << 20);
-        return (size_t)(v > 0 ? v : 1);
-    }();
     SlabPlan p;
     p.width = width;
     p.rows = rows;
     const uint32_t tiles_y = (rows + TILE_H - 1) / TILE_H;
     const size_t bytes = (size_t)width * rows * 3;
-    uint32_t s = (uint32_t)std::min<size_t>((size_t)tunables().slabs, std::max<size_t>(1, bytes / slab_bytes));
+    uint32_t s = (uint32_t)std::min<size_t>(kSlabs, std::max<size_t>(1, bytes / kSlabBytes));
     s = std::max(1u, std::min(s, tiles_y));
     p.tile_rows = (tiles_y + s - 1) / s;
     p.slabs = (tiles_y + p.tile_rows - 1) / p.tile_rows;
@@ -183,7 +181,7 @@ static int read_counters(rt_ctx* ctx) {
     CK(ctx, cudaStreamSynchronize(ctx->stream));
     if (ctx->h_flag[0]) {
         ctx->h_flag[0] = 0;
-        return set_err(ctx, RT_ERR_TIMEOUT, "waited %d ms for a frame counter (the owner's \"consumed\" word, or a slab of the frame)", tunables().wait_timeout_ms);
+        return set_err(ctx, RT_ERR_TIMEOUT, "waited %d ms for a frame counter (the owner's \"consumed\" word, or a slab of the frame)", test_hooks().wait_timeout_ms);
     }
     return RT_OK;
 }
@@ -270,11 +268,10 @@ int finish_stats(rt_ctx* ctx, const Resolved& r, uint64_t pixels, rt_stats* st,
 }
 
 int enqueue_slab_copies(rt_ctx* ctx, const uint8_t* frame_dev, const rt_frame_ctl* ctl, const SlabPlan& plan, uint64_t seq,
-                        uint8_t* out_rgb, bool reverse_order, SlabJob* job) {
+                        uint8_t* out_rgb, SlabJob* job) {
     job->plan = plan;
     job->out = out_rgb;
     job->pinned = out_rgb;
-    job->reverse = reverse_order;
     const size_t bytes = (size_t)plan.rows * plan.width * 3;
     if (out_rgb) {
         cudaPointerAttributes attr;
@@ -305,8 +302,8 @@ int enqueue_slab_copies(rt_ctx* ctx, const uint8_t* frame_dev, const rt_frame_ct
         CK(ctx, launch_wait_all_slabs(ctl->done, (unsigned long long)seq, plan.slabs, plan.tile_rows, plan.rows, plan.width,
                                       ctx->h_flag, ctx->copy_stream));
     for (uint32_t i = 0; (out_rgb || by_value) && i < plan.slabs; i++) {
-        // tickets walk the frame bottom-up by default: the last slab completes first
-        const uint32_t s = reverse_order ? plan.slabs - 1 - i : i;
+        // tickets walk the frame bottom-up: the last slab completes first
+        const uint32_t s = plan.slabs - 1 - i;
         const unsigned long long target = (unsigned long long)seq * plan.pixels(s);
         if (by_value) {  // CU_STREAM_WAIT_VALUE_GEQ = 0: the stream itself waits, no SM involved
             const int wr = ctx->stream_wait_value64((void*)ctx->copy_stream, (unsigned long long)(uintptr_t)&ctl->done[s], target, 0u);
@@ -332,7 +329,7 @@ int enqueue_slab_copies(rt_ctx* ctx, const uint8_t* frame_dev, const rt_frame_ct
 static int host_copy_slabs(rt_ctx* ctx, const SlabJob& job, uint32_t first, bool until_kernel_done, uint32_t* done_out) {
     uint32_t i = first;
     for (; i < job.plan.slabs; i++) {
-        const uint32_t s = job.reverse ? job.plan.slabs - 1 - i : i;
+        const uint32_t s = job.plan.slabs - 1 - i;  // in the order enqueue_slab_copies queued them
         if (until_kernel_done) {
             bool landed = false;
             for (;;) {
@@ -345,7 +342,7 @@ static int host_copy_slabs(rt_ctx* ctx, const SlabJob& job, uint32_t first, bool
         } else {
             const auto t0 = std::chrono::steady_clock::now();
             while (cudaEventQuery(ctx->slab_events[s]) != cudaSuccess) {
-                if (std::chrono::steady_clock::now() - t0 > std::chrono::milliseconds(tunables().wait_timeout_ms)) {
+                if (std::chrono::steady_clock::now() - t0 > std::chrono::milliseconds(test_hooks().wait_timeout_ms)) {
                     (void)cudaGetLastError();
                     *done_out = i;
                     return RT_OK;  // finish_slab_copies' drain reports the timeout
@@ -370,7 +367,7 @@ static int drain_copy_stream(rt_ctx* ctx, const SlabJob& job) {
         const cudaError_t q = cudaStreamQuery(ctx->copy_stream);
         if (q == cudaSuccess) break;
         if (q != cudaErrorNotReady) return set_err(ctx, RT_ERR_CUDA, "copy stream: %s", cudaGetErrorString(q));
-        if (std::chrono::steady_clock::now() - t0 > std::chrono::milliseconds(tunables().wait_timeout_ms)) {
+        if (std::chrono::steady_clock::now() - t0 > std::chrono::milliseconds(test_hooks().wait_timeout_ms)) {
             ctx->h_flag[0] = 1;
             if (job.ctl) {
                 unsigned long long* fill = ctx->h_ctr;  // pinned scratch: RT_CTR_SLOTS >= MAX_SLABS entries
@@ -398,7 +395,7 @@ int finish_slab_copies(rt_ctx* ctx, const SlabJob& job) {
     if (rc) return rc;
     if (ctx->h_flag[0]) {
         ctx->h_flag[0] = 0;  // reported here: the next call starts clean
-        return set_err(ctx, RT_ERR_TIMEOUT, "a slab of the frame did not complete within %d ms", tunables().wait_timeout_ms);
+        return set_err(ctx, RT_ERR_TIMEOUT, "a slab of the frame did not complete within %d ms", test_hooks().wait_timeout_ms);
     }
     return RT_OK;
 }
@@ -419,7 +416,7 @@ int render_and_collect(rt_ctx* ctx, const rt_scene* scene, const Resolved& r, co
     SlabJob job;
     const bool late = ctx->serial_launches;  // launches block: queue the waits once nothing of ours is outstanding
     if (streamed && !late) {
-        rc = enqueue_slab_copies(ctx, frame_dev, a.ctl, a.plan, seq, out_rgb, tunables().tile_order_reverse != 0, &job);
+        rc = enqueue_slab_copies(ctx, frame_dev, a.ctl, a.plan, seq, out_rgb, &job);
         if (rc) return rc;
     }
     if (streamed && !late && job.out && job.pinned != job.out) {  // pageable destination: host copies while the kernel runs
@@ -430,7 +427,7 @@ int render_and_collect(rt_ctx* ctx, const rt_scene* scene, const Resolved& r, co
     rc = finish_redo(ctx, scene, r, a, &redone);  // own kernel done; pixels it still held back are final (and counted) now
     if (rc) return rc;
     if (streamed && late) {
-        rc = enqueue_slab_copies(ctx, frame_dev, a.ctl, a.plan, seq, out_rgb, tunables().tile_order_reverse != 0, &job);
+        rc = enqueue_slab_copies(ctx, frame_dev, a.ctl, a.plan, seq, out_rgb, &job);
         if (rc) return rc;
     }
     if (streamed) {
@@ -483,7 +480,7 @@ static bool launches_block() {
             !strncmp(*e, "CUDA_INJECTION64_PATH=", 22))
             return true;
     const char* b = std::getenv("CUDA_LAUNCH_BLOCKING");
-    return (b && atoi(b) != 0) || std::getenv("RT_B200_SERIAL_LAUNCHES");
+    return b && atoi(b) != 0;
 }
 
 int rt_abi_version(void) { return RT_B200_ABI_VERSION; }
@@ -501,7 +498,7 @@ int rt_init(int device, rt_ctx** out) {
     if (!out) return set_err(nullptr, RT_ERR_INVALID_ARG, "rt_init: out is NULL");
     *out = nullptr;
     RT_GUARD_BEGIN
-    (void)tunables();  // the environment is read here, once
+    (void)test_hooks();  // the environment is read here, once
     int count = 0;
     cudaError_t e = cudaGetDeviceCount(&count);
     if (e != cudaSuccess || count == 0)
@@ -553,7 +550,7 @@ int rt_init(int device, rt_ctx** out) {
         cudaDriverEntryPointQueryResult qr;
         if (cudaDeviceGetAttribute(&can64, static_cast<cudaDeviceAttr>(122) /* CU_DEVICE_ATTRIBUTE_CAN_USE_64_BIT_STREAM_MEM_OPS */, device) == cudaSuccess && can64 &&
             cudaGetDriverEntryPoint("cuStreamWaitValue64", &fn, cudaEnableDefault, &qr) == cudaSuccess &&
-            qr == cudaDriverEntryPointSuccess && fn && !std::getenv("RT_B200_NO_STREAM_WAIT"))
+            qr == cudaDriverEntryPointSuccess && fn && !test_hooks().no_stream_wait)
             ctx->stream_wait_value64 = reinterpret_cast<int (*)(void*, unsigned long long, unsigned long long, unsigned int)>(fn);
         (void)cudaGetLastError();
     }
@@ -931,7 +928,7 @@ int rt_frame_collect(rt_ctx* ctx, const void* frame_dev, const rt_params* params
     const SlabPlan plan = plan_slabs(params->width, params->height);
     const rt_frame_ctl* ctl = reinterpret_cast<const rt_frame_ctl*>((const uint8_t*)frame_dev + rt_frame_ctl_offset(bytes));
     SlabJob job;
-    const int rc = enqueue_slab_copies(ctx, (const uint8_t*)frame_dev, ctl, plan, seq, out_rgb, tunables().tile_order_reverse != 0, &job);
+    const int rc = enqueue_slab_copies(ctx, (const uint8_t*)frame_dev, ctl, plan, seq, out_rgb, &job);
     if (rc) return rc;
     return finish_slab_copies(ctx, job);
     RT_GUARD_END(ctx)

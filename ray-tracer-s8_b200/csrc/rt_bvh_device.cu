@@ -16,7 +16,6 @@
 //   leaf_depths   deepest leaf, for the traversal stack bound (MAX_STACK)
 #include <cub/device/device_radix_sort.cuh>
 
-#include <cstdio>
 #include <cstdlib>
 
 #include "rt_device.cuh"
@@ -215,8 +214,6 @@ cudaError_t build_lbvh_device(DeviceBuild* buf, const float* h_boxes, const uint
         if ((e = cudaMalloc(&buf->mem, cap)) != cudaSuccess) return e;
         buf->bytes = cap;
     }
-    const bool timing = tunables().timing;
-    if (timing) fprintf(stderr, "[build_lbvh_device n=%u] scratch %zu bytes of %zu\n", n, off, buf->bytes);
     uint8_t* m = (uint8_t*)buf->mem;
     float* d_boxes = (float*)(m + o_box);
     uint32_t* d_pid = (uint32_t*)(m + o_pid);

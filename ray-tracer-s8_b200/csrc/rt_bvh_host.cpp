@@ -31,14 +31,10 @@ namespace {
 constexpr int kBuckets = 6;
 // A subtree over n primitives has exactly n - 1 inner nodes and its leaves are idx[lo,hi) in their final order, so
 // every node's slot in the DFS pre-order arrays is known before its subtree is built: node `base`, left subtree from
-// base + 1, right subtree from base + n_left.  Subtrees above this size are built by their own thread.
-static const size_t kParallelMin = [] {
-    // subtree size from which both children get their own thread (RT_B200_BUILD_PAR=N, 0 = never).  Default 2048 on hosts
-    // with >= 8 hardware threads: on the 16-core GPU box the reference build of 65,536 spheres drops from 30 to 6.5 ms.
-    const char* e = std::getenv("RT_B200_BUILD_PAR");
-    const long v = e ? std::atol(e) : (std::thread::hardware_concurrency() >= 8 ? 2048 : 0);
-    return v > 0 ? (size_t)v : (size_t)-1 / 4;
-}();
+// base + 1, right subtree from base + n_left.  Subtrees above this size are built by their own thread: 2048 on hosts
+// with >= 8 hardware threads (on a 16-core host the reference build of 65,536 spheres drops from 30 to 6.5 ms), never
+// on smaller hosts.
+static const size_t kParallelMin = std::thread::hardware_concurrency() >= 8 ? 2048 : (size_t)-1 / 4;
 constexpr float kEpsilon = 0.00001f;  // bvh::EPSILON (lib.rs:80)
 
 // f32::min / f32::max inline (libm's fminf/fmaxf are out-of-line calls under -fno-fast-math and were most of the build

@@ -155,12 +155,11 @@ struct SlabJob {
     SlabPlan plan;
     uint8_t* out = nullptr;       // caller's destination
     uint8_t* pinned = nullptr;    // where the device copies go (== out when out is pinned)
-    bool reverse = false;
     uint32_t host_done = 0;       // pageable path: slabs already copied on to `out`
     const rt_frame_ctl* ctl = nullptr;
 };
 int enqueue_slab_copies(rt_ctx* ctx, const uint8_t* frame_dev, const rt_frame_ctl* ctl, const SlabPlan& plan, uint64_t seq,
-                        uint8_t* out_rgb, bool reverse_order, SlabJob* job);
+                        uint8_t* out_rgb, SlabJob* job);
 int finish_slab_copies(rt_ctx* ctx, const SlabJob& job);
 
 }  // namespace rtb

@@ -16,23 +16,15 @@ struct DevParams;
 
 constexpr int MAX_SLABS = 64;  // completion counters per frame (frame control block)
 
-// Measurement switches, read from the environment once per process (rt_init forces the read).  Not API.
-struct Tunables {
-    int smem_override = -1;      // RT_B200_SMEM=0|1: force the scene out of / into shared memory
-    int tile_order_reverse = 1;  // RT_B200_TILE_ORDER=topdown: tickets walk the tile grid top-down
-    int stage_out = -1;          // RT_B200_STAGE_OUT=0|1: force the output stage + completion counters off / on (-1: shared frames only)
-    int tail_permille = 30;      // RT_B200_TAIL_PERMILLE: share of the tickets handed out pixel by pixel
+// Test hooks, read from the environment once per process (rt_init forces the read).  They let tests reach paths a
+// normal run does not take on a given machine or at a given moment; they are not API.
+struct TestHooks {
     int build_mode = 1;          // RT_B200_BUILD=host|device|auto: who builds the traversal tree
-    int tree_mode = 2;           // RT_B200_TREE=ref|sah|split: which tree is traversed
-    bool timing = false;         // RT_B200_TIMING: stage times of rt_scene_create on stderr
-    int slabs = 16;              // RT_B200_SLABS: slabs a frame download is streamed in
-    bool async_ref = true;       // RT_B200_ASYNC_REF=0: build the reference-topology tree inside rt_scene_create
-    int pid_order = 1;           // RT_B200_PID_ORDER=world: primitive ids in world order instead of the traversal tree's DFS order
-    int aux_delay_ms = 0;        // RT_B200_AUX_DELAY_MS: the builder thread sleeps first (tests: frames rendered before the tables land)
+    int aux_delay_ms = 0;        // RT_B200_AUX_DELAY_MS: the builder thread sleeps first (frames rendered before the tables land)
     int wait_timeout_ms = 20000; // RT_B200_WAIT_TIMEOUT_MS: how long a frame owner waits for a slab / a rank for the owner
-    bool count_done = true;      // RT_B200_COUNT_DONE=0: no completion counters (frames are copied after the kernel)
+    bool no_stream_wait = false; // RT_B200_NO_STREAM_WAIT: slab waits as one-thread kernels instead of cuStreamWaitValue64
 };
-const Tunables& tunables();
+const TestHooks& test_hooks();
 
 struct LaunchInfo {
     unsigned grid = 0, threads = 0;

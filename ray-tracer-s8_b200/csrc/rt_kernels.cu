@@ -241,7 +241,7 @@ __global__ void __launch_bounds__(TPB, MINB) render_kernel_lanes(const DevScene 
     // ticket → tile of this rank: group k of `tile_ranks` tiles, rotated; bottom-up so the sky rows end the launch
     auto tile_of_ticket = [&](uint32_t k) -> uint32_t {
         uint32_t g = k * pr.tile_ranks + (pr.tile_rank + k) % pr.tile_ranks;
-        if (g < total_tiles && pr.tile_order_reverse) g = total_tiles - 1 - g;
+        if (g < total_tiles) g = total_tiles - 1 - g;
         return g;
     };
     auto out_desc = [&]() { return OutDesc{pr.out, pr.done, pr.width, pr.out_row0, pr.row0, pr.slab_tile_rows}; };
@@ -644,7 +644,7 @@ __global__ void __launch_bounds__(256) fp32_peak_kernel(float* out, int iters, f
 }
 
 // ---------------------------------------------------------------------------------------------
-// Tunables: read from the environment ONCE (rt_init forces the read); measurement switches, not API
+// Test hooks: read from the environment ONCE (rt_init forces the read); not API
 // ---------------------------------------------------------------------------------------------
 static int env_int(const char* name, int dflt) {
     const char* e = std::getenv(name);
@@ -654,22 +654,13 @@ static bool env_is(const char* name, const char* value) {
     const char* e = std::getenv(name);
     return e && std::strcmp(e, value) == 0;
 }
-const Tunables& tunables() {
-    static const Tunables t = [] {
-        Tunables v;
-        v.smem_override = env_int("RT_B200_SMEM", -1);
-        v.tile_order_reverse = env_is("RT_B200_TILE_ORDER", "topdown") ? 0 : 1;
-        v.stage_out = env_int("RT_B200_STAGE_OUT", -1);
-        v.tail_permille = std::max(0, std::min(500, env_int("RT_B200_TAIL_PERMILLE", 30)));
+const TestHooks& test_hooks() {
+    static const TestHooks t = [] {
+        TestHooks v;
         v.build_mode = env_is("RT_B200_BUILD", "host") ? 0 : (env_is("RT_B200_BUILD", "device") ? 2 : 1);
-        v.tree_mode = env_is("RT_B200_TREE", "ref") ? 0 : (env_is("RT_B200_TREE", "sah") ? 1 : 2);
-        v.timing = std::getenv("RT_B200_TIMING") != nullptr;
-        v.slabs = std::max(1, std::min(MAX_SLABS, env_int("RT_B200_SLABS", 16)));
-        v.async_ref = env_int("RT_B200_ASYNC_REF", 1) != 0;
-        v.count_done = env_int("RT_B200_COUNT_DONE", 1) != 0;
-        v.pid_order = env_is("RT_B200_PID_ORDER", "world") ? 0 : 1;
         v.aux_delay_ms = std::max(0, env_int("RT_B200_AUX_DELAY_MS", 0));
         v.wait_timeout_ms = std::max(1, env_int("RT_B200_WAIT_TIMEOUT_MS", 20000));
+        v.no_stream_wait = std::getenv("RT_B200_NO_STREAM_WAIT") != nullptr;
         return v;
     }();
     return t;
@@ -752,9 +743,12 @@ cudaError_t preload_kernels() {
     return cudaSuccess;
 }
 
+// Share of a launch's tickets handed out pixel by pixel at its end.  0 to 300 permille measured the same on C3 at 8
+// ranks (4.67 / 4.68 / 4.67 / 4.67 / 4.64 ms), 600 and more slower (profiles/r2_final_tail_sweep.log).
+constexpr uint64_t kTailPermille = 30;
+
 cudaError_t launch_render(const DevScene& sc, const DevCamera& cam, const DevParams& pr, int isect, bool count,
                           int sm_count, int smem_optin, cudaStream_t stream, LaunchInfo* info) {
-    const Tunables& tn = tunables();
     const bool resume = pr.state_out != nullptr;  // rt_render_samples
     if (resume) count = false;
     const size_t static_smem = (SMEM_TPB / 32) * (OUT_SLOTS * (TILE_BYTES + 16) + 4) + 64;
@@ -762,15 +756,12 @@ cudaError_t launch_render(const DevScene& sc, const DevCamera& cam, const DevPar
     // Stage the scene in shared memory when one 1024-thread CTA per SM fits with it (scenes up to ~200 KB); larger
     // scenes are read through L1/L2 (measured on the C5 sweep, profiles/r1_c5_sweep.log)
     if (info) info->counts_done = true;
-    bool smem = !count ? (need + static_smem + 1024 <= (size_t)smem_optin)
-                       : ((need + static_smem + 1024) * 3 <= (size_t)smem_optin);
-    if (tn.smem_override == 0) smem = false;
-    if (tn.smem_override == 1) smem = need + static_smem + 1024 <= (size_t)smem_optin;
+    const bool smem = !count ? (need + static_smem + 1024 <= (size_t)smem_optin)
+                             : ((need + static_smem + 1024) * 3 <= (size_t)smem_optin);
     // The output stage and the completion counters cost ~0.03 ns per pixel (C3: +0.2 ms of 38.0; C2, 1 spp: +0.07 of 0.24);
     // the copy they let the owner overlap costs 0.06 ns per pixel.  On for frames shared between ranks and for frames the
-    // caller streams to the host; a frame that stays on one device keeps round 1's byte stores.
-    // RT_B200_STAGE_OUT=0|1 forces it (profiles/r2_notes.md).
-    const bool stage = !count && !resume && (tn.stage_out < 0 ? ((pr.tile_ranks > 1 || pr.stage_hint) && pr.done != nullptr) : tn.stage_out != 0);
+    // caller streams to the host; a frame that stays on one device keeps round 1's byte stores (profiles/r2_notes.md).
+    const bool stage = !count && !resume && (pr.tile_ranks > 1 || pr.stage_hint) && pr.done != nullptr;
     int threads = THREADS;
     KernelFn fn;
     if (resume) fn = isect == RT_INTERSECT_BRUTE ? (smem ? pick_resume<RT_INTERSECT_BRUTE, true>(&threads) : pick_resume<RT_INTERSECT_BRUTE, false>(&threads))
@@ -791,20 +782,19 @@ cudaError_t launch_render(const DevScene& sc, const DevCamera& cam, const DevPar
     if (grid > want_ctas) grid = want_ctas;
     if (grid < 1) grid = 1;
     DevParams prm = pr;
-    if (!tn.count_done || (!stage && !count)) {  // without the stage every pixel would pay a system-scope release of its
-                                                 // own (the instrumented kernel does: it is not a timed path)
+    if (!stage && !count) {  // without the stage every pixel would pay a system-scope release of its own (the
+                             // instrumented kernel does: it is not a timed path)
         prm.done = nullptr;
         if (info) info->counts_done = false;
     }
-    prm.tile_order_reverse = tn.tile_order_reverse;
     prm.my_tickets = (uint32_t)my_tiles;
     if (pr.pixel_list) {  // second pass over a pixel list: pixel tickets only
         const uint64_t warps = ((uint64_t)pr.list_count + 31) / 32;
         grid = std::max<uint64_t>(1, std::min<uint64_t>(grid, (warps + (threads / 32) - 1) / (threads / 32)));
     }
-    // the tail: the last tail_permille / 1000 of the tickets (at least two tiles per warp-slot of the grid would be
+    // the tail: the last kTailPermille / 1000 of the tickets (at least two tiles per warp-slot of the grid would be
     // pointless to split further: small launches are all tail)
-    uint64_t tail = my_tiles * (uint64_t)tn.tail_permille / 1000;
+    uint64_t tail = my_tiles * kTailPermille / 1000;
     if (my_tiles <= grid * (uint64_t)(threads / 32)) tail = my_tiles;  // fewer tiles than warps: pixel tickets only
     prm.tail_first = (uint32_t)(my_tiles - std::min<uint64_t>(tail, my_tiles));
     if (pr.pixel_list) prm.tail_first = 0;
@@ -821,14 +811,14 @@ cudaError_t launch_render(const DevScene& sc, const DevCamera& cam, const DevPar
 
 cudaError_t launch_wait_slab(const unsigned long long* done, unsigned long long target, unsigned int* timeout_flag,
                              cudaStream_t stream) {
-    wait_slab_kernel<<<1, 1, 0, stream>>>(done, target, timeout_flag, (unsigned long long)tunables().wait_timeout_ms * 1000000ull);
+    wait_slab_kernel<<<1, 1, 0, stream>>>(done, target, timeout_flag, (unsigned long long)test_hooks().wait_timeout_ms * 1000000ull);
     return cudaGetLastError();
 }
 
 cudaError_t launch_wait_all_slabs(const unsigned long long* done, unsigned long long seq, uint32_t slabs, uint32_t tile_rows,
                                   uint32_t rows, uint32_t width, unsigned int* timeout_flag, cudaStream_t stream) {
     wait_all_slabs_kernel<<<1, MAX_SLABS, 0, stream>>>(done, seq, slabs, tile_rows, rows, width, timeout_flag,
-                                                       (unsigned long long)tunables().wait_timeout_ms * 1000000ull);
+                                                       (unsigned long long)test_hooks().wait_timeout_ms * 1000000ull);
     return cudaGetLastError();
 }
 

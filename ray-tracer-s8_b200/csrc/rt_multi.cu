@@ -84,7 +84,7 @@ extern "C" int rt_render_frame_multi(rt_ctx* const* ctxs, const rt_scene* const*
     SlabJob job;
     const bool late = c0->serial_launches;  // blocking launches: the waits go behind the second passes (rt_init)
     if (streamed && !late) {
-        rc = enqueue_slab_copies(c0, c0->d_out, a0.ctl, a0.plan, c0->out_seq, out_rgb, tunables().tile_order_reverse != 0, &job);
+        rc = enqueue_slab_copies(c0, c0->d_out, a0.ctl, a0.plan, c0->out_seq, out_rgb, &job);
         if (rc) return rc;
     }
     // second passes (tie-break tables that had not landed) and counters, context by context
@@ -123,7 +123,7 @@ extern "C" int rt_render_frame_multi(rt_ctx* const* ctxs, const rt_scene* const*
     CK(c0, cudaSetDevice(c0->device));
     if (streamed && late) {
         CK(c0, cudaSetDevice(c0->device));
-        rc = enqueue_slab_copies(c0, c0->d_out, a0.ctl, a0.plan, c0->out_seq, out_rgb, tunables().tile_order_reverse != 0, &job);
+        rc = enqueue_slab_copies(c0, c0->d_out, a0.ctl, a0.plan, c0->out_seq, out_rgb, &job);
         if (rc) return rc;
     }
     if (streamed) {  // every context's held-back pixels are final and counted by now: the last slabs complete

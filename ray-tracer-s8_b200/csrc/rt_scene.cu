@@ -203,14 +203,7 @@ int rt_scene_create(rt_ctx* ctx, const rt_sphere* spheres, uint32_t n_spheres, c
     if ((n_spheres && !spheres) || (n_triangles && !triangles))
         return set_err(ctx, RT_ERR_INVALID_ARG, "rt_scene_create: NULL primitive array");
     const uint32_t n = (uint32_t)n64;
-    const Tunables& tn = tunables();
-    auto t_prev = std::chrono::steady_clock::now();
-    auto lap = [&](const char* what) {
-        if (!tn.timing) return;
-        const auto now = std::chrono::steady_clock::now();
-        fprintf(stderr, "[rt_scene_create n=%u] %-22s %8.3f ms\n", n, what, std::chrono::duration<double, std::milli>(now - t_prev).count());
-        t_prev = now;
-    };
+    const TestHooks& hooks = test_hooks();
 
     static std::atomic<uint64_t> next_serial{1};
     std::unique_ptr<rt_scene> sc(new rt_scene());
@@ -226,14 +219,12 @@ int rt_scene_create(rt_ctx* ctx, const rt_sphere* spheres, uint32_t n_spheres, c
         if (wrc) return set_err(ctx, wrc, "%s", werr.c_str());
     }
     const std::vector<Box>& boxes = aux->boxes;  // shared, read-only from here on
-    lap("world order + boxes");
 
     // ---- which tree will be traversed ---------------------------------------------------------------------
-    const int tree_mode = tn.tree_mode;
     std::vector<uint32_t> big_world;  // split layout: world positions of the primitives kept out of the tree
-    std::vector<Box> rest_store;      // boxes and world positions of the primitives the tree covers (split layout only:
-    std::vector<uint32_t> rest_world; //   without big primitives the tree covers `boxes` itself, no copy)
-    if (tree_mode == 2 && n > 1) {
+    std::vector<Box> rest_store;      // boxes and world positions of the primitives the tree covers (without big
+    std::vector<uint32_t> rest_world; //   primitives the tree covers `boxes` itself, no copy)
+    if (n > 1) {
         auto area_of = [](const Box& b) {
             const double sx = (double)b.max[0] - b.min[0], sy = (double)b.max[1] - b.min[1], sz = (double)b.max[2] - b.min[2];
             return 2.0 * (sx * sy + sx * sz + sy * sz);
@@ -274,11 +265,11 @@ int rt_scene_create(rt_ctx* ctx, const rt_sphere* spheres, uint32_t n_spheres, c
     const std::vector<Box>& rest = big_world.empty() ? boxes : rest_store;
     const bool ltree = !rest.empty();
     constexpr uint32_t kDeviceBuildMin = 8192;
-    const bool device_tree = tree_mode != 0 && rest.size() >= 2 &&
-                             (tn.build_mode == 2 || (tn.build_mode == 1 && rest.size() >= kDeviceBuildMin));
+    const bool device_tree = rest.size() >= 2 &&
+                             (hooks.build_mode == 2 || (hooks.build_mode == 1 && rest.size() >= kDeviceBuildMin));
 
     // ---- the reference-topology tree: beside everything else when it is worth a thread -------------------
-    const bool ref_sync = !tn.async_ref || tree_mode == 0 || n < 256;
+    const bool ref_sync = n < 256;
     HostBVH ref_bvh;  // synchronous case only
     AuxTables ref_tables;
     if (ref_sync) {
@@ -286,30 +277,24 @@ int rt_scene_create(rt_ctx* ctx, const rt_sphere* spheres, uint32_t n_spheres, c
         if (!build_bvh(boxes, &ref_bvh, &berr)) return set_err(ctx, RT_ERR_BVH, "BVH build failed: %s", berr.c_str());
         aux->n_nodes = ref_bvh.node_count;
         aux->depth = ref_bvh.depth;
-        lap("reference tree (sync)");
     }
 
     // ---- host traversal tree ---------------------------------------------------------------------------------
     HostBVH sah;
     const HostBVH* T = nullptr;  // tree to emit as lnode records (leaf codes: world positions)
     if (ltree && !device_tree && rest.size() >= 2) {
-        if (tree_mode == 0) {
-            T = &ref_bvh;
-        } else {
-            if (!build_bvh_sah(rest, &sah)) return set_err(ctx, RT_ERR_BVH, "traversal tree build failed");
-            auto remap = [&](int32_t c) { return c >= 0 ? c : ~(int32_t)rest_world[(uint32_t)~c]; };
-            for (auto& nd : sah.inner) {
-                nd.left = remap(nd.left);
-                nd.right = remap(nd.right);
-            }
-            sah.root = remap(sah.root);
-            T = &sah;
+        if (!build_bvh_sah(rest, &sah)) return set_err(ctx, RT_ERR_BVH, "traversal tree build failed");
+        auto remap = [&](int32_t c) { return c >= 0 ? c : ~(int32_t)rest_world[(uint32_t)~c]; };
+        for (auto& nd : sah.inner) {
+            nd.left = remap(nd.left);
+            nd.right = remap(nd.right);
         }
+        sah.root = remap(sah.root);
+        T = &sah;
         if (T->depth > (uint32_t)MAX_STACK)
             return set_err(ctx, RT_ERR_UNSUPPORTED, "traversal tree depth %u exceeds the traversal stack (%d)", T->depth, MAX_STACK);
         sc->tree_depth = T->depth;
     }
-    lap("traversal tree");
 
     // ---- primitive ids: spheres [0, ns), triangles [ns, n).  In the DFS leaf order of the host-built traversal tree
     // when there is one (neighbours in space are neighbours in memory: the per-hit material / box / rank reads of the
@@ -320,7 +305,7 @@ int rt_scene_create(rt_ctx* ctx, const rt_sphere* spheres, uint32_t n_spheres, c
         auto give = [&](uint32_t w) {
             if (aux->pid_of_world[w] == 0xffffffffu) aux->pid_of_world[w] = world[w].kind == 0 ? next_s++ : next_t++;
         };
-        if (T && tn.pid_order == 1) {
+        if (T) {
             std::vector<int32_t> todo;
             todo.push_back(T->root);
             while (!todo.empty()) {
@@ -341,7 +326,6 @@ int rt_scene_create(rt_ctx* ctx, const rt_sphere* spheres, uint32_t n_spheres, c
     uint32_t lni = 0;
     if (device_tree) lni = (uint32_t)rest.size() - 1;
     else if (T) lni = (uint32_t)T->inner.size();
-    lap("primitive ids");
 
     // ---- blob layout: the shared-memory image first (contiguous, 16-byte granules), then 256-byte aligned sections
     const uint32_t ni_ref = n - 1;
@@ -398,7 +382,6 @@ int rt_scene_create(rt_ctx* ctx, const rt_sphere* spheres, uint32_t n_spheres, c
         if (sc->d_blob) ctx->retired.push_back({sc->d_blob, sc->blob_cap});
         sc->d_blob = nullptr;
     };
-    lap("staging + device blob");
 
     // ---- the builder thread starts now: it knows where its tables go ------------------------------------------
     if (!ref_sync) {
@@ -409,7 +392,7 @@ int rt_scene_create(rt_ctx* ctx, const rt_sphere* spheres, uint32_t n_spheres, c
         rt_ctx* const c = ctx;
         const size_t dr = o_rank, du = o_up, db = o_refbox, df = o_flag;
         uint8_t* const dst = sc->d_blob;
-        const int delay_ms = tn.aux_delay_ms;
+        const int delay_ms = hooks.aux_delay_ms;
         a->worker = std::thread([a, c, dst, dr, du, db, df, delay_ms] {
             try {
                 if (delay_ms > 0) std::this_thread::sleep_for(std::chrono::milliseconds(delay_ms));
@@ -518,7 +501,6 @@ int rt_scene_create(rt_ctx* ctx, const rt_sphere* spheres, uint32_t n_spheres, c
     // the flag lives in the late region: inside the staging copy only when the whole blob is uploaded by this call (the
     // asynchronous path zeroes it on the device above and the builder thread raises it)
     if (ref_sync) *(int32_t*)(h + o_flag) = 1;
-    lap("primitive arrays");
 
     // traversal-tree records from the host tree: DFS pre-order numbering, left subtree first
     int32_t lroot = 0;
@@ -562,7 +544,6 @@ int rt_scene_create(rt_ctx* ctx, const rt_sphere* spheres, uint32_t n_spheres, c
         memcpy(h + o_up, ref_tables.up.data(), ref_tables.up.size() * 4);
         memcpy(h + o_refbox, ref_tables.refbox.data(), ref_tables.refbox.size() * 4);
     }
-    lap("tree records");
 
     cudaError_t e;
     const size_t ln_end = align_up(o_ln + (size_t)lni * NODE_BYTES, 256);
@@ -579,7 +560,6 @@ int rt_scene_create(rt_ctx* ctx, const rt_sphere* spheres, uint32_t n_spheres, c
         give_back();
         return set_err(ctx, RT_ERR_CUDA, "scene upload failed: %s", cudaGetErrorString(e));
     }
-    lap("upload");
     if (device_tree) {
         std::vector<float> dev_boxes(6 * rest.size());
         std::vector<uint32_t> dev_pid(rest.size());
@@ -600,7 +580,6 @@ int rt_scene_create(rt_ctx* ctx, const rt_sphere* spheres, uint32_t n_spheres, c
         }
         sc->tree_depth = depth;
         sc->device_tree = true;
-        lap("device tree build");
     }
     if (ref_sync) aux->state.store(1, std::memory_order_release);
 

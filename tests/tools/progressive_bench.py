@@ -101,7 +101,6 @@ def main():
                    f"every frame starts behind a {FLUSH_BYTES >> 20} MB L2 flush; kernel_ms from CUDA events (per call), "
                    "e2e_ms = host clock around the frame's calls (each returns after the device has finished); pinned "
                    "destination; medians over the rounds"),
-        "RT_B200_STAGE_OUT": os.environ.get("RT_B200_STAGE_OUT", "unset (frame_16 streams its slabs through the output stage)"),
         "state_bytes_note": ("per chunk: pixels x 48 B written, plus pixels x 48 B read from the second chunk on "
                              "(the first chunk seeds its chains); computed from the shape, not measured"),
         "modes": {},
