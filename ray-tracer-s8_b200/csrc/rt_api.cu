@@ -120,20 +120,33 @@ static int ensure_out(rt_ctx* ctx, size_t bytes) {
     return RT_OK;
 }
 
-// The context's own staging frame.  Its counters start from zero for every launch (frame number 1 each time): whether a
-// launch counts at all is the launcher's choice (single-rank frames do not, rt_kernels.cu), so nothing cumulative can be
-// assumed here — unlike the shared frames of rt_frame_alloc, whose ranks always count.
-int own_frame(rt_ctx* ctx, uint32_t width, uint32_t rows, LaunchArgs* a) {
+// The context's own staging frame.  Its counters start from zero for every launch (frame number OWN_FRAME_SEQ = 1 each
+// time): whether a launch counts at all is the launcher's choice (single-rank frames do not, rt_kernels.cu), so nothing
+// cumulative can be assumed here — unlike the shared frames of rt_frame_alloc, whose ranks always count.
+int own_frame(rt_ctx* ctx, uint32_t width, uint32_t rows, Frame* f) {
     const size_t bytes = (size_t)width * rows * 3;
     const int rc = ensure_out(ctx, bytes);
     if (rc) return rc;
-    a->dst = ctx->d_out;
-    a->ctl = reinterpret_cast<rt_frame_ctl*>(ctx->d_out + ctx->d_out_bytes);
-    a->plan = plan_slabs(width, rows);
-    CK(ctx, cudaMemsetAsync(a->ctl, 0, sizeof(rt_frame_ctl), ctx->stream));
+    f->dev = ctx->d_out;
+    f->ctl = reinterpret_cast<rt_frame_ctl*>(ctx->d_out + ctx->d_out_bytes);
+    f->plan = plan_slabs(width, rows);
+    CK(ctx, cudaMemsetAsync(f->ctl, 0, sizeof(rt_frame_ctl), ctx->stream));
     CK(ctx, cudaEventRecord(ctx->ev_sync, ctx->stream));
     CK(ctx, cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_sync, 0));  // slab waits start after the reset
-    ctx->out_seq = 1;
+    return RT_OK;
+}
+
+Frame caller_frame(void* frame_dev, uint32_t width, uint32_t height) {
+    Frame f;
+    f.dev = static_cast<uint8_t*>(frame_dev);
+    f.ctl = reinterpret_cast<rt_frame_ctl*>(f.dev + rt_frame_ctl_offset((size_t)width * height * 3));
+    f.plan = plan_slabs(width, height);
+    return f;
+}
+
+int check_frame_out(rt_ctx* ctx, const uint8_t* out_rgb, size_t out_len, uint32_t width, uint32_t height) {
+    const size_t bytes = (size_t)width * height * 3;
+    if (out_rgb && out_len != bytes) return set_err(ctx, RT_ERR_INVALID_ARG, "out_len %zu != height*width*3 = %zu", out_len, bytes);
     return RT_OK;
 }
 
@@ -148,7 +161,7 @@ int launch(rt_ctx* ctx, const rt_scene* scene, const Resolved& r, const LaunchAr
     pr.seed = r.p.seed;
     pr.tile_rank = a.tile_rank;
     pr.tile_ranks = a.tile_ranks;
-    pr.out = a.dst;
+    pr.out = a.frame.dev;
     pr.out_row0 = a.out_row0;
     pr.tiles_x = (r.p.width + TILE_W - 1) / TILE_W;
     pr.tiles_y = (a.row1 - a.row0 + TILE_H - 1) / TILE_H;
@@ -162,10 +175,10 @@ int launch(rt_ctx* ctx, const rt_scene* scene, const Resolved& r, const LaunchAr
     pr.state_in = static_cast<const uint4*>(a.state_in);
     pr.state_out = static_cast<uint4*>(a.state_out);
     pr.s0 = a.s0;
-    pr.done = a.ctl ? a.ctl->done : nullptr;
+    pr.done = a.frame.ctl ? a.frame.ctl->done : nullptr;
     pr.stage_hint = a.stream ? 1 : 0;
     pr.redo_slab = ctx->d_ctr + RT_CTR_REDO_SLAB;
-    pr.slab_tile_rows = a.plan.tile_rows ? a.plan.tile_rows : 1;
+    pr.slab_tile_rows = a.frame.plan.tile_rows ? a.frame.plan.tile_rows : 1;
     const DevScene dev = scene_view(scene);
     CK(ctx, cudaMemsetAsync(ctx->d_ctr, 0, RT_CTR_SLOTS * sizeof(unsigned long long), ctx->stream));
     if (!a.pixel_list) CK(ctx, cudaMemsetAsync(ctx->d_redo, 0, RT_REDO_CAP * sizeof(unsigned int), ctx->stream));
@@ -186,89 +199,147 @@ static int read_counters(rt_ctx* ctx) {
     return RT_OK;
 }
 
-int finish_redo(rt_ctx* ctx, const rt_scene* scene, const Resolved& r, const LaunchArgs& a, uint32_t* redone) {
-    *redone = 0;
+static float ms_since(std::chrono::steady_clock::time_point t0) {
+    return std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
+}
+
+// Camera rays of `shares` of the tile_ranks equal shares of the launch's rows: one share is what a rank reports alone;
+// all of a frame's ranks together report the whole frame, also when the shares do not divide it evenly.
+static uint64_t primary_rays(const Launch& l, uint32_t shares) {
+    return (uint64_t)(l.a.row1 - l.a.row0) * l.r.p.width * shares / l.a.tile_ranks * (l.r.p.spp - l.a.s0);
+}
+
+// After the kernel of launch() has completed: re-renders the pixels that needed the tie-break tables before they had
+// landed (waits for the tables), then fills l.st (total_ms is the caller's).  kernel_launches counts a second launch
+// whenever the first pass listed pixels, even when the kernel's own redo rounds took all of them.
+static int finish_launch(Launch& l) {
+    rt_ctx* const ctx = l.ctx;
     int rc = read_counters(ctx);
     if (rc) return rc;
     const unsigned long long count = ctx->h_ctr[RT_CTR_REDO];
     const unsigned long long taken = ctx->h_ctr[RT_CTR_TICKET2] & 0xffffffffull;  // second passes done inside the kernel
-    ctx->first_pass_ms = 0.0f;
-    if (count == 0) return RT_OK;
-    *redone = count > RT_REDO_CAP ? 0xffffffffu : (uint32_t)count;
-    if (count <= RT_REDO_CAP && taken >= count) return RT_OK;
-    cudaEventElapsedTime(&ctx->first_pass_ms, ctx->ev0, ctx->ev1);  // the second pass re-records the events
-    unsigned long long first[NUM_COUNTERS], slab_counts[MAX_SLABS];
-    memcpy(first, ctx->h_ctr, sizeof first);
-    memcpy(slab_counts, ctx->h_ctr + RT_CTR_REDO_SLAB, sizeof slab_counts);
-    rc = scene_settle(ctx, scene);  // the tables must be there now
-    if (rc) return rc;
-    LaunchInfo li;
-    LaunchArgs b = a;
-    if (count > RT_REDO_CAP) {
-        // more than the list holds: the whole launch again, without counting (every pixel it had not held back is
-        // counted already); the pixels still held back are then counted slab by slab from the first pass's numbers
-        b.ctl = nullptr;
-        rc = launch(ctx, scene, r, b, &li);
+    const uint32_t redone = count == 0 ? 0u : count > RT_REDO_CAP ? 0xffffffffu : (uint32_t)count;
+    float first_ms = 0.0f;  // kernel time of the first pass when a second one follows (it re-records ev0 / ev1)
+    if (count > RT_REDO_CAP || taken < count) {
+        cudaEventElapsedTime(&first_ms, ctx->ev0, ctx->ev1);
+        unsigned long long first[NUM_COUNTERS], slab_counts[MAX_SLABS];
+        memcpy(first, ctx->h_ctr, sizeof first);
+        memcpy(slab_counts, ctx->h_ctr + RT_CTR_REDO_SLAB, sizeof slab_counts);
+        rc = scene_settle(ctx, l.scene);  // the tables must be there now
         if (rc) return rc;
-        if (a.ctl) {
-            memcpy(ctx->h_ctr + RT_CTR_REDO_SLAB, slab_counts, sizeof slab_counts);
-            CK(ctx, cudaMemcpyAsync(ctx->d_ctr + RT_CTR_REDO_SLAB, ctx->h_ctr + RT_CTR_REDO_SLAB, sizeof slab_counts,
-                                    cudaMemcpyHostToDevice, ctx->stream));
-            CK(ctx, launch_add_counts(a.ctl->done, ctx->d_ctr + RT_CTR_REDO_SLAB, MAX_SLABS, ctx->stream));
+        LaunchInfo li;
+        LaunchArgs b = l.a;
+        if (count > RT_REDO_CAP) {
+            // more than the list holds: the whole launch again, without counting (every pixel it had not held back is
+            // counted already); the pixels still held back are then counted slab by slab from the first pass's numbers
+            b.frame.ctl = nullptr;
+            rc = launch(ctx, l.scene, l.r, b, &li);
+            if (rc) return rc;
+            if (l.a.frame.ctl) {
+                memcpy(ctx->h_ctr + RT_CTR_REDO_SLAB, slab_counts, sizeof slab_counts);
+                CK(ctx, cudaMemcpyAsync(ctx->d_ctr + RT_CTR_REDO_SLAB, ctx->h_ctr + RT_CTR_REDO_SLAB, sizeof slab_counts,
+                                        cudaMemcpyHostToDevice, ctx->stream));
+                CK(ctx, launch_add_counts(l.a.frame.ctl->done, ctx->d_ctr + RT_CTR_REDO_SLAB, MAX_SLABS, ctx->stream));
+            }
+            rc = read_counters(ctx);  // the counters of the repeated launch are the frame's
+            if (rc) return rc;
+        } else {
+            // the listed pixels nobody got to inside the kernel, with the tables: counted now (their first pass held
+            // them back)
+            b.pixel_list = ctx->d_redo + taken;
+            b.list_count = (uint32_t)(count - taken);
+            rc = launch(ctx, l.scene, l.r, b, &li);
+            if (rc) return rc;
+            rc = read_counters(ctx);
+            if (rc) return rc;
+            for (int i = 0; i < NUM_COUNTERS; i++) ctx->h_ctr[i] += first[i];  // queries of both passes (redo_pixels says so)
         }
-        return read_counters(ctx);  // the counters of the repeated launch are the frame's
     }
-    // the listed pixels nobody got to inside the kernel, with the tables: counted now (their first pass held them back)
-    b.pixel_list = ctx->d_redo + taken;
-    b.list_count = (uint32_t)(count - taken);
-    rc = launch(ctx, scene, r, b, &li);
-    if (rc) return rc;
-    rc = read_counters(ctx);
-    if (rc) return rc;
-    for (int i = 0; i < NUM_COUNTERS; i++) ctx->h_ctr[i] += first[i];  // queries of both passes (stats.redo_pixels says so)
-    return RT_OK;
-}
-
-int finish_stats(rt_ctx* ctx, const Resolved& r, uint64_t pixels, rt_stats* st,
-                 std::chrono::steady_clock::time_point t0, const LaunchInfo& li) {
-    if (!st) return RT_OK;
-    const uint32_t redo = st->redo_pixels;  // set by the caller before
-    memset(st, 0, sizeof *st);
-    const unsigned long long* c = ctx->h_ctr;  // read by finish_redo
-    st->rays = c[CTR_RAYS];
-    st->primary = pixels * r.p.spp;
-    st->slab_tests = c[CTR_SLAB];
-    st->sphere_tests = c[CTR_SPH_TEST];
-    st->sphere_exact = c[CTR_SPH_EXACT];
-    st->sphere_hits = c[CTR_SPH_HIT];
-    st->tri_tests = c[CTR_TRI_TEST];
-    st->tri_stage[0] = c[CTR_TRI_S1];
-    st->tri_stage[1] = c[CTR_TRI_S2];
-    st->tri_stage[2] = c[CTR_TRI_S3];
-    st->tri_hits = c[CTR_TRI_HIT];
-    st->shades_sphere = c[CTR_SHADE_SPH];
-    st->shades_tri = c[CTR_SHADE_TRI];
-    st->emissive = c[CTR_EMISSIVE];
-    st->sky = c[CTR_SKY];
-    st->active_lane_iters = c[CTR_ACTIVE_LANES];
-    st->total_lane_iters = c[CTR_TOTAL_LANES];
+    rt_stats& st = l.st;
+    memset(&st, 0, sizeof st);
+    const unsigned long long* c = ctx->h_ctr;
+    st.rays = c[CTR_RAYS];
+    st.primary = primary_rays(l, 1);
+    st.slab_tests = c[CTR_SLAB];
+    st.sphere_tests = c[CTR_SPH_TEST];
+    st.sphere_exact = c[CTR_SPH_EXACT];
+    st.sphere_hits = c[CTR_SPH_HIT];
+    st.tri_tests = c[CTR_TRI_TEST];
+    st.tri_stage[0] = c[CTR_TRI_S1];
+    st.tri_stage[1] = c[CTR_TRI_S2];
+    st.tri_stage[2] = c[CTR_TRI_S3];
+    st.tri_hits = c[CTR_TRI_HIT];
+    st.shades_sphere = c[CTR_SHADE_SPH];
+    st.shades_tri = c[CTR_SHADE_TRI];
+    st.emissive = c[CTR_EMISSIVE];
+    st.sky = c[CTR_SKY];
+    st.active_lane_iters = c[CTR_ACTIVE_LANES];
+    st.total_lane_iters = c[CTR_TOTAL_LANES];
     float ms = 0.0f;
     CK(ctx, cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
-    st->kernel_ms = ms + ctx->first_pass_ms;
-    st->total_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
-    st->intersector_used = (uint32_t)r.isect;
-    st->kernel_launches = 1u + (redo ? 1u : 0u);
-    st->grid_ctas = li.grid;
-    st->cta_threads = li.threads;
-    st->ctas_per_sm = (uint32_t)li.ctas_per_sm;
-    st->scene_in_smem = li.scene_in_smem ? 1u : 0u;
-    st->dyn_smem_bytes = (uint32_t)li.dyn_smem;
-    st->redo_pixels = redo;
+    st.kernel_ms = ms + first_ms;
+    st.intersector_used = (uint32_t)l.r.isect;
+    st.kernel_launches = 1u + (redone ? 1u : 0u);
+    st.grid_ctas = l.info.grid;
+    st.cta_threads = l.info.threads;
+    st.ctas_per_sm = (uint32_t)l.info.ctas_per_sm;
+    st.scene_in_smem = l.info.scene_in_smem ? 1u : 0u;
+    st.dyn_smem_bytes = (uint32_t)l.info.dyn_smem;
+    st.redo_pixels = redone;
     return RT_OK;
 }
 
-int enqueue_slab_copies(rt_ctx* ctx, const uint8_t* frame_dev, const rt_frame_ctl* ctl, const SlabPlan& plan, uint64_t seq,
-                        uint8_t* out_rgb, SlabJob* job) {
+// The statistics of the n launches of one call together (n = 1: the launch's own).  The counters, kernel_launches and
+// redo_pixels add up (redo_pixels stays at 0xffffffff, "more than the list held", once a launch reports it); kernel_ms is
+// the longest launch's, as the launches run side by side; intersector_used and the launch shape are the first launch's
+// (context 0's); primary counts the launches' shares together.  total_ms is the caller's.
+static rt_stats combine_stats(const Launch* l, uint32_t n) {
+    rt_stats t;
+    memset(&t, 0, sizeof t);
+    for (uint32_t i = 0; i < n; i++) {
+        const rt_stats& s = l[i].st;
+        t.rays += s.rays;
+        t.slab_tests += s.slab_tests;
+        t.sphere_tests += s.sphere_tests;
+        t.sphere_exact += s.sphere_exact;
+        t.sphere_hits += s.sphere_hits;
+        t.tri_tests += s.tri_tests;
+        for (int k = 0; k < 3; k++) t.tri_stage[k] += s.tri_stage[k];
+        t.tri_hits += s.tri_hits;
+        t.shades_sphere += s.shades_sphere;
+        t.shades_tri += s.shades_tri;
+        t.emissive += s.emissive;
+        t.sky += s.sky;
+        t.active_lane_iters += s.active_lane_iters;
+        t.total_lane_iters += s.total_lane_iters;
+        t.kernel_launches += s.kernel_launches;
+        t.redo_pixels = (t.redo_pixels == 0xffffffffu || s.redo_pixels == 0xffffffffu) ? 0xffffffffu : t.redo_pixels + s.redo_pixels;
+        t.kernel_ms = std::max(t.kernel_ms, s.kernel_ms);
+    }
+    t.primary = primary_rays(l[0], n);
+    t.intersector_used = l[0].st.intersector_used;
+    t.grid_ctas = l[0].st.grid_ctas;
+    t.cta_threads = l[0].st.cta_threads;
+    t.ctas_per_sm = l[0].st.ctas_per_sm;
+    t.scene_in_smem = l[0].st.scene_in_smem;
+    t.dyn_smem_bytes = l[0].st.dyn_smem_bytes;
+    return t;
+}
+
+// On the frame owner.  enqueue: for every slab, on the copy stream, wait (on the device) until frame number `seq` of it
+// is complete, then copy it towards out_rgb (nullptr: only wait) — asynchronous; a pageable out_rgb is reached through a
+// pinned staging frame.  finish: host side of the same — returns when every slab is in out_rgb.  Between the two the
+// caller is free to finish its own kernel (second pass included): nothing here blocks the render stream.
+struct SlabJob {
+    SlabPlan plan;
+    uint8_t* out = nullptr;       // caller's destination
+    uint8_t* pinned = nullptr;    // where the device copies go (== out when out is pinned)
+    uint32_t host_done = 0;       // pageable path: slabs already copied on to `out`
+    const rt_frame_ctl* ctl = nullptr;
+};
+
+static int enqueue_slab_copies(rt_ctx* ctx, const uint8_t* frame_dev, const rt_frame_ctl* ctl, const SlabPlan& plan, uint64_t seq,
+                               uint8_t* out_rgb, SlabJob* job) {
     job->plan = plan;
     job->out = out_rgb;
     job->pinned = out_rgb;
@@ -385,7 +456,7 @@ static int drain_copy_stream(rt_ctx* ctx, const SlabJob& job) {
     return RT_OK;
 }
 
-int finish_slab_copies(rt_ctx* ctx, const SlabJob& job) {
+static int finish_slab_copies(rt_ctx* ctx, const SlabJob& job) {
     if (job.out && job.pinned != job.out) {
         uint32_t done = 0;
         const int rc = host_copy_slabs(ctx, job, job.host_done, false, &done);
@@ -400,46 +471,65 @@ int finish_slab_copies(rt_ctx* ctx, const SlabJob& job) {
     return RT_OK;
 }
 
-}  // namespace rtb
-
-namespace {
-
-// Owner side of a frame: launch this context's share of it, stream finished slabs (all ranks') to the host while it
-// renders, run the own second pass if one is needed, and leave the complete frame in out_rgb.
-int render_and_collect(rt_ctx* ctx, const rt_scene* scene, const Resolved& r, const LaunchArgs& a, const uint8_t* frame_dev,
-                       uint64_t seq, uint8_t* out_rgb, size_t bytes, uint64_t my_pixels, rt_stats* stats,
-                       std::chrono::steady_clock::time_point t0) {
-    LaunchInfo li;
-    int rc = launch(ctx, scene, r, a, &li);
-    if (rc) return rc;
-    const bool streamed = li.counts_done && a.ctl && (a.plan.slabs > 1 || a.tile_ranks > 1);
+int collect_frame(rt_ctx* owner, const Frame& f, uint64_t seq, uint8_t* out_rgb, Launch* l, uint32_t n, rt_stats* stats,
+                  std::chrono::steady_clock::time_point t0) {
+    const auto relay = [&](uint32_t i, int rc) {
+        if (rc && l[i].ctx != owner) set_err(owner, rc, "context %u: %s", i, l[i].ctx->err.c_str());
+        return rc;
+    };
+    int rc;
+    for (uint32_t i = 0; i < n; i++) {
+        CK(owner, cudaSetDevice(l[i].ctx->device));
+        if ((rc = relay(i, launch(l[i].ctx, l[i].scene, l[i].r, l[i].a, &l[i].info)))) return rc;
+    }
+    CK(owner, cudaSetDevice(owner->device));
+    // The frame streams when every launch counts its finished pixels into the frame's control block and there is more
+    // than one slab or rank to wait for.  Streaming waits on the device for the kernels; contexts that share a device
+    // also share its hardware queues, where a wait could sit in front of the very kernel it waits for, so such frames
+    // are copied after the kernels instead.  With no launch the ranks elsewhere count: the frame always streams.
+    bool streamed = true;
+    for (uint32_t i = 0; i < n; i++) {
+        streamed = streamed && l[i].info.counts_done && f.ctl && (f.plan.slabs > 1 || l[i].a.tile_ranks > 1);
+        for (uint32_t j = 0; j < i; j++) streamed = streamed && l[i].ctx->device != l[j].ctx->device;
+    }
     SlabJob job;
-    const bool late = ctx->serial_launches;  // launches block: queue the waits once nothing of ours is outstanding
+    const bool late = owner->serial_launches;  // launches block: queue the waits once nothing of ours is outstanding
     if (streamed && !late) {
-        rc = enqueue_slab_copies(ctx, frame_dev, a.ctl, a.plan, seq, out_rgb, &job);
+        rc = enqueue_slab_copies(owner, f.dev, f.ctl, f.plan, seq, out_rgb, &job);
         if (rc) return rc;
+        // pageable destination: host copies while the owner's kernel runs (it stops there, never waiting on a second
+        // pass that only the loop below runs)
+        if (n && job.out && job.pinned != job.out) {
+            rc = host_copy_slabs(owner, job, 0, true, &job.host_done);
+            if (rc) return rc;
+        }
     }
-    if (streamed && !late && job.out && job.pinned != job.out) {  // pageable destination: host copies while the kernel runs
-        rc = host_copy_slabs(ctx, job, 0, true, &job.host_done);
-        if (rc) return rc;
+    for (uint32_t i = 0; i < n; i++) {  // kernels done: the pixels they still held back are final (and counted) now
+        CK(owner, cudaSetDevice(l[i].ctx->device));
+        if ((rc = relay(i, finish_launch(l[i])))) return rc;
     }
-    uint32_t redone = 0;
-    rc = finish_redo(ctx, scene, r, a, &redone);  // own kernel done; pixels it still held back are final (and counted) now
-    if (rc) return rc;
+    CK(owner, cudaSetDevice(owner->device));
     if (streamed && late) {
-        rc = enqueue_slab_copies(ctx, frame_dev, a.ctl, a.plan, seq, out_rgb, &job);
+        rc = enqueue_slab_copies(owner, f.dev, f.ctl, f.plan, seq, out_rgb, &job);
         if (rc) return rc;
     }
     if (streamed) {
-        rc = finish_slab_copies(ctx, job);
+        rc = finish_slab_copies(owner, job);
         if (rc) return rc;
     } else if (out_rgb) {
-        CK(ctx, cudaMemcpyAsync(out_rgb, frame_dev, bytes, cudaMemcpyDeviceToHost, ctx->stream));
-        CK(ctx, cudaStreamSynchronize(ctx->stream));
+        CK(owner, cudaMemcpyAsync(out_rgb, f.dev, (size_t)f.plan.rows * f.plan.width * 3, cudaMemcpyDeviceToHost, owner->stream));
+        CK(owner, cudaStreamSynchronize(owner->stream));
     }
-    if (stats) stats->redo_pixels = redone;
-    return finish_stats(ctx, r, my_pixels, stats, t0, li);
+    if (stats && n) {
+        *stats = combine_stats(l, n);
+        stats->total_ms = ms_since(t0);
+    }
+    return RT_OK;
 }
+
+}  // namespace rtb
+
+namespace {
 
 int render_rows_to_host(rt_ctx* ctx, const rt_scene* scene, const Resolved& r, uint32_t row0, uint32_t row1,
                         uint8_t* out_rgb, size_t out_len, rt_stats* stats) {
@@ -450,18 +540,30 @@ int render_rows_to_host(rt_ctx* ctx, const rt_scene* scene, const Resolved& r, u
         return set_err(ctx, RT_ERR_INVALID_ARG, "out_len %zu != (rows %u * width %u * 3) = %zu", out_len, row1 - row0,
                        r.p.width, bytes);
     CK(ctx, cudaSetDevice(ctx->device));
-    LaunchArgs a;
-    a.row0 = row0;
-    a.row1 = row1;
-    a.out_row0 = row0;
-    const int rc = own_frame(ctx, r.p.width, row1 - row0, &a);
+    Launch l{ctx, scene, r};
+    l.a.row0 = row0;
+    l.a.row1 = row1;
+    l.a.out_row0 = row0;
+    const int rc = own_frame(ctx, r.p.width, row1 - row0, &l.a.frame);
     if (rc) return rc;
     // Streaming the frame out slab by slab while it renders beats one copy after the kernel on a single GPU when a pixel
     // is many samples of work (C3, 16 spp: stage + counters +0.2 ms, the 25 MB copy 0.5 ms); at few samples per pixel
     // the stage costs more than the copy (C2, 1 spp: +0.09 vs 0.12 ms incl. the slab waits; C4, 4 spp: +2.2 vs 2.0 ms)
-    a.stream = bytes >= ((size_t)4 << 20) && a.plan.slabs > 1 && r.p.spp >= 8;
-    return render_and_collect(ctx, scene, r, a, ctx->d_out, ctx->out_seq, out_rgb, bytes, (uint64_t)(row1 - row0) * r.p.width,
-                              stats, t0);
+    l.a.stream = bytes >= ((size_t)4 << 20) && l.a.frame.plan.slabs > 1 && r.p.spp >= 8;
+    return collect_frame(ctx, l.a.frame, OWN_FRAME_SEQ, out_rgb, &l, 1, stats, t0);
+}
+
+// Rank tile_rank of tile_ranks of a caller's whole frame.  seq (nullable: not the frame owner's call) must not be 0.
+int tiles_args(rt_ctx* ctx, const Resolved& r, void* frame_dev, uint32_t tile_rank, uint32_t tile_ranks, const uint64_t* seq,
+               LaunchArgs* a) {
+    if (!frame_dev) return set_err(ctx, RT_ERR_INVALID_ARG, "frame_dev is NULL");
+    if (tile_ranks == 0 || tile_rank >= tile_ranks || (seq && *seq == 0))
+        return set_err(ctx, RT_ERR_INVALID_ARG, seq ? "bad tile_rank/tile_ranks/seq" : "bad tile_rank/tile_ranks");
+    a->row1 = r.p.height;
+    a->tile_rank = tile_rank;
+    a->tile_ranks = tile_ranks;
+    a->frame = caller_frame(frame_dev, r.p.width, r.p.height);
+    return RT_OK;
 }
 
 }  // namespace
@@ -469,7 +571,7 @@ int render_rows_to_host(rt_ctx* ctx, const rt_scene* scene, const Resolved& r, u
 extern "C" {
 
 // Nsight Compute (and CUDA_LAUNCH_BLOCKING=1) make every kernel launch synchronous.  The frame owner normally queues
-// its slab waits, then runs the second pass that releases the pixels its first pass held back (finish_redo); with
+// its slab waits, then runs the second pass that releases the pixels its first pass held back (finish_launch); with
 // blocking launches the host would sit in the launch of a wait (or of the kernel behind the value waits) that only its
 // own next step can satisfy — measured: bench.py under ncu stopped at the first streamed frame.  So when launches
 // block, the waits are queued after the second pass.
@@ -643,35 +745,23 @@ int rt_render_tiles_device(rt_ctx* ctx, const rt_scene* scene, const rt_params* 
     if (!ctx) return RT_ERR_INVALID_ARG;
     RT_GUARD_BEGIN
     const auto t0 = std::chrono::steady_clock::now();
-    Resolved r;
-    int rc = resolve(ctx, scene, params, true, &r);
+    Launch l{ctx, scene};
+    int rc = resolve(ctx, scene, params, true, &l.r);
     if (rc) return rc;
-    if (!frame_dev) return set_err(ctx, RT_ERR_INVALID_ARG, "frame_dev is NULL");
-    if (tile_ranks == 0 || tile_rank >= tile_ranks) return set_err(ctx, RT_ERR_INVALID_ARG, "bad tile_rank/tile_ranks");
+    rc = tiles_args(ctx, l.r, frame_dev, tile_rank, tile_ranks, nullptr, &l.a);
+    if (rc) return rc;
     CK(ctx, cudaSetDevice(ctx->device));
     if (!sync) {  // nobody will be there for a second pass: have the tie-break tables first
         rc = scene_settle(ctx, scene);
         if (rc) return rc;
     }
-    LaunchArgs a;
-    a.row0 = 0;
-    a.row1 = r.p.height;
-    a.tile_rank = tile_rank;
-    a.tile_ranks = tile_ranks;
-    a.dst = (uint8_t*)frame_dev;
-    a.out_row0 = 0;
-    a.plan = plan_slabs(r.p.width, r.p.height);
-    a.ctl = reinterpret_cast<rt_frame_ctl*>((uint8_t*)frame_dev + rt_frame_ctl_offset((size_t)r.p.width * r.p.height * 3));
-    LaunchInfo li;
-    rc = launch(ctx, scene, r, a, &li);
+    rc = launch(ctx, scene, l.r, l.a, &l.info);
+    if (rc || !sync) return rc;
+    rc = finish_launch(l);
     if (rc) return rc;
-    if (sync) {
-        uint32_t redone = 0;
-        rc = finish_redo(ctx, scene, r, a, &redone);
-        if (rc) return rc;
-        if (stats) stats->redo_pixels = redone;
-        // pixel count of this rank's tiles is not needed by callers; report the frame total / ranks
-        return finish_stats(ctx, r, (uint64_t)r.p.width * r.p.height / tile_ranks, stats, t0, li);
+    if (stats) {
+        *stats = l.st;  // primary: the frame's pixels / ranks (the exact count of this rank's tiles is not needed)
+        stats->total_ms = ms_since(t0);
     }
     return RT_OK;
     RT_GUARD_END(ctx)
@@ -683,25 +773,15 @@ int rt_render_tiles_collect(rt_ctx* ctx, const rt_scene* scene, const rt_params*
     if (!ctx) return RT_ERR_INVALID_ARG;
     RT_GUARD_BEGIN
     const auto t0 = std::chrono::steady_clock::now();
-    Resolved r;
-    int rc = resolve(ctx, scene, params, true, &r);
+    Launch l{ctx, scene};
+    int rc = resolve(ctx, scene, params, true, &l.r);
     if (rc) return rc;
-    if (!frame_dev) return set_err(ctx, RT_ERR_INVALID_ARG, "frame_dev is NULL");
-    if (tile_ranks == 0 || tile_rank >= tile_ranks || seq == 0) return set_err(ctx, RT_ERR_INVALID_ARG, "bad tile_rank/tile_ranks/seq");
-    const size_t bytes = (size_t)r.p.width * r.p.height * 3;
-    if (out_rgb && out_len != bytes) return set_err(ctx, RT_ERR_INVALID_ARG, "out_len %zu != height*width*3 = %zu", out_len, bytes);
+    rc = tiles_args(ctx, l.r, frame_dev, tile_rank, tile_ranks, &seq, &l.a);
+    if (rc) return rc;
+    rc = check_frame_out(ctx, out_rgb, out_len, l.r.p.width, l.r.p.height);
+    if (rc) return rc;
     CK(ctx, cudaSetDevice(ctx->device));
-    LaunchArgs a;
-    a.row0 = 0;
-    a.row1 = r.p.height;
-    a.tile_rank = tile_rank;
-    a.tile_ranks = tile_ranks;
-    a.dst = (uint8_t*)frame_dev;
-    a.out_row0 = 0;
-    a.plan = plan_slabs(r.p.width, r.p.height);
-    a.ctl = reinterpret_cast<rt_frame_ctl*>((uint8_t*)frame_dev + rt_frame_ctl_offset(bytes));
-    return render_and_collect(ctx, scene, r, a, (const uint8_t*)frame_dev, seq, out_rgb, bytes,
-                              (uint64_t)r.p.width * r.p.height / tile_ranks, stats, t0);
+    return collect_frame(ctx, l.a.frame, seq, out_rgb, &l, 1, stats, t0);
     RT_GUARD_END(ctx)
 }
 
@@ -792,31 +872,28 @@ int rt_render_samples(rt_ctx* ctx, const rt_scene* scene, rt_accum* acc, uint32_
         return set_err(ctx, RT_ERR_INVALID_ARG, "rt_render_samples: not the scene of the chunks since the last create / reset");
     rt_params p = acc->params;
     p.spp = acc->samples + n_samples;
-    Resolved r;
-    int rc = resolve(ctx, scene, &p, false, &r);
+    Launch l{ctx, scene};
+    int rc = resolve(ctx, scene, &p, false, &l.r);
     if (rc) return rc;
-    const uint32_t rows = acc->row1 - acc->row0;
-    const size_t bytes = (size_t)rows * r.p.width * 3;
+    const uint32_t rows = acc->row1 - acc->row0, width = l.r.p.width;
+    const size_t bytes = (size_t)rows * width * 3;
     if (out_rgb && out_len != bytes)
-        return set_err(ctx, RT_ERR_INVALID_ARG, "out_len %zu != (rows %u * width %u * 3) = %zu", out_len, rows, r.p.width, bytes);
+        return set_err(ctx, RT_ERR_INVALID_ARG, "out_len %zu != (rows %u * width %u * 3) = %zu", out_len, rows, width, bytes);
     CK(ctx, cudaSetDevice(ctx->device));
-    LaunchArgs a;
-    a.row0 = acc->row0;
-    a.row1 = acc->row1;
-    a.out_row0 = acc->row0;
-    rc = own_frame(ctx, r.p.width, rows, &a);
+    l.a.row0 = acc->row0;
+    l.a.row1 = acc->row1;
+    l.a.out_row0 = acc->row0;
+    rc = own_frame(ctx, width, rows, &l.a.frame);
     if (rc) return rc;
-    a.stream = false;  // the band is copied after the kernel
-    a.state_in = acc->state[acc->cur];
-    a.state_out = acc->state[acc->cur ^ 1];
-    a.s0 = acc->samples;
-    const uint64_t pixels = (uint64_t)rows * r.p.width;
-    rc = render_and_collect(ctx, scene, r, a, ctx->d_out, ctx->out_seq, out_rgb, bytes, pixels, stats, t0);
+    l.a.stream = false;  // the band is copied after the kernel
+    l.a.state_in = acc->state[acc->cur];
+    l.a.state_out = acc->state[acc->cur ^ 1];
+    l.a.s0 = acc->samples;
+    rc = collect_frame(ctx, l.a.frame, OWN_FRAME_SEQ, out_rgb, &l, 1, stats, t0);
     if (rc) return rc;
     acc->cur ^= 1;
     acc->samples += n_samples;
     acc->scene_serial = scene->serial;
-    if (stats) stats->primary = pixels * n_samples;
     return RT_OK;
     RT_GUARD_END(ctx)
 }
@@ -921,16 +998,14 @@ int rt_frame_collect(rt_ctx* ctx, const void* frame_dev, const rt_params* params
                      size_t out_len) {
     if (!ctx || !frame_dev || !params) return RT_ERR_INVALID_ARG;
     RT_GUARD_BEGIN
+    const auto t0 = std::chrono::steady_clock::now();
     if (params->width == 0 || params->height == 0 || seq == 0) return set_err(ctx, RT_ERR_INVALID_ARG, "rt_frame_collect: zero size or seq");
-    const size_t bytes = (size_t)params->width * params->height * 3;
-    if (out_rgb && out_len != bytes) return set_err(ctx, RT_ERR_INVALID_ARG, "out_len %zu != height*width*3 = %zu", out_len, bytes);
-    CK(ctx, cudaSetDevice(ctx->device));
-    const SlabPlan plan = plan_slabs(params->width, params->height);
-    const rt_frame_ctl* ctl = reinterpret_cast<const rt_frame_ctl*>((const uint8_t*)frame_dev + rt_frame_ctl_offset(bytes));
-    SlabJob job;
-    const int rc = enqueue_slab_copies(ctx, (const uint8_t*)frame_dev, ctl, plan, seq, out_rgb, &job);
+    const int rc = check_frame_out(ctx, out_rgb, out_len, params->width, params->height);
     if (rc) return rc;
-    return finish_slab_copies(ctx, job);
+    CK(ctx, cudaSetDevice(ctx->device));
+    // read only here: the ranks elsewhere render into the frame
+    const Frame f = caller_frame(const_cast<void*>(frame_dev), params->width, params->height);
+    return collect_frame(ctx, f, seq, out_rgb, nullptr, 0, nullptr, t0);
     RT_GUARD_END(ctx)
 }
 

@@ -36,7 +36,6 @@ struct rt_ctx {
     char name[64] = {0};
     uint8_t* d_out = nullptr;  // band / frame staging in HBM + control block
     size_t d_out_bytes = 0;    // capacity for pixels (the control block follows at rt_frame_ctl_offset(capacity))
-    uint64_t out_seq = 1;      // frame number the counters of d_out count towards (reset per launch: always 1)
     unsigned long long* d_ctr = nullptr;  // NUM_COUNTERS counters | 2 tickets (one u64) | redo count (one u64)
     unsigned long long* h_ctr = nullptr;  // pinned mirror
     unsigned int* d_redo = nullptr;       // pixels to render again once the tie-break tables are up (REDO_CAP entries)
@@ -52,7 +51,6 @@ struct rt_ctx {
     float* d_scratch = nullptr;
     void* d_flush = nullptr;              // rt_l2_flush: a buffer larger than L2
     size_t flush_bytes = 0;
-    float first_pass_ms = 0.0f;           // kernel time of the first pass when a second one followed (finish_redo)
     rtb::DeviceBuild dbuild;
     // scene upload: one pinned staging buffer the blob is assembled in, and a few retired device blobs kept for the
     // next rt_scene_create (a slave makes one scene per job: cudaMalloc/cudaFree per job were a third of a small job)
@@ -125,12 +123,25 @@ struct SlabPlan {
 };
 SlabPlan plan_slabs(uint32_t width, uint32_t rows);
 
+// A frame buffer on the device (possibly a peer's) with its control block and slab plan.
+struct Frame {
+    uint8_t* dev = nullptr;
+    rt_frame_ctl* ctl = nullptr;  // nullable: no completion counting
+    SlabPlan plan;
+};
+// The context's own staging frame for `rows` rows, its counters reset on ctx->stream: its frame number is always
+// OWN_FRAME_SEQ (see own_frame in rt_api.cu).
+constexpr uint64_t OWN_FRAME_SEQ = 1;
+int own_frame(rt_ctx* ctx, uint32_t width, uint32_t rows, Frame* f);
+// A caller's whole frame of width x height (rt_frame_alloc / rt_frame_open): the control block follows the pixels.
+Frame caller_frame(void* frame_dev, uint32_t width, uint32_t height);
+// out_rgb (nullable: no download) must hold a whole frame of width x height.
+int check_frame_out(rt_ctx* ctx, const uint8_t* out_rgb, size_t out_len, uint32_t width, uint32_t height);
+
 struct LaunchArgs {
     uint32_t row0 = 0, row1 = 0, tile_rank = 0, tile_ranks = 1;
-    uint8_t* dst = nullptr;       // frame / band buffer (device, possibly a peer's)
+    Frame frame;                  // where the launch's rows go
     uint32_t out_row0 = 0;
-    rt_frame_ctl* ctl = nullptr;  // its control block (nullable: no completion counting)
-    SlabPlan plan;
     bool stream = false;          // the frame goes to the host slab by slab while it renders (stage + counters wanted)
     const unsigned int* pixel_list = nullptr;  // redo launch: render exactly these pixels (y * width + x)
     uint32_t list_count = 0;
@@ -138,29 +149,25 @@ struct LaunchArgs {
     void* state_out = nullptr;
     uint32_t s0 = 0;
 };
-// The context's own staging frame (+ control block) for a launch of `rows` rows: fills dst / ctl / plan, bumps out_seq.
-int own_frame(rt_ctx* ctx, uint32_t width, uint32_t rows, LaunchArgs* a);
 // Launches the render on ctx->stream; timing events ev0 / ev1 are recorded around the kernel.
 int launch(rt_ctx* ctx, const rt_scene* scene, const Resolved& r, const LaunchArgs& a, LaunchInfo* info);
-// After the kernel of `launch` has completed: re-renders the pixels that needed the tie-break tables before they had
-// landed (waits for the tables).  *redone = number of pixels rendered again.
-int finish_redo(rt_ctx* ctx, const rt_scene* scene, const Resolved& r, const LaunchArgs& a, uint32_t* redone);
-int finish_stats(rt_ctx* ctx, const Resolved& r, uint64_t pixels, rt_stats* st,
-                 std::chrono::steady_clock::time_point t0, const LaunchInfo& li);
-// On the frame owner.  enqueue: for every slab, on the copy stream, wait (on the device) until frame number `seq` of it
-// is complete, then copy it towards out_rgb (nullptr: only wait) — asynchronous; a pageable out_rgb is reached through a
-// pinned staging frame.  finish: host side of the same — returns when every slab is in out_rgb.  Between the two the
-// caller is free to finish its own kernel (second pass included): nothing here blocks the render stream.
-struct SlabJob {
-    SlabPlan plan;
-    uint8_t* out = nullptr;       // caller's destination
-    uint8_t* pinned = nullptr;    // where the device copies go (== out when out is pinned)
-    uint32_t host_done = 0;       // pageable path: slabs already copied on to `out`
-    const rt_frame_ctl* ctl = nullptr;
+
+// One context's launch towards a frame, and what it reports: `info` from launch(), `st` from its finish (rt_api.cu).
+struct Launch {
+    rt_ctx* ctx = nullptr;
+    const rt_scene* scene = nullptr;
+    Resolved r;
+    LaunchArgs a;
+    LaunchInfo info;
+    rt_stats st{};
 };
-int enqueue_slab_copies(rt_ctx* ctx, const uint8_t* frame_dev, const rt_frame_ctl* ctl, const SlabPlan& plan, uint64_t seq,
-                        uint8_t* out_rgb, SlabJob* job);
-int finish_slab_copies(rt_ctx* ctx, const SlabJob& job);
+// The frame owner's sequence, on `owner` (the context whose memory holds frame f): launches the n entries of l (none:
+// the frame is rendered by ranks elsewhere), streams frame number `seq` of f to out_rgb (nullptr: none) slab by slab
+// while it renders, finishes every launch (second pass, statistics) and returns when the whole frame is in out_rgb.
+// Errors of a launch on another context are reported on `owner` as "context i: ...".  stats (nullable; filled when
+// n >= 1): the launches' statistics combined, total_ms counted from t0.
+int collect_frame(rt_ctx* owner, const Frame& f, uint64_t seq, uint8_t* out_rgb, Launch* l, uint32_t n, rt_stats* stats,
+                  std::chrono::steady_clock::time_point t0);
 
 }  // namespace rtb
 

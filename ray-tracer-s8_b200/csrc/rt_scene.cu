@@ -9,7 +9,7 @@
 //     alone defines: the DFS leaf rank that breaks exact-distance ties (shapes/mod.rs:177-182) and the ancestor boxes a
 //     ray with a zero direction component must pass (ray.rs:174-194).  A builder thread makes it beside the upload and
 //     sends its tables (rank | ref_up | ref_box) to the device when they are done; a render that starts earlier marks
-//     the (measure-zero) pixels that needed them and renders those again (rt_api.cu finish_redo).
+//     the (measure-zero) pixels that needed them and renders those again (rt_api.cu finish_launch).
 #include <algorithm>
 #include <cmath>
 #include <cstring>
