@@ -12,7 +12,7 @@
 //   radix sort    cub::DeviceRadixSort::SortKeys on the 62 significant bits (library sort: not a path kernel)
 //   karras_nodes  inner node i ↔ keys [first,last], split by the highest differing bit; children + parents
 //   refit         one thread per leaf walks up; the second arrival at a node joins its two child boxes, writes the
-//                 node record (centre / half-extent form, padded exactly like the host's centre_half_of) and goes on
+//                 node record (centre / half-extent form: centre_half, as on the host) and goes on
 //   leaf_depths   deepest leaf, for the traversal stack bound (MAX_STACK)
 #include <cub/device/device_radix_sort.cuh>
 
@@ -85,18 +85,6 @@ struct B6 {
     float lo[3], hi[3];
 };
 
-// centre / half-extent form, padded for the FILTER-domain slab arithmetic — the host's centre_half_of, verbatim
-__device__ __forceinline__ void centre_half_dev(const B6& b, float c[3], float h[3]) {
-    double m = 0.0;
-    for (int a = 0; a < 3; a++) m = fmax(m, fmax(fabs((double)b.lo[a]), fabs((double)b.hi[a])));
-    for (int a = 0; a < 3; a++) {
-        const double cc = 0.5 * ((double)b.lo[a] + (double)b.hi[a]);
-        const double hh = 0.5 * ((double)b.hi[a] - (double)b.lo[a]);
-        c[a] = (float)cc;
-        h[a] = (float)(hh * (1.0 + 4e-6) + 2e-6 * m + 1e-30);
-    }
-}
-
 __global__ void refit(const unsigned long long* __restrict__ keys, const float* __restrict__ boxes,
                       const uint32_t* __restrict__ pid_of, int n, const int2* __restrict__ child,
                       const int* __restrict__ parent, unsigned int* __restrict__ arrived, B6* nbox,
@@ -134,8 +122,8 @@ __global__ void refit(const unsigned long long* __restrict__ keys, const float* 
         fetch(ch.x, &bl, &cl);
         fetch(ch.y, &br, &cr);
         float lc[3], lh[3], rc[3], rh[3];
-        centre_half_dev(bl, lc, lh);
-        centre_half_dev(br, rc, rh);
+        centre_half(bl.lo, bl.hi, lc, lh);
+        centre_half(br.lo, br.hi, rc, rh);
         float w[12];
         node_box_words(lc, lh, rc, rh, w);
         lnode[NODE_F4 * (size_t)node + 0] = make_float4(w[0], w[1], w[2], w[3]);
@@ -173,17 +161,18 @@ void free_device_build(DeviceBuild* b) {
     *b = DeviceBuild();
 }
 
-// boxes: n x (min xyz, max xyz) of the primitives the tree covers (host); pid_of: their primitive ids (host).
+// h_boxes: the boxes of the n primitives the tree covers (host); pid_of: their primitive ids (host).
 // Writes n - 1 node records to lnode (device); the root is node 0.
 // *depth_out = deepest leaf.
-cudaError_t build_lbvh_device(DeviceBuild* buf, const float* h_boxes, const uint32_t* h_pid_of, uint32_t n,
+static_assert(sizeof(Box) == 6 * sizeof(float), "the kernels read a Box as min xyz | max xyz");
+cudaError_t build_lbvh_device(DeviceBuild* buf, const Box* h_boxes, const uint32_t* h_pid_of, uint32_t n,
                               float4* lnode, uint32_t* depth_out, cudaStream_t stream) {
     if (n < 2) return cudaErrorInvalidValue;
     // centroid bounds on the host: one pass over data the host already holds
     float cmin[3] = {3.0e38f, 3.0e38f, 3.0e38f}, cmax[3] = {-3.0e38f, -3.0e38f, -3.0e38f};
     for (uint32_t i = 0; i < n; i++)
         for (int a = 0; a < 3; a++) {
-            const float c = 0.5f * (h_boxes[6 * (size_t)i + a] + h_boxes[6 * (size_t)i + 3 + a]);
+            const float c = 0.5f * (h_boxes[i].min[a] + h_boxes[i].max[a]);
             cmin[a] = c < cmin[a] ? c : cmin[a];
             cmax[a] = c > cmax[a] ? c : cmax[a];
         }
@@ -223,7 +212,7 @@ cudaError_t build_lbvh_device(DeviceBuild* buf, const float* h_boxes, const uint
     int* d_parent = (int*)(m + o_parent);
     unsigned int* d_arr = (unsigned int*)(m + o_arr);
     B6* d_nbox = (B6*)(m + o_nbox);
-    if ((e = cudaMemcpyAsync(d_boxes, h_boxes, (size_t)n * 24, cudaMemcpyHostToDevice, stream)) != cudaSuccess) return e;
+    if ((e = cudaMemcpyAsync(d_boxes, h_boxes, (size_t)n * sizeof(Box), cudaMemcpyHostToDevice, stream)) != cudaSuccess) return e;
     if ((e = cudaMemcpyAsync(d_pid, h_pid_of, (size_t)n * 4, cudaMemcpyHostToDevice, stream)) != cudaSuccess) return e;
     if ((e = cudaMemsetAsync(d_arr, 0, (size_t)n * 4 + 4, stream)) != cudaSuccess) return e;
     const unsigned T = 256, G = (n + T - 1) / T;

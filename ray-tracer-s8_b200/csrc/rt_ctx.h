@@ -89,9 +89,6 @@ struct rt_scene {
     size_t blob_bytes = 0, blob_cap = 0;
     rtb::DevScene dev{};
     uint32_t n = 0;
-    uint32_t tree_depth = 0;   // depth of the tree the kernels traverse
-    bool device_tree = false;  // it was built on the device (LBVH)
-    size_t o_rank = 0, o_up = 0, o_refbox = 0;  // blob offsets of the late tables
     std::unique_ptr<rt_aux> aux;
     uint64_t serial = 0;  // unique per process (rt_scene_create): a re-created scene may reuse a destroyed one's address
 };

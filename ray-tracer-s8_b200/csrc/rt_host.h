@@ -13,6 +13,7 @@ namespace rtb {
 struct DevScene;
 struct DevCamera;
 struct DevParams;
+struct Box;
 
 constexpr int MAX_SLABS = 64;  // completion counters per frame (frame control block)
 
@@ -40,7 +41,7 @@ struct DeviceBuild {
     size_t bytes = 0;
 };
 void free_device_build(DeviceBuild* b);
-cudaError_t build_lbvh_device(DeviceBuild* buf, const float* h_boxes, const uint32_t* h_pid_of, uint32_t n,
+cudaError_t build_lbvh_device(DeviceBuild* buf, const Box* h_boxes, const uint32_t* h_pid_of, uint32_t n,
                               float4* lnode, uint32_t* depth_out, cudaStream_t stream);
 
 // rt_kernels.cu
@@ -57,7 +58,6 @@ cudaError_t launch_fp32_peak(float* scratch, int sm_count, int iters, cudaStream
 // rows * width * 3 floats: sum / samples of each pixel's state record (rt_accum_read_linear)
 cudaError_t launch_accum_linear(const void* state, float* out, unsigned long long pixels, uint32_t samples, int sm_count,
                                 cudaStream_t stream);
-size_t scene_smem_bytes(const DevScene& sc, int isect);
 
 // ---- rt_bvh_host.cpp: SAH BVH with the reference's topology ------------------------------------------
 struct Box {

@@ -170,7 +170,7 @@ __global__ void __launch_bounds__(TPB, MINB) render_kernel_lanes(const DevScene 
 
     SceneView sv;
     if (SMEM) {
-        // image layout = blob layout: sph | tri | lnode (BVH) or sph | tri + sph2 (brute force)
+        // image = blob layout, scene_image_bytes long: sph | tri | lnode (BVH) or sph | tri + sph2 (brute force)
         const uint32_t geom = sc.ns * 16u + sc.nt * 64u;
         const uint32_t rest = (ISECT == RT_INTERSECT_BVH) ? sc.lni * (uint32_t)NODE_BYTES
                                                           : ((sc.ns + 7u) & ~7u) * 16u;
@@ -708,13 +708,6 @@ static KernelFn pick_resume(int* threads) {
     }
 }
 
-size_t scene_smem_bytes(const DevScene& sc, int isect) {
-    size_t b = (size_t)sc.ns * 16 + (size_t)sc.nt * 64;
-    if (isect == RT_INTERSECT_BVH) b += (size_t)sc.lni * NODE_BYTES;
-    else b += (size_t)((sc.ns + 7u) & ~7u) * 16;  // pair-packed spheres
-    return b;
-}
-
 // Resolves every kernel variant once per context so that the first render does not pay the lazy module load.
 cudaError_t preload_kernels() {
     cudaFuncAttributes a;
@@ -752,7 +745,7 @@ cudaError_t launch_render(const DevScene& sc, const DevCamera& cam, const DevPar
     const bool resume = pr.state_out != nullptr;  // rt_render_samples
     if (resume) count = false;
     const size_t static_smem = (SMEM_TPB / 32) * (OUT_SLOTS * (TILE_BYTES + 16) + 4) + 64;
-    const size_t need = scene_smem_bytes(sc, isect);
+    const size_t need = scene_image_bytes(sc.ns, sc.nt, sc.lni, isect == RT_INTERSECT_BVH);
     // Stage the scene in shared memory when one 1024-thread CTA per SM fits with it (scenes up to ~200 KB); larger
     // scenes are read through L1/L2 (measured on the C5 sweep, profiles/r1_c5_sweep.log)
     if (info) info->counts_done = true;

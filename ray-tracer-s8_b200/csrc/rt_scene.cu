@@ -13,7 +13,6 @@
 #include <algorithm>
 #include <cmath>
 #include <cstring>
-#include <functional>
 #include <limits>
 
 #include "rt_ctx.h"
@@ -21,6 +20,12 @@
 using namespace rtb;
 
 namespace {
+
+// leaf codes are ~(pid << 5) in 32 bits: 26-bit primitive ids
+constexpr uint64_t MAX_PRIMS = 0x3ffffffu;
+constexpr uint32_t kDeviceBuildMin = 8192;  // RT_B200_BUILD=auto: the traversal tree is built on the device from here
+constexpr uint32_t kRefSyncBelow = 256;     // the reference tree is built inline below this many primitives
+constexpr size_t kRetiredBlobs = 4;         // retired device blobs a context keeps
 
 struct PrimRef {
     uint8_t kind;  // 0 sphere, 1 triangle
@@ -34,24 +39,16 @@ inline float ref_max(float x, float y) { return (x > y) ? x : y; }
 inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 inline bool finite3(const float* v) { return std::isfinite(v[0]) && std::isfinite(v[1]) && std::isfinite(v[2]); }
 
-// centre / half-extent form of a box (FILTER domain): t = (c - o)*inv -/+ h*|inv|.  h is padded for the rounding of
-// the c- and h-terms (<= 2^-24 * (2|c| + h) per axis); the o-term is covered per ray by the kernels.
-void centre_half_of(const Box& b, float c[3], float h[3]) {
-    double m = 0.0;
-    for (int a = 0; a < 3; a++) m = std::fmax(m, std::fmax(std::fabs((double)b.min[a]), std::fabs((double)b.max[a])));
-    for (int a = 0; a < 3; a++) {
-        const double cc = 0.5 * ((double)b.min[a] + (double)b.max[a]);
-        const double hh = 0.5 * ((double)b.max[a] - (double)b.min[a]);
-        c[a] = (float)cc;
-        h[a] = (float)(hh * (1.0 + 4e-6) + 2e-6 * m + 1e-30);
-    }
-}
-
 // World order + bounds (Sphere::aabb sphere.rs:65-72, Triangle::aabb mesh.rs:46-95).
 int world_and_boxes(const rt_sphere* spheres, uint32_t n_spheres, const rt_triangle* triangles, uint32_t n_triangles,
                     const uint32_t* world_index, std::vector<PrimRef>* world_out, std::vector<Box>* boxes_out,
                     std::string* err) {
-    char buf[256];
+    auto fail = [err](int rc, const char* fmt, uint32_t v) {
+        char buf[256];
+        snprintf(buf, sizeof buf, fmt, v);
+        *err = buf;
+        return rc;
+    };
     const uint32_t n = n_spheres + n_triangles;
     std::vector<PrimRef>& world = *world_out;
     world.assign(n, PrimRef{0, 0});
@@ -59,11 +56,7 @@ int world_and_boxes(const rt_sphere* spheres, uint32_t n_spheres, const rt_trian
         std::vector<uint8_t> seen(n, 0);
         for (uint32_t i = 0; i < n; i++) {
             const uint32_t pos = world_index ? world_index[i] : i;
-            if (pos >= n || seen[pos]) {
-                snprintf(buf, sizeof buf, "world_index is not a permutation of 0..%u", n - 1);
-                *err = buf;
-                return RT_ERR_INVALID_ARG;
-            }
+            if (pos >= n || seen[pos]) return fail(RT_ERR_INVALID_ARG, "world_index is not a permutation of 0..%u", n - 1);
             seen[pos] = 1;
             world[pos] = i < n_spheres ? PrimRef{0, i} : PrimRef{1, i - n_spheres};
         }
@@ -74,156 +67,72 @@ int world_and_boxes(const rt_sphere* spheres, uint32_t n_spheres, const rt_trian
         Box& b = boxes[w];
         if (world[w].kind == 0) {
             const rt_sphere& s = spheres[world[w].idx];
-            if (!finite3(s.center) || !std::isfinite(s.radius)) {
-                snprintf(buf, sizeof buf, "sphere %u has non-finite geometry", world[w].idx);
-                *err = buf;
-                return RT_ERR_BVH;
-            }
+            if (!finite3(s.center) || !std::isfinite(s.radius))
+                return fail(RT_ERR_BVH, "sphere %u has non-finite geometry", world[w].idx);
             for (int a = 0; a < 3; a++) {
                 b.min[a] = s.center[a] - s.radius;
                 b.max[a] = s.center[a] + s.radius;
             }
         } else {
             const rt_triangle& t = triangles[world[w].idx];
-            if (!finite3(t.a) || !finite3(t.b) || !finite3(t.c)) {
-                snprintf(buf, sizeof buf, "triangle %u has non-finite geometry", world[w].idx);
-                *err = buf;
-                return RT_ERR_BVH;
-            }
+            if (!finite3(t.a) || !finite3(t.b) || !finite3(t.c))
+                return fail(RT_ERR_BVH, "triangle %u has non-finite geometry", world[w].idx);
             for (int a = 0; a < 3; a++) {
                 b.min[a] = ref_min(ref_min(t.a[a], t.c[a]), t.b[a]);
                 b.max[a] = ref_max(ref_max(t.a[a], t.c[a]), t.b[a]);
             }
         }
-        if (!finite3(b.min) || !finite3(b.max)) {  // centre +- radius overflowed: the reference's bucket index would panic
-            snprintf(buf, sizeof buf, "primitive at world position %u has non-finite bounds", w);
-            *err = buf;
-            return RT_ERR_BVH;
-        }
+        if (!finite3(b.min) || !finite3(b.max))  // centre +- radius overflowed: the reference's bucket index would panic
+            return fail(RT_ERR_BVH, "primitive at world position %u has non-finite bounds", w);
     }
     return RT_OK;
 }
 
-// The late tables, in pid indexing, from the reference tree.
-struct AuxTables {
-    std::vector<uint32_t> rank, up;
-    std::vector<float> refbox;  // [ni][side][min xyz . | max xyz .]
+// The scene blob, the one statement of its layout: the shared-memory image first (sph | tri | lnode, contiguous, each a
+// multiple of 16 bytes, scene_image_bytes long), then 256-byte aligned sections.  rt_scene_create uploads everything
+// before sync_bytes; the reference tables and the flag that announces them follow.
+struct BlobLayout {
+    size_t sph, tri, lnode, sph2, mat, emis, box, big, rank, up, refbox, flag;
+    size_t sync_bytes, blob_bytes;
 };
-void tables_from_tree(const HostBVH& bvh, const std::vector<uint32_t>& pid_of_world, AuxTables* t,
-                      std::vector<uint32_t>* rank_by_world) {
-    const uint32_t n = (uint32_t)pid_of_world.size(), ni = (uint32_t)bvh.inner.size();
-    t->rank.assign(n, 0);
-    t->up.assign((size_t)n + std::max(ni, 1u), UP_ROOT);
-    t->refbox.assign((size_t)std::max(ni, 1u) * 16, 0.0f);
-    rank_by_world->assign(n, 0);
-    for (uint32_t r = 0; r < n; r++) {
-        const uint32_t w = bvh.leaf_order[r];
-        (*rank_by_world)[w] = r;
-        t->rank[pid_of_world[w]] = r;
-    }
-    for (uint32_t i = 0; i < ni; i++) {
-        const HostNode& hn = bvh.inner[i];
-        for (uint32_t side = 0; side < 2; side++) {
-            const int32_t code = side ? hn.right : hn.left;
-            const Box& b = side ? hn.box_r : hn.box_l;
-            float* o = t->refbox.data() + ((size_t)2 * i + side) * 8;
-            for (int a = 0; a < 3; a++) {
-                o[a] = b.min[a];
-                o[4 + a] = b.max[a];
-            }
-            const uint32_t slot = (i << 1) | side;
-            if (code >= 0) t->up[(size_t)n + (uint32_t)code] = slot;
-            else t->up[pid_of_world[(uint32_t)~code]] = slot;
-        }
-    }
+BlobLayout blob_layout(uint32_t n_spheres, uint32_t n_triangles, uint32_t lni) {
+    const size_t n = (size_t)n_spheres + n_triangles, ni_ref = std::max<size_t>(n - 1, 1);
+    BlobLayout L;
+    size_t off = 0;
+    auto take = [&](size_t bytes) {
+        const size_t o = off;
+        off = align_up(off + bytes, 256);
+        return o;
+    };
+    L.sph = 0;
+    L.tri = L.sph + (size_t)n_spheres * 16;
+    L.lnode = L.tri + (size_t)n_triangles * 64;
+    off = align_up(scene_image_bytes(n_spheres, n_triangles, lni, true), 256);
+    L.sph2 = take((size_t)((n_spheres + 7u) & ~7u) * 16);
+    L.mat = take(n * 16);
+    L.emis = take(n * 4);
+    L.box = take(n * 32);
+    L.big = take((size_t)MAX_BIG * 4);
+    L.sync_bytes = off;
+    L.rank = take(n * 4);
+    L.up = take((n + ni_ref) * 4);
+    L.refbox = take(ni_ref * 64);
+    L.flag = take(4);
+    L.blob_bytes = off;
+    return L;
 }
 
-}  // namespace
-
-namespace rtb {
-
-int scene_settle(rt_ctx* ctx, const rt_scene* scene) {
-    rt_aux* aux = scene->aux.get();
-    if (!aux) return RT_OK;
-    if (aux->worker.joinable()) aux->worker.join();
-    if (aux->state.load(std::memory_order_acquire) < 0) return set_err(ctx, RT_ERR_BVH, "BVH build failed: %s", aux->err.c_str());
-    return RT_OK;
-}
-
-DevScene scene_view(const rt_scene* scene) {
-    DevScene d = scene->dev;
-    d.aux_ready = (!scene->aux || scene->aux->state.load(std::memory_order_acquire) == 1) ? 1 : 0;
-    return d;
-}
-
-}  // namespace rtb
-
-extern "C" {
-
-int rt_bvh_build_host(const rt_sphere* spheres, uint32_t n_spheres, const rt_triangle* triangles, uint32_t n_triangles,
-                      const uint32_t* world_index, uint32_t* rank_out, uint32_t* n_nodes, uint32_t* depth) {
-    RT_GUARD_BEGIN
-    const uint64_t n64 = (uint64_t)n_spheres + n_triangles;
-    if (n64 == 0) return RT_ERR_EMPTY_SCENE;
-    if (n64 > 0x3ffffffu) return RT_ERR_UNSUPPORTED;  // leaf codes hold a 26-bit primitive id
-    if ((n_spheres && !spheres) || (n_triangles && !triangles)) return RT_ERR_INVALID_ARG;
-    std::vector<PrimRef> world;
-    std::vector<Box> boxes;
-    std::string err;
-    int rc = world_and_boxes(spheres, n_spheres, triangles, n_triangles, world_index, &world, &boxes, &err);
-    HostBVH bvh;
-    if (rc == RT_OK && !build_bvh(boxes, &bvh, &err)) {
-        err = "BVH build failed: " + err;
-        rc = RT_ERR_BVH;
-    }
-    if (rc) return set_err(nullptr, rc, "%s", err.c_str());
-    if (rank_out)
-        for (uint32_t r = 0; r < (uint32_t)n64; r++) rank_out[bvh.leaf_order[r]] = r;
-    if (n_nodes) *n_nodes = bvh.node_count;
-    if (depth) *depth = bvh.depth;
-    return RT_OK;
-    RT_GUARD_END(nullptr)
-}
-
-int rt_scene_create(rt_ctx* ctx, const rt_sphere* spheres, uint32_t n_spheres, const rt_triangle* triangles,
-                    uint32_t n_triangles, const uint32_t* world_index, rt_scene** out) {
-    if (!ctx) return RT_ERR_INVALID_ARG;
-    RT_GUARD_BEGIN
-    if (!out) return set_err(ctx, RT_ERR_INVALID_ARG, "rt_scene_create: out is NULL");
-    *out = nullptr;
-    const uint64_t n64 = (uint64_t)n_spheres + n_triangles;
-    if (n64 == 0)
-        return set_err(ctx, RT_ERR_EMPTY_SCENE,
-                       "empty world: the reference's BVHNode::build never terminates on zero shapes");
-    // leaf codes are ~(pid << 5) in 32 bits (26-bit ids); inner codes are the byte offset of a 64-byte node record and
-    // must stay positive (n - 1 records: 25 bits of nodes)
-    if (n64 > 0x3ffffffu || (n64 - 1) * (uint64_t)NODE_BYTES > 0x7fffffffull)
-        return set_err(ctx, RT_ERR_UNSUPPORTED, "too many primitives (%llu; this build addresses %llu)", (unsigned long long)n64,
-                       (unsigned long long)(0x7fffffffull / NODE_BYTES + 1));
-    if ((n_spheres && !spheres) || (n_triangles && !triangles))
-        return set_err(ctx, RT_ERR_INVALID_ARG, "rt_scene_create: NULL primitive array");
-    const uint32_t n = (uint32_t)n64;
-    const TestHooks& hooks = test_hooks();
-
-    static std::atomic<uint64_t> next_serial{1};
-    std::unique_ptr<rt_scene> sc(new rt_scene());
-    sc->ctx = ctx;
-    sc->serial = next_serial++;
-    sc->n = n;
-    sc->aux.reset(new rt_aux());
-    rt_aux* aux = sc->aux.get();
-    std::vector<PrimRef> world;
-    {
-        std::string werr;
-        const int wrc = world_and_boxes(spheres, n_spheres, triangles, n_triangles, world_index, &world, &aux->boxes, &werr);
-        if (wrc) return set_err(ctx, wrc, "%s", werr.c_str());
-    }
-    const std::vector<Box>& boxes = aux->boxes;  // shared, read-only from here on
-
-    // ---- which tree will be traversed ---------------------------------------------------------------------
-    std::vector<uint32_t> big_world;  // split layout: world positions of the primitives kept out of the tree
-    std::vector<Box> rest_store;      // boxes and world positions of the primitives the tree covers (without big
-    std::vector<uint32_t> rest_world; //   primitives the tree covers `boxes` itself, no copy)
+// The split layout: the primitives whose box is a large share of the scene's (at most MAX_BIG, the largest) are kept
+// out of the traversal tree and tested first; the tree covers the rest.
+struct Split {
+    std::vector<uint32_t> big_world;   // world positions of the primitives kept out of the tree, ascending
+    std::vector<uint32_t> rest_world;  // world positions of the primitives the tree covers
+    std::vector<Box> rest_store;       // their boxes, when some primitives are big
+    // boxes of the primitives the tree covers (without big primitives, `boxes` itself: no copy)
+    const std::vector<Box>& rest(const std::vector<Box>& boxes) const { return big_world.empty() ? boxes : rest_store; }
+};
+void split_big(const std::vector<Box>& boxes, Split* s) {
+    const uint32_t n = (uint32_t)boxes.size();
     if (n > 1) {
         auto area_of = [](const Box& b) {
             const double sx = (double)b.max[0] - b.min[0], sy = (double)b.max[1] - b.min[1], sz = (double)b.max[2] - b.min[2];
@@ -243,200 +152,187 @@ int rt_scene_create(rt_ctx* ctx, const rt_sphere* spheres, uint32_t n_spheres, c
         }
         std::sort(cand.begin(), cand.end());
         if (cand.size() > (size_t)MAX_BIG) cand.resize(MAX_BIG);
-        for (auto& c : cand) big_world.push_back(c.second);
-        std::sort(big_world.begin(), big_world.end());
+        for (auto& c : cand) s->big_world.push_back(c.second);
+        std::sort(s->big_world.begin(), s->big_world.end());
     }
-    if (big_world.empty()) {
-        rest_world.resize(n);
-        for (uint32_t w = 0; w < n; w++) rest_world[w] = w;
-    } else {
-        size_t bi = 0;
-        rest_store.reserve(n - big_world.size());
-        rest_world.reserve(n - big_world.size());
-        for (uint32_t w = 0; w < n; w++) {
-            if (bi < big_world.size() && big_world[bi] == w) {
-                bi++;
-                continue;
-            }
-            rest_store.push_back(boxes[w]);
-            rest_world.push_back(w);
-        }
+    size_t bi = 0;
+    s->rest_world.reserve(n - s->big_world.size());
+    for (uint32_t w = 0; w < n; w++) {
+        if (bi < s->big_world.size() && s->big_world[bi] == w) bi++;
+        else s->rest_world.push_back(w);
     }
-    const std::vector<Box>& rest = big_world.empty() ? boxes : rest_store;
-    const bool ltree = !rest.empty();
-    constexpr uint32_t kDeviceBuildMin = 8192;
-    const bool device_tree = rest.size() >= 2 &&
-                             (hooks.build_mode == 2 || (hooks.build_mode == 1 && rest.size() >= kDeviceBuildMin));
+    if (!s->big_world.empty()) {
+        s->rest_store.reserve(s->rest_world.size());
+        for (uint32_t w : s->rest_world) s->rest_store.push_back(boxes[w]);
+    }
+}
 
-    // ---- the reference-topology tree: beside everything else when it is worth a thread -------------------
-    const bool ref_sync = n < 256;
-    HostBVH ref_bvh;  // synchronous case only
-    AuxTables ref_tables;
-    if (ref_sync) {
-        std::string berr;
-        if (!build_bvh(boxes, &ref_bvh, &berr)) return set_err(ctx, RT_ERR_BVH, "BVH build failed: %s", berr.c_str());
-        aux->n_nodes = ref_bvh.node_count;
-        aux->depth = ref_bvh.depth;
+// The SAH tree over `rest` (at least two primitives), its leaf codes remapped to world positions.
+int host_traversal_tree(rt_ctx* ctx, const std::vector<Box>& rest, const std::vector<uint32_t>& rest_world, HostBVH* t) {
+    if (!build_bvh_sah(rest, t)) return set_err(ctx, RT_ERR_BVH, "traversal tree build failed");
+    auto remap = [&](int32_t c) { return c >= 0 ? c : ~(int32_t)rest_world[(uint32_t)~c]; };
+    for (auto& nd : t->inner) {
+        nd.left = remap(nd.left);
+        nd.right = remap(nd.right);
     }
+    t->root = remap(t->root);
+    if (t->depth > (uint32_t)MAX_STACK)
+        return set_err(ctx, RT_ERR_UNSUPPORTED, "traversal tree depth %u exceeds the traversal stack (%d)", t->depth, MAX_STACK);
+    return RT_OK;
+}
 
-    // ---- host traversal tree ---------------------------------------------------------------------------------
-    HostBVH sah;
-    const HostBVH* T = nullptr;  // tree to emit as lnode records (leaf codes: world positions)
-    if (ltree && !device_tree && rest.size() >= 2) {
-        if (!build_bvh_sah(rest, &sah)) return set_err(ctx, RT_ERR_BVH, "traversal tree build failed");
-        auto remap = [&](int32_t c) { return c >= 0 ? c : ~(int32_t)rest_world[(uint32_t)~c]; };
-        for (auto& nd : sah.inner) {
-            nd.left = remap(nd.left);
-            nd.right = remap(nd.right);
-        }
-        sah.root = remap(sah.root);
-        T = &sah;
-        if (T->depth > (uint32_t)MAX_STACK)
-            return set_err(ctx, RT_ERR_UNSUPPORTED, "traversal tree depth %u exceeds the traversal stack (%d)", T->depth, MAX_STACK);
-        sc->tree_depth = T->depth;
-    }
-
-    // ---- primitive ids: spheres [0, ns), triangles [ns, n).  In the DFS leaf order of the host-built traversal tree
-    // when there is one (neighbours in space are neighbours in memory: the per-hit material / box / rank reads of the
-    // lanes of a warp share cache lines), else in world order.
-    aux->pid_of_world.assign(n, 0xffffffffu);
-    {
-        uint32_t next_s = 0, next_t = n_spheres;
-        auto give = [&](uint32_t w) {
-            if (aux->pid_of_world[w] == 0xffffffffu) aux->pid_of_world[w] = world[w].kind == 0 ? next_s++ : next_t++;
-        };
-        if (T) {
-            std::vector<int32_t> todo;
-            todo.push_back(T->root);
-            while (!todo.empty()) {
-                const int32_t c = todo.back();
-                todo.pop_back();
-                if (c < 0) {
-                    give((uint32_t)~c);
-                } else {
-                    todo.push_back(T->inner[(size_t)c].right);
-                    todo.push_back(T->inner[(size_t)c].left);
-                }
-            }
-        }
-        for (uint32_t w = 0; w < n; w++) give(w);
-    }
-    const std::vector<uint32_t>& pid_of_world = aux->pid_of_world;
-    if (ref_sync) tables_from_tree(ref_bvh, pid_of_world, &ref_tables, &aux->rank_by_world);
-    uint32_t lni = 0;
-    if (device_tree) lni = (uint32_t)rest.size() - 1;
-    else if (T) lni = (uint32_t)T->inner.size();
-
-    // ---- blob layout: the shared-memory image first (contiguous, 16-byte granules), then 256-byte aligned sections
-    const uint32_t ni_ref = n - 1;
-    const uint32_t ns8 = (n_spheres + 7u) & ~7u;
-    size_t off = 0;
-    auto take = [&](size_t bytes) {
-        const size_t o = off;
-        off = align_up(off + bytes, 256);
-        return o;
+// Primitive ids: spheres [0, ns), triangles [ns, n).  In the DFS leaf order of the host-built traversal tree T when
+// there is one (neighbours in space are neighbours in memory: the per-hit material / box / rank reads of the lanes of a
+// warp share cache lines), else in world order.
+void assign_pids(const std::vector<PrimRef>& world, uint32_t n_spheres, const HostBVH* T, std::vector<uint32_t>* pid_of_world) {
+    const uint32_t n = (uint32_t)world.size();
+    std::vector<uint32_t>& pid = *pid_of_world;
+    pid.assign(n, 0xffffffffu);
+    uint32_t next_s = 0, next_t = n_spheres;
+    auto give = [&](uint32_t w) {
+        if (pid[w] == 0xffffffffu) pid[w] = world[w].kind == 0 ? next_s++ : next_t++;
     };
-    const size_t o_sph = 0, o_tri = o_sph + (size_t)n_spheres * 16, o_ln = o_tri + (size_t)n_triangles * 64;
-    off = align_up(o_ln + (size_t)lni * NODE_BYTES, 256);
-    const size_t o_sph2 = take((size_t)ns8 * 16), o_mat = take((size_t)n * 16), o_em = take((size_t)n * 4),
-                 o_box = take((size_t)n * 32), o_big = take((size_t)MAX_BIG * 4);
-    const size_t sync_bytes = off;  // everything up to here is uploaded by this call
-    const size_t o_rank = take((size_t)n * 4), o_up = take(((size_t)n + std::max(ni_ref, 1u)) * 4),
-                 o_refbox = take((size_t)std::max(ni_ref, 1u) * 64), o_flag = take(4);
-    const size_t blob_bytes = off;
-    sc->o_rank = o_rank;
-    sc->o_up = o_up;
-    sc->o_refbox = o_refbox;
-    sc->blob_bytes = blob_bytes;
-    const size_t stage_bytes = ref_sync ? blob_bytes : sync_bytes;
-
-    CK(ctx, cudaSetDevice(ctx->device));
-    if (ctx->h_stage_bytes < stage_bytes) {
-        if (ctx->h_stage) cudaFreeHost(ctx->h_stage);
-        ctx->h_stage = nullptr;
-        ctx->h_stage_bytes = 0;
-        size_t cap = (size_t)1 << 20;
-        while (cap < stage_bytes) cap <<= 1;
-        CK(ctx, cudaMallocHost(&ctx->h_stage, cap));
-        ctx->h_stage_bytes = cap;
-    }
-    uint8_t* const h = ctx->h_stage;
-    {   // smallest retired device blob that fits, else a new allocation in power-of-two size classes (>= 256 KB): retired
-        // blobs fit the next scene of a similar size, and the driver sees few distinct allocation sizes
-        size_t pick = ctx->retired.size();
-        for (size_t i = 0; i < ctx->retired.size(); i++)
-            if (ctx->retired[i].cap >= blob_bytes && (pick == ctx->retired.size() || ctx->retired[i].cap < ctx->retired[pick].cap)) pick = i;
-        if (pick < ctx->retired.size()) {
-            sc->d_blob = ctx->retired[pick].p;
-            sc->blob_cap = ctx->retired[pick].cap;
-            ctx->retired.erase(ctx->retired.begin() + (long)pick);
-        } else {
-            size_t cap = (size_t)1 << 18;
-            while (cap < blob_bytes) cap <<= 1;
-            CK(ctx, cudaMalloc(&sc->d_blob, cap));
-            sc->blob_cap = cap;
+    if (T) {
+        std::vector<int32_t> todo;
+        todo.push_back(T->root);
+        while (!todo.empty()) {
+            const int32_t c = todo.back();
+            todo.pop_back();
+            if (c < 0) {
+                give((uint32_t)~c);
+            } else {
+                todo.push_back(T->inner[(size_t)c].right);
+                todo.push_back(T->inner[(size_t)c].left);
+            }
         }
     }
-    auto give_back = [&] {
-        if (sc->aux && sc->aux->worker.joinable()) sc->aux->worker.join();
-        if (sc->d_blob) ctx->retired.push_back({sc->d_blob, sc->blob_cap});
-        sc->d_blob = nullptr;
-    };
+    for (uint32_t w = 0; w < n; w++) give(w);
+}
 
-    // ---- the builder thread starts now: it knows where its tables go ------------------------------------------
-    if (!ref_sync) {
-        // the flag kernels poll for the tables: down before anybody can look (device blobs are reused)
-        CK(ctx, cudaMemsetAsync(sc->d_blob + o_flag, 0, 4, ctx->stream));
-        CK(ctx, cudaStreamSynchronize(ctx->stream));
-        rt_aux* const a = aux;
-        rt_ctx* const c = ctx;
-        const size_t dr = o_rank, du = o_up, db = o_refbox, df = o_flag;
-        uint8_t* const dst = sc->d_blob;
-        const int delay_ms = hooks.aux_delay_ms;
-        a->worker = std::thread([a, c, dst, dr, du, db, df, delay_ms] {
-            try {
-                if (delay_ms > 0) std::this_thread::sleep_for(std::chrono::milliseconds(delay_ms));
-                HostBVH bvh;
-                AuxTables t;
-                std::string berr;
-                if (!build_bvh(a->boxes, &bvh, &berr)) {
-                    a->err = berr;
-                    a->state.store(-1, std::memory_order_release);
-                    return;
-                }
-                tables_from_tree(bvh, a->pid_of_world, &t, &a->rank_by_world);
-                a->n_nodes = bvh.node_count;
-                a->depth = bvh.depth;
-                cudaError_t e = cudaSetDevice(c->device);
-                if (e == cudaSuccess) e = cudaMemcpyAsync(dst + dr, t.rank.data(), t.rank.size() * 4, cudaMemcpyHostToDevice, c->aux_stream);
-                if (e == cudaSuccess) e = cudaMemcpyAsync(dst + du, t.up.data(), t.up.size() * 4, cudaMemcpyHostToDevice, c->aux_stream);
-                if (e == cudaSuccess) e = cudaMemcpyAsync(dst + db, t.refbox.data(), t.refbox.size() * 4, cudaMemcpyHostToDevice, c->aux_stream);
-                // ... and then the flag kernels already running poll (stream order: the tables are there before it)
-                static const int one = 1;
-                if (e == cudaSuccess) e = cudaMemcpyAsync(dst + df, &one, 4, cudaMemcpyHostToDevice, c->aux_stream);
-                if (e == cudaSuccess) e = cudaStreamSynchronize(c->aux_stream);
-                if (e != cudaSuccess) {
-                    a->err = std::string("upload of the tie-break tables failed: ") + cudaGetErrorString(e);
-                    a->state.store(-1, std::memory_order_release);
-                    return;
-                }
-                a->state.store(1, std::memory_order_release);
-            } catch (const std::exception& ex) {
-                a->err = ex.what();
-                a->state.store(-1, std::memory_order_release);
-            } catch (...) {
-                a->err = "unknown exception in the builder thread";
-                a->state.store(-1, std::memory_order_release);
-            }
-        });
+// The late tables, in pid indexing, from the reference tree.
+struct AuxTables {
+    std::vector<uint32_t> rank, up;
+    std::vector<float> refbox;  // [ni][side][min xyz . | max xyz .]
+};
+// Builds the reference tree and its tables, and sets aux's n_nodes, depth and rank_by_world.  false (message in *err):
+// the reference's build would panic or never terminate.
+bool build_ref_tables(const std::vector<Box>& boxes, const std::vector<uint32_t>& pid_of_world, rt_aux* aux, AuxTables* t,
+                      std::string* err) {
+    HostBVH bvh;
+    if (!build_bvh(boxes, &bvh, err)) return false;
+    const uint32_t n = (uint32_t)pid_of_world.size(), ni = (uint32_t)bvh.inner.size();
+    t->rank.assign(n, 0);
+    t->up.assign((size_t)n + std::max(ni, 1u), UP_ROOT);
+    t->refbox.assign((size_t)std::max(ni, 1u) * 16, 0.0f);
+    aux->rank_by_world.assign(n, 0);
+    for (uint32_t r = 0; r < n; r++) {
+        const uint32_t w = bvh.leaf_order[r];
+        aux->rank_by_world[w] = r;
+        t->rank[pid_of_world[w]] = r;
     }
+    for (uint32_t i = 0; i < ni; i++) {
+        const HostNode& hn = bvh.inner[i];
+        for (uint32_t side = 0; side < 2; side++) {
+            const int32_t code = side ? hn.right : hn.left;
+            const Box& b = side ? hn.box_r : hn.box_l;
+            float* o = t->refbox.data() + ((size_t)2 * i + side) * 8;
+            for (int a = 0; a < 3; a++) {
+                o[a] = b.min[a];
+                o[4 + a] = b.max[a];
+            }
+            const uint32_t slot = (i << 1) | side;
+            if (code >= 0) t->up[(size_t)n + (uint32_t)code] = slot;
+            else t->up[pid_of_world[(uint32_t)~code]] = slot;
+        }
+    }
+    aux->n_nodes = bvh.node_count;
+    aux->depth = bvh.depth;
+    return true;
+}
 
-    // ---- fill the staging copy ------------------------------------------------------------------------------------
-    float* h_sph = (float*)(h + o_sph);
-    float* h_tri = (float*)(h + o_tri);
-    float* h_mat = (float*)(h + o_mat);
-    float* h_em = (float*)(h + o_em);
-    float* h_box = (float*)(h + o_box);
+// The retired-blob pool: the smallest retired device blob that fits, else a new allocation in power-of-two size classes
+// (>= 256 KB).  Retired blobs fit the next scene of a similar size, and the driver sees few distinct allocation sizes.
+cudaError_t take_blob(rt_ctx* ctx, size_t bytes, uint8_t** p, size_t* cap) {
+    size_t pick = ctx->retired.size();
+    for (size_t i = 0; i < ctx->retired.size(); i++)
+        if (ctx->retired[i].cap >= bytes && (pick == ctx->retired.size() || ctx->retired[i].cap < ctx->retired[pick].cap)) pick = i;
+    if (pick < ctx->retired.size()) {
+        *p = ctx->retired[pick].p;
+        *cap = ctx->retired[pick].cap;
+        ctx->retired.erase(ctx->retired.begin() + (long)pick);
+        return cudaSuccess;
+    }
+    *cap = (size_t)1 << 18;
+    while (*cap < bytes) *cap <<= 1;
+    return cudaMalloc(p, *cap);
+}
+// ctx may be null (its blobs are then freed)
+void retire_blob(rt_ctx* ctx, uint8_t* p, size_t cap) {
+    if (ctx && ctx->retired.size() < kRetiredBlobs) ctx->retired.push_back({p, cap});
+    else cudaFree(p);
+}
+
+// The pinned staging buffer holds at least `bytes` (power-of-two size classes, >= 1 MB).
+cudaError_t reserve_stage(rt_ctx* ctx, size_t bytes) {
+    if (ctx->h_stage_bytes >= bytes) return cudaSuccess;
+    if (ctx->h_stage) cudaFreeHost(ctx->h_stage);
+    ctx->h_stage = nullptr;
+    ctx->h_stage_bytes = 0;
+    size_t cap = (size_t)1 << 20;
+    while (cap < bytes) cap <<= 1;
+    const cudaError_t e = cudaMallocHost(&ctx->h_stage, cap);
+    if (e == cudaSuccess) ctx->h_stage_bytes = cap;
+    return e;
+}
+
+// The reference tree on a thread of its own: its tables go to the blob on aux_stream, then the flag the kernels poll
+// (stream order: the tables are there before it).  The flag is lowered first, before anybody can look (device blobs are
+// reused).
+int start_ref_builder(rt_ctx* ctx, rt_scene* sc, const BlobLayout& L, int delay_ms) {
+    CK(ctx, cudaMemsetAsync(sc->d_blob + L.flag, 0, 4, ctx->stream));
+    CK(ctx, cudaStreamSynchronize(ctx->stream));
+    sc->aux->worker = std::thread([a = sc->aux.get(), c = ctx, dst = sc->d_blob, L, delay_ms] {
+        try {
+            if (delay_ms > 0) std::this_thread::sleep_for(std::chrono::milliseconds(delay_ms));
+            AuxTables t;
+            if (!build_ref_tables(a->boxes, a->pid_of_world, a, &t, &a->err)) {
+                a->state.store(-1, std::memory_order_release);
+                return;
+            }
+            static const int one = 1;
+            cudaError_t e = cudaSetDevice(c->device);
+            if (e == cudaSuccess) e = cudaMemcpyAsync(dst + L.rank, t.rank.data(), t.rank.size() * 4, cudaMemcpyHostToDevice, c->aux_stream);
+            if (e == cudaSuccess) e = cudaMemcpyAsync(dst + L.up, t.up.data(), t.up.size() * 4, cudaMemcpyHostToDevice, c->aux_stream);
+            if (e == cudaSuccess) e = cudaMemcpyAsync(dst + L.refbox, t.refbox.data(), t.refbox.size() * 4, cudaMemcpyHostToDevice, c->aux_stream);
+            if (e == cudaSuccess) e = cudaMemcpyAsync(dst + L.flag, &one, 4, cudaMemcpyHostToDevice, c->aux_stream);
+            if (e == cudaSuccess) e = cudaStreamSynchronize(c->aux_stream);
+            if (e != cudaSuccess) {
+                a->err = std::string("upload of the tie-break tables failed: ") + cudaGetErrorString(e);
+                a->state.store(-1, std::memory_order_release);
+                return;
+            }
+            a->state.store(1, std::memory_order_release);
+        } catch (const std::exception& ex) {
+            a->err = ex.what();
+            a->state.store(-1, std::memory_order_release);
+        } catch (...) {
+            a->err = "unknown exception in the builder thread";
+            a->state.store(-1, std::memory_order_release);
+        }
+    });
+    return RT_OK;
+}
+
+// Geometry, materials, boxes, sphere pairs and big-primitive codes into the staging image h, in pid order.
+void fill_image(uint8_t* h, const BlobLayout& L, const std::vector<PrimRef>& world, const rt_sphere* spheres,
+                const rt_triangle* triangles, uint32_t n_spheres, const std::vector<Box>& boxes,
+                const std::vector<uint32_t>& pid_of_world, const std::vector<uint32_t>& big_world) {
+    const uint32_t n = (uint32_t)world.size();
+    float* h_sph = (float*)(h + L.sph);
+    float* h_tri = (float*)(h + L.tri);
+    float* h_mat = (float*)(h + L.mat);
+    float* h_em = (float*)(h + L.emis);
+    float* h_box = (float*)(h + L.box);
     for (uint32_t w = 0; w < n; w++) {
         const uint32_t pid = pid_of_world[w];
         float* bx = h_box + 8 * (size_t)pid;
@@ -484,7 +380,8 @@ int rt_scene_create(rt_ctx* ctx, const rt_sphere* spheres, uint32_t n_spheres, c
         }
     }
     {   // pair j = spheres 2j, 2j+1: (-c0.x, -c1.x, -c0.y, -c1.y) | (-c0.z, -c1.z, r0^2, r1^2); pads can never pass
-        float* h2 = (float*)(h + o_sph2);
+        const uint32_t ns8 = (n_spheres + 7u) & ~7u;
+        float* h2 = (float*)(h + L.sph2);
         for (uint32_t j = 0; j < ns8 / 2; j++)
             for (uint32_t k = 0; k < 2; k++) {
                 const uint32_t pid = 2 * j + k;
@@ -497,113 +394,235 @@ int rt_scene_create(rt_ctx* ctx, const rt_sphere* spheres, uint32_t n_spheres, c
             }
     }
     for (size_t i = 0; i < (size_t)MAX_BIG; i++)
-        ((int32_t*)(h + o_big))[i] = i < big_world.size() ? ~(int32_t)(pid_of_world[big_world[i]] << 5) : 0;
-    // the flag lives in the late region: inside the staging copy only when the whole blob is uploaded by this call (the
-    // asynchronous path zeroes it on the device above and the builder thread raises it)
-    if (ref_sync) *(int32_t*)(h + o_flag) = 1;
+        ((int32_t*)(h + L.big))[i] = i < big_world.size() ? ~(int32_t)(pid_of_world[big_world[i]] << 5) : 0;
+}
 
-    // traversal-tree records from the host tree: DFS pre-order numbering, left subtree first
-    int32_t lroot = 0;
+// Traversal-tree records of the host tree T into ln (DFS pre-order numbering, left subtree first); returns the root
+// code.  Without T: a single primitive in the tree (rest_world) is the root leaf itself; otherwise the tree is empty or
+// built on the device (its root is node 0) and the root code is 0.
+int32_t emit_nodes(uint8_t* ln, const HostBVH* T, const std::vector<uint32_t>& rest_world,
+                   const std::vector<uint32_t>& pid_of_world) {
     auto leaf_code = [&](int32_t world_code) { return ~(int32_t)(pid_of_world[(uint32_t)~world_code] << 5); };
-    if (device_tree) {
-        lroot = 0;  // nodes 0 .. n-2 are written on the device after the upload; the root is node 0
-    } else if (T) {
-        float* ln = (float*)(h + o_ln);
-        int32_t* lc = (int32_t*)(h + o_ln);  // the same records: words 12, 13 are the child codes
-        struct Item { int32_t code; uint32_t parent; int side; };
-        std::vector<Item> todo;
-        uint32_t next = 0;
-        todo.push_back(Item{T->root, 0, -1});
-        while (!todo.empty()) {
-            const Item it = todo.back();
-            todo.pop_back();
-            const uint32_t me = next++;
-            if (it.side < 0) lroot = (int32_t)me * NODE_BYTES;
-            else lc[NODE_WORDS * (size_t)it.parent + 12 + it.side] = (int32_t)me * NODE_BYTES;
-            const HostNode& hn = T->inner[(size_t)it.code];
-            float lcn[3], lhh[3], rcn[3], rhh[3];
-            centre_half_of(hn.box_l, lcn, lhh);
-            centre_half_of(hn.box_r, rcn, rhh);
-            float* pa = ln + NODE_WORDS * (size_t)me;
-            node_box_words(lcn, lhh, rcn, rhh, pa);
-            for (int k = 14; k < NODE_WORDS; k++) lc[NODE_WORDS * (size_t)me + k] = 0;
-            const int32_t kids[2] = {hn.left, hn.right};
-            for (int side = 1; side >= 0; side--) {  // push right first so the left subtree is numbered first
-                if (kids[side] < 0) {
-                    lc[NODE_WORDS * (size_t)me + 12 + side] = leaf_code(kids[side]);
-                } else {
-                    todo.push_back(Item{kids[side], me, side});
-                }
+    if (!T) return rest_world.size() == 1 ? leaf_code(~(int32_t)rest_world[0]) : 0;
+    int32_t* lc = (int32_t*)ln;  // the same records: words 12, 13 are the child codes
+    struct Item { int32_t code; uint32_t parent; int side; };
+    std::vector<Item> todo;
+    uint32_t next = 0;
+    int32_t lroot = 0;
+    todo.push_back(Item{T->root, 0, -1});
+    while (!todo.empty()) {
+        const Item it = todo.back();
+        todo.pop_back();
+        const uint32_t me = next++;
+        if (it.side < 0) lroot = (int32_t)me * NODE_BYTES;
+        else lc[NODE_WORDS * (size_t)it.parent + 12 + it.side] = (int32_t)me * NODE_BYTES;
+        const HostNode& hn = T->inner[(size_t)it.code];
+        float lcn[3], lhh[3], rcn[3], rhh[3];
+        centre_half(hn.box_l.min, hn.box_l.max, lcn, lhh);
+        centre_half(hn.box_r.min, hn.box_r.max, rcn, rhh);
+        node_box_words(lcn, lhh, rcn, rhh, (float*)ln + NODE_WORDS * (size_t)me);
+        for (int k = 14; k < NODE_WORDS; k++) lc[NODE_WORDS * (size_t)me + k] = 0;
+        const int32_t kids[2] = {hn.left, hn.right};
+        for (int side = 1; side >= 0; side--) {  // push right first so the left subtree is numbered first
+            if (kids[side] < 0) {
+                lc[NODE_WORDS * (size_t)me + 12 + side] = leaf_code(kids[side]);
+            } else {
+                todo.push_back(Item{kids[side], me, side});
             }
         }
-    } else if (ltree) {  // a single primitive in the tree: the root is its leaf
-        lroot = leaf_code(~(int32_t)rest_world[0]);
     }
-    if (ref_sync) {
-        memcpy(h + o_rank, ref_tables.rank.data(), ref_tables.rank.size() * 4);
-        memcpy(h + o_up, ref_tables.up.data(), ref_tables.up.size() * 4);
-        memcpy(h + o_refbox, ref_tables.refbox.data(), ref_tables.refbox.size() * 4);
-    }
+    return lroot;
+}
 
+// The staging image's first stage_bytes to the device blob, then, with device_tree, the LBVH over `rest` into the
+// node-record region (which the staging image leaves out).  The staging buffer is free again on return; on an error the
+// caller still owns the blob.
+int upload(rt_ctx* ctx, rt_scene* sc, const uint8_t* h, const BlobLayout& L, size_t stage_bytes, bool device_tree,
+           const std::vector<Box>& rest, const std::vector<uint32_t>& rest_world, const std::vector<uint32_t>& pid_of_world) {
     cudaError_t e;
-    const size_t ln_end = align_up(o_ln + (size_t)lni * NODE_BYTES, 256);
-    if (device_tree && ln_end < stage_bytes) {
-        // the node records are written on the device: nothing of that region is in the staging copy (4 MB at 65,536)
-        e = o_ln ? cudaMemcpyAsync(sc->d_blob, h, o_ln, cudaMemcpyHostToDevice, ctx->stream) : cudaSuccess;
+    if (device_tree) {  // 4 MB of node records at 65,536 primitives are not copied
+        e = cudaMemcpyAsync(sc->d_blob, h, L.lnode, cudaMemcpyHostToDevice, ctx->stream);
         if (e == cudaSuccess)
-            e = cudaMemcpyAsync(sc->d_blob + ln_end, h + ln_end, stage_bytes - ln_end, cudaMemcpyHostToDevice, ctx->stream);
+            e = cudaMemcpyAsync(sc->d_blob + L.sph2, h + L.sph2, stage_bytes - L.sph2, cudaMemcpyHostToDevice, ctx->stream);
     } else {
         e = cudaMemcpyAsync(sc->d_blob, h, stage_bytes, cudaMemcpyHostToDevice, ctx->stream);
     }
     if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);  // the staging buffer is reused by the next scene
-    if (e != cudaSuccess) {
-        give_back();
-        return set_err(ctx, RT_ERR_CUDA, "scene upload failed: %s", cudaGetErrorString(e));
-    }
-    if (device_tree) {
-        std::vector<float> dev_boxes(6 * rest.size());
-        std::vector<uint32_t> dev_pid(rest.size());
-        for (size_t i = 0; i < rest.size(); i++) {
-            for (int a = 0; a < 3; a++) {
-                dev_boxes[6 * i + a] = rest[i].min[a];
-                dev_boxes[6 * i + 3 + a] = rest[i].max[a];
-            }
-            dev_pid[i] = pid_of_world[rest_world[i]];
-        }
-        uint32_t depth = 0;
-        e = build_lbvh_device(&ctx->dbuild, dev_boxes.data(), dev_pid.data(), (uint32_t)dev_pid.size(),
-                              (float4*)(sc->d_blob + o_ln), &depth, ctx->stream);
-        if (e != cudaSuccess || depth > (uint32_t)MAX_STACK) {
-            give_back();
-            if (e != cudaSuccess) return set_err(ctx, RT_ERR_CUDA, "device BVH build failed: %s", cudaGetErrorString(e));
-            return set_err(ctx, RT_ERR_UNSUPPORTED, "device-built tree depth %u exceeds the traversal stack (%d)", depth, MAX_STACK);
-        }
-        sc->tree_depth = depth;
-        sc->device_tree = true;
-    }
-    if (ref_sync) aux->state.store(1, std::memory_order_release);
+    if (e != cudaSuccess) return set_err(ctx, RT_ERR_CUDA, "scene upload failed: %s", cudaGetErrorString(e));
+    if (!device_tree) return RT_OK;
+    std::vector<uint32_t> dev_pid(rest.size());
+    for (size_t i = 0; i < rest.size(); i++) dev_pid[i] = pid_of_world[rest_world[i]];
+    uint32_t depth = 0;
+    e = build_lbvh_device(&ctx->dbuild, rest.data(), dev_pid.data(), (uint32_t)dev_pid.size(),
+                          (float4*)(sc->d_blob + L.lnode), &depth, ctx->stream);
+    if (e != cudaSuccess) return set_err(ctx, RT_ERR_CUDA, "device BVH build failed: %s", cudaGetErrorString(e));
+    if (depth > (uint32_t)MAX_STACK)
+        return set_err(ctx, RT_ERR_UNSUPPORTED, "device-built tree depth %u exceeds the traversal stack (%d)", depth, MAX_STACK);
+    return RT_OK;
+}
 
-    DevScene& d = sc->dev;
-    d.sph = (const float4*)(sc->d_blob + o_sph);
-    d.tri = (const float4*)(sc->d_blob + o_tri);
-    d.lnode = (const float4*)(sc->d_blob + o_ln);
-    d.sph2 = (const float4*)(sc->d_blob + o_sph2);
+DevScene make_dev_scene(const uint8_t* blob, const BlobLayout& L, uint32_t n_spheres, uint32_t n_triangles, uint32_t lni,
+                        int32_t lroot, bool ltree, uint32_t nbig) {
+    DevScene d{};
+    d.sph = (const float4*)(blob + L.sph);
+    d.tri = (const float4*)(blob + L.tri);
+    d.lnode = (const float4*)(blob + L.lnode);
+    d.sph2 = (const float4*)(blob + L.sph2);
     d.lni = lni;
     d.lroot = lroot;
     d.ltree = ltree ? 1 : 0;
-    d.nbig = (uint32_t)big_world.size();
-    d.big_code = (const int*)(sc->d_blob + o_big);
-    d.mat = (const float4*)(sc->d_blob + o_mat);
-    d.emis = (const float*)(sc->d_blob + o_em);
-    d.rank = (const uint32_t*)(sc->d_blob + o_rank);
-    d.leaf_box = (const float4*)(sc->d_blob + o_box);
-    d.ref_up = (const uint32_t*)(sc->d_blob + o_up);
-    d.ref_box = (const float4*)(sc->d_blob + o_refbox);
+    d.nbig = nbig;
+    d.big_code = (const int*)(blob + L.big);
+    d.mat = (const float4*)(blob + L.mat);
+    d.emis = (const float*)(blob + L.emis);
+    d.rank = (const uint32_t*)(blob + L.rank);
+    d.leaf_box = (const float4*)(blob + L.box);
+    d.ref_up = (const uint32_t*)(blob + L.up);
+    d.ref_box = (const float4*)(blob + L.refbox);
     d.aux_ready = 0;
-    d.aux_flag = (const int*)(sc->d_blob + o_flag);
+    d.aux_flag = (const int*)(blob + L.flag);
     d.ns = n_spheres;
     d.nt = n_triangles;
-    d.ni = ni_ref;
+    d.ni = n_spheres + n_triangles - 1;
+    return d;
+}
+
+}  // namespace
+
+namespace rtb {
+
+int scene_settle(rt_ctx* ctx, const rt_scene* scene) {
+    rt_aux* aux = scene->aux.get();
+    if (!aux) return RT_OK;
+    if (aux->worker.joinable()) aux->worker.join();
+    if (aux->state.load(std::memory_order_acquire) < 0) return set_err(ctx, RT_ERR_BVH, "BVH build failed: %s", aux->err.c_str());
+    return RT_OK;
+}
+
+DevScene scene_view(const rt_scene* scene) {
+    DevScene d = scene->dev;
+    d.aux_ready = (!scene->aux || scene->aux->state.load(std::memory_order_acquire) == 1) ? 1 : 0;
+    return d;
+}
+
+}  // namespace rtb
+
+extern "C" {
+
+int rt_bvh_build_host(const rt_sphere* spheres, uint32_t n_spheres, const rt_triangle* triangles, uint32_t n_triangles,
+                      const uint32_t* world_index, uint32_t* rank_out, uint32_t* n_nodes, uint32_t* depth) {
+    RT_GUARD_BEGIN
+    const uint64_t n64 = (uint64_t)n_spheres + n_triangles;
+    if (n64 == 0) return RT_ERR_EMPTY_SCENE;
+    if (n64 > MAX_PRIMS) return RT_ERR_UNSUPPORTED;
+    if ((n_spheres && !spheres) || (n_triangles && !triangles)) return RT_ERR_INVALID_ARG;
+    std::vector<PrimRef> world;
+    std::vector<Box> boxes;
+    std::string err;
+    int rc = world_and_boxes(spheres, n_spheres, triangles, n_triangles, world_index, &world, &boxes, &err);
+    HostBVH bvh;
+    if (rc == RT_OK && !build_bvh(boxes, &bvh, &err)) {
+        err = "BVH build failed: " + err;
+        rc = RT_ERR_BVH;
+    }
+    if (rc) return set_err(nullptr, rc, "%s", err.c_str());
+    if (rank_out)
+        for (uint32_t r = 0; r < (uint32_t)n64; r++) rank_out[bvh.leaf_order[r]] = r;
+    if (n_nodes) *n_nodes = bvh.node_count;
+    if (depth) *depth = bvh.depth;
+    return RT_OK;
+    RT_GUARD_END(nullptr)
+}
+
+int rt_scene_create(rt_ctx* ctx, const rt_sphere* spheres, uint32_t n_spheres, const rt_triangle* triangles,
+                    uint32_t n_triangles, const uint32_t* world_index, rt_scene** out) {
+    if (!ctx) return RT_ERR_INVALID_ARG;
+    RT_GUARD_BEGIN
+    if (!out) return set_err(ctx, RT_ERR_INVALID_ARG, "rt_scene_create: out is NULL");
+    *out = nullptr;
+    const uint64_t n64 = (uint64_t)n_spheres + n_triangles;
+    if (n64 == 0)
+        return set_err(ctx, RT_ERR_EMPTY_SCENE,
+                       "empty world: the reference's BVHNode::build never terminates on zero shapes");
+    // inner codes are the byte offset of a 64-byte node record and must stay positive (n - 1 records: 25 bits of nodes)
+    if (n64 > MAX_PRIMS || (n64 - 1) * (uint64_t)NODE_BYTES > 0x7fffffffull)
+        return set_err(ctx, RT_ERR_UNSUPPORTED, "too many primitives (%llu; this build addresses %llu)", (unsigned long long)n64,
+                       (unsigned long long)(0x7fffffffull / NODE_BYTES + 1));
+    if ((n_spheres && !spheres) || (n_triangles && !triangles))
+        return set_err(ctx, RT_ERR_INVALID_ARG, "rt_scene_create: NULL primitive array");
+    const uint32_t n = (uint32_t)n64;
+    const TestHooks& hooks = test_hooks();
+
+    static std::atomic<uint64_t> next_serial{1};
+    std::unique_ptr<rt_scene> sc(new rt_scene());
+    sc->ctx = ctx;
+    sc->serial = next_serial++;
+    sc->n = n;
+    sc->aux.reset(new rt_aux());
+    rt_aux* aux = sc->aux.get();
+    std::vector<PrimRef> world;
+    std::string werr;
+    const int wrc = world_and_boxes(spheres, n_spheres, triangles, n_triangles, world_index, &world, &aux->boxes, &werr);
+    if (wrc) return set_err(ctx, wrc, "%s", werr.c_str());
+    const std::vector<Box>& boxes = aux->boxes;  // shared, read-only from here on
+
+    // which tree will be traversed, and who builds it
+    Split split;
+    split_big(boxes, &split);
+    const std::vector<Box>& rest = split.rest(boxes);
+    const bool device_tree = rest.size() >= 2 &&
+                             (hooks.build_mode == 2 || (hooks.build_mode == 1 && rest.size() >= kDeviceBuildMin));
+    HostBVH sah;
+    const HostBVH* T = nullptr;  // the host-built traversal tree (leaf codes: world positions)
+    if (!device_tree && rest.size() >= 2) {
+        const int rc = host_traversal_tree(ctx, rest, split.rest_world, &sah);
+        if (rc) return rc;
+        T = &sah;
+    }
+    assign_pids(world, n_spheres, T, &aux->pid_of_world);
+    const std::vector<uint32_t>& pid_of_world = aux->pid_of_world;
+
+    // the reference tree: inline for small scenes, else on the builder thread below
+    const bool ref_sync = n < kRefSyncBelow;
+    AuxTables ref_tables;
+    if (ref_sync) {
+        std::string berr;
+        if (!build_ref_tables(boxes, pid_of_world, aux, &ref_tables, &berr))
+            return set_err(ctx, RT_ERR_BVH, "BVH build failed: %s", berr.c_str());
+    }
+
+    const uint32_t lni = device_tree ? (uint32_t)rest.size() - 1 : T ? (uint32_t)T->inner.size() : 0;
+    const BlobLayout L = blob_layout(n_spheres, n_triangles, lni);
+    sc->blob_bytes = L.blob_bytes;
+    const size_t stage_bytes = ref_sync ? L.blob_bytes : L.sync_bytes;
+    CK(ctx, cudaSetDevice(ctx->device));
+    CK(ctx, reserve_stage(ctx, stage_bytes));
+    CK(ctx, take_blob(ctx, L.blob_bytes, &sc->d_blob, &sc->blob_cap));
+    // the builder thread starts now, with pid_of_world final: it overlaps the fill and the upload
+    if (!ref_sync) {
+        const int rc = start_ref_builder(ctx, sc.get(), L, hooks.aux_delay_ms);
+        if (rc) return rc;
+    }
+
+    uint8_t* const h = ctx->h_stage;
+    fill_image(h, L, world, spheres, triangles, n_spheres, boxes, pid_of_world, split.big_world);
+    const int32_t lroot = emit_nodes(h + L.lnode, T, split.rest_world, pid_of_world);
+    if (ref_sync) {  // the whole blob is uploaded by this call: the tables and the raised flag go with it
+        memcpy(h + L.rank, ref_tables.rank.data(), ref_tables.rank.size() * 4);
+        memcpy(h + L.up, ref_tables.up.data(), ref_tables.up.size() * 4);
+        memcpy(h + L.refbox, ref_tables.refbox.data(), ref_tables.refbox.size() * 4);
+        *(int32_t*)(h + L.flag) = 1;
+    }
+    const int rc = upload(ctx, sc.get(), h, L, stage_bytes, device_tree, rest, split.rest_world, pid_of_world);
+    if (rc) {  // the builder thread may still write to the blob
+        if (aux->worker.joinable()) aux->worker.join();
+        retire_blob(ctx, sc->d_blob, sc->blob_cap);
+        return rc;
+    }
+    if (ref_sync) aux->state.store(1, std::memory_order_release);
+
+    sc->dev = make_dev_scene(sc->d_blob, L, n_spheres, n_triangles, lni, lroot, !rest.empty(),
+                             (uint32_t)split.big_world.size());
     *out = sc.release();
     return RT_OK;
     RT_GUARD_END(ctx)
@@ -617,10 +636,7 @@ void rt_scene_destroy(rt_ctx* ctx, rt_scene* scene) {
         cudaStreamSynchronize(ctx->stream);
         cudaStreamSynchronize(ctx->copy_stream);
     }
-    if (scene->d_blob) {
-        if (ctx && ctx->retired.size() < 4) ctx->retired.push_back({scene->d_blob, scene->blob_cap});
-        else cudaFree(scene->d_blob);
-    }
+    if (scene->d_blob) retire_blob(ctx, scene->d_blob, scene->blob_cap);
     delete scene;
 }
 
