@@ -147,6 +147,21 @@ const char* rt_last_error(const rt_ctx* ctx);
 int rt_scene_create(rt_ctx* ctx, const rt_sphere* spheres, uint32_t n_spheres, const rt_triangle* triangles,
                     uint32_t n_triangles, const uint32_t* world_index, rt_scene** out);
 void rt_scene_destroy(rt_ctx* ctx, rt_scene* scene);
+/* Replaces the primitives of `scene` with a world of the same shape: n_spheres and n_triangles as created, the
+ * world_index given at creation still applies.  Geometry, materials and emission may all change.  Renders queued on
+ * ctx before the call see the old world, renders after it the new one, byte-identical to a scene created from it.
+ * The traversal tree keeps its topology and is refitted to the new boxes on the device (a tree that motion has made
+ * loose costs time, never correctness; re-create the scene to rebuild it); when no primitive's box changes (materials
+ * only) only the primitive data is uploaded.  The reference-topology tree is rebuilt as by rt_scene_create, beside the
+ * upload from 256 primitives on; a failure of that build is reported by rt_scene_wait_ready, rt_scene_info or a render
+ * that needs it.  rt_scene_info then reports the new world; rt_scene_device_bytes does not change.
+ * Every successful update gives the scene a new serial: an rt_accum with samples of the old world refuses it
+ * (RT_ERR_INVALID_ARG from rt_render_samples) until rt_accum_reset.
+ * RT_ERR_INVALID_ARG: NULL ctx or scene, a scene of another context, counts other than the creation counts, a NULL array
+ * with a nonzero count.  RT_ERR_BVH: non-finite geometry or bounds.  On either the scene is untouched and still renders
+ * the old world.  RT_ERR_CUDA leaves the scene undefined: destroy it. */
+int rt_scene_update(rt_ctx* ctx, rt_scene* scene, const rt_sphere* spheres, uint32_t n_spheres,
+                    const rt_triangle* triangles, uint32_t n_triangles);
 /* rt_scene_create returns as soon as the geometry and the tree the kernels traverse are on the device.  The reference-
  * topology tree (bvh_impl.rs:229-364), which only decides exact-distance ties and the fate of rays with a zero direction
  * component, is finished by a builder thread; renders started before it lands are correct all the same (the few pixels

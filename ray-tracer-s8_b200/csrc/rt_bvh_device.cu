@@ -1,5 +1,7 @@
-// rt_bvh_device.cu — device-side build of the TRAVERSAL tree (SURVEY.md §8f row f3): Morton-code LBVH
-// (Karras 2012: one thread per inner node finds its key range and split from common prefixes) + bottom-up refit.
+// rt_bvh_device.cu — device-side build and refit of the TRAVERSAL tree (SURVEY.md §8f row f3): Morton-code LBVH
+// (Karras 2012: one thread per inner node finds its key range and split from common prefixes) + bottom-up refit.  The
+// refit reads nothing but the scene blob (child codes of the node records, exact leaf boxes), so it serves any tree in
+// it: the LBVH below, and rt_scene_update's refit of a host-built or device-built tree to moved primitives.
 //
 // What it replaces: the host's 3-axis binned-SAH build of the product kernels' culling tree (rt_bvh_host.cpp,
 // build_bvh_sah), serial O(N log N) — 42 ms at 65,536 spheres against a 3 ms frame.  What it does NOT replace: the
@@ -10,10 +12,11 @@
 // Pipeline (one stream, no host round trip except the depth check):
 //   morton_keys   key = 30-bit Morton code of the box centre (10 bits per axis inside the centroid bounds) << 32 | i
 //   radix sort    cub::DeviceRadixSort::SortKeys on the 62 significant bits (library sort: not a path kernel)
-//   karras_nodes  inner node i ↔ keys [first,last], split by the highest differing bit; children + parents
-//   refit         one thread per leaf walks up; the second arrival at a node joins its two child boxes, writes the
-//                 node record (centre / half-extent form: centre_half, as on the host) and goes on
-//   leaf_depths   deepest leaf, for the traversal stack bound (MAX_STACK)
+//   karras_nodes  inner node i ↔ keys [first,last], split by the highest differing bit; the child codes of record i
+//   link_nodes    parents of every record's children, from the child codes           (refit from here on)
+//   refit_nodes   one thread per leaf walks up; the second arrival at a node joins its two child boxes, writes the
+//                 node record's boxes (centre / half-extent form: centre_half, as on the host) and goes on
+//   leaf_depths   deepest leaf, for the traversal stack bound (MAX_STACK)               (build only)
 #include <cub/device/device_radix_sort.cuh>
 
 #include <cstdlib>
@@ -52,9 +55,10 @@ __device__ __forceinline__ int delta(const unsigned long long* keys, int n, int 
 }
 
 // Karras 2012, Algorithm "construct binary radix tree": inner node i (0 = root) covers sorted keys [first, last].
-// Children: index < n-1 → inner node, else leaf (sorted position = index - (n-1)).
-__global__ void karras_nodes(const unsigned long long* __restrict__ keys, int n, int2* __restrict__ child,
-                             int* __restrict__ parent /* [2n-1]: inner nodes then leaves */) {
+// Children: index < n-1 → inner node, else leaf (sorted position = index - (n-1)).  Writes the child codes of record i
+// (inner: the byte offset of its record; leaf: ~(pid << 5), one primitive per leaf); refit_nodes fills in the boxes.
+__global__ void karras_nodes(const unsigned long long* __restrict__ keys, const uint32_t* __restrict__ pid_of, int n,
+                             int4* __restrict__ lnode4) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n - 1) return;
     const int d = (delta(keys, n, i, i + 1) - delta(keys, n, i, i - 1)) >= 0 ? 1 : -1;
@@ -75,52 +79,62 @@ __global__ void karras_nodes(const unsigned long long* __restrict__ keys, int n,
     const int lo = min(i, j), hi = max(i, j);
     const int left = (lo == gamma) ? (n - 1 + gamma) : gamma;
     const int right = (hi == gamma + 1) ? (n - 1 + gamma + 1) : gamma + 1;
-    child[i] = make_int2(left, right);
-    parent[left] = i;
-    parent[right] = i;
-    if (i == 0) parent[0] = -1;
+    auto code = [&](int c) {
+        return c < n - 1 ? c * NODE_BYTES : ~(int)(pid_of[(uint32_t)(keys[c - (n - 1)] & 0xffffffffull)] << 5);
+    };
+    lnode4[NODE_F4 * (size_t)i + 3] = make_int4(code(left), code(right), 0, 0);
 }
 
 struct B6 {
     float lo[3], hi[3];
 };
 
-__global__ void refit(const unsigned long long* __restrict__ keys, const float* __restrict__ boxes,
-                      const uint32_t* __restrict__ pid_of, int n, const int2* __restrict__ child,
-                      const int* __restrict__ parent, unsigned int* __restrict__ arrived, B6* nbox,
-                      float4* __restrict__ lnode) {
-    const int p = blockIdx.x * blockDim.x + threadIdx.x;
-    if (p >= n) return;
-    int node = parent[n - 1 + p];
+// The parents of every record's children, from the child codes (words 12, 13 of the record): parent[node] for inner
+// children, leaf_parent[pid] for leaves.  What no record names keeps the -1 it was set to: the root, big primitives.
+__global__ void link_nodes(const int4* __restrict__ lnode4, uint32_t lni, int* __restrict__ parent,
+                           int* __restrict__ leaf_parent) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= lni) return;
+    const int4 ch = lnode4[NODE_F4 * (size_t)i + 3];
+    for (const int c : {ch.x, ch.y}) {
+        if (c >= 0) parent[c / NODE_BYTES] = (int)i;
+        else leaf_parent[(uint32_t)~c >> 5] = (int)i;
+    }
+}
+
+// One thread per primitive walks up from its leaf; the second arrival at a node joins its two child boxes (leaves: the
+// exact AABB leaf_box[pid]), writes the node record's boxes (centre / half-extent form: centre_half, as on the host)
+// and goes on.  The child codes of the records stay as they are.
+__global__ void refit_nodes(const float4* __restrict__ leaf_box, uint32_t n_prims, const int* __restrict__ parent,
+                            const int* __restrict__ leaf_parent, unsigned int* __restrict__ arrived, B6* nbox,
+                            float4* __restrict__ lnode) {
+    const uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= n_prims) return;
+    int node = leaf_parent[p];
     while (node >= 0) {
         __threadfence();
         if (atomicAdd(&arrived[node], 1u) == 0u) return;  // the sibling subtree is not finished: its thread goes on
         __threadfence();
-        const int2 ch = child[node];
+        const int4 ch = reinterpret_cast<const int4*>(lnode)[NODE_F4 * (size_t)node + 3];
         B6 bl, br;
-        int cl, cr;
-        auto fetch = [&](int c, B6* out, int* code) {
-            if (c >= n - 1) {
-                const uint32_t id = (uint32_t)(keys[c - (n - 1)] & 0xffffffffull);
-                const float* b = boxes + 6 * (size_t)id;
-                for (int a = 0; a < 3; a++) {
-                    out->lo[a] = b[a];
-                    out->hi[a] = b[3 + a];
-                }
-                *code = ~(int)((pid_of[id] << 5) | 0u);  // one primitive per leaf
+        auto fetch = [&](int c, B6* out) {
+            if (c < 0) {
+                const uint32_t pid = (uint32_t)~c >> 5;
+                const float4 lo = __ldg(leaf_box + 2 * (size_t)pid), hi = __ldg(leaf_box + 2 * (size_t)pid + 1);
+                out->lo[0] = lo.x; out->lo[1] = lo.y; out->lo[2] = lo.z;
+                out->hi[0] = hi.x; out->hi[1] = hi.y; out->hi[2] = hi.z;
             } else {
                 // written by another SM's thread before its atomicAdd: read past L1 (a neighbour in the same line may
                 // have been cached earlier in this launch)
-                const float* q = reinterpret_cast<const float*>(nbox + c);
+                const float* q = reinterpret_cast<const float*>(nbox + c / NODE_BYTES);
                 for (int a = 0; a < 3; a++) {
                     out->lo[a] = __ldcg(q + a);
                     out->hi[a] = __ldcg(q + 3 + a);
                 }
-                *code = c;
             }
         };
-        fetch(ch.x, &bl, &cl);
-        fetch(ch.y, &br, &cr);
+        fetch(ch.x, &bl);
+        fetch(ch.y, &br);
         float lc[3], lh[3], rc[3], rh[3];
         centre_half(bl.lo, bl.hi, lc, lh);
         centre_half(br.lo, br.hi, rc, rh);
@@ -129,10 +143,6 @@ __global__ void refit(const unsigned long long* __restrict__ keys, const float* 
         lnode[NODE_F4 * (size_t)node + 0] = make_float4(w[0], w[1], w[2], w[3]);
         lnode[NODE_F4 * (size_t)node + 1] = make_float4(w[4], w[5], w[6], w[7]);
         lnode[NODE_F4 * (size_t)node + 2] = make_float4(w[8], w[9], w[10], w[11]);
-        // inner children by the byte offset of their record (rt_device.cuh)
-        reinterpret_cast<int4*>(lnode)[NODE_F4 * (size_t)node + 3] =
-            make_int4(cl >= 0 ? cl * NODE_BYTES : cl, cr >= 0 ? cr * NODE_BYTES : cr, 0, 0);
-        for (int k = 4; k < NODE_F4; k++) lnode[NODE_F4 * (size_t)node + k] = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
         B6 u;
         for (int a = 0; a < 3; a++) {
             u.lo[a] = fminf(bl.lo[a], br.lo[a]);
@@ -143,16 +153,65 @@ __global__ void refit(const unsigned long long* __restrict__ keys, const float* 
     }
 }
 
-__global__ void leaf_depths(const int* __restrict__ parent, int n, unsigned int* __restrict__ max_depth) {
-    const int p = blockIdx.x * blockDim.x + threadIdx.x;
+__global__ void leaf_depths(const int* __restrict__ parent, const int* __restrict__ leaf_parent, uint32_t n_prims,
+                            unsigned int* __restrict__ max_depth) {
+    const uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
     unsigned int d = 0;
-    if (p < n)
-        for (int node = parent[n - 1 + p]; node >= 0; node = parent[node]) d++;
+    if (p < n_prims)
+        for (int node = leaf_parent[p]; node >= 0; node = parent[node]) d++;
     for (int ofs = 16; ofs > 0; ofs >>= 1) d = max(d, __shfl_xor_sync(0xffffffffu, d, ofs));
     if ((threadIdx.x & 31) == 0 && d) atomicMax(max_depth, d);
 }
 
 size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
+
+// Sections of the one scratch allocation, 256-byte aligned.
+struct Carve {
+    size_t off = 0;
+    size_t take(size_t bytes) {
+        const size_t o = off;
+        off = align256(off + bytes);
+        return o;
+    }
+};
+
+// The refit's scratch: parent | leaf_parent (adjacent: one reset to -1) | arrival counters + the deepest leaf | unions.
+struct RefitScratch {
+    size_t parent, leaf_parent, arrived, nbox;
+    RefitScratch(Carve* c, uint32_t n_prims, uint32_t lni)
+        : parent(c->take((size_t)lni * 4)), leaf_parent(c->take((size_t)n_prims * 4)), arrived(c->take((size_t)lni * 4 + 4)),
+          nbox(c->take((size_t)lni * sizeof(B6))) {}
+};
+
+// The scratch buffer holds at least `bytes` (power-of-two size classes, >= 1 MB).
+cudaError_t reserve(DeviceBuild* buf, size_t bytes, cudaStream_t stream) {
+    if (buf->bytes >= bytes) return cudaSuccess;
+    cudaStreamSynchronize(stream);
+    free_device_build(buf);
+    size_t cap = (size_t)1 << 20;
+    while (cap < bytes) cap <<= 1;
+    const cudaError_t e = cudaMalloc(&buf->mem, cap);
+    if (e == cudaSuccess) buf->bytes = cap;
+    return e;
+}
+
+// Refit of the lni records at lnode to the leaf boxes; with want_depth, the deepest leaf goes to the word after the
+// arrival counters too.  Queued on `stream`.
+cudaError_t run_refit(uint8_t* m, const RefitScratch& r, const float4* leaf_box, uint32_t n_prims, float4* lnode,
+                      uint32_t lni, bool want_depth, cudaStream_t stream) {
+    int* parent = (int*)(m + r.parent);
+    int* leaf_parent = (int*)(m + r.leaf_parent);
+    unsigned int* arrived = (unsigned int*)(m + r.arrived);
+    cudaError_t e = cudaMemsetAsync(parent, 0xff, r.leaf_parent - r.parent + (size_t)n_prims * 4, stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(arrived, 0, (size_t)lni * 4 + 4, stream);
+    if (e != cudaSuccess) return e;
+    const unsigned T = 256;
+    link_nodes<<<(lni + T - 1) / T, T, 0, stream>>>((const int4*)lnode, lni, parent, leaf_parent);
+    refit_nodes<<<(n_prims + T - 1) / T, T, 0, stream>>>(leaf_box, n_prims, parent, leaf_parent, arrived,
+                                                         (B6*)(m + r.nbox), lnode);
+    if (want_depth) leaf_depths<<<(n_prims + T - 1) / T, T, 0, stream>>>(parent, leaf_parent, n_prims, arrived + lni);
+    return cudaGetLastError();
+}
 
 }  // namespace
 
@@ -161,12 +220,13 @@ void free_device_build(DeviceBuild* b) {
     *b = DeviceBuild();
 }
 
-// h_boxes: the boxes of the n primitives the tree covers (host); pid_of: their primitive ids (host).
-// Writes n - 1 node records to lnode (device); the root is node 0.
-// *depth_out = deepest leaf.
+// h_boxes: the boxes of the n primitives the tree covers (host); pid_of: their primitive ids (host).  leaf_box (device,
+// n_prims pairs min | max by pid) must hold their boxes already.  Writes n - 1 node records to lnode (device); the root is
+// node 0.  *depth_out = deepest leaf.
 static_assert(sizeof(Box) == 6 * sizeof(float), "the kernels read a Box as min xyz | max xyz");
 cudaError_t build_lbvh_device(DeviceBuild* buf, const Box* h_boxes, const uint32_t* h_pid_of, uint32_t n,
-                              float4* lnode, uint32_t* depth_out, cudaStream_t stream) {
+                              const float4* leaf_box, uint32_t n_prims, float4* lnode, uint32_t* depth_out,
+                              cudaStream_t stream) {
     if (n < 2) return cudaErrorInvalidValue;
     // centroid bounds on the host: one pass over data the host already holds
     float cmin[3] = {3.0e38f, 3.0e38f, 3.0e38f}, cmax[3] = {-3.0e38f, -3.0e38f, -3.0e38f};
@@ -185,47 +245,41 @@ cudaError_t build_lbvh_device(DeviceBuild* buf, const Box* h_boxes, const uint32
     cudaError_t e = cub::DeviceRadixSort::SortKeys(nullptr, sort_bytes, (const unsigned long long*)nullptr,
                                                    (unsigned long long*)nullptr, (int)n, 0, 62, stream);
     if (e != cudaSuccess) return e;
-    // one allocation: boxes | pid_of | keys in | keys out | child | parent | arrived + depth | node boxes | sort scratch
-    size_t off = 0;
-    auto take = [&](size_t bytes) {
-        const size_t o = off;
-        off = align256(off + bytes);
-        return o;
-    };
-    const size_t o_box = take((size_t)n * 24), o_pid = take((size_t)n * 4), o_k0 = take((size_t)n * 8),
-                 o_k1 = take((size_t)n * 8), o_child = take((size_t)(n - 1) * 8), o_parent = take((size_t)(2 * n - 1) * 4),
-                 o_arr = take((size_t)n * 4 + 4), o_nbox = take((size_t)(n - 1) * sizeof(B6)), o_sort = take(sort_bytes);
-    if (buf->bytes < off) {
-        cudaStreamSynchronize(stream);
-        free_device_build(buf);
-        size_t cap = (size_t)1 << 20;
-        while (cap < off) cap <<= 1;
-        if ((e = cudaMalloc(&buf->mem, cap)) != cudaSuccess) return e;
-        buf->bytes = cap;
-    }
+    // one allocation: boxes | pid_of | keys in | keys out | sort scratch | the refit's scratch
+    Carve c;
+    const size_t o_box = c.take((size_t)n * 24), o_pid = c.take((size_t)n * 4), o_k0 = c.take((size_t)n * 8),
+                 o_k1 = c.take((size_t)n * 8), o_sort = c.take(sort_bytes);
+    const RefitScratch r(&c, n_prims, n - 1);
+    if ((e = reserve(buf, c.off, stream)) != cudaSuccess) return e;
     uint8_t* m = (uint8_t*)buf->mem;
     float* d_boxes = (float*)(m + o_box);
     uint32_t* d_pid = (uint32_t*)(m + o_pid);
     unsigned long long* k0 = (unsigned long long*)(m + o_k0);
     unsigned long long* k1 = (unsigned long long*)(m + o_k1);
-    int2* d_child = (int2*)(m + o_child);
-    int* d_parent = (int*)(m + o_parent);
-    unsigned int* d_arr = (unsigned int*)(m + o_arr);
-    B6* d_nbox = (B6*)(m + o_nbox);
     if ((e = cudaMemcpyAsync(d_boxes, h_boxes, (size_t)n * sizeof(Box), cudaMemcpyHostToDevice, stream)) != cudaSuccess) return e;
     if ((e = cudaMemcpyAsync(d_pid, h_pid_of, (size_t)n * 4, cudaMemcpyHostToDevice, stream)) != cudaSuccess) return e;
-    if ((e = cudaMemsetAsync(d_arr, 0, (size_t)n * 4 + 4, stream)) != cudaSuccess) return e;
     const unsigned T = 256, G = (n + T - 1) / T;
     morton_keys<<<G, T, 0, stream>>>(d_boxes, n, lo, sc, k0);
     if ((e = cub::DeviceRadixSort::SortKeys(m + o_sort, sort_bytes, k0, k1, (int)n, 0, 62, stream)) != cudaSuccess) return e;
-    karras_nodes<<<G, T, 0, stream>>>(k1, (int)n, d_child, d_parent);
-    refit<<<G, T, 0, stream>>>(k1, d_boxes, d_pid, (int)n, d_child, d_parent, d_arr, d_nbox, lnode);
-    leaf_depths<<<G, T, 0, stream>>>(d_parent, (int)n, d_arr + n);
+    karras_nodes<<<G, T, 0, stream>>>(k1, d_pid, (int)n, (int4*)lnode);
+    if ((e = run_refit(m, r, leaf_box, n_prims, lnode, n - 1, true, stream)) != cudaSuccess) return e;
     unsigned int depth = 0;
-    if ((e = cudaMemcpyAsync(&depth, d_arr + n, 4, cudaMemcpyDeviceToHost, stream)) != cudaSuccess) return e;
+    if ((e = cudaMemcpyAsync(&depth, (unsigned int*)(m + r.arrived) + (n - 1), 4, cudaMemcpyDeviceToHost, stream)) != cudaSuccess)
+        return e;
     if ((e = cudaStreamSynchronize(stream)) != cudaSuccess) return e;
     *depth_out = depth;
     return cudaGetLastError();
+}
+
+cudaError_t refit_device(DeviceBuild* buf, const float4* leaf_box, uint32_t n_prims, float4* lnode, uint32_t lni,
+                         cudaStream_t stream) {
+    if (lni == 0) return cudaSuccess;
+    Carve c;
+    const RefitScratch r(&c, n_prims, lni);
+    cudaError_t e = reserve(buf, c.off, stream);
+    if (e == cudaSuccess) e = run_refit((uint8_t*)buf->mem, r, leaf_box, n_prims, lnode, lni, false, stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(stream);
+    return e;
 }
 
 }  // namespace rtb

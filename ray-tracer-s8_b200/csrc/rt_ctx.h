@@ -75,7 +75,7 @@ struct rt_aux {
     std::thread worker;
     std::atomic<int> state{0};  // 0 running, 1 tables on the device, -1 failed
     std::string err;
-    // inputs (owned)
+    // inputs (owned; rt_scene_update replaces boxes once the thread has been joined)
     std::vector<rtb::Box> boxes;            // by world position
     std::vector<uint32_t> pid_of_world;
     // outputs
@@ -90,7 +90,11 @@ struct rt_scene {
     rtb::DevScene dev{};
     uint32_t n = 0;
     std::unique_ptr<rt_aux> aux;
-    uint64_t serial = 0;  // unique per process (rt_scene_create): a re-created scene may reuse a destroyed one's address
+    uint64_t serial = 0;  // unique per process (rt_scene_create, rt_scene_update): a re-created scene may reuse a destroyed
+                          // one's address, an updated one keeps its own
+    // the topology rt_scene_update keeps (the traversal tree's lni / lroot / ltree are in dev)
+    std::vector<uint32_t> world_index;  // as given to rt_scene_create (empty: none)
+    std::vector<uint32_t> big_world;    // world positions of the primitives kept out of the traversal tree
 };
 
 namespace rtb {

@@ -42,7 +42,12 @@ struct DeviceBuild {
 };
 void free_device_build(DeviceBuild* b);
 cudaError_t build_lbvh_device(DeviceBuild* buf, const Box* h_boxes, const uint32_t* h_pid_of, uint32_t n,
-                              float4* lnode, uint32_t* depth_out, cudaStream_t stream);
+                              const float4* leaf_box, uint32_t n_prims, float4* lnode, uint32_t* depth_out,
+                              cudaStream_t stream);
+// The boxes of the lni node records at lnode (any traversal tree of a scene blob: root node 0) recomputed from the leaf
+// boxes leaf_box (n_prims pairs min | max by pid); topology and child codes unchanged.  Returns synchronised.
+cudaError_t refit_device(DeviceBuild* buf, const float4* leaf_box, uint32_t n_prims, float4* lnode, uint32_t lni,
+                         cudaStream_t stream);
 
 // rt_kernels.cu
 cudaError_t preload_kernels();

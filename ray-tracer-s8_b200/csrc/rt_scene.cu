@@ -398,12 +398,9 @@ void fill_image(uint8_t* h, const BlobLayout& L, const std::vector<PrimRef>& wor
 }
 
 // Traversal-tree records of the host tree T into ln (DFS pre-order numbering, left subtree first); returns the root
-// code.  Without T: a single primitive in the tree (rest_world) is the root leaf itself; otherwise the tree is empty or
-// built on the device (its root is node 0) and the root code is 0.
-int32_t emit_nodes(uint8_t* ln, const HostBVH* T, const std::vector<uint32_t>& rest_world,
-                   const std::vector<uint32_t>& pid_of_world) {
+// code.
+int32_t emit_nodes(uint8_t* ln, const HostBVH* T, const std::vector<uint32_t>& pid_of_world) {
     auto leaf_code = [&](int32_t world_code) { return ~(int32_t)(pid_of_world[(uint32_t)~world_code] << 5); };
-    if (!T) return rest_world.size() == 1 ? leaf_code(~(int32_t)rest_world[0]) : 0;
     int32_t* lc = (int32_t*)ln;  // the same records: words 12, 13 are the child codes
     struct Item { int32_t code; uint32_t parent; int side; };
     std::vector<Item> todo;
@@ -434,27 +431,55 @@ int32_t emit_nodes(uint8_t* ln, const HostBVH* T, const std::vector<uint32_t>& r
     return lroot;
 }
 
-// The staging image's first stage_bytes to the device blob, then, with device_tree, the LBVH over `rest` into the
-// node-record region (which the staging image leaves out).  The staging buffer is free again on return; on an error the
-// caller still owns the blob.
-int upload(rt_ctx* ctx, rt_scene* sc, const uint8_t* h, const BlobLayout& L, size_t stage_bytes, bool device_tree,
-           const std::vector<Box>& rest, const std::vector<uint32_t>& rest_world, const std::vector<uint32_t>& pid_of_world) {
+// The part of an ingest that rt_scene_create and rt_scene_update share: aux->boxes and aux->pid_of_world are final and
+// sc->d_blob is laid out as L.  The reference tables are either `inline_tables` (uploaded with the image, the flag
+// raised) or made by the builder thread (start_builder); with neither (an update that leaves every box as it was) the
+// tables already in the blob stay.  Then the staging image is filled and uploaded.  T (nullable): a host-built traversal
+// tree whose records go up with the image, *lroot = its root code; without T no node record crosses PCIe (the device
+// writes them).  The staging buffer is free again on return; on an error the builder thread may still write to the blob.
+int fill_and_upload(rt_ctx* ctx, rt_scene* sc, const BlobLayout& L, const std::vector<PrimRef>& world,
+                    const rt_sphere* spheres, uint32_t n_spheres, const rt_triangle* triangles, const AuxTables* inline_tables,
+                    bool start_builder, const HostBVH* T, int32_t* lroot) {
+    const rt_aux* aux = sc->aux.get();
+    const size_t stage_bytes = inline_tables ? L.blob_bytes : L.sync_bytes;
+    CK(ctx, reserve_stage(ctx, stage_bytes));
+    // the builder thread starts now, with pid_of_world final: it overlaps the fill and the upload
+    if (start_builder) {
+        const int rc = start_ref_builder(ctx, sc, L, test_hooks().aux_delay_ms);
+        if (rc) return rc;
+    }
+    uint8_t* const h = ctx->h_stage;
+    fill_image(h, L, world, spheres, triangles, n_spheres, aux->boxes, aux->pid_of_world, sc->big_world);
+    if (T) *lroot = emit_nodes(h + L.lnode, T, aux->pid_of_world);
+    if (inline_tables) {  // the whole blob is uploaded by this call: the tables and the raised flag go with it
+        memcpy(h + L.rank, inline_tables->rank.data(), inline_tables->rank.size() * 4);
+        memcpy(h + L.up, inline_tables->up.data(), inline_tables->up.size() * 4);
+        memcpy(h + L.refbox, inline_tables->refbox.data(), inline_tables->refbox.size() * 4);
+        *(int32_t*)(h + L.flag) = 1;
+    }
     cudaError_t e;
-    if (device_tree) {  // 4 MB of node records at 65,536 primitives are not copied
+    if (T) {
+        e = cudaMemcpyAsync(sc->d_blob, h, stage_bytes, cudaMemcpyHostToDevice, ctx->stream);
+    } else {  // 4 MB of node records at 65,536 primitives are not copied
         e = cudaMemcpyAsync(sc->d_blob, h, L.lnode, cudaMemcpyHostToDevice, ctx->stream);
         if (e == cudaSuccess)
             e = cudaMemcpyAsync(sc->d_blob + L.sph2, h + L.sph2, stage_bytes - L.sph2, cudaMemcpyHostToDevice, ctx->stream);
-    } else {
-        e = cudaMemcpyAsync(sc->d_blob, h, stage_bytes, cudaMemcpyHostToDevice, ctx->stream);
     }
     if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);  // the staging buffer is reused by the next scene
     if (e != cudaSuccess) return set_err(ctx, RT_ERR_CUDA, "scene upload failed: %s", cudaGetErrorString(e));
-    if (!device_tree) return RT_OK;
+    return RT_OK;
+}
+
+// The LBVH over `rest` into the node-record region of the blob (leaf boxes uploaded already).
+int device_traversal_tree(rt_ctx* ctx, rt_scene* sc, const BlobLayout& L, const std::vector<Box>& rest,
+                          const std::vector<uint32_t>& rest_world) {
+    const std::vector<uint32_t>& pid_of_world = sc->aux->pid_of_world;
     std::vector<uint32_t> dev_pid(rest.size());
     for (size_t i = 0; i < rest.size(); i++) dev_pid[i] = pid_of_world[rest_world[i]];
     uint32_t depth = 0;
-    e = build_lbvh_device(&ctx->dbuild, rest.data(), dev_pid.data(), (uint32_t)dev_pid.size(),
-                          (float4*)(sc->d_blob + L.lnode), &depth, ctx->stream);
+    const cudaError_t e = build_lbvh_device(&ctx->dbuild, rest.data(), dev_pid.data(), (uint32_t)dev_pid.size(),
+                                            (const float4*)(sc->d_blob + L.box), sc->n, (float4*)(sc->d_blob + L.lnode),
+                                            &depth, ctx->stream);
     if (e != cudaSuccess) return set_err(ctx, RT_ERR_CUDA, "device BVH build failed: %s", cudaGetErrorString(e));
     if (depth > (uint32_t)MAX_STACK)
         return set_err(ctx, RT_ERR_UNSUPPORTED, "device-built tree depth %u exceeds the traversal stack (%d)", depth, MAX_STACK);
@@ -486,6 +511,8 @@ DevScene make_dev_scene(const uint8_t* blob, const BlobLayout& L, uint32_t n_sph
     d.ni = n_spheres + n_triangles - 1;
     return d;
 }
+
+std::atomic<uint64_t> next_serial{1};  // scene serials (rt_scene_create, rt_scene_update)
 
 }  // namespace
 
@@ -553,11 +580,11 @@ int rt_scene_create(rt_ctx* ctx, const rt_sphere* spheres, uint32_t n_spheres, c
     const uint32_t n = (uint32_t)n64;
     const TestHooks& hooks = test_hooks();
 
-    static std::atomic<uint64_t> next_serial{1};
     std::unique_ptr<rt_scene> sc(new rt_scene());
     sc->ctx = ctx;
     sc->serial = next_serial++;
     sc->n = n;
+    if (world_index) sc->world_index.assign(world_index, world_index + n);
     sc->aux.reset(new rt_aux());
     rt_aux* aux = sc->aux.get();
     std::vector<PrimRef> world;
@@ -569,6 +596,7 @@ int rt_scene_create(rt_ctx* ctx, const rt_sphere* spheres, uint32_t n_spheres, c
     // which tree will be traversed, and who builds it
     Split split;
     split_big(boxes, &split);
+    sc->big_world = split.big_world;
     const std::vector<Box>& rest = split.rest(boxes);
     const bool device_tree = rest.size() >= 2 &&
                              (hooks.build_mode == 2 || (hooks.build_mode == 1 && rest.size() >= kDeviceBuildMin));
@@ -582,7 +610,7 @@ int rt_scene_create(rt_ctx* ctx, const rt_sphere* spheres, uint32_t n_spheres, c
     assign_pids(world, n_spheres, T, &aux->pid_of_world);
     const std::vector<uint32_t>& pid_of_world = aux->pid_of_world;
 
-    // the reference tree: inline for small scenes, else on the builder thread below
+    // the reference tree: inline for small scenes, else on the builder thread
     const bool ref_sync = n < kRefSyncBelow;
     AuxTables ref_tables;
     if (ref_sync) {
@@ -594,26 +622,14 @@ int rt_scene_create(rt_ctx* ctx, const rt_sphere* spheres, uint32_t n_spheres, c
     const uint32_t lni = device_tree ? (uint32_t)rest.size() - 1 : T ? (uint32_t)T->inner.size() : 0;
     const BlobLayout L = blob_layout(n_spheres, n_triangles, lni);
     sc->blob_bytes = L.blob_bytes;
-    const size_t stage_bytes = ref_sync ? L.blob_bytes : L.sync_bytes;
+    // without a host tree: a single primitive in the tree is the root leaf itself; otherwise the tree is empty or built
+    // on the device (its root is node 0)
+    int32_t lroot = split.rest_world.size() == 1 ? ~(int32_t)(pid_of_world[split.rest_world[0]] << 5) : 0;
     CK(ctx, cudaSetDevice(ctx->device));
-    CK(ctx, reserve_stage(ctx, stage_bytes));
     CK(ctx, take_blob(ctx, L.blob_bytes, &sc->d_blob, &sc->blob_cap));
-    // the builder thread starts now, with pid_of_world final: it overlaps the fill and the upload
-    if (!ref_sync) {
-        const int rc = start_ref_builder(ctx, sc.get(), L, hooks.aux_delay_ms);
-        if (rc) return rc;
-    }
-
-    uint8_t* const h = ctx->h_stage;
-    fill_image(h, L, world, spheres, triangles, n_spheres, boxes, pid_of_world, split.big_world);
-    const int32_t lroot = emit_nodes(h + L.lnode, T, split.rest_world, pid_of_world);
-    if (ref_sync) {  // the whole blob is uploaded by this call: the tables and the raised flag go with it
-        memcpy(h + L.rank, ref_tables.rank.data(), ref_tables.rank.size() * 4);
-        memcpy(h + L.up, ref_tables.up.data(), ref_tables.up.size() * 4);
-        memcpy(h + L.refbox, ref_tables.refbox.data(), ref_tables.refbox.size() * 4);
-        *(int32_t*)(h + L.flag) = 1;
-    }
-    const int rc = upload(ctx, sc.get(), h, L, stage_bytes, device_tree, rest, split.rest_world, pid_of_world);
+    int rc = fill_and_upload(ctx, sc.get(), L, world, spheres, n_spheres, triangles, ref_sync ? &ref_tables : nullptr, !ref_sync, T,
+                             &lroot);
+    if (!rc && device_tree) rc = device_traversal_tree(ctx, sc.get(), L, rest, split.rest_world);
     if (rc) {  // the builder thread may still write to the blob
         if (aux->worker.joinable()) aux->worker.join();
         retire_blob(ctx, sc->d_blob, sc->blob_cap);
@@ -624,6 +640,65 @@ int rt_scene_create(rt_ctx* ctx, const rt_sphere* spheres, uint32_t n_spheres, c
     sc->dev = make_dev_scene(sc->d_blob, L, n_spheres, n_triangles, lni, lroot, !rest.empty(),
                              (uint32_t)split.big_world.size());
     *out = sc.release();
+    return RT_OK;
+    RT_GUARD_END(ctx)
+}
+
+int rt_scene_update(rt_ctx* ctx, rt_scene* scene, const rt_sphere* spheres, uint32_t n_spheres,
+                    const rt_triangle* triangles, uint32_t n_triangles) {
+    if (!ctx) return RT_ERR_INVALID_ARG;
+    RT_GUARD_BEGIN
+    if (!scene) return set_err(ctx, RT_ERR_INVALID_ARG, "rt_scene_update: scene is NULL");
+    if (scene->ctx != ctx) return set_err(ctx, RT_ERR_INVALID_ARG, "rt_scene_update: the scene belongs to another context");
+    const DevScene& d = scene->dev;
+    if (n_spheres != d.ns || n_triangles != d.nt)
+        return set_err(ctx, RT_ERR_INVALID_ARG, "rt_scene_update: %u spheres and %u triangles for a scene of %u and %u",
+                       n_spheres, n_triangles, d.ns, d.nt);
+    if ((n_spheres && !spheres) || (n_triangles && !triangles))
+        return set_err(ctx, RT_ERR_INVALID_ARG, "rt_scene_update: NULL primitive array");
+    rt_aux* aux = scene->aux.get();
+    std::vector<PrimRef> world;
+    std::vector<Box> boxes;
+    std::string werr;
+    const int wrc = world_and_boxes(spheres, n_spheres, triangles, n_triangles,
+                                    scene->world_index.empty() ? nullptr : scene->world_index.data(), &world, &boxes, &werr);
+    if (wrc) return set_err(ctx, wrc, "%s", werr.c_str());
+    // The topology stays as created: split set, pids, node count and depth.  Both are conservative for any geometry
+    // (DESIGN.md section 2), so only the boxes of the traversal tree's records change.
+    const bool same_boxes = memcmp(boxes.data(), aux->boxes.data(), boxes.size() * sizeof(Box)) == 0;
+    const bool ref_sync = scene->n < kRefSyncBelow;
+    AuxTables ref_tables;
+    if (!same_boxes && ref_sync) {  // on failure aux is untouched
+        std::string berr;
+        if (!build_ref_tables(boxes, aux->pid_of_world, aux, &ref_tables, &berr))
+            return set_err(ctx, RT_ERR_BVH, "BVH build failed: %s", berr.c_str());
+    }
+    const BlobLayout L = blob_layout(n_spheres, n_triangles, d.lni);
+    CK(ctx, cudaSetDevice(ctx->device));
+    int rc;
+    if (same_boxes) {
+        // traversal tree and reference tables depend on the boxes alone: both stay, and a builder thread that still runs
+        // is left alone (it writes nothing but the tables)
+        rc = fill_and_upload(ctx, scene, L, world, spheres, n_spheres, triangles, nullptr, false, nullptr, nullptr);
+    } else {
+        if (aux->worker.joinable()) aux->worker.join();  // it reads aux->boxes and writes the tables
+        aux->boxes.swap(boxes);
+        aux->err.clear();
+        aux->state.store(0, std::memory_order_release);
+        // With the tables on the builder thread, start_ref_builder lowers the flag on ctx->stream and synchronises before
+        // the thread starts: no kernel queued before this update can see new tables next to the old geometry, and none
+        // queued after it (aux_ready 0 from here on) can take the old tables for the new ones.
+        rc = fill_and_upload(ctx, scene, L, world, spheres, n_spheres, triangles, ref_sync ? &ref_tables : nullptr, !ref_sync,
+                             nullptr, nullptr);
+        if (!rc) {
+            const cudaError_t e = refit_device(&ctx->dbuild, (const float4*)(scene->d_blob + L.box), scene->n,
+                                               (float4*)(scene->d_blob + L.lnode), d.lni, ctx->stream);
+            if (e != cudaSuccess) rc = set_err(ctx, RT_ERR_CUDA, "traversal tree refit failed: %s", cudaGetErrorString(e));
+        }
+        if (!rc && ref_sync) aux->state.store(1, std::memory_order_release);
+    }
+    if (rc) return rc;
+    scene->serial = next_serial++;
     return RT_OK;
     RT_GUARD_END(ctx)
 }

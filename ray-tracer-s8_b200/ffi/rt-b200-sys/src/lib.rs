@@ -115,6 +115,14 @@ extern "C" {
         out: *mut *mut rt_scene,
     ) -> c_int;
     pub fn rt_scene_destroy(ctx: *mut rt_ctx, scene: *mut rt_scene);
+    pub fn rt_scene_update(
+        ctx: *mut rt_ctx,
+        scene: *mut rt_scene,
+        spheres: *const rt_sphere,
+        n_spheres: u32,
+        triangles: *const rt_triangle,
+        n_triangles: u32,
+    ) -> c_int;
     pub fn rt_render_division(
         ctx: *mut rt_ctx,
         scene: *const rt_scene,
@@ -268,6 +276,19 @@ impl Context {
         let mut raw = ptr::null_mut();
         self.check(unsafe { rt_accum_create(self.raw, params, &mut raw) })?;
         Ok(Accum { ctx: self, raw, len: (params.height / div) as usize * params.width as usize * 3 })
+    }
+}
+
+impl Scene<'_> {
+    /// Replaces the world with one of the same shape (as many spheres and triangles as created; the creation's
+    /// `world_index` still applies).  Later renders are byte-identical to those of a scene created from the new world;
+    /// an `Accum` with samples of the old world needs `reset`.  On an error other than status -4 (CUDA) the scene still
+    /// holds the old world; after -4 drop it.
+    pub fn update(&mut self, spheres: &[rt_sphere], triangles: &[rt_triangle]) -> Result<(), Error> {
+        let rc = unsafe {
+            rt_scene_update(self.ctx.raw, self.raw, spheres.as_ptr(), spheres.len() as u32, triangles.as_ptr(), triangles.len() as u32)
+        };
+        self.ctx.check(rc)
     }
 }
 

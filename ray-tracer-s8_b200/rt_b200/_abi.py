@@ -74,6 +74,7 @@ EXPORTS = [
     "rt_frame_download", "rt_measure_fp32_peak", "rt_device_info", "rt_bvh_build_host", "rt_struct_sizes", "rt_scene_device_bytes",
     "rt_scene_wait_ready", "rt_render_frame_multi", "rt_frame_collect", "rt_render_tiles_collect", "rt_frame_wait_consumed", "rt_l2_flush",
     "rt_accum_create", "rt_accum_destroy", "rt_accum_reset", "rt_accum_samples", "rt_render_samples", "rt_accum_read_linear",
+    "rt_scene_update",
 ]
 
 _lib = None
@@ -107,6 +108,8 @@ def lib():
     L.rt_scene_create.restype = i32
     L.rt_scene_destroy.argtypes = [vp, vp]
     L.rt_scene_destroy.restype = None
+    L.rt_scene_update.argtypes = [vp, vp, vp, u32, vp, u32]
+    L.rt_scene_update.restype = i32
     L.rt_scene_info.argtypes = [vp, C.POINTER(u32), C.POINTER(u32), C.POINTER(u32), vp]
     L.rt_scene_info.restype = i32
     L.rt_render_division.argtypes = [vp, vp, C.POINTER(RtParams), vp, sz, C.POINTER(RtStats)]

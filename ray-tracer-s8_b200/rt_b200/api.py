@@ -334,6 +334,18 @@ class Scene:
         self._h = h
         self.n_spheres, self.n_triangles = len(sp), len(tr)
 
+    def update(self, spheres=None, triangles=None) -> "Scene":
+        """Replace the world with one of the same shape (as many spheres and triangles as created; the creation's
+        world_index still applies): geometry, materials and emission may all change.  Later renders are byte-identical
+        to those of a scene created from the new world; an Accum with samples of the old one needs reset()."""
+        sp = np.ascontiguousarray(spheres if spheres is not None else np.zeros(0, SPHERE_DTYPE), dtype=SPHERE_DTYPE)
+        tr = np.ascontiguousarray(triangles if triangles is not None else np.zeros(0, TRIANGLE_DTYPE), dtype=TRIANGLE_DTYPE)
+        if (len(sp), len(tr)) != (self.n_spheres, self.n_triangles):
+            raise RtError(_abi.RT_ERR_INVALID_ARG, f"{len(sp)} spheres and {len(tr)} triangles for a scene of "
+                                                   f"{self.n_spheres} and {self.n_triangles}")
+        self._ctx._check(self._ctx._lib.rt_scene_update(self._ctx._h, self._h, _ptr(sp), len(sp), _ptr(tr), len(tr)))
+        return self
+
     def info(self):
         n, nn, d = C.c_uint32(), C.c_uint32(), C.c_uint32()
         rank = np.zeros(self.n_spheres + self.n_triangles, dtype=np.uint32)
