@@ -234,14 +234,30 @@ int rt_accum_samples(const rt_accum* acc, uint32_t* samples_out);
  * must render the same scene (another one, a re-created one included, is RT_ERR_INVALID_ARG; RT_INTERSECT_AUTO is
  * resolved against the scene of each call).  RT_ERR_INVALID_ARG also for n_samples == 0, done + n_samples above
  * 2^32 - 1, out_len != rows*width*3 with out_rgb != NULL, and an accum of another context.  On any error the state is
- * unchanged.  stats (nullable): rays, primary (pixels * n_samples), kernel_ms, total_ms, intersector_used,
+ * unchanged.  RT_ERR_INVALID_ARG for an accum bound to several ranks by rt_render_samples_multi until it is reset.
+ * stats (nullable): rays, primary (pixels * n_samples), kernel_ms, total_ms, intersector_used,
  * kernel_launches, the launch shape and redo_pixels; the counters of collect_counters are not filled (0). */
 int rt_render_samples(rt_ctx* ctx, const rt_scene* scene, rt_accum* acc, uint32_t n_samples, uint8_t* out_rgb,
                       size_t out_len, rt_stats* stats);
 /* Linear radiance of the band: rows*width*3 float32 (out_len in bytes), sum / samples per channel (the exact-domain
  * division quantise() does: sqrt, * 255.999, truncate, saturate, NaN -> 0 give the RGB8 band).  RT_ERR_INVALID_ARG before
- * the first chunk. */
+ * the first chunk, and for an accum bound to several ranks by rt_render_samples_multi (each holds only its rank's tiles;
+ * there is no multi-GPU linear readback). */
 int rt_accum_read_linear(rt_ctx* ctx, const rt_accum* acc, float* out, size_t out_len);
+/* One progressive frame on n contexts: accs[i] (rt_accum_create on ctxs[i], whole frame: divisions 1) holds the chains of
+ * rank i's tiles (the interleave of rt_render_frame_multi).  Advances every pixel by n_samples and, if out_rgb != NULL,
+ * streams the frame (height*width*3 bytes) to the host: byte-identical to rt_render_frame at spp = done + n_samples.
+ * Context i renders its tiles of scenes[i] (the same world, created on ctxs[i]) into a frame in ctxs[0]'s memory, as
+ * rt_render_frame_multi does; each accum keeps a whole-frame state buffer, of which only its rank's records are used.
+ * An accum is bound to the tile share of its first chunk after create / reset: rank 0 of 1 for rt_render_samples, rank
+ * i of n here; until rt_accum_reset any other share is refused (n = 1 is the share of rt_render_samples).
+ * RT_ERR_INVALID_ARG, before anything is launched: a NULL handle, accs[i] not of ctxs[i], an accum that is not whole-frame,
+ * bound to another rank or n, bound params (size, seed, camera, max_bounces, flags, intersector) or sample counts that
+ * differ between the accums, a scene other than the one of the chunks since the last reset, n_samples == 0, done +
+ * n_samples above 2^32 - 1, out_len != height*width*3 with out_rgb != NULL.  On any error no accum moves.  stats
+ * (nullable): as rt_render_samples, counters summed over the contexts, kernel_ms the slowest context's. */
+int rt_render_samples_multi(rt_ctx* const* ctxs, const rt_scene* const* scenes, rt_accum* const* accs, uint32_t n,
+                            uint32_t n_samples, uint8_t* out_rgb, size_t out_len, rt_stats* stats);
 
 int rt_sync(rt_ctx* ctx);
 /* The ctx stream as a cudaStream_t, for callers that order their own work (NCCL, copies) after a render. */

@@ -848,6 +848,7 @@ int rt_accum_reset(rt_ctx* ctx, rt_accum* acc, const rt_params* params) {
     }
     acc->samples = 0;
     acc->scene_serial = 0;
+    acc->tile_rank = acc->tile_ranks = 0;
     return RT_OK;
     RT_GUARD_END(ctx)
 }
@@ -864,6 +865,9 @@ int rt_render_samples(rt_ctx* ctx, const rt_scene* scene, rt_accum* acc, uint32_
     RT_GUARD_BEGIN
     const auto t0 = std::chrono::steady_clock::now();
     if (!acc || acc->ctx != ctx) return set_err(ctx, RT_ERR_INVALID_ARG, "rt_render_samples: accum is NULL or of another context");
+    if (acc->tile_ranks > 1)
+        return set_err(ctx, RT_ERR_INVALID_ARG, "rt_render_samples: the accum holds rank %u of %u (rt_render_samples_multi) until reset",
+                       acc->tile_rank, acc->tile_ranks);
     if (!scene) return set_err(ctx, RT_ERR_INVALID_ARG, "rt_render_samples: scene is NULL");
     if (n_samples == 0) return set_err(ctx, RT_ERR_INVALID_ARG, "rt_render_samples: n_samples is 0");
     if ((uint64_t)acc->samples + n_samples > 0xffffffffull)
@@ -894,6 +898,8 @@ int rt_render_samples(rt_ctx* ctx, const rt_scene* scene, rt_accum* acc, uint32_
     acc->cur ^= 1;
     acc->samples += n_samples;
     acc->scene_serial = scene->serial;
+    acc->tile_rank = 0;
+    acc->tile_ranks = 1;
     return RT_OK;
     RT_GUARD_END(ctx)
 }
@@ -904,6 +910,9 @@ int rt_accum_read_linear(rt_ctx* ctx, const rt_accum* acc, float* out, size_t ou
     if (!acc || acc->ctx != ctx) return set_err(ctx, RT_ERR_INVALID_ARG, "rt_accum_read_linear: accum is NULL or of another context");
     if (!out) return set_err(ctx, RT_ERR_INVALID_ARG, "rt_accum_read_linear: out is NULL");
     if (acc->samples == 0) return set_err(ctx, RT_ERR_INVALID_ARG, "rt_accum_read_linear: no samples rendered yet");
+    if (acc->tile_ranks > 1)
+        return set_err(ctx, RT_ERR_INVALID_ARG, "rt_accum_read_linear: the accum holds only rank %u of %u's tiles", acc->tile_rank,
+                       acc->tile_ranks);
     const uint64_t pixels = (uint64_t)(acc->row1 - acc->row0) * acc->params.width;
     const size_t bytes = (size_t)pixels * 3 * sizeof(float);
     if (out_len != bytes) return set_err(ctx, RT_ERR_INVALID_ARG, "out_len %zu != rows * width * 3 * 4 = %zu", out_len, bytes);

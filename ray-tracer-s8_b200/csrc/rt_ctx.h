@@ -183,6 +183,9 @@ struct rt_accum {
     int cur = 0;
     uint32_t samples = 0;       // samples of every pixel's chain done so far
     uint64_t scene_serial = 0;  // the scene of the chunks since the last create / reset (0: none yet)
+    // the tile share of the chunks since the last create / reset (tile_ranks 0: none yet): rt_render_samples is rank 0
+    // of 1; rank i of n (rt_render_samples_multi) holds the chains of that rank's tiles only
+    uint32_t tile_rank = 0, tile_ranks = 0;
 };
 
 #define CK(ctx, call)                                                                                        \

@@ -150,7 +150,9 @@ constexpr int L_SLOT_SHIFT = 4;           // 3 bits: output-stage slot + 1 of th
 constexpr uint32_t L_SECOND = 128u;       // this pixel comes from the redo list: its first pass was held back, not counted
 
 // RESUME: the launch renders samples [pr.s0, pr.spp) of each pixel's chain from the state in pr.state_in and leaves the
-// state in pr.state_out (rt_render_samples); the other instantiations render samples [0, pr.spp).
+// state in pr.state_out (rt_render_samples, rt_render_samples_multi); the other instantiations render samples [0, pr.spp).
+// With the output stage (a frame shared between ranks) a held-back pixel stores no state but is counted in s_hold like
+// any other: its second pass, in the kernel or by the host, starts over from the same state_in and counts it then.
 template <int ISECT, bool SMEM, bool COUNT, bool STAGE, int MINB, int TPB, bool RESUME = false>
 __global__ void __launch_bounds__(TPB, MINB) render_kernel_lanes(const DevScene sc, const DevCamera cam,
                                                                 const DevParams pr) {
@@ -695,16 +697,22 @@ static KernelFn pick_lanes(bool count, bool stage, int* threads) {
                  : (KernelFn)render_kernel_lanes<ISECT, SMEM, false, false, 3, THREADS>;
 }
 
-// the resumable form (rt_render_samples): the same CTA shapes, no output stage and no instrumented variant
+// the resumable form (rt_render_samples, rt_render_samples_multi): the same CTA shapes with and without the output
+// stage, no instrumented variant
 template <int ISECT, bool SMEM>
-static KernelFn pick_resume(int* threads) {
+static KernelFn pick_resume(bool stage, int* threads) {
     if constexpr (SMEM) {
         *threads = SMEM_TPB;
-        return (KernelFn)render_kernel_lanes<ISECT, SMEM, false, false, 1, SMEM_TPB, true>;
+        return stage ? (KernelFn)render_kernel_lanes<ISECT, SMEM, false, true, 1, SMEM_TPB, true>
+                     : (KernelFn)render_kernel_lanes<ISECT, SMEM, false, false, 1, SMEM_TPB, true>;
     } else {
         *threads = THREADS;
-        if constexpr (ISECT == RT_INTERSECT_BVH) return (KernelFn)render_kernel_lanes<ISECT, SMEM, false, false, 4, THREADS, true>;
-        else return (KernelFn)render_kernel_lanes<ISECT, SMEM, false, false, 3, THREADS, true>;
+        if constexpr (ISECT == RT_INTERSECT_BVH)
+            return stage ? (KernelFn)render_kernel_lanes<ISECT, SMEM, false, true, 4, THREADS, true>
+                         : (KernelFn)render_kernel_lanes<ISECT, SMEM, false, false, 4, THREADS, true>;
+        else
+            return stage ? (KernelFn)render_kernel_lanes<ISECT, SMEM, false, true, 3, THREADS, true>
+                         : (KernelFn)render_kernel_lanes<ISECT, SMEM, false, false, 3, THREADS, true>;
     }
 }
 
@@ -722,10 +730,12 @@ cudaError_t preload_kernels() {
             RT_TOUCH((pick_lanes<RT_INTERSECT_BRUTE, true>(count, stage, &th)));
             RT_TOUCH((pick_lanes<RT_INTERSECT_BRUTE, false>(count, stage, &th)));
         }
-    RT_TOUCH((pick_resume<RT_INTERSECT_BVH, true>(&th)));
-    RT_TOUCH((pick_resume<RT_INTERSECT_BVH, false>(&th)));
-    RT_TOUCH((pick_resume<RT_INTERSECT_BRUTE, true>(&th)));
-    RT_TOUCH((pick_resume<RT_INTERSECT_BRUTE, false>(&th)));
+    for (int stage = 0; stage < 2; stage++) {
+        RT_TOUCH((pick_resume<RT_INTERSECT_BVH, true>(stage, &th)));
+        RT_TOUCH((pick_resume<RT_INTERSECT_BVH, false>(stage, &th)));
+        RT_TOUCH((pick_resume<RT_INTERSECT_BRUTE, true>(stage, &th)));
+        RT_TOUCH((pick_resume<RT_INTERSECT_BRUTE, false>(stage, &th)));
+    }
     RT_TOUCH(accum_linear_kernel);
     RT_TOUCH(wait_slab_kernel);
     RT_TOUCH(wait_all_slabs_kernel);
@@ -754,11 +764,12 @@ cudaError_t launch_render(const DevScene& sc, const DevCamera& cam, const DevPar
     // The output stage and the completion counters cost ~0.03 ns per pixel (C3: +0.2 ms of 38.0; C2, 1 spp: +0.07 of 0.24);
     // the copy they let the owner overlap costs 0.06 ns per pixel.  On for frames shared between ranks and for frames the
     // caller streams to the host; a frame that stays on one device keeps round 1's byte stores (profiles/r2_notes.md).
-    const bool stage = !count && !resume && (pr.tile_ranks > 1 || pr.stage_hint) && pr.done != nullptr;
+    // The same for the resumable form: rt_render_samples_multi's shared frames stage, rt_render_samples' bands do not.
+    const bool stage = !count && (pr.tile_ranks > 1 || pr.stage_hint) && pr.done != nullptr;
     int threads = THREADS;
     KernelFn fn;
-    if (resume) fn = isect == RT_INTERSECT_BRUTE ? (smem ? pick_resume<RT_INTERSECT_BRUTE, true>(&threads) : pick_resume<RT_INTERSECT_BRUTE, false>(&threads))
-                                                 : (smem ? pick_resume<RT_INTERSECT_BVH, true>(&threads) : pick_resume<RT_INTERSECT_BVH, false>(&threads));
+    if (resume) fn = isect == RT_INTERSECT_BRUTE ? (smem ? pick_resume<RT_INTERSECT_BRUTE, true>(stage, &threads) : pick_resume<RT_INTERSECT_BRUTE, false>(stage, &threads))
+                                                 : (smem ? pick_resume<RT_INTERSECT_BVH, true>(stage, &threads) : pick_resume<RT_INTERSECT_BVH, false>(stage, &threads));
     else if (isect == RT_INTERSECT_BRUTE) fn = smem ? pick_lanes<RT_INTERSECT_BRUTE, true>(count, stage, &threads) : pick_lanes<RT_INTERSECT_BRUTE, false>(count, stage, &threads);
     else fn = smem ? pick_lanes<RT_INTERSECT_BVH, true>(count, stage, &threads) : pick_lanes<RT_INTERSECT_BVH, false>(count, stage, &threads);
     const size_t dyn = smem ? need : 0;

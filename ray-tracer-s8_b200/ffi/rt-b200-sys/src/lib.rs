@@ -173,6 +173,16 @@ extern "C" {
         stats: *mut rt_stats,
     ) -> c_int;
     pub fn rt_accum_read_linear(ctx: *mut rt_ctx, acc: *const rt_accum, out: *mut f32, out_len: usize) -> c_int;
+    pub fn rt_render_samples_multi(
+        ctxs: *const *mut rt_ctx,
+        scenes: *const *const rt_scene,
+        accs: *const *mut rt_accum,
+        n: u32,
+        n_samples: u32,
+        out_rgb: *mut u8,
+        out_len: usize,
+        stats: *mut rt_stats,
+    ) -> c_int;
 }
 
 /// Error of any call: the negative `rt_status` and the library's message.
@@ -325,6 +335,22 @@ pub fn render_frame_multi(ctxs: &[&Context], scenes: &[&Scene<'_>], params: &rt_
     let s: Vec<*const rt_scene> = scenes.iter().map(|s| s.raw as *const rt_scene).collect();
     let mut out = vec![0u8; params.height as usize * params.width as usize * 3];
     let rc = unsafe { rt_render_frame_multi(c.as_ptr(), s.as_ptr(), c.len() as u32, params, out.as_mut_ptr(), out.len(), ptr::null_mut()) };
+    ctxs[0].check(rc)?;
+    Ok(out)
+}
+
+/// One progressive frame over several GPUs (`rt_render_samples_multi`): `accs[i]` (a whole-frame `Accum` of `ctxs[i]`)
+/// holds the chains of rank i's tiles of `scenes[i]`; every pixel advances by `n_samples` and the returned frame is the
+/// bytes of `render_frame_multi` at `spp = accs[0].samples()`.  On an error no accum moves.
+pub fn render_samples_multi(ctxs: &[&Context], scenes: &[&Scene<'_>], accs: &mut [&mut Accum<'_>], n_samples: u32) -> Result<Vec<u8>, Error> {
+    assert!(!ctxs.is_empty() && ctxs.len() == scenes.len() && ctxs.len() == accs.len(), "one scene and one accum per context");
+    let c: Vec<*mut rt_ctx> = ctxs.iter().map(|c| c.raw).collect();
+    let s: Vec<*const rt_scene> = scenes.iter().map(|s| s.raw as *const rt_scene).collect();
+    let a: Vec<*mut rt_accum> = accs.iter().map(|a| a.raw).collect();
+    let mut out = vec![0u8; accs[0].len];
+    let rc = unsafe {
+        rt_render_samples_multi(c.as_ptr(), s.as_ptr(), a.as_ptr(), c.len() as u32, n_samples, out.as_mut_ptr(), out.len(), ptr::null_mut())
+    };
     ctxs[0].check(rc)?;
     Ok(out)
 }

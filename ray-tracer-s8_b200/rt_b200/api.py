@@ -268,6 +268,25 @@ def render_frame_multi(ctxs, scenes, params: RtParams, out: np.ndarray | None = 
     return (out, st.as_dict()) if want_stats else out
 
 
+def render_samples_multi(ctxs, scenes, accs, n: int, out: np.ndarray | None = None, download=True, want_stats=False):
+    """One progressive frame on several contexts (rt_render_samples_multi): accs[i] (a whole-frame Accum of ctxs[i])
+    holds the chains of rank i's tiles; every pixel advances by `n` samples and the frame as it now stands (byte-identical
+    to render_frame at spp = accs[0].samples) goes to `out` (None: a new array); download=False skips the copy and returns
+    None in its place."""
+    if not ctxs or not (len(ctxs) == len(scenes) == len(accs)):
+        raise RtError(_abi.RT_ERR_INVALID_ARG, "one scene and one accum per context")
+    k = len(ctxs)
+    out = Context._out_buffer(out, (accs[0].rows, accs[0].width, 3)) if download else None
+    ch = (C.c_void_p * k)(*[c._h for c in ctxs])
+    sh = (C.c_void_p * k)(*[s._h for s in scenes])
+    ah = (C.c_void_p * k)(*[a._h for a in accs])
+    st = RtStats()
+    ctxs[0]._check(ctxs[0]._lib.rt_render_samples_multi(ch, sh, ah, k, int(n),
+                                                        None if out is None else out.ctypes.data_as(C.c_void_p),
+                                                        0 if out is None else out.nbytes, C.byref(st)))
+    return (out, st.as_dict()) if want_stats else out
+
+
 class Accum:
     """Resumable per-pixel sample chains of one frame or division (rt_accum): chunks rendered with
     Context.render_samples add up to the frame render_division renders at the cumulative sample count."""

@@ -179,6 +179,18 @@ class MultiDeviceRenderer:
     def render(self, scenes, params, out: np.ndarray | None = None, want_stats: bool = False):
         return self._api.render_frame_multi(self.ctxs, scenes, params, out=out, want_stats=want_stats)
 
+    def render_progressive(self, scene_per_ctx, params, schedule=(1, 1, 2, 4, 8)):
+        """Preview that improves, on every GPU: yields (samples_done, frame) after each chunk of `schedule` samples; each
+        frame equals render() at spp = samples_done (rt_render_samples_multi; params.divisions must be 1)."""
+        accs = [c.accum(params) for c in self.ctxs]
+        try:
+            for n in schedule:
+                frame = self._api.render_samples_multi(self.ctxs, scene_per_ctx, accs, n)
+                yield accs[0].samples, frame
+        finally:
+            for a in accs:
+                a.close()
+
     def close(self):
         for c in self.ctxs:
             c.close()
