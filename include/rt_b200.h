@@ -184,6 +184,16 @@ int rt_bvh_build_host(const rt_sphere* spheres, uint32_t n_spheres, const rt_tri
  * top of the band.  Returns after out_rgb is complete.  stats is nullable. */
 int rt_render_division(rt_ctx* ctx, const rt_scene* scene, const rt_params* params, uint8_t* out_rgb,
                        size_t out_len, rt_stats* stats);
+/* Several divisions of one job in one launch: band division_nos[k] of *params (params->division_no is ignored) is
+ * written to out_rgb + k * rows * width * 3, rows = height / divisions, byte-identical to rt_render_division with
+ * division_no = division_nos[k].  out_len = n * rows * width * 3.  A list that is one ascending run of bands renders as
+ * that row range (the path of rt_render_division and rt_render_frame); any other list renders its bands stacked in list
+ * order in one banded launch.  RT_ERR_INVALID_ARG, before anything is launched: a NULL pointer, n == 0, a division
+ * number >= divisions or listed twice, a wrong out_len, and every check of rt_render_division.  Returns after all n
+ * bands are in out_rgb.  stats (nullable): as rt_render_division for all n bands (primary = n * rows * width * spp); the
+ * counters of collect_counters are not filled (0), as for rt_render_samples. */
+int rt_render_divisions(rt_ctx* ctx, const rt_scene* scene, const rt_params* params, const uint32_t* division_nos,
+                        uint32_t n, uint8_t* out_rgb, size_t out_len, rt_stats* stats);
 /* All divisions in one launch: height*width*3 bytes into host memory (what the controller stitches at
  * ray-tracer-controller/src/main.rs:109-119). params->division_no is ignored. */
 int rt_render_frame(rt_ctx* ctx, const rt_scene* scene, const rt_params* params, uint8_t* out_rgb,

@@ -179,6 +179,8 @@ int launch(rt_ctx* ctx, const rt_scene* scene, const Resolved& r, const LaunchAr
     pr.stage_hint = a.stream ? 1 : 0;
     pr.redo_slab = ctx->d_ctr + RT_CTR_REDO_SLAB;
     pr.slab_tile_rows = a.frame.plan.tile_rows ? a.frame.plan.tile_rows : 1;
+    pr.band_table = a.band_table;
+    pr.band_rows = a.band_rows;
     const DevScene dev = scene_view(scene);
     CK(ctx, cudaMemsetAsync(ctx->d_ctr, 0, RT_CTR_SLOTS * sizeof(unsigned long long), ctx->stream));
     if (!a.pixel_list) CK(ctx, cudaMemsetAsync(ctx->d_redo, 0, RT_REDO_CAP * sizeof(unsigned int), ctx->stream));
@@ -531,8 +533,11 @@ int collect_frame(rt_ctx* owner, const Frame& f, uint64_t seq, uint8_t* out_rgb,
 
 namespace {
 
+// Rows [row0, row1) of the launch space into host memory: image rows, or with a band table (device memory) the bands of
+// band_rows rows it lists, stacked (row0 = 0).
 int render_rows_to_host(rt_ctx* ctx, const rt_scene* scene, const Resolved& r, uint32_t row0, uint32_t row1,
-                        uint8_t* out_rgb, size_t out_len, rt_stats* stats) {
+                        uint8_t* out_rgb, size_t out_len, rt_stats* stats, const uint32_t* band_table = nullptr,
+                        uint32_t band_rows = 0) {
     const auto t0 = std::chrono::steady_clock::now();
     const size_t bytes = (size_t)(row1 - row0) * r.p.width * 3;
     if (!out_rgb) return set_err(ctx, RT_ERR_INVALID_ARG, "out_rgb is NULL");
@@ -544,6 +549,8 @@ int render_rows_to_host(rt_ctx* ctx, const rt_scene* scene, const Resolved& r, u
     l.a.row0 = row0;
     l.a.row1 = row1;
     l.a.out_row0 = row0;
+    l.a.band_table = band_table;
+    l.a.band_rows = band_rows;
     const int rc = own_frame(ctx, r.p.width, row1 - row0, &l.a.frame);
     if (rc) return rc;
     // Streaming the frame out slab by slab while it renders beats one copy after the kernel on a single GPU when a pixel
@@ -669,6 +676,7 @@ void rt_shutdown(rt_ctx* ctx) {
     if (ctx->copy_stream) cudaStreamSynchronize(ctx->copy_stream);
     if (ctx->aux_stream) cudaStreamSynchronize(ctx->aux_stream);
     if (ctx->d_out) cudaFree(ctx->d_out);
+    if (ctx->d_bands) cudaFree(ctx->d_bands);
     if (ctx->d_ctr) cudaFree(ctx->d_ctr);
     if (ctx->h_ctr) cudaFreeHost(ctx->h_ctr);
     if (ctx->d_redo) cudaFree(ctx->d_redo);
@@ -726,6 +734,53 @@ int rt_render_division(rt_ctx* ctx, const rt_scene* scene, const rt_params* para
     const uint32_t band = r.p.height / r.p.divisions;  // main.rs:55-56
     const uint32_t row0 = band * r.p.division_no;      // main.rs:66-68
     return render_rows_to_host(ctx, scene, r, row0, row0 + band, out_rgb, out_len, stats);
+    RT_GUARD_END(ctx)
+}
+
+int rt_render_divisions(rt_ctx* ctx, const rt_scene* scene, const rt_params* params, const uint32_t* division_nos,
+                        uint32_t n, uint8_t* out_rgb, size_t out_len, rt_stats* stats) {
+    if (!ctx) return RT_ERR_INVALID_ARG;
+    RT_GUARD_BEGIN
+    if (!params) return set_err(ctx, RT_ERR_INVALID_ARG, "NULL scene or params");
+    if (!division_nos || n == 0) return set_err(ctx, RT_ERR_INVALID_ARG, "rt_render_divisions: no division numbers");
+    rt_params p = *params;
+    p.division_no = 0;         // the list says which bands
+    p.collect_counters = 0;    // as rt_render_samples: the banded form has no instrumented variant
+    Resolved r;
+    int rc = resolve(ctx, scene, &p, false, &r);
+    if (rc) return rc;
+    std::vector<bool> seen(r.p.divisions, false);
+    bool contiguous = true;
+    for (uint32_t k = 0; k < n; k++) {
+        const uint32_t d = division_nos[k];
+        if (d >= r.p.divisions)
+            return set_err(ctx, RT_ERR_INVALID_ARG, "rt_render_divisions: division %u out of range (%u divisions)", d, r.p.divisions);
+        if (seen[d]) return set_err(ctx, RT_ERR_INVALID_ARG, "rt_render_divisions: division %u listed twice", d);
+        seen[d] = true;
+        contiguous = contiguous && d == division_nos[0] + k;
+    }
+    const uint32_t band = r.p.height / r.p.divisions;  // main.rs:55-56
+    const size_t bytes = (size_t)n * band * r.p.width * 3;
+    if (!out_rgb) return set_err(ctx, RT_ERR_INVALID_ARG, "out_rgb is NULL");
+    if (out_len != bytes)
+        return set_err(ctx, RT_ERR_INVALID_ARG, "out_len %zu != (n %u * rows %u * width %u * 3) = %zu", out_len, n, band,
+                       r.p.width, bytes);
+    // one ascending run of bands is a plain row range: the path of rt_render_division / rt_render_frame, no table
+    if (contiguous) return render_rows_to_host(ctx, scene, r, band * division_nos[0], band * (division_nos[0] + n), out_rgb, out_len, stats);
+    CK(ctx, cudaSetDevice(ctx->device));
+    if (ctx->d_bands_cap < n) {
+        if (ctx->d_bands) {
+            CK(ctx, cudaStreamSynchronize(ctx->stream));
+            CK(ctx, cudaFree(ctx->d_bands));
+            ctx->d_bands = nullptr;
+            ctx->d_bands_cap = 0;
+        }
+        CK(ctx, cudaMalloc(&ctx->d_bands, (size_t)r.p.divisions * sizeof(uint32_t)));
+        ctx->d_bands_cap = r.p.divisions;
+    }
+    // stream-ordered in front of the launch and of any second pass, which read the same table
+    CK(ctx, cudaMemcpyAsync(ctx->d_bands, division_nos, (size_t)n * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+    return render_rows_to_host(ctx, scene, r, 0, n * band, out_rgb, out_len, stats, ctx->d_bands, band);
     RT_GUARD_END(ctx)
 }
 

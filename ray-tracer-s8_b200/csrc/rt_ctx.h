@@ -36,6 +36,8 @@ struct rt_ctx {
     char name[64] = {0};
     uint8_t* d_out = nullptr;  // band / frame staging in HBM + control block
     size_t d_out_bytes = 0;    // capacity for pixels (the control block follows at rt_frame_ctl_offset(capacity))
+    uint32_t* d_bands = nullptr;  // band table of rt_render_divisions' banded launches
+    size_t d_bands_cap = 0;       // entries
     unsigned long long* d_ctr = nullptr;  // NUM_COUNTERS counters | 2 tickets (one u64) | redo count (one u64)
     unsigned long long* h_ctr = nullptr;  // pinned mirror
     unsigned int* d_redo = nullptr;       // pixels to render again once the tie-break tables are up (REDO_CAP entries)
@@ -149,6 +151,8 @@ struct LaunchArgs {
     const void* state_in = nullptr;  // resumable chains (rt_render_samples): samples [s0, spp) from state_in to state_out
     void* state_out = nullptr;
     uint32_t s0 = 0;
+    const uint32_t* band_table = nullptr;  // banded launch (rt_render_divisions): row0 = 0, rows = bands of band_rows
+    uint32_t band_rows = 0;                // stacked in table order (device memory of the context, see DevParams)
 };
 // Launches the render on ctx->stream; timing events ev0 / ev1 are recorded around the kernel.
 int launch(rt_ctx* ctx, const rt_scene* scene, const Resolved& r, const LaunchArgs& a, LaunchInfo* info);

@@ -153,7 +153,10 @@ constexpr uint32_t L_SECOND = 128u;       // this pixel comes from the redo list
 // state in pr.state_out (rt_render_samples, rt_render_samples_multi); the other instantiations render samples [0, pr.spp).
 // With the output stage (a frame shared between ranks) a held-back pixel stores no state but is counted in s_hold like
 // any other: its second pass, in the kernel or by the host, starts over from the same state_in and counts it then.
-template <int ISECT, bool SMEM, bool COUNT, bool STAGE, int MINB, int TPB, bool RESUME = false>
+// BANDS: the launch's rows are the bands of pr.band_table stacked (rt_render_divisions).  px / py stay in launch rows for
+// the stage, the counters, the redo list and the output; the image row, which only the seed and the camera ray need, is
+// looked up where it is used rather than held through the traversal.
+template <int ISECT, bool SMEM, bool COUNT, bool STAGE, int MINB, int TPB, bool RESUME = false, bool BANDS = false>
 __global__ void __launch_bounds__(TPB, MINB) render_kernel_lanes(const DevScene sc, const DevCamera cam,
                                                                 const DevParams pr) {
     extern __shared__ float4 smem_dyn[];
@@ -247,6 +250,11 @@ __global__ void __launch_bounds__(TPB, MINB) render_kernel_lanes(const DevScene 
         return g;
     };
     auto out_desc = [&]() { return OutDesc{pr.out, pr.done, pr.width, pr.out_row0, pr.row0, pr.slab_tile_rows}; };
+    // launch row → image row (the identity outside BANDS)
+    auto image_row = [&](uint32_t y) -> uint32_t {
+        if constexpr (BANDS) return __ldg(&pr.band_table[y / pr.band_rows]) * pr.band_rows + y % pr.band_rows;
+        else return y;
+    };
 
     for (;;) {
         // ---- hand out pixels: warp-cooperative, tile by tile ----
@@ -403,7 +411,7 @@ __global__ void __launch_bounds__(TPB, MINB) render_kernel_lanes(const DevScene 
                         }
                         s = pr.s0;
                     } else {
-                        rng.seed_from_u64(pr.seed + ((uint64_t)y * pr.width + x));
+                        rng.seed_from_u64(pr.seed + ((uint64_t)image_row(y) * pr.width + x));
                         sr = sg = sb = 0.0f;
                         s = 0;
                     }
@@ -416,7 +424,7 @@ __global__ void __launch_bounds__(TPB, MINB) render_kernel_lanes(const DevScene 
 
         if (st & L_HAVE) {
             if (left == 0) {  // start sample s
-                primary_ray(cam, px, pr.height - py - 1, rng, &o, &d);  // y_cam = h - y - 1 (main.rs:71)
+                primary_ray(cam, px, pr.height - image_row(py) - 1, rng, &o, &d);  // y_cam = h - y - 1 (main.rs:71)
                 left = pr.depth;
                 np = 0;
             }
@@ -716,6 +724,25 @@ static KernelFn pick_resume(bool stage, int* threads) {
     }
 }
 
+// the banded form (rt_render_divisions with a list that is not one contiguous run): the product CTA shapes with and
+// without the output stage, no instrumented or resumable variant
+template <int ISECT, bool SMEM>
+static KernelFn pick_bands(bool stage, int* threads) {
+    if constexpr (SMEM) {
+        *threads = SMEM_TPB;
+        return stage ? (KernelFn)render_kernel_lanes<ISECT, SMEM, false, true, 1, SMEM_TPB, false, true>
+                     : (KernelFn)render_kernel_lanes<ISECT, SMEM, false, false, 1, SMEM_TPB, false, true>;
+    } else {
+        *threads = THREADS;
+        if constexpr (ISECT == RT_INTERSECT_BVH)
+            return stage ? (KernelFn)render_kernel_lanes<ISECT, SMEM, false, true, 4, THREADS, false, true>
+                         : (KernelFn)render_kernel_lanes<ISECT, SMEM, false, false, 4, THREADS, false, true>;
+        else
+            return stage ? (KernelFn)render_kernel_lanes<ISECT, SMEM, false, true, 3, THREADS, false, true>
+                         : (KernelFn)render_kernel_lanes<ISECT, SMEM, false, false, 3, THREADS, false, true>;
+    }
+}
+
 // Resolves every kernel variant once per context so that the first render does not pay the lazy module load.
 cudaError_t preload_kernels() {
     cudaFuncAttributes a;
@@ -735,6 +762,10 @@ cudaError_t preload_kernels() {
         RT_TOUCH((pick_resume<RT_INTERSECT_BVH, false>(stage, &th)));
         RT_TOUCH((pick_resume<RT_INTERSECT_BRUTE, true>(stage, &th)));
         RT_TOUCH((pick_resume<RT_INTERSECT_BRUTE, false>(stage, &th)));
+        RT_TOUCH((pick_bands<RT_INTERSECT_BVH, true>(stage, &th)));
+        RT_TOUCH((pick_bands<RT_INTERSECT_BVH, false>(stage, &th)));
+        RT_TOUCH((pick_bands<RT_INTERSECT_BRUTE, true>(stage, &th)));
+        RT_TOUCH((pick_bands<RT_INTERSECT_BRUTE, false>(stage, &th)));
     }
     RT_TOUCH(accum_linear_kernel);
     RT_TOUCH(wait_slab_kernel);
@@ -753,7 +784,8 @@ constexpr uint64_t kTailPermille = 30;
 cudaError_t launch_render(const DevScene& sc, const DevCamera& cam, const DevParams& pr, int isect, bool count,
                           int sm_count, int smem_optin, cudaStream_t stream, LaunchInfo* info) {
     const bool resume = pr.state_out != nullptr;  // rt_render_samples
-    if (resume) count = false;
+    const bool bands = pr.band_table != nullptr;  // rt_render_divisions
+    if (resume || bands) count = false;
     const size_t static_smem = (SMEM_TPB / 32) * (OUT_SLOTS * (TILE_BYTES + 16) + 4) + 64;
     const size_t need = scene_image_bytes(sc.ns, sc.nt, sc.lni, isect == RT_INTERSECT_BVH);
     // Stage the scene in shared memory when one 1024-thread CTA per SM fits with it (scenes up to ~200 KB); larger
@@ -770,6 +802,8 @@ cudaError_t launch_render(const DevScene& sc, const DevCamera& cam, const DevPar
     KernelFn fn;
     if (resume) fn = isect == RT_INTERSECT_BRUTE ? (smem ? pick_resume<RT_INTERSECT_BRUTE, true>(stage, &threads) : pick_resume<RT_INTERSECT_BRUTE, false>(stage, &threads))
                                                  : (smem ? pick_resume<RT_INTERSECT_BVH, true>(stage, &threads) : pick_resume<RT_INTERSECT_BVH, false>(stage, &threads));
+    else if (bands) fn = isect == RT_INTERSECT_BRUTE ? (smem ? pick_bands<RT_INTERSECT_BRUTE, true>(stage, &threads) : pick_bands<RT_INTERSECT_BRUTE, false>(stage, &threads))
+                                                     : (smem ? pick_bands<RT_INTERSECT_BVH, true>(stage, &threads) : pick_bands<RT_INTERSECT_BVH, false>(stage, &threads));
     else if (isect == RT_INTERSECT_BRUTE) fn = smem ? pick_lanes<RT_INTERSECT_BRUTE, true>(count, stage, &threads) : pick_lanes<RT_INTERSECT_BRUTE, false>(count, stage, &threads);
     else fn = smem ? pick_lanes<RT_INTERSECT_BVH, true>(count, stage, &threads) : pick_lanes<RT_INTERSECT_BVH, false>(count, stage, &threads);
     const size_t dyn = smem ? need : 0;

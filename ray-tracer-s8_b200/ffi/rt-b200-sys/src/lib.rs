@@ -131,6 +131,16 @@ extern "C" {
         out_len: usize,
         stats: *mut rt_stats,
     ) -> c_int;
+    pub fn rt_render_divisions(
+        ctx: *mut rt_ctx,
+        scene: *const rt_scene,
+        params: *const rt_params,
+        division_nos: *const u32,
+        n: u32,
+        out_rgb: *mut u8,
+        out_len: usize,
+        stats: *mut rt_stats,
+    ) -> c_int;
     pub fn rt_render_frame(
         ctx: *mut rt_ctx,
         scene: *const rt_scene,
@@ -276,6 +286,20 @@ impl Context {
         let len = (params.height / div) as usize * params.width as usize * 3;
         let mut out = vec![0u8; len];
         let rc = unsafe { rt_render_division(self.raw, scene.raw, params, out.as_mut_ptr(), out.len(), ptr::null_mut()) };
+        self.check(rc)?;
+        Ok(out)
+    }
+
+    /// Bands `division_nos` of one job in one launch (`params.division_no` is ignored): band `division_nos[k]` is
+    /// `out[k * rows * width * 3..][..rows * width * 3]`, the bytes `render_division` gives for it.
+    pub fn render_divisions(&self, scene: &Scene<'_>, params: &rt_params, division_nos: &[u32]) -> Result<Vec<u8>, Error> {
+        let div = params.divisions.max(1);
+        let len = division_nos.len() * (params.height / div) as usize * params.width as usize * 3;
+        let mut out = vec![0u8; len];
+        let rc = unsafe {
+            rt_render_divisions(self.raw, scene.raw, params, division_nos.as_ptr(), division_nos.len() as u32, out.as_mut_ptr(),
+                                out.len(), ptr::null_mut())
+        };
         self.check(rc)?;
         Ok(out)
     }

@@ -74,7 +74,7 @@ EXPORTS = [
     "rt_frame_download", "rt_measure_fp32_peak", "rt_device_info", "rt_bvh_build_host", "rt_struct_sizes", "rt_scene_device_bytes",
     "rt_scene_wait_ready", "rt_render_frame_multi", "rt_frame_collect", "rt_render_tiles_collect", "rt_frame_wait_consumed", "rt_l2_flush",
     "rt_accum_create", "rt_accum_destroy", "rt_accum_reset", "rt_accum_samples", "rt_render_samples", "rt_accum_read_linear",
-    "rt_scene_update", "rt_render_samples_multi",
+    "rt_scene_update", "rt_render_samples_multi", "rt_render_divisions",
 ]
 
 _lib = None
@@ -114,6 +114,8 @@ def lib():
     L.rt_scene_info.restype = i32
     L.rt_render_division.argtypes = [vp, vp, C.POINTER(RtParams), vp, sz, C.POINTER(RtStats)]
     L.rt_render_division.restype = i32
+    L.rt_render_divisions.argtypes = [vp, vp, C.POINTER(RtParams), vp, u32, vp, sz, C.POINTER(RtStats)]
+    L.rt_render_divisions.restype = i32
     L.rt_render_frame.argtypes = [vp, vp, C.POINTER(RtParams), vp, sz, C.POINTER(RtStats)]
     L.rt_render_frame.restype = i32
     L.rt_render_tiles_device.argtypes = [vp, vp, C.POINTER(RtParams), u32, u32, vp, i32, C.POINTER(RtStats)]

@@ -157,6 +157,23 @@ class Context:
                                                  out.nbytes, C.byref(st)))
         return (out, st.as_dict()) if want_stats else out
 
+    def render_divisions(self, scene: "Scene", params: RtParams, division_nos, out: np.ndarray | None = None,
+                         want_stats=False):
+        """Bands `division_nos` of one job in one launch → uint8 (n, height/divisions, width, 3); out[k] is
+        render_division of band division_nos[k] (params.division_no is ignored)."""
+        div = params.divisions or 1
+        if params.height % div != 0:
+            raise RtError(_abi.RT_ERR_INVALID_ARG, f"height {params.height} is not a multiple of divisions {div}")
+        nos = np.asarray(division_nos, dtype=np.int64).reshape(-1)
+        if ((nos < 0) | (nos > 0xFFFFFFFF)).any():
+            raise RtError(_abi.RT_ERR_INVALID_ARG, "division numbers must fit 32 bits unsigned")
+        nos = np.ascontiguousarray(nos, dtype=np.uint32)
+        out = self._out_buffer(out, (len(nos), params.height // div, params.width, 3))
+        st = RtStats()
+        self._check(self._lib.rt_render_divisions(self._h, scene._h, C.byref(params), _ptr(nos), len(nos),
+                                                  out.ctypes.data_as(C.c_void_p), out.nbytes, C.byref(st)))
+        return (out, st.as_dict()) if want_stats else out
+
     def render_frame(self, scene: "Scene", params: RtParams, out: np.ndarray | None = None, want_stats=False):
         """All divisions in one launch → uint8 (height, width, 3)."""
         out = self._out_buffer(out, (params.height, params.width, 3))

@@ -79,8 +79,11 @@ class Controller:
                 self.result(sl)
         elif self.worker is not None:
             world = wire.World(np.zeros(0, wire.SPHERE_DTYPE), triangles, np.arange(len(triangles), dtype=np.uint32))
-            for d in range(self.divisions):
-                self.result(self.worker.render(wire.RenderInfo(world, meta, d)))
+            infos = [wire.RenderInfo(world, meta, d) for d in range(self.divisions)]
+            # all divisions in one call (rt_render_divisions) when the worker can; any object with render() still works
+            render_many = getattr(self.worker, "render_many", None)
+            for sl in render_many(infos) if render_many else map(self.worker.render, infos):
+                self.result(sl)
         else:
             for d in range(self.divisions):                      # join_all over 0..divisions (main.rs:47-75)
                 text = wire.render_info_to_json(None, triangles, meta, d)

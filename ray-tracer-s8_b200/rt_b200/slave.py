@@ -7,7 +7,9 @@ Mirrors ray-tracer-slave/src/main.rs:
     BVH per request, main.rs:60).
   * `serve()` = main() + index() (main.rs:148-174): `POST /` with a RenderInfo body answers
     "i'll get you a slice at once" immediately and queues the job for the single worker thread, which
-    POSTs the ImageSlice JSON to `http://master:8080/result` (main.rs:85-101).
+    POSTs the ImageSlice JSON to `http://master:8080/result` (main.rs:85-101).  The worker thread takes every request
+    already queued with the one it waited for and renders those of one job together (`Worker.render_many`, one
+    `rt_render_divisions` call); each still gets its own ImageSlice POST.
 spp / max_bounces / camera default to the reference's literals (main.rs:39-51).
 """
 from __future__ import annotations
@@ -79,6 +81,24 @@ class Worker:
         sl = wire.ImageSlice(info.division_no, np.ascontiguousarray(img).reshape(-1), m.id)
         return (sl, st) if want_stats else sl
 
+    def render_many(self, infos, want_stats: bool = False):
+        """Requests of one world and one (width, height, divisions) in one call (rt_render_divisions): one ImageSlice per
+        request, in order, each equal to render(info)'s.  A division requested twice is rendered once.  The world is
+        infos[0]'s (the caller groups by _world_key, which checksums it)."""
+        m = infos[0].render_meta
+        key = (m.id, m.width, m.height, m.divisions)
+        if any((i.render_meta.id, i.render_meta.width, i.render_meta.height, i.render_meta.divisions) != key for i in infos):
+            raise ValueError("render_many takes requests of one job: one id, width, height and divisions")
+        nos = list(dict.fromkeys(i.division_no for i in infos))
+        p = api.make_params(m.width, m.height, divisions=m.divisions, spp=self.spp, max_bounces=self.max_bounces,
+                            seed=self.seed, intersector=self.intersector)
+        with self.lock:
+            out = self.ctx.render_divisions(self._scene_for(infos[0]), p, nos, want_stats=want_stats)
+        imgs, st = out if want_stats else (out, None)
+        at = {d: k for k, d in enumerate(nos)}
+        slices = [wire.ImageSlice(i.division_no, imgs[at[i.division_no]].reshape(-1), i.render_meta.id) for i in infos]
+        return (slices, st) if want_stats else slices
+
     def render_json(self, body: str | bytes) -> str:
         """RenderInfo JSON in → ImageSlice JSON out."""
         return self.render(wire.parse_render_info(body)).to_json()
@@ -102,16 +122,55 @@ def serve(host: str = "0.0.0.0", port: int = 8081, result_url: str = MASTER_RESU
     wk = worker or Worker()
     jobs: "queue.Queue[wire.RenderInfo | None]" = queue.Queue()  # crossbeam unbounded channel (main.rs:159)
 
+    def post_slice(sl):
+        try:
+            post(result_url, sl.to_json())
+        except Exception as e:  # the reference unwrap()s and dies; we log and keep serving
+            print(f"[rt_b200.slave] job failed: {e}", flush=True)
+
+    def render_alone(info):
+        try:
+            sl = wk.render(info)
+        except Exception as e:
+            print(f"[rt_b200.slave] job failed: {e}", flush=True)
+            return
+        post_slice(sl)
+
     def worker_loop():
         while True:
             info = jobs.get()
             if info is None:
                 return
-            try:
-                body = wk.render(info).to_json()
-                post(result_url, body)
-            except Exception as e:  # the reference unwrap()s and dies; we log and keep serving
-                print(f"[rt_b200.slave] job failed: {e}", flush=True)
+            # every request already queued goes along: the controller POSTs a job's divisions at once, and one launch
+            # over several bands keeps the GPU busier than one launch per band
+            batch, stopping = [info], False
+            while True:
+                try:
+                    nxt = jobs.get_nowait()
+                except queue.Empty:
+                    break
+                if nxt is None:
+                    stopping = True
+                    break
+                batch.append(nxt)
+            groups: dict = {}  # insertion order: groups in the arrival order of their first request
+            for i in batch:
+                m = i.render_meta
+                groups.setdefault((Worker._world_key(i), m.width, m.height, m.divisions), []).append(i)
+            for g in groups.values():
+                try:
+                    slices = wk.render_many(g)
+                except Exception as e:
+                    if len(g) == 1:
+                        print(f"[rt_b200.slave] job failed: {e}", flush=True)
+                    else:  # a request that fails on its own (a bad division_no) must not sink the others
+                        for i in g:
+                            render_alone(i)
+                    continue
+                for sl in slices:
+                    post_slice(sl)
+            if stopping:
+                return
 
     class Handler(BaseHTTPRequestHandler):
         def do_POST(self):  # noqa: N802
