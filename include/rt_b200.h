@@ -208,6 +208,27 @@ int rt_render_frame(rt_ctx* ctx, const rt_scene* scene, const rt_params* params,
 int rt_render_frame_multi(rt_ctx* const* ctxs, const rt_scene* const* scenes, uint32_t n, const rt_params* params,
                           uint8_t* out_rgb, size_t out_len, rt_stats* stats);
 
+/* ---- JPEG ------------------------------------------------------------------------------------------ */
+/* The controller's output format (ray-tracer-controller/src/main.rs:95-142 encodes the stitched frame as JPEG(90)),
+ * encoded on the device.  The bytes are identical to libjpeg's defaults at the same quality (what PIL's
+ * save(format="JPEG", quality=q) writes): JFIF 1.01, 4:2:0, the standard Huffman tables, no restart markers.
+ * RT_ERR_INVALID_ARG, before anything is launched: a NULL pointer, a width or height of 0 or above 65535, a quality
+ * outside 1..100, out_cap < rt_jpeg_bound(width, height).  *out_len: the bytes written to out. */
+
+/* Bytes enough for any JPEG the two calls below write for width x height, at any quality. */
+size_t rt_jpeg_bound(uint32_t width, uint32_t height);
+/* Baseline JPEG of an RGB8 frame in host memory (height*width*3 bytes, row-major, row 0 on top), byte-identical to
+ * libjpeg's defaults at this quality (JFIF, 4:2:0, standard Huffman tables, no restart markers).  ms_out (nullable):
+ * device time of the encode. */
+int rt_jpeg_encode(rt_ctx* ctx, const uint8_t* rgb, uint32_t width, uint32_t height, uint32_t quality,
+                   uint8_t* out, size_t out_cap, size_t* out_len, float* ms_out);
+/* Renders the whole frame as rt_render_frame (n == 1) or rt_render_frame_multi (n > 1), then encodes it on ctxs[0]
+ * from device memory: the RGB frame never reaches the host.  The bytes equal rt_jpeg_encode of that call's frame.
+ * Refused as rt_jpeg_encode and as the render entry it wraps.  stats (nullable): the render's, with total_ms including
+ * the encode and the download. */
+int rt_render_frame_jpeg(rt_ctx* const* ctxs, const rt_scene* const* scenes, uint32_t n, const rt_params* params,
+                         uint32_t quality, uint8_t* out, size_t out_cap, size_t* out_len, rt_stats* stats);
+
 /* Device-side entry for the multi-GPU tile scheduler: renders the 8x4-pixel tiles of the whole frame that belong to
  * rank tile_rank of tile_ranks (tile t, row-major over the tile grid, belongs to rank (t % ranks - t / ranks) mod ranks:
  * a rotating interleave) into a full-frame DEVICE buffer `frame_dev` (height*width*3 bytes;

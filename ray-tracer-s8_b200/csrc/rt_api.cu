@@ -652,6 +652,7 @@ int rt_init(int device, rt_ctx** out) {
     ctx->h_flag[0] = 0;
     // load the module and resolve every kernel now: the first division of a job must not pay the lazy load
     CKI(preload_kernels());
+    CKI(jpeg_preload());
     ctx->serial_launches = launches_block();
     {   // stream memory operations, if this driver and device have them (64-bit waits)
         int can64 = 0;
@@ -691,6 +692,8 @@ void rt_shutdown(rt_ctx* ctx) {
     for (void* p : ctx->host_allocs) cudaFreeHost(p);
     ctx->host_allocs.clear();
     if (ctx->h_stage) cudaFreeHost(ctx->h_stage);
+    if (ctx->d_jpeg) cudaFree(ctx->d_jpeg);
+    if (ctx->h_jpeg_len) cudaFreeHost(ctx->h_jpeg_len);
     if (ctx->ev0) cudaEventDestroy(ctx->ev0);
     if (ctx->ev1) cudaEventDestroy(ctx->ev1);
     if (ctx->ev_sync) cudaEventDestroy(ctx->ev_sync);

@@ -61,6 +61,9 @@ struct rt_ctx {
     struct Retired { uint8_t* p; size_t cap; };
     std::vector<Retired> retired;
     std::vector<void*> host_allocs;  // rt_host_alloc'ed buffers still alive (freed at shutdown)
+    uint8_t* d_jpeg = nullptr;       // JPEG encoder scratch (rt_jpeg.cu): coefficients, bit offsets, coded and stuffed bytes
+    size_t d_jpeg_bytes = 0;
+    unsigned long long* h_jpeg_len = nullptr;  // pinned: length of the last encoded segment
     std::string err;
 };
 constexpr uint32_t RT_REDO_CAP = 1u << 16;
@@ -173,6 +176,16 @@ struct Launch {
 // n >= 1): the launches' statistics combined, total_ms counted from t0.
 int collect_frame(rt_ctx* owner, const Frame& f, uint64_t seq, uint8_t* out_rgb, Launch* l, uint32_t n, rt_stats* stats,
                   std::chrono::steady_clock::time_point t0);
+
+// JPEG (rt_jpeg.cu).  jpeg_check: the refusals shared by every JPEG entry (NULL out, size, quality, out_cap below
+// rt_jpeg_bound).  jpeg_encode_device: encodes the width x height RGB8 frame at rgb_dev (device memory of ctx, ordered
+// on ctx->stream) into out (checked by jpeg_check) and returns when out holds all *out_len bytes; ms_out (nullable): the
+// device time of the encode.
+int jpeg_check(rt_ctx* ctx, uint32_t width, uint32_t height, uint32_t quality, const uint8_t* out, size_t out_cap,
+               const size_t* out_len);
+int jpeg_encode_device(rt_ctx* ctx, const uint8_t* rgb_dev, uint32_t width, uint32_t height, uint32_t quality,
+                       uint8_t* out, size_t* out_len, float* ms_out);
+cudaError_t jpeg_preload();
 
 }  // namespace rtb
 

@@ -7,6 +7,7 @@
 // control block counts finished pixels per slab (system-scope releases from every GPU), so the copy of a slab to the
 // caller's host buffer starts as soon as all ranks have finished that slab, while the rest of the frame still renders.
 // rt_render_samples_multi is the same frame rendered in chunks of samples: each context resumes its tiles' chains.
+// rt_render_frame_jpeg renders the frame (on one context or on n) and encodes it where it lies, in context 0's memory.
 #include <cstring>
 #include <vector>
 
@@ -153,6 +154,50 @@ extern "C" int rt_render_samples_multi(rt_ctx* const* ctxs, const rt_scene* cons
         a->tile_rank = i;
         a->tile_ranks = n;
     }
+    return RT_OK;
+    RT_GUARD_END(c0)
+}
+
+extern "C" int rt_render_frame_jpeg(rt_ctx* const* ctxs, const rt_scene* const* scenes, uint32_t n, const rt_params* params,
+                                    uint32_t quality, uint8_t* out, size_t out_cap, size_t* out_len, rt_stats* stats) {
+    if (!ctxs || !scenes || n == 0 || !ctxs[0]) return RT_ERR_INVALID_ARG;
+    rt_ctx* const c0 = ctxs[0];
+    RT_GUARD_BEGIN
+    const auto t0 = std::chrono::steady_clock::now();
+    for (uint32_t i = 0; i < n; i++)
+        if (!ctxs[i] || !scenes[i]) return set_err(c0, RT_ERR_INVALID_ARG, "rt_render_frame_jpeg: NULL context or scene %u", i);
+    std::vector<Launch> l;
+    for (uint32_t i = 0; i < n; i++) {
+        l.push_back({ctxs[i], scenes[i]});
+        const int rc = resolve(ctxs[i], scenes[i], params, true, &l[i].r);
+        if (rc) {
+            if (i) set_err(c0, rc, "context %u: %s", i, ctxs[i]->err.c_str());
+            return rc;
+        }
+    }
+    const uint32_t W = l[0].r.p.width, H = l[0].r.p.height;
+    int rc = jpeg_check(c0, W, H, quality, out, out_cap, out_len);
+    if (rc) return rc;
+    // the frame stays in context 0's staging frame: with no host destination a single launch does not stream
+    if (n == 1) {
+        CK(c0, cudaSetDevice(c0->device));
+        l[0].a.row1 = H;
+        rc = own_frame(c0, W, H, &l[0].a.frame);
+    } else {
+        rc = shared_frame(ctxs, n, W, H, l.data());
+    }
+    if (rc) return rc;
+    rc = collect_frame(c0, l[0].a.frame, OWN_FRAME_SEQ, nullptr, l.data(), n, stats, t0);
+    if (rc) return rc;
+    for (uint32_t i = 1; i < n; i++) {  // the encode on context 0's stream comes after every rank's last store
+        CK(c0, cudaSetDevice(ctxs[i]->device));
+        CK(c0, cudaEventRecord(ctxs[i]->ev_sync, ctxs[i]->stream));
+        CK(c0, cudaSetDevice(c0->device));
+        CK(c0, cudaStreamWaitEvent(c0->stream, ctxs[i]->ev_sync, 0));
+    }
+    rc = jpeg_encode_device(c0, l[0].a.frame.dev, W, H, quality, out, out_len, nullptr);
+    if (rc) return rc;
+    if (stats) stats->total_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
     return RT_OK;
     RT_GUARD_END(c0)
 }

@@ -159,6 +159,29 @@ extern "C" {
         out_len: usize,
         stats: *mut rt_stats,
     ) -> c_int;
+    pub fn rt_jpeg_bound(width: u32, height: u32) -> usize;
+    pub fn rt_jpeg_encode(
+        ctx: *mut rt_ctx,
+        rgb: *const u8,
+        width: u32,
+        height: u32,
+        quality: u32,
+        out: *mut u8,
+        out_cap: usize,
+        out_len: *mut usize,
+        ms_out: *mut f32,
+    ) -> c_int;
+    pub fn rt_render_frame_jpeg(
+        ctxs: *const *mut rt_ctx,
+        scenes: *const *const rt_scene,
+        n: u32,
+        params: *const rt_params,
+        quality: u32,
+        out: *mut u8,
+        out_cap: usize,
+        out_len: *mut usize,
+        stats: *mut rt_stats,
+    ) -> c_int;
     pub fn rt_render_tiles_device(
         ctx: *mut rt_ctx,
         scene: *const rt_scene,
@@ -304,6 +327,26 @@ impl Context {
         Ok(out)
     }
 
+    /// Baseline JPEG of an RGB8 frame (`height * width * 3` bytes, row 0 on top), encoded on this context's GPU: the
+    /// bytes libjpeg writes with its defaults at `quality` (1..100), i.e. the controller's JPEG(90) at 90.
+    pub fn encode_jpeg(&self, rgb: &[u8], width: u32, height: u32, quality: u32) -> Result<Vec<u8>, Error> {
+        assert_eq!(rgb.len(), width as usize * height as usize * 3, "rgb must hold height * width * 3 bytes");
+        let mut out = vec![0u8; unsafe { rt_jpeg_bound(width, height) }];
+        let mut len = 0usize;
+        let rc = unsafe {
+            rt_jpeg_encode(self.raw, rgb.as_ptr(), width, height, quality, out.as_mut_ptr(), out.len(), &mut len, ptr::null_mut())
+        };
+        self.check(rc)?;
+        out.truncate(len);
+        Ok(out)
+    }
+
+    /// The whole frame of `render_frame` as JPEG bytes, encoded on the device where it was rendered: equal to
+    /// `encode_jpeg(&render_frame(..)?, ..)` without the RGB frame crossing to the host.
+    pub fn render_frame_jpeg(&self, scene: &Scene<'_>, params: &rt_params, quality: u32) -> Result<Vec<u8>, Error> {
+        render_frame_jpeg(&[self], &[scene], params, quality)
+    }
+
     /// Sample state of the band `params` selects (`params.spp` is ignored), every pixel at sample 0.
     pub fn accum(&self, params: &rt_params) -> Result<Accum<'_>, Error> {
         let div = params.divisions.max(1);
@@ -360,6 +403,23 @@ pub fn render_frame_multi(ctxs: &[&Context], scenes: &[&Scene<'_>], params: &rt_
     let mut out = vec![0u8; params.height as usize * params.width as usize * 3];
     let rc = unsafe { rt_render_frame_multi(c.as_ptr(), s.as_ptr(), c.len() as u32, params, out.as_mut_ptr(), out.len(), ptr::null_mut()) };
     ctxs[0].check(rc)?;
+    Ok(out)
+}
+
+/// The frame of `render_frame_multi` (or of `Context::render_frame` for one context) as JPEG bytes at `quality`,
+/// encoded on `ctxs[0]`'s GPU where the frame lies (`rt_render_frame_jpeg`).  What a controller returns from `/poll`.
+pub fn render_frame_jpeg(ctxs: &[&Context], scenes: &[&Scene<'_>], params: &rt_params, quality: u32) -> Result<Vec<u8>, Error> {
+    assert!(!ctxs.is_empty() && ctxs.len() == scenes.len(), "one scene per context");
+    let c: Vec<*mut rt_ctx> = ctxs.iter().map(|c| c.raw).collect();
+    let s: Vec<*const rt_scene> = scenes.iter().map(|s| s.raw as *const rt_scene).collect();
+    let mut out = vec![0u8; unsafe { rt_jpeg_bound(params.width, params.height) }];
+    let mut len = 0usize;
+    let rc = unsafe {
+        rt_render_frame_jpeg(c.as_ptr(), s.as_ptr(), c.len() as u32, params, quality, out.as_mut_ptr(), out.len(), &mut len,
+                             ptr::null_mut())
+    };
+    ctxs[0].check(rc)?;
+    out.truncate(len);
     Ok(out)
 }
 

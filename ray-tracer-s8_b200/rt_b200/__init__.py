@@ -11,5 +11,5 @@
 from . import scenes  # noqa: F401
 from .api import (  # noqa: F401
     INTERSECT_AUTO, INTERSECT_BRUTE, INTERSECT_BVH, Accum, Context, RtError, RtParams, RtStats, Scene, make_params,
-    render_frame_multi, render_samples_multi,
+    render_frame_jpeg, render_frame_multi, render_samples_multi,
 )

@@ -74,7 +74,8 @@ EXPORTS = [
     "rt_frame_download", "rt_measure_fp32_peak", "rt_device_info", "rt_bvh_build_host", "rt_struct_sizes", "rt_scene_device_bytes",
     "rt_scene_wait_ready", "rt_render_frame_multi", "rt_frame_collect", "rt_render_tiles_collect", "rt_frame_wait_consumed", "rt_l2_flush",
     "rt_accum_create", "rt_accum_destroy", "rt_accum_reset", "rt_accum_samples", "rt_render_samples", "rt_accum_read_linear",
-    "rt_scene_update", "rt_render_samples_multi", "rt_render_divisions",
+    "rt_scene_update", "rt_render_samples_multi", "rt_render_divisions", "rt_jpeg_bound", "rt_jpeg_encode",
+    "rt_render_frame_jpeg",
 ]
 
 _lib = None
@@ -172,6 +173,12 @@ def lib():
     L.rt_accum_read_linear.restype = i32
     L.rt_render_samples_multi.argtypes = [pp, pp, pp, u32, u32, vp, sz, C.POINTER(RtStats)]
     L.rt_render_samples_multi.restype = i32
+    L.rt_jpeg_bound.argtypes = [u32, u32]
+    L.rt_jpeg_bound.restype = sz
+    L.rt_jpeg_encode.argtypes = [vp, vp, u32, u32, u32, vp, sz, C.POINTER(sz), C.POINTER(C.c_float)]
+    L.rt_jpeg_encode.restype = i32
+    L.rt_render_frame_jpeg.argtypes = [pp, pp, u32, C.POINTER(RtParams), u32, vp, sz, C.POINTER(sz), C.POINTER(RtStats)]
+    L.rt_render_frame_jpeg.restype = i32
     L.rt_struct_sizes.argtypes = [C.POINTER(sz)]
     L.rt_struct_sizes.restype = None
     sizes = (sz * 4)()

@@ -182,6 +182,25 @@ class Context:
                                               out.nbytes, C.byref(st)))
         return (out, st.as_dict()) if want_stats else out
 
+    def encode_jpeg(self, frame: np.ndarray, quality: int = 90, want_ms=False):
+        """Baseline JPEG of a uint8 (height, width, 3) frame, encoded on this context's GPU (rt_jpeg_encode): the bytes
+        PIL's save(format="JPEG", quality=quality) writes.  want_ms: also the device time of the encode."""
+        frame = np.ascontiguousarray(frame, dtype=np.uint8)
+        if frame.ndim != 3 or frame.shape[2] != 3:
+            raise RtError(_abi.RT_ERR_INVALID_ARG, f"frame must be (height, width, 3), not {frame.shape}")
+        h, w = frame.shape[:2]
+        buf = np.empty(self._lib.rt_jpeg_bound(w, h), dtype=np.uint8)
+        n, ms = C.c_size_t(0), C.c_float(0.0)
+        self._check(self._lib.rt_jpeg_encode(self._h, _ptr(frame), w, h, int(quality), _ptr(buf), buf.nbytes,
+                                             C.byref(n), C.byref(ms)))
+        data = buf[: n.value].tobytes()
+        return (data, ms.value) if want_ms else data
+
+    def render_frame_jpeg(self, scene: "Scene", params: RtParams, quality: int = 90, want_stats=False):
+        """render_frame, then the frame encoded as JPEG on the device (rt_render_frame_jpeg): the bytes of
+        encode_jpeg(render_frame(...)); the RGB frame never reaches the host."""
+        return render_frame_jpeg([self], [scene], params, quality=quality, want_stats=want_stats)
+
     def render_tiles_device(self, scene: "Scene", params: RtParams, tile_rank: int, tile_ranks: int, frame_dev: int,
                             sync=True, want_stats=False):
         """This rank's tiles of the whole frame into a device (possibly peer-mapped) frame buffer."""
@@ -283,6 +302,23 @@ def render_frame_multi(ctxs, scenes, params: RtParams, out: np.ndarray | None = 
     ctxs[0]._check(ctxs[0]._lib.rt_render_frame_multi(ch, sh, n, C.byref(params), out.ctypes.data_as(C.c_void_p),
                                                       out.nbytes, C.byref(st)))
     return (out, st.as_dict()) if want_stats else out
+
+
+def render_frame_jpeg(ctxs, scenes, params: RtParams, quality: int = 90, want_stats=False):
+    """The frame of render_frame (one context) or render_frame_multi (several) as JPEG bytes, encoded on ctxs[0]'s GPU
+    where the frame lies (rt_render_frame_jpeg).  Stats: the render's, total_ms including the encode."""
+    if len(ctxs) != len(scenes) or not ctxs:
+        raise RtError(_abi.RT_ERR_INVALID_ARG, "one scene per context")
+    L = ctxs[0]._lib
+    n = len(ctxs)
+    ch = (C.c_void_p * n)(*[c._h for c in ctxs])
+    sh = (C.c_void_p * n)(*[s._h for s in scenes])
+    buf = np.empty(L.rt_jpeg_bound(params.width, params.height), dtype=np.uint8)
+    size, st = C.c_size_t(0), RtStats()
+    ctxs[0]._check(L.rt_render_frame_jpeg(ch, sh, n, C.byref(params), int(quality), _ptr(buf), buf.nbytes, C.byref(size),
+                                          C.byref(st)))
+    data = buf[: size.value].tobytes()
+    return (data, st.as_dict()) if want_stats else data
 
 
 def render_samples_multi(ctxs, scenes, accs, n: int, out: np.ndarray | None = None, download=True, want_stats=False):

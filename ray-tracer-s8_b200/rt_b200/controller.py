@@ -10,6 +10,9 @@ Same literals as the reference: 1920x1080, 20 divisions (main.rs:33-36), the sam
   * `devices=[...]`: the tile scheduler — the whole frame in ONE call over all listed GPUs (`rt_render_frame_multi`:
     every GPU renders an interleaved share of the 8x4 tiles straight into GPU 0's frame over NVLink), then cut into
     the job's divisions so /poll stitches them exactly as it stitches slave slices (main.rs:109-119).
+/poll's JPEG(90) is encoded on the GPU where there is one: in `devices=` mode the frame is encoded where it was rendered
+(`rt_render_frame_jpeg`) and never reaches the host as RGB; in `worker=` mode the stitched frame is encoded with the
+worker's context (`rt_jpeg_encode`).  The bytes are the same as PIL's, which the HTTP-slave mode keeps using.
 GPU work from concurrent /upload requests is serialised (one rt_ctx has one owner at a time).
 """
 from __future__ import annotations
@@ -65,6 +68,19 @@ class Controller:
         rows = meta.height // meta.divisions          # main.rs:55-56
         return [wire.ImageSlice(d, frame[d * rows:(d + 1) * rows].reshape(-1), meta.id) for d in range(meta.divisions)]
 
+    def _render_all_gpus_jpeg(self, triangles, meta: "wire.RenderMeta") -> bytes:
+        """devices= mode: one frame over all GPUs, encoded as JPEG(90) on the first GPU, where the frame lies."""
+        from . import api
+
+        p = api.make_params(meta.width, meta.height, spp=self.spp, max_bounces=self.max_bounces, seed=self.seed)
+        with self.gpu_lock:
+            scenes = self.multi.scenes(None, triangles, np.arange(len(triangles), dtype=np.uint32))
+            try:
+                return self.multi.render_jpeg(scenes, p, quality=90)
+            finally:
+                for sc in scenes:
+                    sc.close()
+
     # -- /upload ---------------------------------------------------------------------------------------
     def upload(self, body: bytes, obj_size: int) -> str:
         job_id = str(uuid.uuid4())
@@ -75,8 +91,10 @@ class Controller:
         if self.multi is not None:
             if self.height % self.divisions != 0:
                 raise ValueError(f"height {self.height} is not a multiple of divisions {self.divisions}")
-            for sl in self._render_all_gpus(triangles, meta):
-                self.result(sl)
+            jpeg = self._render_all_gpus_jpeg(triangles, meta)
+            with self.lock:
+                if job_id in self.jobs:
+                    self.jobs[job_id]["jpeg"] = jpeg
         elif self.worker is not None:
             world = wire.World(np.zeros(0, wire.SPHERE_DTYPE), triangles, np.arange(len(triangles), dtype=np.uint32))
             infos = [wire.RenderInfo(world, meta, d) for d in range(self.divisions)]
@@ -111,16 +129,24 @@ class Controller:
             job = self.jobs.get(job_id)
             if job is None:
                 return b"No such job", False
+            if "jpeg" in job:                        # devices= mode: the whole frame, already encoded
+                del self.jobs[job_id]
+                return job["jpeg"], True
             have = sum(1 for d in range(job["meta"].divisions) if d in job["result"])
             if have < job["meta"].divisions:
                 return f"Job not finished yet {have}/{job['meta'].divisions}".encode(), False
             frame = np.concatenate([job["result"][d] for d in range(job["meta"].divisions)])   # sorted by division_no
             del self.jobs[job_id]                                                                # main.rs:122
         frame = frame.reshape(job["meta"].height, job["meta"].width, 3)
+        ctx = getattr(self.worker, "ctx", None)
+        if ctx is not None:                          # worker= mode: encoded on the worker's GPU, same bytes as PIL
+            with self.worker.lock:
+                return ctx.encode_jpeg(frame, 90), True
         return encode_jpeg(frame, 90), True
 
 
 def encode_jpeg(frame: np.ndarray, quality: int = 90) -> bytes:
+    """Host encoder of the HTTP-slave mode (no GPU context here): libjpeg's defaults, the bytes rt_jpeg_encode writes."""
     from PIL import Image  # image 0.24's JPEG encoder in the reference; any baseline JPEG encoder here
 
     buf = io.BytesIO()

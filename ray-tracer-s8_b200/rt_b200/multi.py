@@ -179,6 +179,10 @@ class MultiDeviceRenderer:
     def render(self, scenes, params, out: np.ndarray | None = None, want_stats: bool = False):
         return self._api.render_frame_multi(self.ctxs, scenes, params, out=out, want_stats=want_stats)
 
+    def render_jpeg(self, scenes, params, quality: int = 90, want_stats: bool = False):
+        """The frame of render() as JPEG bytes, encoded on the first GPU where the frame lies (rt_render_frame_jpeg)."""
+        return self._api.render_frame_jpeg(self.ctxs, scenes, params, quality=quality, want_stats=want_stats)
+
     def render_progressive(self, scene_per_ctx, params, schedule=(1, 1, 2, 4, 8)):
         """Preview that improves, on every GPU: yields (samples_done, frame) after each chunk of `schedule` samples; each
         frame equals render() at spp = samples_done (rt_render_samples_multi; params.divisions must be 1)."""
