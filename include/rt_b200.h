@@ -229,6 +229,35 @@ int rt_jpeg_encode(rt_ctx* ctx, const uint8_t* rgb, uint32_t width, uint32_t hei
 int rt_render_frame_jpeg(rt_ctx* const* ctxs, const rt_scene* const* scenes, uint32_t n, const rt_params* params,
                          uint32_t quality, uint8_t* out, size_t out_cap, size_t* out_len, rt_stats* stats);
 
+/* ---- wire format: the slave's request and result bodies (ray-tracer-slave/src/lib.rs:10-30) --------- */
+/* Upper bound on the Objects in `len` bytes of world JSON (len / the shortest accepted Object, derived in rt_wire.cu). */
+size_t rt_world_json_max_objects(size_t len);
+/* Parses the JSON array of Object that starts at text[0] (leading JSON whitespace allowed): the "world" value of a
+ * RenderInfo.  Writes the spheres and the triangles in world order and the world position of each (spheres first, then
+ * triangles), exactly the arrays rt_b200/wire.py's parse_render_info puts in its World, and *consumed = the offset just
+ * past the array's ']'.  spheres, triangles and world_index must each hold cap >= rt_world_json_max_objects(len) entries.
+ * The device grammar is a strict subset of JSON, serde's canonical layout: every Object {"Sphere":{...}} or
+ * {"Triangle":{...}} with its fields in declaration order, JSON whitespace anywhere, JSON numbers of at most 19 significant
+ * digits, node_index a non-negative integer (its value is ignored).  Numbers convert as Python's json + float32 do: an
+ * integer exactly to f64, then to f32; any other token correctly rounded to f64, then to f32 (both to nearest).
+ * RT_ERR_UNSUPPORTED: the text is outside the device grammar (a backslash, an unknown, missing, repeated or reordered key,
+ * NaN / Infinity, a number of more than 19 digits or with an exponent outside the conversion table, malformed JSON ...);
+ * nothing is promised about the outputs, and the caller parses the text on the host, which decides whether it is valid.
+ * RT_ERR_INVALID_ARG: a NULL pointer, cap below the bound. */
+int rt_world_parse_json(rt_ctx* ctx, const char* text, size_t len, rt_sphere* spheres, rt_triangle* triangles,
+                        uint32_t* world_index, size_t cap, uint32_t* n_spheres, uint32_t* n_triangles, size_t* consumed);
+/* Bytes enough for the ImageSlice JSON of one band of rows x width. */
+size_t rt_slice_json_bound(uint32_t rows, uint32_t width);
+/* rt_render_divisions, then band k written on the device as the body the slave POSTs to /result,
+ * {"division_no":D,"image":[v,v,...],"id":"ID"} with no spaces: the bytes of serde_json's json!(ImageSlice) and of
+ * wire.ImageSlice(D, band, ID).to_json().  The bodies are packed back to back in out, body k (band division_nos[k]) first
+ * after body k - 1; out_lens[k] is its length.  id: the 36-character hyphenated lowercase uuid.  The RGB bands never reach
+ * the host.  Refused as rt_render_divisions (out_rgb / out_len aside), and with RT_ERR_INVALID_ARG, before anything is
+ * launched: a NULL id, out or out_lens, an id not of that form, out_cap < n * rt_slice_json_bound(rows, width).  stats
+ * (nullable): as rt_render_divisions, with total_ms including the bodies and their download. */
+int rt_render_divisions_json(rt_ctx* ctx, const rt_scene* scene, const rt_params* params, const uint32_t* division_nos,
+                             uint32_t n, const char* id, uint8_t* out, size_t out_cap, size_t* out_lens, rt_stats* stats);
+
 /* Device-side entry for the multi-GPU tile scheduler: renders the 8x4-pixel tiles of the whole frame that belong to
  * rank tile_rank of tile_ranks (tile t, row-major over the tile grid, belongs to rank (t % ranks - t / ranks) mod ranks:
  * a rotating interleave) into a full-frame DEVICE buffer `frame_dev` (height*width*3 bytes;

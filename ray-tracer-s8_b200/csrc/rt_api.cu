@@ -534,14 +534,15 @@ int collect_frame(rt_ctx* owner, const Frame& f, uint64_t seq, uint8_t* out_rgb,
 namespace {
 
 // Rows [row0, row1) of the launch space into host memory: image rows, or with a band table (device memory) the bands of
-// band_rows rows it lists, stacked (row0 = 0).
+// band_rows rows it lists, stacked (row0 = 0).  on_device: no host destination (out_rgb NULL, out_len 0); the rows stay
+// in the context's staging frame, ctx->d_out, ordered on ctx->stream.
 int render_rows_to_host(rt_ctx* ctx, const rt_scene* scene, const Resolved& r, uint32_t row0, uint32_t row1,
                         uint8_t* out_rgb, size_t out_len, rt_stats* stats, const uint32_t* band_table = nullptr,
-                        uint32_t band_rows = 0) {
+                        uint32_t band_rows = 0, bool on_device = false) {
     const auto t0 = std::chrono::steady_clock::now();
     const size_t bytes = (size_t)(row1 - row0) * r.p.width * 3;
-    if (!out_rgb) return set_err(ctx, RT_ERR_INVALID_ARG, "out_rgb is NULL");
-    if (out_len != bytes)
+    if (!on_device && !out_rgb) return set_err(ctx, RT_ERR_INVALID_ARG, "out_rgb is NULL");
+    if (!on_device && out_len != bytes)
         return set_err(ctx, RT_ERR_INVALID_ARG, "out_len %zu != (rows %u * width %u * 3) = %zu", out_len, row1 - row0,
                        r.p.width, bytes);
     CK(ctx, cudaSetDevice(ctx->device));
@@ -556,8 +557,56 @@ int render_rows_to_host(rt_ctx* ctx, const rt_scene* scene, const Resolved& r, u
     // Streaming the frame out slab by slab while it renders beats one copy after the kernel on a single GPU when a pixel
     // is many samples of work (C3, 16 spp: stage + counters +0.2 ms, the 25 MB copy 0.5 ms); at few samples per pixel
     // the stage costs more than the copy (C2, 1 spp: +0.09 vs 0.12 ms incl. the slab waits; C4, 4 spp: +2.2 vs 2.0 ms)
-    l.a.stream = bytes >= ((size_t)4 << 20) && l.a.frame.plan.slabs > 1 && r.p.spp >= 8;
-    return collect_frame(ctx, l.a.frame, OWN_FRAME_SEQ, out_rgb, &l, 1, stats, t0);
+    l.a.stream = !on_device && bytes >= ((size_t)4 << 20) && l.a.frame.plan.slabs > 1 && r.p.spp >= 8;
+    return collect_frame(ctx, l.a.frame, OWN_FRAME_SEQ, on_device ? nullptr : out_rgb, &l, 1, stats, t0);
+}
+
+// The checks of rt_render_divisions up to its output (params, list, everything rt_render_division checks); *contiguous:
+// the list is one ascending run of bands.
+int divisions_check(rt_ctx* ctx, const rt_scene* scene, const rt_params* params, const uint32_t* division_nos, uint32_t n,
+                    Resolved* r, bool* contiguous) {
+    if (!params) return set_err(ctx, RT_ERR_INVALID_ARG, "NULL scene or params");
+    if (!division_nos || n == 0) return set_err(ctx, RT_ERR_INVALID_ARG, "rt_render_divisions: no division numbers");
+    rt_params p = *params;
+    p.division_no = 0;         // the list says which bands
+    p.collect_counters = 0;    // as rt_render_samples: the banded form has no instrumented variant
+    int rc = resolve(ctx, scene, &p, false, r);
+    if (rc) return rc;
+    std::vector<bool> seen(r->p.divisions, false);
+    *contiguous = true;
+    for (uint32_t k = 0; k < n; k++) {
+        const uint32_t d = division_nos[k];
+        if (d >= r->p.divisions)
+            return set_err(ctx, RT_ERR_INVALID_ARG, "rt_render_divisions: division %u out of range (%u divisions)", d, r->p.divisions);
+        if (seen[d]) return set_err(ctx, RT_ERR_INVALID_ARG, "rt_render_divisions: division %u listed twice", d);
+        seen[d] = true;
+        *contiguous = *contiguous && d == division_nos[0] + k;
+    }
+    return RT_OK;
+}
+
+// The n checked bands stacked in list order: into out_rgb (host), or with on_device into the context's staging frame.
+int divisions_render(rt_ctx* ctx, const rt_scene* scene, const Resolved& r, const uint32_t* division_nos, uint32_t n,
+                     bool contiguous, uint8_t* out_rgb, size_t out_len, rt_stats* stats, bool on_device) {
+    const uint32_t band = r.p.height / r.p.divisions;  // main.rs:55-56
+    // one ascending run of bands is a plain row range: the path of rt_render_division / rt_render_frame, no table
+    if (contiguous)
+        return render_rows_to_host(ctx, scene, r, band * division_nos[0], band * (division_nos[0] + n), out_rgb, out_len,
+                                   stats, nullptr, 0, on_device);
+    CK(ctx, cudaSetDevice(ctx->device));
+    if (ctx->d_bands_cap < n) {
+        if (ctx->d_bands) {
+            CK(ctx, cudaStreamSynchronize(ctx->stream));
+            CK(ctx, cudaFree(ctx->d_bands));
+            ctx->d_bands = nullptr;
+            ctx->d_bands_cap = 0;
+        }
+        CK(ctx, cudaMalloc(&ctx->d_bands, (size_t)r.p.divisions * sizeof(uint32_t)));
+        ctx->d_bands_cap = r.p.divisions;
+    }
+    // stream-ordered in front of the launch and of any second pass, which read the same table
+    CK(ctx, cudaMemcpyAsync(ctx->d_bands, division_nos, (size_t)n * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+    return render_rows_to_host(ctx, scene, r, 0, n * band, out_rgb, out_len, stats, ctx->d_bands, band, on_device);
 }
 
 // Rank tile_rank of tile_ranks of a caller's whole frame.  seq (nullable: not the frame owner's call) must not be 0.
@@ -653,6 +702,7 @@ int rt_init(int device, rt_ctx** out) {
     // load the module and resolve every kernel now: the first division of a job must not pay the lazy load
     CKI(preload_kernels());
     CKI(jpeg_preload());
+    CKI(wire_preload());
     ctx->serial_launches = launches_block();
     {   // stream memory operations, if this driver and device have them (64-bit waits)
         int can64 = 0;
@@ -694,6 +744,8 @@ void rt_shutdown(rt_ctx* ctx) {
     if (ctx->h_stage) cudaFreeHost(ctx->h_stage);
     if (ctx->d_jpeg) cudaFree(ctx->d_jpeg);
     if (ctx->h_jpeg_len) cudaFreeHost(ctx->h_jpeg_len);
+    if (ctx->d_wire) cudaFree(ctx->d_wire);
+    if (ctx->h_wire) cudaFreeHost(ctx->h_wire);
     if (ctx->ev0) cudaEventDestroy(ctx->ev0);
     if (ctx->ev1) cudaEventDestroy(ctx->ev1);
     if (ctx->ev_sync) cudaEventDestroy(ctx->ev_sync);
@@ -744,46 +796,35 @@ int rt_render_divisions(rt_ctx* ctx, const rt_scene* scene, const rt_params* par
                         uint32_t n, uint8_t* out_rgb, size_t out_len, rt_stats* stats) {
     if (!ctx) return RT_ERR_INVALID_ARG;
     RT_GUARD_BEGIN
-    if (!params) return set_err(ctx, RT_ERR_INVALID_ARG, "NULL scene or params");
-    if (!division_nos || n == 0) return set_err(ctx, RT_ERR_INVALID_ARG, "rt_render_divisions: no division numbers");
-    rt_params p = *params;
-    p.division_no = 0;         // the list says which bands
-    p.collect_counters = 0;    // as rt_render_samples: the banded form has no instrumented variant
     Resolved r;
-    int rc = resolve(ctx, scene, &p, false, &r);
-    if (rc) return rc;
-    std::vector<bool> seen(r.p.divisions, false);
     bool contiguous = true;
-    for (uint32_t k = 0; k < n; k++) {
-        const uint32_t d = division_nos[k];
-        if (d >= r.p.divisions)
-            return set_err(ctx, RT_ERR_INVALID_ARG, "rt_render_divisions: division %u out of range (%u divisions)", d, r.p.divisions);
-        if (seen[d]) return set_err(ctx, RT_ERR_INVALID_ARG, "rt_render_divisions: division %u listed twice", d);
-        seen[d] = true;
-        contiguous = contiguous && d == division_nos[0] + k;
-    }
+    int rc = divisions_check(ctx, scene, params, division_nos, n, &r, &contiguous);
+    if (rc) return rc;
     const uint32_t band = r.p.height / r.p.divisions;  // main.rs:55-56
     const size_t bytes = (size_t)n * band * r.p.width * 3;
     if (!out_rgb) return set_err(ctx, RT_ERR_INVALID_ARG, "out_rgb is NULL");
     if (out_len != bytes)
         return set_err(ctx, RT_ERR_INVALID_ARG, "out_len %zu != (n %u * rows %u * width %u * 3) = %zu", out_len, n, band,
                        r.p.width, bytes);
-    // one ascending run of bands is a plain row range: the path of rt_render_division / rt_render_frame, no table
-    if (contiguous) return render_rows_to_host(ctx, scene, r, band * division_nos[0], band * (division_nos[0] + n), out_rgb, out_len, stats);
-    CK(ctx, cudaSetDevice(ctx->device));
-    if (ctx->d_bands_cap < n) {
-        if (ctx->d_bands) {
-            CK(ctx, cudaStreamSynchronize(ctx->stream));
-            CK(ctx, cudaFree(ctx->d_bands));
-            ctx->d_bands = nullptr;
-            ctx->d_bands_cap = 0;
-        }
-        CK(ctx, cudaMalloc(&ctx->d_bands, (size_t)r.p.divisions * sizeof(uint32_t)));
-        ctx->d_bands_cap = r.p.divisions;
-    }
-    // stream-ordered in front of the launch and of any second pass, which read the same table
-    CK(ctx, cudaMemcpyAsync(ctx->d_bands, division_nos, (size_t)n * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
-    return render_rows_to_host(ctx, scene, r, 0, n * band, out_rgb, out_len, stats, ctx->d_bands, band);
+    return divisions_render(ctx, scene, r, division_nos, n, contiguous, out_rgb, out_len, stats, false);
+    RT_GUARD_END(ctx)
+}
+
+int rt_render_divisions_json(rt_ctx* ctx, const rt_scene* scene, const rt_params* params, const uint32_t* division_nos,
+                             uint32_t n, const char* id, uint8_t* out, size_t out_cap, size_t* out_lens, rt_stats* stats) {
+    if (!ctx) return RT_ERR_INVALID_ARG;
+    RT_GUARD_BEGIN
+    const auto t0 = std::chrono::steady_clock::now();
+    Resolved r;
+    bool contiguous = true;
+    int rc = divisions_check(ctx, scene, params, division_nos, n, &r, &contiguous);
+    if (rc) return rc;
+    const uint32_t band = r.p.height / r.p.divisions;  // main.rs:55-56
+    if ((rc = slice_json_check(ctx, n, band, r.p.width, id, out, out_cap, out_lens))) return rc;
+    if ((rc = divisions_render(ctx, scene, r, division_nos, n, contiguous, nullptr, 0, stats, true))) return rc;
+    if ((rc = slice_json_device(ctx, ctx->d_out, n, band, r.p.width, division_nos, id, out, out_lens))) return rc;
+    if (stats) stats->total_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    return RT_OK;
     RT_GUARD_END(ctx)
 }
 

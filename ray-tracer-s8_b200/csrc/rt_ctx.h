@@ -64,6 +64,9 @@ struct rt_ctx {
     uint8_t* d_jpeg = nullptr;       // JPEG encoder scratch (rt_jpeg.cu): coefficients, bit offsets, coded and stuffed bytes
     size_t d_jpeg_bytes = 0;
     unsigned long long* h_jpeg_len = nullptr;  // pinned: length of the last encoded segment
+    uint8_t* d_wire = nullptr;       // wire format scratch (rt_wire.cu): the world's text and records, ImageSlice bodies
+    size_t d_wire_bytes = 0;
+    unsigned long long* h_wire = nullptr;  // pinned: a parse's outcome (array end, decline, sphere count)
     std::string err;
 };
 constexpr uint32_t RT_REDO_CAP = 1u << 16;
@@ -186,6 +189,19 @@ int jpeg_check(rt_ctx* ctx, uint32_t width, uint32_t height, uint32_t quality, c
 int jpeg_encode_device(rt_ctx* ctx, const uint8_t* rgb_dev, uint32_t width, uint32_t height, uint32_t quality,
                        uint8_t* out, size_t* out_len, float* ms_out);
 cudaError_t jpeg_preload();
+// In place: sums[0..n) → their exclusive sum, sums[n] = the total (the carry pass behind the CTA scans of rt_jpeg.cu and
+// rt_wire.cu), on stream s.
+cudaError_t scan_carry(unsigned long long* sums, uint32_t n, cudaStream_t s);
+
+// Wire format (rt_wire.cu).  slice_json_check: the refusals of rt_render_divisions_json beyond those of
+// rt_render_divisions.  slice_json_device: the ImageSlice bodies of the n bands of rows x width stacked at rgb_dev (device
+// memory of ctx, ordered on ctx->stream), band k with division_no division_nos[k], packed into out with their lengths in
+// out_lens; returns when both are complete.
+cudaError_t wire_preload();
+int slice_json_check(rt_ctx* ctx, uint32_t n, uint32_t rows, uint32_t width, const char* id, const uint8_t* out,
+                     size_t out_cap, const size_t* out_lens);
+int slice_json_device(rt_ctx* ctx, const uint8_t* rgb_dev, uint32_t n, uint32_t rows, uint32_t width,
+                      const uint32_t* division_nos, const char* id, uint8_t* out, size_t* out_lens);
 
 }  // namespace rtb
 

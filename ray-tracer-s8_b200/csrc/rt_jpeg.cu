@@ -568,6 +568,11 @@ int jpeg_encode_device(rt_ctx* ctx, const uint8_t* rgb_dev, uint32_t width, uint
     return RT_OK;
 }
 
+cudaError_t scan_carry(unsigned long long* sums, uint32_t n, cudaStream_t s) {
+    jpeg_carry_kernel<<<1, kCarryThreads, 0, s>>>(sums, n);
+    return cudaGetLastError();
+}
+
 cudaError_t jpeg_preload() {
     cudaFuncAttributes a;
     cudaError_t e;

@@ -182,6 +182,32 @@ extern "C" {
         out_len: *mut usize,
         stats: *mut rt_stats,
     ) -> c_int;
+    pub fn rt_world_json_max_objects(len: usize) -> usize;
+    pub fn rt_world_parse_json(
+        ctx: *mut rt_ctx,
+        text: *const c_char,
+        len: usize,
+        spheres: *mut rt_sphere,
+        triangles: *mut rt_triangle,
+        world_index: *mut u32,
+        cap: usize,
+        n_spheres: *mut u32,
+        n_triangles: *mut u32,
+        consumed: *mut usize,
+    ) -> c_int;
+    pub fn rt_slice_json_bound(rows: u32, width: u32) -> usize;
+    pub fn rt_render_divisions_json(
+        ctx: *mut rt_ctx,
+        scene: *const rt_scene,
+        params: *const rt_params,
+        division_nos: *const u32,
+        n: u32,
+        id: *const c_char,
+        out: *mut u8,
+        out_cap: usize,
+        out_lens: *mut usize,
+        stats: *mut rt_stats,
+    ) -> c_int;
     pub fn rt_render_tiles_device(
         ctx: *mut rt_ctx,
         scene: *const rt_scene,
@@ -325,6 +351,48 @@ impl Context {
         };
         self.check(rc)?;
         Ok(out)
+    }
+
+    /// The `world` of a RenderInfo body (the raw JSON text of the array) parsed on the GPU: spheres, triangles and the
+    /// world position of each (spheres first), what `Vec<Object>` holds.  `None` when the text is outside the device
+    /// grammar (serde's own layout of `Object`, numbers of at most 19 digits): deserialize `Vec<Object>` then, which
+    /// decides whether the body is valid.
+    pub fn parse_world_json(&self, text: &str) -> Option<(Vec<rt_sphere>, Vec<rt_triangle>, Vec<u32>)> {
+        let cap = unsafe { rt_world_json_max_objects(text.len()) };
+        let (mut sp, mut tr, mut wi) = (Vec::with_capacity(cap), Vec::with_capacity(cap), Vec::with_capacity(cap));
+        let (mut ns, mut nt, mut used) = (0u32, 0u32, 0usize);
+        let rc = unsafe {
+            rt_world_parse_json(self.raw, text.as_ptr() as *const c_char, text.len(), sp.as_mut_ptr(), tr.as_mut_ptr(),
+                                wi.as_mut_ptr(), cap, &mut ns, &mut nt, &mut used)
+        };
+        // a text with more after the array is not a world value (serde's RawValue holds exactly the value)
+        if rc != 0 || !text[used..].trim_matches(|c| matches!(c, ' ' | '\t' | '\n' | '\r')).is_empty() {
+            return None;
+        }
+        unsafe {
+            sp.set_len(ns as usize);
+            tr.set_len(nt as usize);
+            wi.set_len((ns + nt) as usize);
+        }
+        Some((sp, tr, wi))
+    }
+
+    /// `render_divisions`, then each band as the ImageSlice body the slave POSTs to /result, written on the device: body
+    /// k is `serde_json::to_vec(&ImageSlice { division_no: division_nos[k], image, id })`.  `id`: the hyphenated
+    /// lowercase uuid (`Uuid::to_string`).
+    pub fn render_divisions_json(&self, scene: &Scene<'_>, params: &rt_params, division_nos: &[u32], id: &str)
+                                 -> Result<Vec<Vec<u8>>, Error> {
+        let rows = params.height / params.divisions.max(1);
+        let mut out = vec![0u8; division_nos.len() * unsafe { rt_slice_json_bound(rows, params.width) }];
+        let mut lens = vec![0usize; division_nos.len()];
+        let id = std::ffi::CString::new(id).map_err(|_| Error { status: -1, message: "id holds a NUL".into() })?;
+        let rc = unsafe {
+            rt_render_divisions_json(self.raw, scene.raw, params, division_nos.as_ptr(), division_nos.len() as u32,
+                                     id.as_ptr(), out.as_mut_ptr(), out.len(), lens.as_mut_ptr(), ptr::null_mut())
+        };
+        self.check(rc)?;
+        let mut at = 0;
+        Ok(lens.iter().map(|&n| { let b = out[at..at + n].to_vec(); at += n; b }).collect())
     }
 
     /// Baseline JPEG of an RGB8 frame (`height * width * 3` bytes, row 0 on top), encoded on this context's GPU: the

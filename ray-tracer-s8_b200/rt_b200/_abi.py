@@ -75,7 +75,8 @@ EXPORTS = [
     "rt_scene_wait_ready", "rt_render_frame_multi", "rt_frame_collect", "rt_render_tiles_collect", "rt_frame_wait_consumed", "rt_l2_flush",
     "rt_accum_create", "rt_accum_destroy", "rt_accum_reset", "rt_accum_samples", "rt_render_samples", "rt_accum_read_linear",
     "rt_scene_update", "rt_render_samples_multi", "rt_render_divisions", "rt_jpeg_bound", "rt_jpeg_encode",
-    "rt_render_frame_jpeg",
+    "rt_render_frame_jpeg", "rt_world_json_max_objects", "rt_world_parse_json", "rt_slice_json_bound",
+    "rt_render_divisions_json",
 ]
 
 _lib = None
@@ -179,6 +180,15 @@ def lib():
     L.rt_jpeg_encode.restype = i32
     L.rt_render_frame_jpeg.argtypes = [pp, pp, u32, C.POINTER(RtParams), u32, vp, sz, C.POINTER(sz), C.POINTER(RtStats)]
     L.rt_render_frame_jpeg.restype = i32
+    L.rt_world_json_max_objects.argtypes = [sz]
+    L.rt_world_json_max_objects.restype = sz
+    L.rt_world_parse_json.argtypes = [vp, vp, sz, vp, vp, vp, sz, C.POINTER(u32), C.POINTER(u32), C.POINTER(sz)]
+    L.rt_world_parse_json.restype = i32
+    L.rt_slice_json_bound.argtypes = [u32, u32]
+    L.rt_slice_json_bound.restype = sz
+    L.rt_render_divisions_json.argtypes = [vp, vp, C.POINTER(RtParams), vp, u32, C.c_char_p, vp, sz, C.POINTER(sz),
+                                           C.POINTER(RtStats)]
+    L.rt_render_divisions_json.restype = i32
     L.rt_struct_sizes.argtypes = [C.POINTER(sz)]
     L.rt_struct_sizes.restype = None
     sizes = (sz * 4)()

@@ -174,6 +174,50 @@ class Context:
                                                   out.ctypes.data_as(C.c_void_p), out.nbytes, C.byref(st)))
         return (out, st.as_dict()) if want_stats else out
 
+    def render_divisions_json(self, scene: "Scene", params: RtParams, division_nos, id: str, want_stats=False):
+        """Bands `division_nos` of one job as the ImageSlice bodies the slave POSTs to /result, written on the device
+        (rt_render_divisions_json): body k is wire.ImageSlice(division_nos[k], band, id).to_json().encode() of the band
+        render_divisions gives; the RGB never reaches the host."""
+        div = params.divisions or 1
+        if params.height % div != 0:
+            raise RtError(_abi.RT_ERR_INVALID_ARG, f"height {params.height} is not a multiple of divisions {div}")
+        nos = np.asarray(division_nos, dtype=np.int64).reshape(-1)
+        if ((nos < 0) | (nos > 0xFFFFFFFF)).any():
+            raise RtError(_abi.RT_ERR_INVALID_ARG, "division numbers must fit 32 bits unsigned")
+        nos = np.ascontiguousarray(nos, dtype=np.uint32)
+        buf = np.empty(max(1, len(nos) * self._lib.rt_slice_json_bound(params.height // div, params.width)), np.uint8)
+        lens = np.zeros(max(1, len(nos)), dtype=np.uintp)
+        st = RtStats()
+        self._check(self._lib.rt_render_divisions_json(self._h, scene._h, C.byref(params), _ptr(nos), len(nos),
+                                                       str(id).encode(), _ptr(buf), buf.nbytes,
+                                                       lens.ctypes.data_as(C.POINTER(C.c_size_t)), C.byref(st)))
+        ends = np.cumsum(lens[: len(nos)])
+        bodies = [buf[e - n: e].tobytes() for e, n in zip(ends.tolist(), lens[: len(nos)].tolist())]
+        return (bodies, st.as_dict()) if want_stats else bodies
+
+    def parse_world_json(self, text, start: int = 0):
+        """The "world" array at text[start:] (bytes or str; leading JSON whitespace allowed) parsed on the device
+        (rt_world_parse_json): (wire.World, offset in text just past the array's ']'), the arrays
+        wire.parse_render_info builds.  None when the text is outside the device grammar; the host parser then decides."""
+        from .wire import World
+
+        data = text.encode("utf-8", "surrogatepass") if isinstance(text, str) else bytes(text)
+        if not 0 <= start <= len(data):
+            raise RtError(_abi.RT_ERR_INVALID_ARG, f"start {start} outside the text")
+        n_bytes = len(data) - start
+        base = C.c_void_p(C.cast(C.c_char_p(data), C.c_void_p).value + start)
+        cap = self._lib.rt_world_json_max_objects(n_bytes)
+        sp, tr = np.empty(cap, SPHERE_DTYPE), np.empty(cap, TRIANGLE_DTYPE)
+        wi = np.empty(cap, np.uint32)
+        ns, nt, used = C.c_uint32(), C.c_uint32(), C.c_size_t()
+        rc = self._lib.rt_world_parse_json(self._h, base, n_bytes, _ptr(sp), _ptr(tr), _ptr(wi), cap, C.byref(ns),
+                                           C.byref(nt), C.byref(used))
+        if rc == _abi.RT_ERR_UNSUPPORTED:
+            return None
+        self._check(rc)
+        n = ns.value + nt.value
+        return World(sp[: ns.value].copy(), tr[: nt.value].copy(), wi[:n].copy()), start + used.value
+
     def render_frame(self, scene: "Scene", params: RtParams, out: np.ndarray | None = None, want_stats=False):
         """All divisions in one launch → uint8 (height, width, 3)."""
         out = self._out_buffer(out, (params.height, params.width, 3))

@@ -8,8 +8,9 @@ Mirrors ray-tracer-slave/src/main.rs:
   * `serve()` = main() + index() (main.rs:148-174): `POST /` with a RenderInfo body answers
     "i'll get you a slice at once" immediately and queues the job for the single worker thread, which
     POSTs the ImageSlice JSON to `http://master:8080/result` (main.rs:85-101).  The worker thread takes every request
-    already queued with the one it waited for and renders those of one job together (`Worker.render_many`, one
-    `rt_render_divisions` call); each still gets its own ImageSlice POST.
+    already queued with the one it waited for and renders those of one job together (`Worker.render_many_json`, one
+    `rt_render_divisions_json` call, which also writes the ImageSlice bodies on the GPU); each still gets its own
+    ImageSlice POST.  The request's world is parsed on the worker's GPU when it is in serde's layout (`Worker.parse`).
 spp / max_bounces / camera default to the reference's literals (main.rs:39-51).
 """
 from __future__ import annotations
@@ -99,6 +100,37 @@ class Worker:
         slices = [wire.ImageSlice(i.division_no, imgs[at[i.division_no]].reshape(-1), i.render_meta.id) for i in infos]
         return (slices, st) if want_stats else slices
 
+    def render_many_json(self, infos):
+        """render_many, as the ImageSlice bodies the slave POSTs (bytes, one per request, in order), written on the device
+        by rt_render_divisions_json: each equals render(info).to_json().encode()."""
+        to_json = getattr(self.ctx, "render_divisions_json", None)
+        if to_json is None:  # a context without the device writer (a stand-in): the host encoder, same bytes
+            return [sl.to_json().encode() for sl in self.render_many(infos)]
+        m = infos[0].render_meta
+        key = (m.id, m.width, m.height, m.divisions)
+        if any((i.render_meta.id, i.render_meta.width, i.render_meta.height, i.render_meta.divisions) != key for i in infos):
+            raise ValueError("render_many_json takes requests of one job: one id, width, height and divisions")
+        nos = list(dict.fromkeys(i.division_no for i in infos))
+        p = api.make_params(m.width, m.height, divisions=m.divisions, spp=self.spp, max_bounces=self.max_bounces,
+                            seed=self.seed, intersector=self.intersector)
+        with self.lock:
+            bodies = to_json(self._scene_for(infos[0]), p, nos, m.id)
+        at = {d: k for k, d in enumerate(nos)}
+        return [bodies[at[i.division_no]] for i in infos]
+
+    def parse(self, body: str | bytes) -> wire.RenderInfo:
+        """wire.parse_render_info with the world parsed on this worker's GPU when the device grammar covers it (same
+        result, same WireError)."""
+        parse_world = getattr(self.ctx, "parse_world_json", None)
+        if parse_world is None:  # a context without the device parser (a stand-in)
+            return wire.parse_render_info(body)
+
+        def world_parser(data, start):
+            with self.lock:
+                return parse_world(data, start)
+
+        return wire.parse_render_info(body, world_parser=world_parser)
+
     def render_json(self, body: str | bytes) -> str:
         """RenderInfo JSON in → ImageSlice JSON out."""
         return self.render(wire.parse_render_info(body)).to_json()
@@ -110,8 +142,9 @@ class Worker:
         self.ctx.close()
 
 
-def _post(url: str, body: str, timeout: float = 60.0) -> str:
-    req = urllib.request.Request(url, data=body.encode(), headers={"Content-Type": "application/json"}, method="POST")
+def _post(url: str, body: str | bytes, timeout: float = 60.0) -> str:
+    data = body if isinstance(body, bytes) else body.encode()
+    req = urllib.request.Request(url, data=data, headers={"Content-Type": "application/json"}, method="POST")
     with urllib.request.urlopen(req, timeout=timeout) as r:
         return r.read().decode(errors="replace")
 
@@ -122,9 +155,9 @@ def serve(host: str = "0.0.0.0", port: int = 8081, result_url: str = MASTER_RESU
     wk = worker or Worker()
     jobs: "queue.Queue[wire.RenderInfo | None]" = queue.Queue()  # crossbeam unbounded channel (main.rs:159)
 
-    def post_slice(sl):
+    def post_body(body):
         try:
-            post(result_url, sl.to_json())
+            post(result_url, body)
         except Exception as e:  # the reference unwrap()s and dies; we log and keep serving
             print(f"[rt_b200.slave] job failed: {e}", flush=True)
 
@@ -134,7 +167,7 @@ def serve(host: str = "0.0.0.0", port: int = 8081, result_url: str = MASTER_RESU
         except Exception as e:
             print(f"[rt_b200.slave] job failed: {e}", flush=True)
             return
-        post_slice(sl)
+        post_body(sl.to_json())
 
     def worker_loop():
         while True:
@@ -159,7 +192,7 @@ def serve(host: str = "0.0.0.0", port: int = 8081, result_url: str = MASTER_RESU
                 groups.setdefault((Worker._world_key(i), m.width, m.height, m.divisions), []).append(i)
             for g in groups.values():
                 try:
-                    slices = wk.render_many(g)
+                    bodies = wk.render_many_json(g)
                 except Exception as e:
                     if len(g) == 1:
                         print(f"[rt_b200.slave] job failed: {e}", flush=True)
@@ -167,8 +200,8 @@ def serve(host: str = "0.0.0.0", port: int = 8081, result_url: str = MASTER_RESU
                         for i in g:
                             render_alone(i)
                     continue
-                for sl in slices:
-                    post_slice(sl)
+                for body in bodies:
+                    post_body(body)
             if stopping:
                 return
 
@@ -182,7 +215,7 @@ def serve(host: str = "0.0.0.0", port: int = 8081, result_url: str = MASTER_RESU
                 self.send_error(413)
                 return
             try:
-                info = wire.parse_render_info(self.rfile.read(n))
+                info = wk.parse(self.rfile.read(n))
             except wire.WireError as e:
                 self.send_error(400, str(e))
                 return

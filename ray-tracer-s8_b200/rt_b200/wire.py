@@ -14,6 +14,7 @@ tagged `enum Object`), shapes/sphere.rs:13-20, shapes/mesh.rs:15-23, color.rs:5-
 from __future__ import annotations
 
 import json
+import re
 import uuid as _uuid
 from dataclasses import dataclass, field
 
@@ -132,18 +133,60 @@ def world_from_objects(objs) -> World:
     return World(spheres, triangles, np.array(sph_pos + tri_pos, dtype=np.uint32))
 
 
-def parse_render_info(text: str | bytes) -> RenderInfo:
+# serde's layout of a RenderInfo starts with its world: {"world":[
+_WORLD_FIRST = re.compile(rb'[ \t\n\r]*\{[ \t\n\r]*"world"[ \t\n\r]*:')
+
+
+def _device_world(body, world_parser):
+    """(World, the body's other members as json parses them) when the world went through `world_parser`, else None.
+
+    world_parser(data, start) parses the array at data[start:] and returns (World, end offset) or None (declined).  The
+    rest of the body is parsed by json with [] in place of the world, so it meets exactly the host path's checks; any
+    doubt (a decline, a JSON error, a second "world" key, which json resolves to the last) leaves the body to the host
+    path, which then gives today's result or error text."""
+    data = body.encode("utf-8", "surrogatepass") if isinstance(body, str) else bytes(body)
+    m = _WORLD_FIRST.match(data)
+    if m is None:
+        return None
+    got = world_parser(data, m.end())
+    if got is None:
+        return None
+    world, end = got
+    last_pairs = []
+
+    def pairs(kv):
+        last_pairs[:] = kv
+        return dict(kv)
+
     try:
-        o = json.loads(text)
-    except json.JSONDecodeError as e:
-        raise WireError(f"invalid JSON: {e}") from e
+        o = json.loads(data[: m.end()] + b"[]" + data[end:], object_pairs_hook=pairs)  # the outermost object comes last
+    except (json.JSONDecodeError, UnicodeDecodeError):
+        return None
+    if sum(k == "world" for k, _ in last_pairs) != 1:
+        return None
+    return world, o
+
+
+def parse_render_info(text: str | bytes, world_parser=None) -> RenderInfo:
+    """RenderInfo from a request body.  world_parser (optional, e.g. a GPU context's parse_world_json) parses the world
+    array when the body starts with it; the result and every WireError are those of the host path alone."""
+    device = _device_world(text, world_parser) if world_parser is not None else None
+    if device is not None:
+        world, o = device
+    else:
+        world = None
+        try:
+            o = json.loads(text)
+        except json.JSONDecodeError as e:
+            raise WireError(f"invalid JSON: {e}") from e
     if not isinstance(o, dict):
         raise WireError("RenderInfo: expected an object")
     try:
         m = o["render_meta"]
         meta = RenderMeta(_u32(m["height"], "height"), _u32(m["width"], "width"), _u32(m["divisions"], "divisions"),
                           str(_uuid.UUID(str(m["id"]))))
-        return RenderInfo(world_from_objects(o["world"]), meta, _u32(o["division_no"], "division_no"))
+        return RenderInfo(world if world is not None else world_from_objects(o["world"]), meta,
+                          _u32(o["division_no"], "division_no"))
     except KeyError as e:
         raise WireError(f"RenderInfo: missing field {e}") from e
     except (TypeError, ValueError) as e:
