@@ -258,6 +258,29 @@ size_t rt_slice_json_bound(uint32_t rows, uint32_t width);
 int rt_render_divisions_json(rt_ctx* ctx, const rt_scene* scene, const rt_params* params, const uint32_t* division_nos,
                              uint32_t n, const char* id, uint8_t* out, size_t out_cap, size_t* out_lens, rt_stats* stats);
 
+/* ---- OBJ ingest: the controller's /upload body (ray-tracer-controller/src/obj.rs:10-53) ------------------------- */
+/* Bytes-derived upper bound on the triangles of an OBJ section of obj_size bytes (obj_size / 6, derived in rt_obj.cu). */
+size_t rt_obj_max_triangles(size_t obj_size);
+/* obj::build_world (ray-tracer-controller/src/obj.rs:10-53) on the device: body[0, obj_size) is the OBJ, body[obj_size,
+ * len) the MTL.  Writes the triangles in world order, exactly the TRIANGLE_DTYPE array rt_b200/obj.py's build_world
+ * returns (a, b, c from the corner triples of each model, albedo = Kd, roughness = f32(Ns) / 1000 in f32, emission 0),
+ * and *n_triangles.  triangles must hold cap >= rt_obj_max_triangles(obj_size) entries.  A body without faces gives
+ * RT_OK and 0 triangles.
+ * The device grammar is ASCII, lines broken at \n \r \v \f \x1c \x1d \x1e, '#' cutting the rest of a line, tokens
+ * separated by space, \t and \x1f; keys v, f, o, g, usemtl in the OBJ and newmtl, Kd, Ns in the MTL (any other line is
+ * ignored); numbers [+-]? (digits [. digits] | . digits) ([eE] [+-]? digits)? of at most 19 significant digits, converted
+ * as float(np.float32(token)) (correctly rounded to f64, then to f32, both to nearest); face indices [+-]? digits of at
+ * most 10 digits, then the corner's end or a '/'.
+ * RT_ERR_UNSUPPORTED: the body is outside the device grammar (a byte above 0x7F, inf / nan, a number with '_' or of
+ * more than 19 digits, a non-finite result, an exponent outside the conversion table, a longer face index, a material
+ * named __order__) or is one the host rejects (a v of fewer than 3 coordinates, an f of fewer than 3 corners, a bad
+ * number or an index out of range, a model with faces and no material, a bad Kd or Ns after a newmtl), or positions
+ * would not fit 32 bits.  Nothing is promised about the outputs, and the caller builds the world on the host, which
+ * decides whether the body is valid and what its error is.
+ * RT_ERR_INVALID_ARG, before anything is launched: a NULL pointer, obj_size > len, cap below the bound. */
+int rt_obj_build_world(rt_ctx* ctx, const uint8_t* body, size_t len, size_t obj_size, rt_triangle* triangles, size_t cap,
+                       uint32_t* n_triangles);
+
 /* Device-side entry for the multi-GPU tile scheduler: renders the 8x4-pixel tiles of the whole frame that belong to
  * rank tile_rank of tile_ranks (tile t, row-major over the tile grid, belongs to rank (t % ranks - t / ranks) mod ranks:
  * a rotating interleave) into a full-frame DEVICE buffer `frame_dev` (height*width*3 bytes;

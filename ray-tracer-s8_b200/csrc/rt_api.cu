@@ -703,6 +703,7 @@ int rt_init(int device, rt_ctx** out) {
     CKI(preload_kernels());
     CKI(jpeg_preload());
     CKI(wire_preload());
+    CKI(obj_preload());
     ctx->serial_launches = launches_block();
     {   // stream memory operations, if this driver and device have them (64-bit waits)
         int can64 = 0;
@@ -746,6 +747,8 @@ void rt_shutdown(rt_ctx* ctx) {
     if (ctx->h_jpeg_len) cudaFreeHost(ctx->h_jpeg_len);
     if (ctx->d_wire) cudaFree(ctx->d_wire);
     if (ctx->h_wire) cudaFreeHost(ctx->h_wire);
+    if (ctx->d_obj) cudaFree(ctx->d_obj);
+    if (ctx->h_obj) cudaFreeHost(ctx->h_obj);
     if (ctx->ev0) cudaEventDestroy(ctx->ev0);
     if (ctx->ev1) cudaEventDestroy(ctx->ev1);
     if (ctx->ev_sync) cudaEventDestroy(ctx->ev_sync);

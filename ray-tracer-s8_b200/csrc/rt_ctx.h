@@ -67,6 +67,9 @@ struct rt_ctx {
     uint8_t* d_wire = nullptr;       // wire format scratch (rt_wire.cu): the world's text and records, ImageSlice bodies
     size_t d_wire_bytes = 0;
     unsigned long long* h_wire = nullptr;  // pinned: a parse's outcome (array end, decline, sphere count)
+    uint8_t* d_obj = nullptr;        // OBJ ingest scratch (rt_obj.cu): the body's text, its lines, vertices, corners, triangles
+    size_t d_obj_bytes = 0;
+    unsigned long long* h_obj = nullptr;   // pinned: counts and the decline flag between the stages of a parse
     std::string err;
 };
 constexpr uint32_t RT_REDO_CAP = 1u << 16;
@@ -202,6 +205,9 @@ int slice_json_check(rt_ctx* ctx, uint32_t n, uint32_t rows, uint32_t width, con
                      size_t out_cap, const size_t* out_lens);
 int slice_json_device(rt_ctx* ctx, const uint8_t* rgb_dev, uint32_t n, uint32_t rows, uint32_t width,
                       const uint32_t* division_nos, const char* id, uint8_t* out, size_t* out_lens);
+
+// OBJ ingest (rt_obj.cu).
+cudaError_t obj_preload();
 
 }  // namespace rtb
 

@@ -6,6 +6,7 @@
 // Declined (the host decides): more than 19 significant digits, a nonzero significand with a decimal exponent outside
 // the table (rt_wire_pow5.h), and the one case the 128-bit product cannot decide.  Host and device code, so the
 // conversion can be checked on a CPU.
+// obj_number reads the number tokens of OBJ / MTL lines (rt_obj.cu) with the same conversion: see there.
 #pragma once
 #include <cstdint>
 #include <cstring>
@@ -131,6 +132,58 @@ __host__ __device__ inline bool json_number(const uint8_t*& p, float* out) {
         *out = f64_bits_to_f32(bits | (neg ? 1ull << 63 : 0));
     }
     p = s;
+    return true;
+}
+
+// The OBJ / MTL number token [p, end), converted as rt_b200/obj.py does: float(np.float32(token)), i.e. Python's
+// correctly rounded float(token), then f32 to nearest ("-0" is -0.0).  The device form is
+// [+-]? (digits [. digits*] | . digits) ([eE] [+-]? digits)?; false: any other token (Python also takes "inf", "nan",
+// "1_0" ...: the host decides), more than 19 significant digits, a nonzero significand with a decimal exponent outside
+// the table, an undecided product, or a result that is not finite.
+__host__ __device__ inline bool obj_number(const uint8_t* p, const uint8_t* end, float* out) {
+    const bool neg = p < end && *p == '-';
+    p += p < end && (*p == '-' || *p == '+');
+    uint64_t w = 0;
+    int sig = 0, nfrac = 0, ndig = 0;
+    const auto digit = [&](uint8_t c) {
+        if (w || c != '0') {  // leading zeros are not significant
+            sig += sig <= 19;
+            w = w * 10 + (c - '0');
+        }
+        ndig += ndig <= 1;
+    };
+    while (p < end && json_digit(*p)) digit(*p++);
+    if (p < end && *p == '.') {
+        p++;
+        while (p < end && json_digit(*p)) {
+            digit(*p++);
+            nfrac += nfrac <= 100000;
+        }
+    }
+    if (!ndig) return false;  // "." or no digits at all
+    int e = 0;
+    if (p < end && (*p == 'e' || *p == 'E')) {
+        p++;
+        const bool eneg = p < end && *p == '-';
+        p += p < end && (*p == '-' || *p == '+');
+        if (p == end || !json_digit(*p)) return false;
+        while (p < end && json_digit(*p)) {
+            if (e < 100000) e = e * 10 + (*p - '0');
+            p++;
+        }
+        e = eneg ? -e : e;
+    }
+    if (p != end || sig > 19 || nfrac > 100000) return false;
+    if (w == 0) {
+        *out = neg ? -0.0f : 0.0f;
+        return true;
+    }
+    const int q = e - nfrac;
+    uint64_t bits;
+    if (q < RT_POW5_QMIN || q > RT_POW5_QMAX || !eisel_lemire(w, q, &bits)) return false;
+    const float f = f64_bits_to_f32(bits | (neg ? 1ull << 63 : 0));
+    if (!(f >= -3.40282347e38f && f <= 3.40282347e38f)) return false;  // the host gives inf (with a warning)
+    *out = f;
     return true;
 }
 

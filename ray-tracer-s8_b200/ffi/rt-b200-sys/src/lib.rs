@@ -196,6 +196,16 @@ extern "C" {
         consumed: *mut usize,
     ) -> c_int;
     pub fn rt_slice_json_bound(rows: u32, width: u32) -> usize;
+    pub fn rt_obj_max_triangles(obj_size: usize) -> usize;
+    pub fn rt_obj_build_world(
+        ctx: *mut rt_ctx,
+        body: *const u8,
+        len: usize,
+        obj_size: usize,
+        triangles: *mut rt_triangle,
+        cap: usize,
+        n_triangles: *mut u32,
+    ) -> c_int;
     pub fn rt_render_divisions_json(
         ctx: *mut rt_ctx,
         scene: *const rt_scene,
@@ -375,6 +385,25 @@ impl Context {
             wi.set_len((ns + nt) as usize);
         }
         Some((sp, tr, wi))
+    }
+
+    /// The controller's `/upload` body (`body[..obj_size]` the OBJ, the rest the MTL) built into its world on the GPU:
+    /// the triangles `obj::build_world` returns (obj.rs:10-53), in its order.  `None` when the body is outside the device
+    /// grammar, which includes every body `obj::build_world` rejects: call it then, which decides whether the body is
+    /// valid.
+    pub fn build_world_obj(&self, body: &[u8], obj_size: usize) -> Option<Vec<rt_triangle>> {
+        if obj_size > body.len() {
+            return None;
+        }
+        let cap = unsafe { rt_obj_max_triangles(obj_size) };
+        let mut tr = Vec::with_capacity(cap);
+        let mut n = 0u32;
+        let rc = unsafe { rt_obj_build_world(self.raw, body.as_ptr(), body.len(), obj_size, tr.as_mut_ptr(), cap, &mut n) };
+        if rc != 0 {
+            return None;
+        }
+        unsafe { tr.set_len(n as usize) };
+        Some(tr)
     }
 
     /// `render_divisions`, then each band as the ImageSlice body the slave POSTs to /result, written on the device: body

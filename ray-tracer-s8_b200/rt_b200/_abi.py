@@ -76,7 +76,7 @@ EXPORTS = [
     "rt_accum_create", "rt_accum_destroy", "rt_accum_reset", "rt_accum_samples", "rt_render_samples", "rt_accum_read_linear",
     "rt_scene_update", "rt_render_samples_multi", "rt_render_divisions", "rt_jpeg_bound", "rt_jpeg_encode",
     "rt_render_frame_jpeg", "rt_world_json_max_objects", "rt_world_parse_json", "rt_slice_json_bound",
-    "rt_render_divisions_json",
+    "rt_render_divisions_json", "rt_obj_max_triangles", "rt_obj_build_world",
 ]
 
 _lib = None
@@ -189,6 +189,10 @@ def lib():
     L.rt_render_divisions_json.argtypes = [vp, vp, C.POINTER(RtParams), vp, u32, C.c_char_p, vp, sz, C.POINTER(sz),
                                            C.POINTER(RtStats)]
     L.rt_render_divisions_json.restype = i32
+    L.rt_obj_max_triangles.argtypes = [sz]
+    L.rt_obj_max_triangles.restype = sz
+    L.rt_obj_build_world.argtypes = [vp, vp, sz, sz, vp, sz, C.POINTER(u32)]
+    L.rt_obj_build_world.restype = i32
     L.rt_struct_sizes.argtypes = [C.POINTER(sz)]
     L.rt_struct_sizes.restype = None
     sizes = (sz * 4)()

@@ -218,6 +218,23 @@ class Context:
         n = ns.value + nt.value
         return World(sp[: ns.value].copy(), tr[: nt.value].copy(), wi[:n].copy()), start + used.value
 
+    def parse_obj(self, body: bytes, obj_size: int):
+        """The controller's /upload body (OBJ = body[:obj_size], MTL = the rest) built into its world on the device
+        (rt_obj_build_world): the TRIANGLE_DTYPE array obj.build_world returns, byte for byte.  None when the body is
+        outside the device grammar, which includes every body the host rejects; obj.build_world then decides."""
+        data = body if isinstance(body, bytes) else bytes(body)
+        if not 0 <= obj_size <= len(data):
+            raise RtError(_abi.RT_ERR_INVALID_ARG, f"obj_size {obj_size} outside the body")
+        cap = self._lib.rt_obj_max_triangles(obj_size)
+        tr = np.empty(max(cap, 1), TRIANGLE_DTYPE)
+        n = C.c_uint32()
+        rc = self._lib.rt_obj_build_world(self._h, C.cast(C.c_char_p(data), C.c_void_p), len(data), obj_size,
+                                          tr.ctypes.data_as(C.c_void_p), cap, C.byref(n))
+        if rc == _abi.RT_ERR_UNSUPPORTED:
+            return None
+        self._check(rc)
+        return tr[: n.value].copy()
+
     def render_frame(self, scene: "Scene", params: RtParams, out: np.ndarray | None = None, want_stats=False):
         """All divisions in one launch → uint8 (height, width, 3)."""
         out = self._out_buffer(out, (params.height, params.width, 3))

@@ -13,6 +13,8 @@ Same literals as the reference: 1920x1080, 20 divisions (main.rs:33-36), the sam
 /poll's JPEG(90) is encoded on the GPU where there is one: in `devices=` mode the frame is encoded where it was rendered
 (`rt_render_frame_jpeg`) and never reaches the host as RGB; in `worker=` mode the stitched frame is encoded with the
 worker's context (`rt_jpeg_encode`).  The bytes are the same as PIL's, which the HTTP-slave mode keeps using.
+/upload builds the world on the GPU in the same two modes (`Context.parse_obj`: the first GPU's context, or the worker's),
+falling back to obj.build_world's host code when the device declines; the HTTP-slave mode parses on the host.
 GPU work from concurrent /upload requests is serialised (one rt_ctx has one owner at a time).
 """
 from __future__ import annotations
@@ -81,13 +83,27 @@ class Controller:
                 for sc in scenes:
                     sc.close()
 
+    def _obj_parser(self):
+        """The device OBJ parser of this mode (None: host only), taken under the lock of the context it uses."""
+        if self.multi is not None:
+            ctx, lock = self.multi.ctxs[0], self.gpu_lock
+        else:
+            ctx, lock = getattr(self.worker, "ctx", None), getattr(self.worker, "lock", None)
+        if getattr(ctx, "parse_obj", None) is None or lock is None:
+            return None
+
+        def parse(data, obj_size):
+            with lock:
+                return ctx.parse_obj(data, obj_size)
+        return parse
+
     # -- /upload ---------------------------------------------------------------------------------------
     def upload(self, body: bytes, obj_size: int) -> str:
         job_id = str(uuid.uuid4())
         meta = wire.RenderMeta(self.height, self.width, self.divisions, job_id)
         with self.lock:
             self.jobs[job_id] = {"meta": meta, "result": {}}
-        triangles = objmod.build_world(body, obj_size)          # obj::build_world (main.rs:46)
+        triangles = objmod.build_world(body, obj_size, parser=self._obj_parser())   # obj::build_world (main.rs:46)
         if self.multi is not None:
             if self.height % self.divisions != 0:
                 raise ValueError(f"height {self.height} is not a multiple of divisions {self.divisions}")

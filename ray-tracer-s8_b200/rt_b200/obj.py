@@ -49,10 +49,18 @@ def parse_mtl(data: bytes) -> dict:
     return mats
 
 
-def build_world(data: bytes, obj_size: int) -> np.ndarray:
-    """`data[:obj_size]` = OBJ, `data[obj_size:]` = MTL → TRIANGLE_DTYPE array in the reference's world order."""
+def build_world(data: bytes, obj_size: int, parser=None) -> np.ndarray:
+    """`data[:obj_size]` = OBJ, `data[obj_size:]` = MTL → TRIANGLE_DTYPE array in the reference's world order.
+
+    parser: optional `parser(data, obj_size)` (e.g. `Context.parse_obj`, which builds the world on the GPU) returning
+    this function's array or None when it declines; a decline falls through to the host code below, which decides
+    whether the body is valid and what its error is."""
     if obj_size < 0 or obj_size > len(data):
         raise ObjError("obj_size out of range")
+    if parser is not None:
+        out = parser(data, obj_size)
+        if out is not None:
+            return out
     mats = parse_mtl(data[obj_size:])
     verts: list = []
     tris: list = []
